@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """Headline benchmark: agent-steps/sec (env step + cost + returns) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step of `value` returned (a fixed sample of envs, see
+dump_closed_loop) as DIR/<name>.npy, so that two builds can be compared output for output.
 
 One "step" = one batch of episodes of the named workload (default: BASELINE.json configs[3],
 CoverageDiscrete 32x32 / 16 agents / T=50 with 2^22 envs PER GPU, weak scaling):
@@ -49,7 +52,10 @@ def emit(obj):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps (batches) of the headline closed loop and of its policy-path, lean, fused, "
+                         "strong-scaled and host-buffer variants; the extra named configs and the policy loops "
+                         "size their own repeat counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--n_envs", type=int, default=1 << 22, help="envs per GPU")
@@ -63,7 +69,12 @@ def parse():
     ap.add_argument("--no_fused", action="store_true")
     ap.add_argument("--no_configs", action="store_true", help="skip the extra named configs (c2, c3, c4_strong)")
     ap.add_argument("--no_policy", action="store_true", help="skip the policy-in-the-loop timing")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0's envs)")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times CPU episodes and returns no arrays")
+    return a
 
 
 def workload_name(a):
@@ -314,9 +325,8 @@ def bench_strong(s, _lib, lib, sd, comm, a, rank, world, dev, peak, timed):
                                              P(buf.stats_scratch), A, A, E, ld, stream))
         comm.allreduce(buf.stats_vec)
         _lib.check(lib.smarl_lambda_update(P(lam), P(buf.stats_vec), P(thr), 0.002, A, A, stream))
-    steps = max(a.steps, 10)
-    ms, _ = timed(loop, steps, a.warmup)
-    ms /= steps
+    ms, _ = timed(loop, a.steps, a.warmup)
+    ms /= a.steps
     count = float(buf.stats_vec[-1].item())
     return {"value": float(total) * A * T / (ms * 1e-3), "unit": UNIT, "ms_per_step": ms, "scaling": "strong",
             "n_envs_total": total, "n_envs_per_rank": E, "world": world, "episodes_reduced": count,
@@ -459,6 +469,29 @@ def bench_policy_loop(s, a, dev):
     return out
 
 
+DUMP_BYTES = 48 << 20
+
+
+def dump_closed_loop(out_dir, env, buf, lambdas, n_envs):
+    """--dump-outputs: what the last timed closed-loop step handed its caller.  Per-env arrays keep a fixed, seeded,
+    sorted sample of env columns sized to stay under DUMP_BYTES (the full per-step slabs of 2^22 envs are GBs):
+    per-step rewards / costs / penalties and reward-to-go G [T, rows, n], the final observations and positions,
+    episode returns R / modR and cost sums C [rows, n].  The reduced stats vector and the updated lambdas are whole.
+    Integer outputs are written as float32 (exact), f64 outputs as float64."""
+    import numpy as np
+    import torch
+    per_env = {"reward": buf.reward, "cost": buf.cost, "penalty": buf.penalty, "G": buf.G, "obs": env.obs,
+               "pos_x": env.pos_x, "pos_y": env.pos_y, "R": buf.R, "modR": buf.modR, "C": buf.Csum}
+    col_bytes = sum(4 * t[..., 0].numel() for t in per_env.values())
+    n = min(n_envs, DUMP_BYTES // col_bytes)
+    cols = torch.as_tensor(np.sort(np.random.default_rng(0).choice(n_envs, n, replace=False)), device=buf.R.device)
+    os.makedirs(out_dir, exist_ok=True)
+    whole = {"stats": buf.stats_vec, "lambdas": lambdas}
+    for name, t in [*((k, v.index_select(-1, cols)) for k, v in per_env.items()), *whole.items()]:
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def run_ours(a):
     import numpy as np
@@ -552,6 +585,8 @@ def run_ours(a):
         sampler.start()
     total_ms, step_kernel_ms = timed(closed_loop, a.steps, a.warmup, per_step_events=True)
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_closed_loop(a.dump_outputs, env, buf, meta.lambdas, E)
 
     agent_steps = float(E) * A * T
     ms_per_step = total_ms / a.steps
@@ -718,7 +753,7 @@ def run_ours(a):
                                                        sy_h.data_ptr(), actions_h.data_ptr(), lam_h.data_ptr(),
                                                        R_h.data_ptr(), M_h.data_ptr(), C_h.data_ptr(),
                                                        st_h.data_ptr()))
-        e2e_steps = max(2, min(a.steps, 5))
+        e2e_steps = a.steps
         for _ in range(2):
             host_call()
         torch.cuda.synchronize()

@@ -1,9 +1,9 @@
 """Drive the UNMODIFIED reference (/root/reference) on injected states and recorded actions.
 
-TEST INFRASTRUCTURE ONLY, and usable only where the reference tree is mounted (this
-container).  Nothing here is imported on the GPU box: the ``-m gpu`` tests, smoke()
-and bench.py use tests/golden/*.npz produced from these functions by
-tests/golden/make_golden.py.
+TEST INFRASTRUCTURE ONLY.  The run_* functions need the reference tree; where it is
+absent, reference_side() serves the differential tests the reference outputs recorded in
+tests/golden/reference_record.npz.  The ``-m gpu`` tests, smoke() and bench.py use
+tests/golden/*.npz produced from these functions by tests/golden/make_golden.py.
 
 The reference is imported read-only (no bytecode written).  ``matplotlib`` is absent
 in this image and only needed by Buffer.save_results, so an empty stub module is
@@ -52,6 +52,27 @@ def load():
                                 MetaAgent=MetaAgent, Buffer=Buffer, ACAgent=ACAgent,
                                 AbstractAgent=AbstractAgent, PPOAgent=PPOAgent)
     return _ns
+
+
+RECORD = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden",
+                      "reference_record.npz")
+_record = None
+
+
+def reference_side(key, live, e=None):
+    """The reference's outputs for one test case: ``live()`` where the reference tree is present, else the entries
+    ``<key>/<name>`` of tests/golden/reference_record.npz (made by tests/golden/make_reference_record.py, which states
+    their provenance).  ``e`` selects one env of a case recorded per env."""
+    global _record
+    if available():
+        return live()
+    if _record is None:
+        with np.load(RECORD) as g:
+            _record = {k: g[k] for k in g.files}
+    rec = {k[len(key) + 1:]: v for k, v in _record.items() if k.startswith(key + "/")}
+    if not rec:
+        raise KeyError(f"no recorded reference outputs for {key}")
+    return rec if e is None else {k: v[e] for k, v in rec.items()}
 
 
 def _f64(x):

@@ -1,9 +1,12 @@
-"""Pin the numpy oracle against the live, unmodified reference (this container only).
+"""Pin the numpy oracle against the unmodified reference.
 
 The reference ships no tests (SURVEY.md section 4), so these differential runs -- and the
 golden fixtures generated from the same harness -- are what pins parity.  Integer
 dynamics and f64 rewards are compared bit-exactly (the oracle restates the reference's
 own f64 arithmetic in the same order); only BLAS-ordered reductions get a tolerance.
+Every test runs everywhere: the differential cases take the reference's side from the live
+reference tree where it is present and from tests/golden/reference_record.npz elsewhere
+(``rh.reference_side``); the known answers (SURVEY.md 4.2) are the reference's own outputs.
 """
 import numpy as np
 import pytest
@@ -11,42 +14,48 @@ import pytest
 from oracle import numpy_oracle as no
 from oracle import reference_harness as rh
 
-pytestmark = pytest.mark.reference
 
-
-# ------------------------------------------------------------------ survey KATs (SURVEY.md 4.2)
+# ------------------------------------------------------------------ the reference's known answers (SURVEY.md 4.2)
 def test_kat_coverage_discrete():
-    tr = rh.run_coverage_discrete(5, 3, [[2, 2]] * 3, [[0, 4, 4]], weights=[1, 2, 3])
-    assert tr["pos"][0].tolist() == [[3, 2], [2, 2], [2, 2]]
-    assert tr["cost"][0].tolist() == [1, 0, 0]
-    assert tr["reward"][0].tolist() == [-15.452994616207489, -30.905989232414978, -46.358983848622465]
-    tr = rh.run_coverage_discrete(5, 3, [[2, 2]] * 3, [[4, 4, 4]], weights=[1, 2, 3])
-    assert tr["reward"][0].tolist() == [-25.000000000000007, -50.000000000000014, -75.00000000000003]
-    assert tr["fieldview"] == 2.886751345948129
+    fv = no.coverage_fieldview(5, 3)
+    assert fv == 2.886751345948129
+    lut = no.coverage_penalty_lut(5, fv)
+    pos, r, c, _ = no.coverage_discrete_step([[[2, 2]] * 3], [[0, 4, 4]], 5, lut, [1, 2, 3])
+    assert pos[0].tolist() == [[3, 2], [2, 2], [2, 2]]
+    assert c[0].tolist() == [1, 0, 0]
+    assert r[0].tolist() == [-15.452994616207489, -30.905989232414978, -46.358983848622465]
+    _, r, _, _ = no.coverage_discrete_step([[[2, 2]] * 3], [[4, 4, 4]], 5, lut, [1, 2, 3])
+    assert r[0].tolist() == [-25.000000000000007, -50.000000000000014, -75.00000000000003]
 
 
 def test_kat_congestion():
     dem = np.array([[2, 2, 4, 4], [3, 6, 10, 5], [3, 8, 3, 4], [4, 6, 7, 8]])
-    tr = rh.run_congestion(3, 2, [[0, 0], [0, 0]], [[1, 4]], dem)
-    assert tr["reward"][0].tolist() == [-6.0, -26.5] and tr["congestions"][0].tolist() == [1, 1]
-    assert tr["cost"][0].tolist() == [0]
-    tr = rh.run_congestion(3, 2, [[0, 0], [0, 0]], [[4, 1]], dem)
-    assert tr["reward"][0].tolist() == [-11.5, -4.0] and tr["congestions"][0].tolist() == [0, 0]
-    tr = rh.run_congestion(3, 3, [[1, 1]] * 3, [[0, 0, 0]], dem)
-    assert tr["reward"][0].tolist() == [-8, -8, -8] and tr["cost"][0].tolist() == [1]
-    tr = rh.run_congestion(3, 2, [[1, 1], [2, 1]], [[0, 1]], dem)
-    assert tr["reward"][0].tolist() == [-4, -4]
+
+    def step(starts, actions):                                  # noise 0: the moves are the intended actions
+        _, r, c, _, con = no.congestion_step([starts], [actions], [actions], 3, dem)
+        return r[0].tolist(), c[0].tolist(), con[0].tolist()
+    r, c, con = step([[0, 0], [0, 0]], [1, 4])
+    assert r == [-6.0, -26.5] and con == [1, 1] and c == [0]
+    r, c, con = step([[0, 0], [0, 0]], [4, 1])
+    assert r == [-11.5, -4.0] and con == [0, 0]
+    r, c, con = step([[1, 1]] * 3, [0, 0, 0])
+    assert r == [-8, -8, -8] and c == [1]
+    r, c, con = step([[1, 1], [2, 1]], [0, 1])
+    assert r == [-4, -4]
 
 
 def test_kat_accounting():
-    out = rh.run_accounting([[-1, -2], [-3, -4], [-5, -6]], [[1, 0], [1, 1], [0, 1]],
-                            [0.5, 0.5], 0.9, [1, 1], 0.5)
-    assert out["mod_reward"].tolist() == [[-1.5, -2.5], [-4, -5], [-5.5, -6.5]]
-    assert out["R"].tolist() == [-7.750000000000001, -10.46]
-    np.testing.assert_allclose(out["modR"], [-9.555, -12.265], rtol=1e-14)
-    assert out["C"].tolist() == [2, 2]
-    assert out["lambdas_after"].tolist() == [1, 1]
-    np.testing.assert_allclose(out["G"][:, 0], [-9.555, -8.95, -5.5], rtol=1e-14)
+    rew = np.array([[-1, -2], [-3, -4], [-5, -6]], dtype=np.float64)[:, None]      # [T, E=1, A]
+    cost = np.array([[1, 0], [1, 1], [0, 1]], dtype=np.float64)[:, None]
+    lam = np.array([0.5, 0.5])
+    mod = no.modified_reward(rew, cost, lam)
+    assert mod[:, 0].tolist() == [[-1.5, -2.5], [-4, -5], [-5.5, -6.5]]
+    assert no.episode_returns(rew, 0.9)[0].tolist() == [-7.750000000000001, -10.46]
+    np.testing.assert_allclose(no.episode_returns(mod, 0.9)[0], [-9.555, -12.265], rtol=1e-14)
+    C = no.episode_cost_sums(cost)[0]
+    assert C.tolist() == [2, 2]
+    assert no.lambda_update(lam, C, [1, 1], 0.5).tolist() == [1, 1]
+    np.testing.assert_allclose(no.reward_to_go(mod, 0.9)[:, 0, 0], [-9.555, -8.95, -5.5], rtol=1e-14)
 
 
 # ------------------------------------------------------------------ differential: Coverage
@@ -64,7 +73,8 @@ def test_coverage_discrete_matches_reference(size, A, T, fv, seed):
         if e == 0:
             starts[:] = size - 1                      # everyone stacked near the wall
         actions = rng.integers(0, 5, size=(T, A))
-        tr = rh.run_coverage_discrete(size, A, starts, actions, weights=weights, fieldview_size=fv)
+        tr = rh.reference_side(f"coverage_discrete/{size},{A},{T},{fv},{seed}", lambda: rh.run_coverage_discrete(
+            size, A, starts, actions, weights=weights, fieldview_size=fv), e)
         pos = starts[None].copy()
         for t in range(T):
             pos, r, c, d = no.coverage_discrete_step(pos, actions[t][None], size, lut, weights)
@@ -106,7 +116,8 @@ def test_congestion_matches_reference(size, A, T, noise, seed):
         starts[0] = 0                                           # congestion.py:215-216
         actions = rng.integers(0, 5, size=(T, A))
         u = rng.random((T, A, 2))
-        tr = rh.run_congestion(size, A, starts, actions, demand, noise=noise, uniforms=u)
+        tr = rh.reference_side(f"congestion/{size},{A},{T},{noise},{seed}", lambda: rh.run_congestion(
+            size, A, starts, actions, demand, noise=noise, uniforms=u), e)
         pos = starts[None].copy()
         for t in range(T):
             moves = no.congestion_noise_moves(actions[t][None], u[t, :, 0][None], u[t, :, 1][None], noise)
@@ -136,7 +147,8 @@ def test_collision_matches_reference(size, A, L, T, seed):
         if e == 2:   # crowd the agents to provoke collisions
             starts = landmarks[0][None] + rng.normal(0, 0.4, size=(A, 2))
             starts = np.clip(starts, 0, size)
-        tr = rh.run_collision(size, A, starts, landmarks, actions, n_landmarks=L)
+        tr = rh.reference_side(f"collision/{size},{A},{L},{T},{seed}", lambda: rh.run_collision(
+            size, A, starts, landmarks, actions, n_landmarks=L), e)
         pos = starts[None].copy()
         done = np.zeros((1, A), dtype=bool)
         for t in range(T):
@@ -157,7 +169,8 @@ def test_accounting_matches_reference(A, K, T, gamma, seed):
     costs = rng.integers(0, 3, size=(T, K)).astype(np.float64)
     lam = rng.random(K)
     thr = rng.random(K) * 10
-    out = rh.run_accounting(rewards, costs, lam, gamma, thr, 0.05)
+    out = rh.reference_side(f"accounting/{A},{K},{T},{gamma},{seed}",
+                            lambda: rh.run_accounting(rewards, costs, lam, gamma, thr, 0.05))
     mod = no.modified_reward(rewards[:, None, :], costs[:, None, :], lam)      # [T,1,A]
     np.testing.assert_allclose(mod[:, 0], out["mod_reward"], rtol=1e-13, atol=1e-13)
     assert np.array_equal(no.episode_returns(rewards[:, None, :], gamma)[0], out["R"])   # same order => exact
@@ -179,7 +192,8 @@ def test_coverage_continuous_matches_reference(size, A, T, coarse, seed):
     for e in range(4):
         starts = rng.random((A, 2)) * size
         actions = rng.normal(0, 0.8, size=(T, A, 2)).astype(np.float32).astype(np.float64)
-        tr = rh.run_coverage_float("continuous", size, A, starts, actions, weights=w, coarseness=coarse)
+        tr = rh.reference_side(f"coverage_continuous/{size},{A},{T},{coarse},{seed}", lambda: rh.run_coverage_float(
+            "continuous", size, A, starts, actions, weights=w, coarseness=coarse), e)
         pos = starts[None].copy()
         for t in range(T):
             pos, r, c, d = no.coverage_continuous_step(pos, actions[t][None], size, fv, w, coarse)
@@ -199,7 +213,8 @@ def test_coverage_discretized_matches_reference(size, A, T, coarse, seed):
     for e in range(4):
         starts = np.floor(rng.random((A, 2)) * size * zoom) / zoom        # coverage.py:270-272
         actions = rng.integers(0, 9, size=(T, A))
-        tr = rh.run_coverage_float("discretized", size, A, starts, actions, weights=w, coarseness=coarse)
+        tr = rh.reference_side(f"coverage_discretized/{size},{A},{T},{coarse},{seed}", lambda: rh.run_coverage_float(
+            "discretized", size, A, starts, actions, weights=w, coarseness=coarse), e)
         pos = starts[None].copy()
         for t in range(T):
             pos, r, c, d = no.coverage_discretized_step(pos, actions[t][None], size, coarse, fv, w)
@@ -212,7 +227,7 @@ def test_ppo_standardised_returns_match_reference():
     rng = np.random.default_rng(0)
     for T, gamma in [(50, 0.999), (8, 0.99), (100, 0.9), (2, 0.5)]:
         m = rng.normal(-3, 4, size=T)
-        want = rh.run_ppo_returns(m, gamma)                          # torch float32
+        want = rh.reference_side(f"ppo/{T},{gamma}", lambda: {"returns": rh.run_ppo_returns(m, gamma)})["returns"]
         got = no.ppo_standardised_returns(m[:, None, None], gamma)[:, 0, 0]
         np.testing.assert_allclose(got, want, rtol=2e-5, atol=2e-5)
 
@@ -230,43 +245,53 @@ def test_batched_buffer_save_results_matches_reference_files(tmp_path, monkeypat
 
     from safe_multiagent_rl_b200.rollout import BatchedBuffer
 
-    ref = rh.load()
     rng = np.random.default_rng(5)
     A, K, T, batches, bsz = 3, 2, 7, 4, 5
     params = argparse.Namespace(gamma=0.95, thresholds=[1.5, 2.0], batch_size=bsz, n_agents_learning_cycles=1,
                                 environment="ExploreDiscrete", size=5, n_agents=A, numpy_seed=3, torch_seed=4,
                                 algo="AC")
     monkeypatch.chdir(tmp_path)
-    rb = ref.Buffer(params, constrained=True, save_path=str(tmp_path / "ref"))
-    (tmp_path / "ref").mkdir()
     mine = BatchedBuffer(params, constrained=True)            # default path: results/<name>_<i>
+    fed = []
     for b in range(batches):
         rew = rng.normal(size=(T, bsz, A))
         cost = rng.integers(0, 3, size=(T, bsz, K)).astype(np.float64)
         lam = rng.random(K)
         mod = rew - (cost @ lam)[:, :, None]
-        for e in range(bsz):
-            for t in range(T):
-                rb.append(list(rew[t, e]), list(mod[t, e]), list(cost[t, e]))
-            rb.step()
+        fed.append((rew, mod, cost, lam))
         for t in range(T):                                     # compat path: per-step [E, A] / [E, K] tensors
             mine.append(torch.from_numpy(rew[t]), torch.from_numpy(mod[t]), torch.from_numpy(cost[t]))
         mine.step()
-        rb.append_lambdas(lam)
         mine.append_lambdas(lam)
-    plt = mock.MagicMock()
-    with mock.patch.object(sys.modules[ref.Buffer.__module__], "plt", plt), mock.patch("builtins.print"):
-        rb.save_results()
+
+    def live():
+        ref = rh.load()
+        rb = ref.Buffer(params, constrained=True, save_path=str(tmp_path / "ref"))
+        (tmp_path / "ref").mkdir()
+        for rew, mod, cost, lam in fed:
+            for e in range(bsz):
+                for t in range(T):
+                    rb.append(list(rew[t, e]), list(mod[t, e]), list(cost[t, e]))
+                rb.step()
+            rb.append_lambdas(lam)
+        plt = mock.MagicMock()
+        with mock.patch.object(sys.modules[ref.Buffer.__module__], "plt", plt), mock.patch("builtins.print"):
+            rb.save_results()
+        out = {n: np.load(tmp_path / "ref" / (n + ".npy")) for n in ("constr3", "scores3", "lambdas")}
+        out["params_json"] = (tmp_path / "ref" / "params.json").read_text()
+        bs, bm = rb._get_batch_scores()
+        return dict(out, batch_scores=np.array(bs), batch_means=np.array(bm),
+                    batch_constraints=np.array(rb._get_batch_constraints()))
+    want = rh.reference_side("buffer", live)
     out = mine.save_results()
     assert out == "results/ExploreDiscrete_s5_n3_3-4_AC_0" and mine.save_results() == out
-    for name in ("constr3.npy", "scores3.npy", "lambdas.npy"):
-        np.testing.assert_allclose(np.load(tmp_path / out / name), np.load(tmp_path / "ref" / name), rtol=1e-13, atol=0)
-    assert json.load(open(tmp_path / out / "params.json")) == json.load(open(tmp_path / "ref" / "params.json"))
-    bs, bm = rb._get_batch_scores()
+    for name in ("constr3", "scores3", "lambdas"):
+        np.testing.assert_allclose(np.load(tmp_path / out / (name + ".npy")), want[name], rtol=1e-13, atol=0)
+    assert json.load(open(tmp_path / out / "params.json")) == json.loads(str(want["params_json"]))
     ms, mm = mine.batch_scores()
-    np.testing.assert_allclose(ms, np.array(bs), rtol=1e-13)
-    np.testing.assert_allclose(mm, np.array(bm), rtol=1e-13)
-    np.testing.assert_allclose(mine.batch_constraints(), np.array(rb._get_batch_constraints()), rtol=1e-13)
+    np.testing.assert_allclose(ms, want["batch_scores"], rtol=1e-13)
+    np.testing.assert_allclose(mm, want["batch_means"], rtol=1e-13)
+    np.testing.assert_allclose(mine.batch_constraints(), want["batch_constraints"], rtol=1e-13)
     # unconstrained runs get their own directory stem and no lambdas file (buffer.py:56-57,152-153)
     un = BatchedBuffer(params, constrained=False)
     un.extend(torch.zeros(2, A), torch.zeros(2, A), torch.zeros(2, K))
