@@ -7,6 +7,7 @@
 #include <stdarg.h>
 #include <stdlib.h>
 
+#include "mbarrier.cuh"
 #include "stats.cuh"
 
 namespace smarl {
@@ -41,12 +42,17 @@ int check_layout(int64_t n_envs, int64_t ld) {
 
 constexpr int kAccThreads = 128;
 constexpr int kReturnsThreads = 128;   // default CTA size of returns_kernel (>= 64: stats scratch rows are sized for 64)
+constexpr int kReturnsStages = 6;      // returns_kernel's ring depth: up to kReturnsStages - 1 steps in flight per CTA
 
 template <typename CT> struct CostVec;
 template <> struct CostVec<float> {   // float costs are summed in f64 like the reference and stored as f32
   typedef double acc_t;
   static __device__ __forceinline__ void load(const float* p, double (&c)[4]) {
     const float4 f = ld_stream_f4(p);
+    c[0] = f.x; c[1] = f.y; c[2] = f.z; c[3] = f.w;
+  }
+  static __device__ __forceinline__ void load_shared(const float* p, double (&c)[4]) {
+    const float4 f = *reinterpret_cast<const float4*>(p);
     c[0] = f.x; c[1] = f.y; c[2] = f.z; c[3] = f.w;
   }
   static __device__ __forceinline__ int4 pack(const double (&s)[4]) {
@@ -61,6 +67,10 @@ template <> struct CostVec<uint8_t> {
     const uint32_t w = ld_stream_u32(p);
     c[0] = w & 0xFF; c[1] = (w >> 8) & 0xFF; c[2] = (w >> 16) & 0xFF; c[3] = w >> 24;
   }
+  static __device__ __forceinline__ void load_shared(const uint8_t* p, int (&c)[4]) {
+    const uint32_t w = *reinterpret_cast<const uint32_t*>(p);
+    c[0] = w & 0xFF; c[1] = (w >> 8) & 0xFF; c[2] = (w >> 16) & 0xFF; c[3] = w >> 24;
+  }
 };
 template <> struct CostVec<int32_t> {
   typedef int acc_t;
@@ -68,6 +78,10 @@ template <> struct CostVec<int32_t> {
   static __device__ __forceinline__ void load(const int32_t* p, int (&c)[4]) {
     const float4 f = ld_stream_f4(p);
     c[0] = __float_as_int(f.x); c[1] = __float_as_int(f.y); c[2] = __float_as_int(f.z); c[3] = __float_as_int(f.w);
+  }
+  static __device__ __forceinline__ void load_shared(const int32_t* p, int (&c)[4]) {
+    const int4 v = *reinterpret_cast<const int4*>(p);
+    c[0] = v.x; c[1] = v.y; c[2] = v.z; c[3] = v.w;
   }
 };
 
@@ -111,13 +125,39 @@ struct ReturnsArgs {
   const float* weights;    // shared-reward kernel: [A] or NULL
 };
 
+// Per-step input tiles of one returns_kernel CTA: an agent row's reward and penalty tiles, or kCostSteps consecutive
+// time steps of a constraint row's cost tiles (so that a u8 row keeps as many bytes in flight as an agent row).
+// Thread 0 fills the stages with cp.async.bulk; `full` counts the bytes landed, `empty` the THREADS threads that
+// have read the stage.  Bytes in flight sit in shared memory, not in registers, so the depth of the
+// ring does not cost occupancy.
+template <typename CT, int THREADS, int S>
+struct ReturnsRing {
+  static constexpr int kCostSteps = 8 / (int)sizeof(CT);
+  union Stage {
+    struct {
+      float4 reward[THREADS];
+      float4 penalty[THREADS];
+    } agent;
+    CT cost[kCostSteps][4 * THREADS];
+  };
+  Stage stage[S];
+  uint64_t full[S], empty[S];
+};
+
 // One CTA = one row (agent a, or constraint k) x 512 envs.  Rows of the same env chunk get
 // consecutive block ids so that they run together and share the chunk's penalty rows in L2.
 // GM = 1 serves g_mode 0 and 1 (backward Horner, G written iff g_mode == 1), 2 and 3 their own paths;
 // a template parameter so that the PPO path's extra registers do not cut the occupancy of the others.
+// The CTA walks a sequence of steps i (an agent row's time steps in the order the path visits them, GM 3 visits
+// them twice; a constraint row's groups of kCostSteps time steps) and reads step i's tiles from ring stage i % S.
+// The minimum of 4 CTAs per SM is what lets ptxas give the GM 3 instance the registers it needs without spilling
+// (it spills at the 80 it picks unasked).
 template <typename CT, int THREADS, int GM>
-__global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
+__global__ void __launch_bounds__(THREADS, 4) returns_kernel(const ReturnsArgs a) {
+  constexpr int S = kReturnsStages;
   __shared__ double s_red[THREADS / 32];
+  __shared__ alignas(128) ReturnsRing<CT, THREADS, S> ring;
+  constexpr int CS = ReturnsRing<CT, THREADS, S>::kCostSteps;
   const int rows = (a.cost_rows_only ? 0 : a.A) + a.K;
   const int row = (int)(blockIdx.x % rows) + (a.cost_rows_only ? a.A : 0);
   const int64_t chunk = blockIdx.x / rows;
@@ -131,7 +171,60 @@ __global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
   for (int k = 0; k < 4; ++k) valid[k] = live && (e0 + k < a.n_envs);
   double* out = a.partials ? a.partials + chunk * stats_len(a.A, a.K) : nullptr;
 
-  if (row < a.A) {
+  const bool agent = row < a.A;
+  const int n_steps = agent ? (GM == 3 ? 2 * T : T) : (T + CS - 1) / CS;
+  // The chunk's envs rounded up to 16 (a multiple of 16 bytes for every element type) and never past ld.
+  const int64_t c0 = chunk * 4 * THREADS;
+  const uint32_t tile_envs = (uint32_t)min((int64_t)4 * THREADS, (a.n_envs - c0 + 15) & ~(int64_t)15);
+  auto issue = [&](int i) {
+    const int slot = i % S;
+    const uint64_t read_once = l2_evict_first_policy();
+    if (agent) {
+      const int t = GM == 2 ? i : T - 1 - (i < T ? i : i - T);
+      const uint32_t bytes = tile_envs * 4;
+      mbar_arrive_expect_tx(&ring.full[slot], a.penalty ? 2 * bytes : bytes);
+      bulk_load(ring.stage[slot].agent.reward, a.reward + ((int64_t)t * a.A + row) * ld + c0, bytes, &ring.full[slot],
+                read_once);
+      // the penalty row is shared by the chunk's A agent CTAs: left to L2's default policy
+      if (a.penalty)
+        bulk_load(ring.stage[slot].agent.penalty, a.penalty + (int64_t)t * ld + c0, bytes, &ring.full[slot],
+                  l2_evict_normal_policy());
+    } else {
+      const uint32_t bytes = tile_envs * (uint32_t)sizeof(CT);
+      const int t0 = i * CS, nt = min(CS, T - t0);
+      mbar_arrive_expect_tx(&ring.full[slot], nt * bytes);
+      for (int j = 0; j < nt; ++j)
+        bulk_load(ring.stage[slot].cost[j], static_cast<const CT*>(a.cost) + ((int64_t)(t0 + j) * a.K + (row - a.A)) * ld + c0,
+                  bytes, &ring.full[slot], read_once);
+    }
+  };
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < S; ++s) {
+      mbar_init(&ring.full[s], 1);
+      mbar_init(&ring.empty[s], THREADS);
+    }
+    for (int i = 0; i < min(S, n_steps); ++i) issue(i);
+  }
+  __syncthreads();
+  auto wait_full = [&](int i) { mbar_wait(&ring.full[i % S], (uint32_t)(i / S) & 1u); };
+  // Done reading step i.  Thread 0 then refills the stage of step i - 1 (which the other threads have most
+  // likely left by now) with step i - 1 + S.
+  auto release = [&](int i) {
+    mbar_arrive(&ring.empty[i % S]);
+    if (threadIdx.x == 0 && i >= 1 && i - 1 + S < n_steps) {
+      mbar_wait(&ring.empty[(i - 1) % S], (uint32_t)((i - 1) / S) & 1u);
+      issue(i - 1 + S);
+    }
+  };
+  auto load_agent = [&](int i, float4& r, float4& p) {
+    wait_full(i);
+    r = ring.stage[i % S].agent.reward[threadIdx.x];
+    p = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (a.penalty) p = ring.stage[i % S].agent.penalty[threadIdx.x];
+    release(i);
+  };
+
+  if (agent) {
     double raw[4] = {0, 0, 0, 0}, mod[4] = {0, 0, 0, 0};
     const double gamma = a.gamma;
     if (GM == 3) {
@@ -147,9 +240,8 @@ __global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
       }
       double sum[4] = {0, 0, 0, 0}, sq[4] = {0, 0, 0, 0};
       for (int t = T - 1; t >= 0; --t) {
-        const float4 r = ld_stream_f4(a.reward + ((int64_t)t * a.A + row) * ld + e0);
-        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.penalty) p = ld_stream_f4(a.penalty + (int64_t)t * ld + e0);
+        float4 r, p;
+        load_agent(T - 1 - t, r, p);
         const float rr[4] = {r.x, r.y, r.z, r.w}, pp[4] = {p.x, p.y, p.z, p.w};
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -171,9 +263,8 @@ __global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
         if (n_act[k] < 2) inv[k] = __longlong_as_double(0x7ff8000000000000ll);   // torch: std of one sample is nan
       }
       for (int t = T - 1; t >= 0; --t) {
-        const float4 r = ld_stream_f4(a.reward + ((int64_t)t * a.A + row) * ld + e0);
-        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.penalty) p = ld_stream_f4(a.penalty + (int64_t)t * ld + e0);
+        float4 r, p;
+        load_agent(2 * T - 1 - t, r, p);
         const float rr[4] = {r.x, r.y, r.z, r.w}, pp[4] = {p.x, p.y, p.z, p.w};
         float o[4];
 #pragma unroll
@@ -186,11 +277,9 @@ __global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
     } else if (GM != 2) {
       // Backward Horner: G_t = m_t + gamma G_{t+1} (agent.py:200-206); G_0 is the discounted
       // episode return of buffer.py:31-35.
-#pragma unroll 4
       for (int t = T - 1; t >= 0; --t) {
-        const float4 r = ld_stream_f4(a.reward + ((int64_t)t * a.A + row) * ld + e0);
-        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.penalty) p = ld_stream_f4(a.penalty + (int64_t)t * ld + e0);
+        float4 r, p;
+        load_agent(T - 1 - t, r, p);
         const float rr[4] = {r.x, r.y, r.z, r.w}, pp[4] = {p.x, p.y, p.z, p.w};
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -204,11 +293,9 @@ __global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
     } else {
       // Forward: gamma^t * m_t per step (agent.py:129-132) and their running sums.
       double disc = 1.0;
-#pragma unroll 4
       for (int t = 0; t < T; ++t) {
-        const float4 r = ld_stream_f4(a.reward + ((int64_t)t * a.A + row) * ld + e0);
-        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.penalty) p = ld_stream_f4(a.penalty + (int64_t)t * ld + e0);
+        float4 r, p;
+        load_agent(t, r, p);
         const float rr[4] = {r.x, r.y, r.z, r.w}, pp[4] = {p.x, p.y, p.z, p.w};
         double term[4];
 #pragma unroll
@@ -245,14 +332,17 @@ __global__ void __launch_bounds__(THREADS) returns_kernel(const ReturnsArgs a) {
   } else {
     // C_k = sum_t c[t,k]  (buffer.py:39, meta_agent.py:28)
     const int k = row - a.A;
-    const CT* cost = static_cast<const CT*>(a.cost);
     typename CostVec<CT>::acc_t sum[4] = {0, 0, 0, 0};
-#pragma unroll 4
-    for (int t = 0; t < T; ++t) {
-      typename CostVec<CT>::acc_t c[4];
-      CostVec<CT>::load(cost + ((int64_t)t * a.K + k) * ld + e0, c);
+    for (int i = 0; i < n_steps; ++i) {
+      wait_full(i);
+      const int nt = min(CS, T - i * CS);
+      for (int s = 0; s < nt; ++s) {
+        typename CostVec<CT>::acc_t c[4];
+        CostVec<CT>::load_shared(ring.stage[i % S].cost[s] + 4 * threadIdx.x, c);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) sum[j] += c[j];
+        for (int j = 0; j < 4; ++j) sum[j] += c[j];
+      }
+      release(i);
     }
     if (live) st_stream_i4(a.C + (int64_t)k * ld + e0, CostVec<CT>::pack(sum));
     if (out) {

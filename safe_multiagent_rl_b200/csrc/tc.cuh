@@ -17,10 +17,15 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "mbarrier.cuh"
+
 namespace smarl {
 namespace tc {
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+using ::smarl::mbar_init;
+using ::smarl::mbar_try_wait;
+using ::smarl::mbar_wait;
+using ::smarl::smem_u32;
 
 __host__ __device__ constexpr uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
@@ -92,30 +97,6 @@ __device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t a_desc, uint6
 // All MMAs issued so far by this thread -> one arrival on the mbarrier when they have completed.
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// ---- mbarrier -------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.b32 %0, 1, 0, p;\n\t"
-      "}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-// Bounded wait: a malformed descriptor must surface as a trapped launch, never as a hung GPU.
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  for (uint32_t spin = 0; !mbar_try_wait(bar, parity); ++spin)
-    if (spin > (1u << 26)) __trap();
 }
 
 // ---- packed fp32 pairs (FFMA2 on sm_100: two fused multiply-adds per issue slot) -----------------------------
