@@ -9,6 +9,7 @@
 
 #include <new>
 
+#include "coverage.cuh"
 #include "stats.cuh"
 
 struct SmarlHostSession {
@@ -108,7 +109,7 @@ extern "C" int smarl_host_session_create(SmarlHostSession** out, int32_t kind, i
   SMARL_TRY(cudaMalloc(&s->d_C, sizeof(int32_t) * s->K * s->ld));
   SMARL_TRY(cudaMalloc(&s->d_stats, sizeof(double) * sl * s->n_chunks));
   SMARL_TRY(cudaMalloc(&s->d_scratch, sizeof(double) * s->scratch_per_chunk * s->n_chunks));
-  SMARL_TRY(cudaMalloc(&s->d_lut, sizeof(float) * 12288));
+  SMARL_TRY(cudaMalloc(&s->d_lut, sizeof(float) * kCoverageMaxLut));
   SMARL_TRY(cudaMalloc(&s->d_weights, sizeof(float) * SMARL_MAX_AGENTS));
   SMARL_TRY(cudaMalloc(&s->d_lambdas, sizeof(double) * SMARL_MAX_AGENTS));
   SMARL_TRY(cudaMalloc(&s->d_thresholds, sizeof(double) * SMARL_MAX_AGENTS));
@@ -121,6 +122,8 @@ extern "C" int smarl_host_session_create(SmarlHostSession** out, int32_t kind, i
 extern "C" void smarl_host_session_destroy(SmarlHostSession* s) { free_session(s); }
 
 extern "C" int64_t smarl_host_session_ld(const SmarlHostSession* s) { return s ? s->ld : 0; }
+
+extern "C" int64_t smarl_host_session_pitch5(const SmarlHostSession* s) { return s ? s->pitch5 : 0; }
 
 namespace {
 
@@ -225,16 +228,6 @@ __global__ void __launch_bounds__(256) agentmajor_to_envmajor(const T* __restric
 }
 
 template <typename T>
-int to_agent_major(const T* in, T* out0, T* out1, int R, int64_t n, int64_t outer, int64_t in_outer, int64_t out_outer,
-                   int64_t ld, cudaStream_t st) {
-  const int te = tile_envs<T>(R);
-  dim3 grid((unsigned)((n + te - 1) / te), (unsigned)outer);
-  envmajor_to_agentmajor<T><<<grid, 256, sizeof(T) * te * (R + 1), st>>>(in, out0, out1, R, n, in_outer, out_outer, ld, te);
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
-}
-
-template <typename T>
 int to_env_major(const T* in, T* out, int R, int64_t n, int64_t ld, cudaStream_t st) {
   const int te = tile_envs<T>(R);
   agentmajor_to_envmajor<T><<<(unsigned)((n + te - 1) / te), 256, sizeof(T) * te * (R + 1), st>>>(in, out, R, n, ld, te);
@@ -246,6 +239,8 @@ struct Chunk {
   int index;
   int64_t e0, n, w;   // first env, envs in the chunk, envs copied per row (n rounded up to 16)
   cudaStream_t st;
+  double* stats;      // this chunk's additive stats and their scratch
+  double* scratch;
 };
 
 // rows x w elements of `elem` bytes between pitched [rows][ld] arrays, starting at env e0
@@ -256,31 +251,160 @@ int copy_rows(void* dst, const void* src, size_t elem, int64_t rows, int64_t ld,
   return SMARL_OK;
 }
 
-int upload_small(SmarlHostSession* s, const double* lambdas_h, const double* thresholds_h, int K) {
-  cudaStream_t s0 = s->streams[0];
-  if (lambdas_h) SMARL_CUDA(cudaMemcpyAsync(s->d_lambdas, lambdas_h, sizeof(double) * K, cudaMemcpyHostToDevice, s0));
-  if (thresholds_h) SMARL_CUDA(cudaMemcpyAsync(s->d_thresholds, thresholds_h, sizeof(double) * K, cudaMemcpyHostToDevice, s0));
+// One input array of a rollout.  On the device it is agent-major, [outer][R][ld] elements of `elem` bytes at `dev`,
+// except that with `dev_y` the R values of an env are interleaved (x, y) pairs (outer = 1): x to the R/2 rows of
+// `dev`, y to those of `dev_y`.  The host array is agent-major like the device (x and y of a pair as two arrays,
+// `host` and `host_y`) or env-major [outer][E][R] (`host` only).
+struct Input {
+  const void* host;
+  const void* host_y;
+  void* dev;
+  void* dev_y;
+  int elem, R, outer;
+  size_t stage_off = 0;   // env-major: byte offset of this input's chunk in d_stage_in, set by ensure_staging
+};
+
+// Places the env-major staging of a chunk's inputs back to back in d_stage_in, and allocates it and the staging of
+// the products (R, modR, C: 3 A rows of 4 bytes) for both streams on first use.
+int ensure_staging(SmarlHostSession* s, Input* in, int n_in) {
+  size_t bytes = 0;
+  for (int i = 0; i < n_in; ++i) {
+    in[i].stage_off = bytes;
+    bytes += (size_t)in[i].elem * in[i].R * in[i].outer * s->chunk;
+  }
+  for (int i = 0; i < 2; ++i) {
+    if (!s->d_stage_in[i]) SMARL_CUDA(cudaMalloc(&s->d_stage_in[i], bytes));
+    if (!s->d_stage_out[i]) SMARL_CUDA(cudaMalloc(&s->d_stage_out[i], (size_t)3 * s->A * s->chunk * 4));
+  }
   return SMARL_OK;
 }
 
-// Runs `body(chunk)` for every env chunk on alternating streams, then gathers the additive stats.
+template <typename T>
+int to_agent_major(const Input& x, const uint8_t* stage, int64_t chunk, int64_t ld, const Chunk& c) {
+  const int te = tile_envs<T>(x.R);
+  dim3 grid((unsigned)((c.n + te - 1) / te), (unsigned)x.outer);
+  envmajor_to_agentmajor<T><<<grid, 256, sizeof(T) * te * (x.R + 1), c.st>>>(
+      reinterpret_cast<const T*>(stage + x.stage_off), static_cast<T*>(x.dev) + c.e0,
+      x.dev_y ? static_cast<T*>(x.dev_y) + c.e0 : nullptr, x.R, c.n, chunk * x.R, (int64_t)x.R * ld, ld, te);
+  SMARL_CUDA(cudaGetLastError());
+  return SMARL_OK;
+}
+
+// A chunk of each input into its agent-major device rows: agent-major host rows are copied as they are; env-major
+// ones go to the stream's staging, all copies before the first transpose, then to the rows.
+int to_device(SmarlHostSession* s, const Chunk& c, bool env_major, const Input* in, int n_in) {
+  const int64_t ld = s->ld, chunk = s->chunk;
+  uint8_t* stage = s->d_stage_in[c.index & 1];
+  for (int i = 0; i < n_in; ++i) {
+    const Input& x = in[i];
+    if (!env_major) {
+      const int64_t rows = x.dev_y ? x.R / 2 : (int64_t)x.outer * x.R;
+      if (int rc = copy_rows(x.dev, x.host, x.elem, rows, ld, c, cudaMemcpyHostToDevice)) return rc;
+      if (x.dev_y)
+        if (int rc = copy_rows(x.dev_y, x.host_y, x.elem, rows, ld, c, cudaMemcpyHostToDevice)) return rc;
+    } else {
+      // the env-major host rows of this chunk are contiguous per step: [e0, e0+n) x R
+      const size_t row = (size_t)x.elem * x.R;
+      const char* src = static_cast<const char*>(x.host) + c.e0 * row;
+      if (x.outer == 1)
+        SMARL_CUDA(cudaMemcpyAsync(stage + x.stage_off, src, c.n * row, cudaMemcpyHostToDevice, c.st));
+      else
+        SMARL_CUDA(cudaMemcpy2DAsync(stage + x.stage_off, chunk * row, src, s->n_envs * row, c.n * row,
+                                     (size_t)x.outer, cudaMemcpyHostToDevice, c.st));
+    }
+  }
+  for (int i = 0; env_major && i < n_in; ++i) {
+    const int rc = in[i].elem == 1 ? to_agent_major<uint8_t>(in[i], stage, chunk, ld, c)
+                   : in[i].elem == 4 ? to_agent_major<float>(in[i], stage, chunk, ld, c)
+                                     : to_agent_major<double>(in[i], stage, chunk, ld, c);
+    if (rc) return rc;
+  }
+  return SMARL_OK;
+}
+
+// A chunk's products back to the host: R, modR [A] and C [K] rows, n_active when asked for, then the chunk's stats.
+// Agent-major host arrays take the rows as they are; env-major ones ([E][A], [E][K], [E]) through a transpose into
+// the stream's product staging.
+int from_device(SmarlHostSession* s, const Chunk& c, bool env_major, float* R_h, float* modR_h, int32_t* C_h,
+                int32_t* n_active_h) {
+  const int A = s->A, K = s->K, sl = stats_len(A, K);
+  const int64_t ld = s->ld, chunk = s->chunk;
+  if (!env_major) {
+    if (int rc = copy_rows(R_h, s->d_R, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
+    if (int rc = copy_rows(modR_h, s->d_modR, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
+    if (n_active_h)
+      if (int rc = copy_rows(n_active_h, s->d_n_active, 4, 1, ld, c, cudaMemcpyDeviceToHost)) return rc;
+    if (int rc = copy_rows(C_h, s->d_C, 4, K, ld, c, cudaMemcpyDeviceToHost)) return rc;
+  } else {
+    if (n_active_h)
+      SMARL_CUDA(cudaMemcpyAsync(n_active_h + c.e0, s->d_n_active + c.e0, (size_t)c.n * 4, cudaMemcpyDeviceToHost, c.st));
+    float* st_R = reinterpret_cast<float*>(s->d_stage_out[c.index & 1]);
+    float* st_M = st_R + (size_t)A * chunk;
+    int32_t* st_C = reinterpret_cast<int32_t*>(st_M + (size_t)A * chunk);
+    if (int rc = to_env_major<float>(s->d_R + c.e0, st_R, A, c.n, ld, c.st)) return rc;
+    if (int rc = to_env_major<float>(s->d_modR + c.e0, st_M, A, c.n, ld, c.st)) return rc;
+    if (int rc = to_env_major<int32_t>(s->d_C + c.e0, st_C, K, c.n, ld, c.st)) return rc;
+    SMARL_CUDA(cudaMemcpyAsync(R_h + c.e0 * A, st_R, (size_t)c.n * A * 4, cudaMemcpyDeviceToHost, c.st));
+    SMARL_CUDA(cudaMemcpyAsync(modR_h + c.e0 * A, st_M, (size_t)c.n * A * 4, cudaMemcpyDeviceToHost, c.st));
+    SMARL_CUDA(cudaMemcpyAsync(C_h + c.e0 * K, st_C, (size_t)c.n * K * 4, cudaMemcpyDeviceToHost, c.st));
+  }
+  SMARL_CUDA(cudaMemcpyAsync(s->h_stats + (int64_t)c.index * sl, c.stats, sizeof(double) * sl, cudaMemcpyDeviceToHost,
+                             c.st));
+  return SMARL_OK;
+}
+
+// What every rollout entry does first: checks that the call fits the session, then the env's own parameters
+// (`check`), and only then queues the uploads of lambdas and thresholds, so that a call these checks reject has
+// queued nothing.  *dacc is acc with its thresholds on the device.
+template <class Params, class Check>
+int begin_rollout(SmarlHostSession* s, int kind, const Params* p, const SmarlAccounting* acc, bool have_buffers,
+                  const double* lambdas_h, SmarlAccounting* dacc, Check check) {
+  SMARL_REQUIRE(s && p && acc, "null session / params");
+  SMARL_REQUIRE(s->kind == kind && p->n_agents == s->A && acc->n_steps == s->T,
+                "session was created for kind=%d A=%d T=%d", s->kind, s->A, s->T);
+  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
+  SMARL_REQUIRE(have_buffers, "null host buffer");
+  if (int rc = check()) return rc;
+  cudaStream_t s0 = s->streams[0];
+  if (lambdas_h) SMARL_CUDA(cudaMemcpyAsync(s->d_lambdas, lambdas_h, sizeof(double) * s->K, cudaMemcpyHostToDevice, s0));
+  if (acc->thresholds)
+    SMARL_CUDA(cudaMemcpyAsync(s->d_thresholds, acc->thresholds, sizeof(double) * s->K, cudaMemcpyHostToDevice, s0));
+  *dacc = *acc;
+  dacc->thresholds = acc->thresholds ? s->d_thresholds : nullptr;
+  return SMARL_OK;
+}
+
+// Waits for the first n_streams streams and returns rc, or the first failure to wait if rc is SMARL_OK.
+int sync_streams(SmarlHostSession* s, int n_streams, int rc) {
+  for (int i = 0; i < n_streams; ++i) {
+    const cudaError_t e = cudaStreamSynchronize(s->streams[i]);
+    if (e != cudaSuccess && rc == SMARL_OK) {
+      set_error("cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
+      rc = SMARL_ECUDA;
+    }
+  }
+  return rc;
+}
+
+// Runs `body(chunk)` for every env chunk on alternating streams, then gathers the additive stats.  Both streams are
+// drained before it returns, after an error too, since copies already queued read and write the caller's arrays;
+// the first error is the one reported.
 template <class Body>
 int pipeline(SmarlHostSession* s, double* stats_h, Body body) {
   const int sl = stats_len(s->A, s->K);
-  SMARL_CUDA(cudaStreamSynchronize(s->streams[0]));      // small parameter uploads are visible to both streams
-  for (int c = 0; c < s->n_chunks; ++c) {
+  int rc = sync_streams(s, 1, SMARL_OK);                   // small parameter uploads are visible to both streams
+  for (int c = 0; c < s->n_chunks && rc == SMARL_OK; ++c) {
     Chunk ch;
     ch.index = c;
     ch.st = s->streams[c & 1];
     ch.e0 = (int64_t)c * s->chunk;
     ch.n = (ch.e0 + s->chunk <= s->n_envs) ? s->chunk : (s->n_envs - ch.e0);
     ch.w = (ch.n + 15) / 16 * 16;
-    if (int rc = body(ch)) return rc;
-    SMARL_CUDA(cudaMemcpyAsync(s->h_stats + (int64_t)c * sl, s->d_stats + (int64_t)c * sl, sizeof(double) * sl,
-                               cudaMemcpyDeviceToHost, ch.st));
+    ch.stats = s->d_stats + (int64_t)c * sl;
+    ch.scratch = s->d_scratch + (int64_t)c * s->scratch_per_chunk;
+    rc = body(ch);
   }
-  SMARL_CUDA(cudaStreamSynchronize(s->streams[0]));
-  SMARL_CUDA(cudaStreamSynchronize(s->streams[1]));
+  if (int e = sync_streams(s, 2, rc)) return e;
   if (stats_h) {
     for (int j = 0; j < sl; ++j) {
       double v = 0.0;
@@ -291,46 +415,49 @@ int pipeline(SmarlHostSession* s, double* stats_h, Body body) {
   return SMARL_OK;
 }
 
-}  // namespace
-
-static int host_coverage_rollout(SmarlHostSession* s, const SmarlCoverageParams* p, const SmarlAccounting* acc,
-                                 const uint8_t* start_x_h, const uint8_t* start_y_h, const uint8_t* actions_h,
-                                 int packing /* 0 bytes, 4 nibbles, 5 base-5 triples */, const double* lambdas_h, float* R_h,
-                                 float* modR_h, int32_t* C_h, double* stats_h) {
-  const bool packed4 = packing == 4, packed5 = packing == 5;
-  SMARL_REQUIRE(s && p && acc, "null session / params");
-  SMARL_REQUIRE(s->kind == SMARL_ENV_COVERAGE && p->n_agents == s->A && acc->n_steps == s->T,
-                "session was created for kind=%d A=%d T=%d", s->kind, s->A, s->T);
-  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
-  SMARL_REQUIRE(p->lut_len >= 0 && p->lut_len <= 12287, "lut_len=%d outside 0..12287", p->lut_len);
-  SMARL_REQUIRE(start_x_h && start_y_h && actions_h && R_h && modR_h && C_h, "null host buffer");
-  const int A = s->A, T = s->T, sl = stats_len(A, A);
+// CoverageDiscrete episodes.  Agent-major host arrays (start_y_h given) carry one byte per action or, by `packing`,
+// two 4-bit (4) or three base-5 (5) actions per byte; env-major arrays (start_y_h unused) one byte per action.
+int coverage_rollout(SmarlHostSession* s, const SmarlCoverageParams* p, const SmarlAccounting* acc, bool env_major,
+                     int packing /* 0 bytes, 4 nibbles, 5 base-5 triples */, const uint8_t* starts_h,
+                     const uint8_t* start_y_h, const uint8_t* actions_h, const double* lambdas_h, float* R_h,
+                     float* modR_h, int32_t* C_h, double* stats_h) {
+  SmarlAccounting dacc;
+  const bool have_buffers = starts_h && (env_major || start_y_h) && actions_h && R_h && modR_h && C_h;
+  if (int rc = begin_rollout(s, SMARL_ENV_COVERAGE, p, acc, have_buffers, lambdas_h, &dacc, [&]() -> int {
+        SMARL_REQUIRE(p->lut_len >= 0, "lut_len=%d is negative", p->lut_len);
+        if (p->lut_len > kCoverageMaxLut) {
+          set_error("lut_len=%d exceeds the shared-memory table limit %d", p->lut_len, kCoverageMaxLut);
+          return SMARL_EUNSUPPORTED;
+        }
+        return SMARL_OK;
+      }))
+    return rc;
+  const int A = s->A, T = s->T;
   const int64_t ld = s->ld;
-  cudaStream_t s0 = s->streams[0];
-  if (p->lut_len) SMARL_CUDA(cudaMemcpyAsync(s->d_lut, p->lut, sizeof(float) * p->lut_len, cudaMemcpyHostToDevice, s0));
-  if (p->weights) SMARL_CUDA(cudaMemcpyAsync(s->d_weights, p->weights, sizeof(float) * A, cudaMemcpyHostToDevice, s0));
-  if (int rc = upload_small(s, lambdas_h, acc->thresholds, A)) return rc;
-  SmarlCoverageParams dp = *p;
-  dp.lut = s->d_lut;
-  dp.weights = p->weights ? s->d_weights : nullptr;
-  SmarlAccounting dacc = *acc;
-  dacc.thresholds = acc->thresholds ? s->d_thresholds : nullptr;
   uint8_t* dx = static_cast<uint8_t*>(s->d_start_x);
   uint8_t* dy = static_cast<uint8_t*>(s->d_start_y);
   uint8_t* da = static_cast<uint8_t*>(s->d_actions);
-  if (packed4 && !s->d_packed) SMARL_CUDA(cudaMalloc(&s->d_packed, (size_t)T * A * ld / 2));
-  if (packed5 && !s->d_packed5) SMARL_CUDA(cudaMalloc(&s->d_packed5, (size_t)T * A * s->pitch5));
+  Input in[] = {{starts_h, start_y_h, dx, dy, 1, 2 * A, 1}, {actions_h, nullptr, da, nullptr, 1, A, T}};
+  if (env_major)
+    if (int rc = ensure_staging(s, in, 2)) return rc;
+  if (packing == 4 && !s->d_packed) SMARL_CUDA(cudaMalloc(&s->d_packed, (size_t)T * A * ld / 2));
+  if (packing == 5 && !s->d_packed5) SMARL_CUDA(cudaMalloc(&s->d_packed5, (size_t)T * A * s->pitch5));
+  cudaStream_t s0 = s->streams[0];
+  if (p->lut_len) SMARL_CUDA(cudaMemcpyAsync(s->d_lut, p->lut, sizeof(float) * p->lut_len, cudaMemcpyHostToDevice, s0));
+  if (p->weights) SMARL_CUDA(cudaMemcpyAsync(s->d_weights, p->weights, sizeof(float) * A, cudaMemcpyHostToDevice, s0));
+  SmarlCoverageParams dp = *p;
+  dp.lut = s->d_lut;
+  dp.weights = p->weights ? s->d_weights : nullptr;
   return pipeline(s, stats_h, [&](const Chunk& c) -> int {
-    if (int rc = copy_rows(dx, start_x_h, 1, A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = copy_rows(dy, start_y_h, 1, A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (packed4) {                      // half the PCIe bytes: copy nibbles, expand on the device
+    if (int rc = to_device(s, c, env_major, in, packing ? 1 : 2)) return rc;
+    if (packing == 4) {                 // half the PCIe bytes: copy nibbles, expand on the device
       const int64_t rows = (int64_t)T * A;
       SMARL_CUDA(cudaMemcpy2DAsync(s->d_packed + c.e0 / 2, ld / 2, actions_h + c.e0 / 2, ld / 2, c.w / 2, (size_t)rows,
                                    cudaMemcpyHostToDevice, c.st));
       const int64_t n = rows * (c.w / 16);
       unpack4_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c.st>>>(s->d_packed, da, rows, ld, c.e0, c.w);
       SMARL_CUDA(cudaGetLastError());
-    } else if (packed5) {               // a third of the PCIe bytes: copy base-5 triples, expand on the device
+    } else if (packing == 5) {          // a third of the PCIe bytes: copy base-5 triples, expand on the device
       const int64_t rows = (int64_t)T * A, groups = (c.w + 47) / 48;       // 16 packed bytes = 48 envs per group
       int64_t w5 = groups * 16;
       if (c.e0 / 3 + w5 > s->pitch5) w5 = s->pitch5 - c.e0 / 3;
@@ -339,26 +466,98 @@ static int host_coverage_rollout(SmarlHostSession* s, const SmarlCoverageParams*
       const int64_t n = rows * groups;
       unpack5_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c.st>>>(s->d_packed5, da, rows, ld, s->pitch5, c.e0, groups);
       SMARL_CUDA(cudaGetLastError());
-    } else if (int rc = copy_rows(da, actions_h, 1, (int64_t)T * A, ld, c, cudaMemcpyHostToDevice)) {
-      return rc;
     }
     if (int rc = smarl_coverage_rollout(&dp, &dacc, dx + c.e0, dy + c.e0, da + c.e0, lambdas_h ? s->d_lambdas : nullptr,
                                         nullptr, nullptr, s->d_R + c.e0, s->d_modR + c.e0, s->d_C + c.e0, nullptr,
-                                        nullptr, s->d_stats + (int64_t)c.index * sl,
-                                        s->d_scratch + (int64_t)c.index * s->scratch_per_chunk, c.n, ld, c.st))
+                                        nullptr, c.stats, c.scratch, c.n, ld, c.st))
       return rc;
-    if (int rc = copy_rows(R_h, s->d_R, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    if (int rc = copy_rows(modR_h, s->d_modR, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    return copy_rows(C_h, s->d_C, 4, A, ld, c, cudaMemcpyDeviceToHost);
+    return from_device(s, c, env_major, R_h, modR_h, C_h, nullptr);
   });
 }
+
+// Congestion episodes; the host arrays are agent-major (start_y_h given) or env-major.
+int congestion_rollout(SmarlHostSession* s, const SmarlCongestionParams* p, const SmarlAccounting* acc, bool env_major,
+                       const uint8_t* starts_h, const uint8_t* start_y_h, const uint8_t* actions_h,
+                       const uint8_t* moves_h, const double* lambdas_h, float* R_h, float* modR_h, int32_t* C_h,
+                       double* stats_h) {
+  SmarlAccounting dacc;
+  const bool have_buffers = starts_h && (env_major || start_y_h) && actions_h && R_h && modR_h && C_h;
+  if (int rc = begin_rollout(s, SMARL_ENV_CONGESTION, p, acc, have_buffers, lambdas_h, &dacc, [&]() -> int {
+        SMARL_REQUIRE(p->size >= 1 && p->size <= 254 && p->demand, "bad size or demand table");
+        SMARL_REQUIRE(p->noise_mode != 1 || moves_h, "noise_mode 1 needs the recorded moves");
+        return SMARL_OK;
+      }))
+    return rc;
+  const int A = s->A, T = s->T, W = p->size + 1;
+  const int64_t ld = s->ld;
+  if (moves_h && !s->d_moves) SMARL_CUDA(cudaMalloc(&s->d_moves, (size_t)T * A * ld));
+  uint8_t* dx = static_cast<uint8_t*>(s->d_start_x);
+  uint8_t* dy = static_cast<uint8_t*>(s->d_start_y);
+  uint8_t* da = static_cast<uint8_t*>(s->d_actions);
+  Input in[] = {{starts_h, start_y_h, dx, dy, 1, 2 * A, 1}, {actions_h, nullptr, da, nullptr, 1, A, T},
+                {moves_h, nullptr, s->d_moves, nullptr, 1, A, T}};
+  if (env_major)
+    if (int rc = ensure_staging(s, in, 3)) return rc;
+  SMARL_CUDA(cudaMemcpyAsync(s->d_demand, p->demand, sizeof(double) * W * W, cudaMemcpyHostToDevice, s->streams[0]));
+  SmarlCongestionParams dp = *p;
+  dp.episode_dev = nullptr;                 // host callers pass the episode by value
+  dp.demand = s->d_demand;
+  dp.wait_reward = nullptr;                 // host callers pass the demand table only; the kernel divides
+  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
+    if (int rc = to_device(s, c, env_major, in, 2)) return rc;
+    if (moves_h)
+      if (int rc = to_device(s, c, env_major, in + 2, 1)) return rc;
+    SmarlCongestionParams cp = dp;
+    cp.env_offset = dp.env_offset + c.e0;                 // Philox streams are keyed by the global env id
+    if (int rc = smarl_congestion_rollout(&cp, &dacc, dx + c.e0, dy + c.e0, da + c.e0, moves_h ? s->d_moves + c.e0 : nullptr,
+                                          lambdas_h ? s->d_lambdas : nullptr, nullptr, nullptr, s->d_R + c.e0,
+                                          s->d_modR + c.e0, s->d_C + c.e0, nullptr, nullptr, c.stats, c.scratch, c.n, ld,
+                                          c.st))
+      return rc;
+    return from_device(s, c, env_major, R_h, modR_h, C_h, nullptr);
+  });
+}
+
+// CollisionAvoidance episodes; the host arrays are agent-major (start_y_h given) or env-major.
+int collision_rollout(SmarlHostSession* s, const SmarlCollisionParams* p, const SmarlAccounting* acc, bool env_major,
+                      const double* starts_h, const double* start_y_h, const double* landmarks_h, const float* actions_h,
+                      const double* lambdas_h, float* R_h, float* modR_h, int32_t* C_h, int32_t* n_active_h,
+                      double* stats_h) {
+  SmarlAccounting dacc;
+  const bool have_buffers = starts_h && (env_major || start_y_h) && landmarks_h && actions_h && R_h && modR_h && C_h;
+  if (int rc = begin_rollout(s, SMARL_ENV_COLLISION, p, acc, have_buffers, lambdas_h, &dacc, [&]() -> int {
+        SMARL_REQUIRE(p->n_landmarks == s->L, "session was created for n_landmarks=%d", s->L);
+        return SMARL_OK;
+      }))
+    return rc;
+  const int A = s->A, T = s->T, L = s->L;
+  const int64_t ld = s->ld;
+  double* dx = static_cast<double*>(s->d_start_x);
+  double* dy = static_cast<double*>(s->d_start_y);
+  float* da = static_cast<float*>(s->d_actions);
+  Input in[] = {{starts_h, start_y_h, dx, dy, 8, 2 * A, 1}, {landmarks_h, nullptr, s->d_landmarks, nullptr, 8, 2 * L, 1},
+                {actions_h, nullptr, da, nullptr, 4, 2 * A, T}};
+  if (env_major)
+    if (int rc = ensure_staging(s, in, 3)) return rc;
+  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
+    if (int rc = to_device(s, c, env_major, in, 3)) return rc;
+    if (int rc = smarl_collision_rollout(p, &dacc, dx + c.e0, dy + c.e0, s->d_landmarks + c.e0, da + c.e0,
+                                         lambdas_h ? s->d_lambdas : nullptr, nullptr, nullptr, nullptr,
+                                         s->d_n_active + c.e0, s->d_R + c.e0, s->d_modR + c.e0, s->d_C + c.e0, nullptr,
+                                         nullptr, c.stats, c.scratch, c.n, ld, c.st))
+      return rc;
+    return from_device(s, c, env_major, R_h, modR_h, C_h, n_active_h);
+  });
+}
+
+}  // namespace
 
 extern "C" int smarl_host_coverage_rollout(SmarlHostSession* s, const SmarlCoverageParams* p,
                                            const SmarlAccounting* acc, const uint8_t* start_x_h,
                                            const uint8_t* start_y_h, const uint8_t* actions_h,
                                            const double* lambdas_h, float* R_h, float* modR_h,
                                            int32_t* C_h, double* stats_h) {
-  return host_coverage_rollout(s, p, acc, start_x_h, start_y_h, actions_h, 0, lambdas_h, R_h, modR_h, C_h, stats_h);
+  return coverage_rollout(s, p, acc, false, 0, start_x_h, start_y_h, actions_h, lambdas_h, R_h, modR_h, C_h, stats_h);
 }
 
 extern "C" int smarl_host_coverage_rollout_packed4(SmarlHostSession* s, const SmarlCoverageParams* p,
@@ -366,17 +565,57 @@ extern "C" int smarl_host_coverage_rollout_packed4(SmarlHostSession* s, const Sm
                                                    const uint8_t* start_y_h, const uint8_t* actions4_h,
                                                    const double* lambdas_h, float* R_h, float* modR_h,
                                                    int32_t* C_h, double* stats_h) {
-  return host_coverage_rollout(s, p, acc, start_x_h, start_y_h, actions4_h, 4, lambdas_h, R_h, modR_h, C_h, stats_h);
+  return coverage_rollout(s, p, acc, false, 4, start_x_h, start_y_h, actions4_h, lambdas_h, R_h, modR_h, C_h, stats_h);
 }
-
-extern "C" int64_t smarl_host_session_pitch5(const SmarlHostSession* s) { return s ? s->pitch5 : 0; }
 
 extern "C" int smarl_host_coverage_rollout_packed5(SmarlHostSession* s, const SmarlCoverageParams* p,
                                                    const SmarlAccounting* acc, const uint8_t* start_x_h,
                                                    const uint8_t* start_y_h, const uint8_t* actions5_h,
                                                    const double* lambdas_h, float* R_h, float* modR_h,
                                                    int32_t* C_h, double* stats_h) {
-  return host_coverage_rollout(s, p, acc, start_x_h, start_y_h, actions5_h, 5, lambdas_h, R_h, modR_h, C_h, stats_h);
+  return coverage_rollout(s, p, acc, false, 5, start_x_h, start_y_h, actions5_h, lambdas_h, R_h, modR_h, C_h, stats_h);
+}
+
+extern "C" int smarl_host_coverage_rollout_envmajor(SmarlHostSession* s, const SmarlCoverageParams* p,
+                                                    const SmarlAccounting* acc, const uint8_t* starts_h,
+                                                    const uint8_t* actions_h, const double* lambdas_h, float* R_h,
+                                                    float* modR_h, int32_t* C_h, double* stats_h) {
+  return coverage_rollout(s, p, acc, true, 0, starts_h, nullptr, actions_h, lambdas_h, R_h, modR_h, C_h, stats_h);
+}
+
+extern "C" int smarl_host_congestion_rollout(SmarlHostSession* s, const SmarlCongestionParams* p,
+                                             const SmarlAccounting* acc, const uint8_t* start_x_h,
+                                             const uint8_t* start_y_h, const uint8_t* actions_h,
+                                             const uint8_t* moves_h, const double* lambdas_h, float* R_h,
+                                             float* modR_h, int32_t* C_h, double* stats_h) {
+  return congestion_rollout(s, p, acc, false, start_x_h, start_y_h, actions_h, moves_h, lambdas_h, R_h, modR_h, C_h,
+                            stats_h);
+}
+
+extern "C" int smarl_host_congestion_rollout_envmajor(SmarlHostSession* s, const SmarlCongestionParams* p,
+                                                      const SmarlAccounting* acc, const uint8_t* starts_h,
+                                                      const uint8_t* actions_h, const uint8_t* moves_h,
+                                                      const double* lambdas_h, float* R_h, float* modR_h,
+                                                      int32_t* C_h, double* stats_h) {
+  return congestion_rollout(s, p, acc, true, starts_h, nullptr, actions_h, moves_h, lambdas_h, R_h, modR_h, C_h, stats_h);
+}
+
+extern "C" int smarl_host_collision_rollout(SmarlHostSession* s, const SmarlCollisionParams* p,
+                                            const SmarlAccounting* acc, const double* start_x_h,
+                                            const double* start_y_h, const double* landmarks_h,
+                                            const float* actions_h, const double* lambdas_h, float* R_h,
+                                            float* modR_h, int32_t* C_h, int32_t* n_active_h, double* stats_h) {
+  return collision_rollout(s, p, acc, false, start_x_h, start_y_h, landmarks_h, actions_h, lambdas_h, R_h, modR_h, C_h,
+                           n_active_h, stats_h);
+}
+
+extern "C" int smarl_host_collision_rollout_envmajor(SmarlHostSession* s, const SmarlCollisionParams* p,
+                                                     const SmarlAccounting* acc, const double* starts_h,
+                                                     const double* landmarks_h, const float* actions_h,
+                                                     const double* lambdas_h, float* R_h, float* modR_h,
+                                                     int32_t* C_h, int32_t* n_active_h, double* stats_h) {
+  return collision_rollout(s, p, acc, true, starts_h, nullptr, landmarks_h, actions_h, lambdas_h, R_h, modR_h, C_h,
+                           n_active_h, stats_h);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -429,254 +668,4 @@ extern "C" int smarl_host_alloc_pinned(void** out, size_t bytes, int32_t* numa_n
 
 extern "C" void smarl_host_free_pinned(void* p) {
   if (p) cudaFreeHost(p);
-}
-
-// Per-stream staging of one chunk's env-major inputs / outputs (allocated on first use of an env-major entry).
-static int ensure_staging(SmarlHostSession* s, size_t in_bytes, size_t out_bytes) {
-  for (int i = 0; i < 2; ++i) {
-    if (!s->d_stage_in[i]) SMARL_CUDA(cudaMalloc(&s->d_stage_in[i], in_bytes));
-    if (!s->d_stage_out[i]) SMARL_CUDA(cudaMalloc(&s->d_stage_out[i], out_bytes));
-  }
-  return SMARL_OK;
-}
-
-// Episode products of one chunk back to env-major host arrays: R, modR [E][A] f32 and C [E][K] i32.
-static int download_env_major(SmarlHostSession* s, const Chunk& c, int A, int K, float* R_h, float* modR_h, int32_t* C_h) {
-  const int64_t ld = s->ld, chunk = s->chunk;
-  float* st_R = reinterpret_cast<float*>(s->d_stage_out[c.index & 1]);
-  float* st_M = st_R + (size_t)A * chunk;
-  int32_t* st_C = reinterpret_cast<int32_t*>(st_M + (size_t)A * chunk);
-  if (int rc = to_env_major<float>(s->d_R + c.e0, st_R, A, c.n, ld, c.st)) return rc;
-  if (int rc = to_env_major<float>(s->d_modR + c.e0, st_M, A, c.n, ld, c.st)) return rc;
-  if (int rc = to_env_major<int32_t>(s->d_C + c.e0, st_C, K, c.n, ld, c.st)) return rc;
-  SMARL_CUDA(cudaMemcpyAsync(R_h + c.e0 * A, st_R, (size_t)c.n * A * 4, cudaMemcpyDeviceToHost, c.st));
-  SMARL_CUDA(cudaMemcpyAsync(modR_h + c.e0 * A, st_M, (size_t)c.n * A * 4, cudaMemcpyDeviceToHost, c.st));
-  SMARL_CUDA(cudaMemcpyAsync(C_h + c.e0 * K, st_C, (size_t)c.n * K * 4, cudaMemcpyDeviceToHost, c.st));
-  return SMARL_OK;
-}
-
-extern "C" int smarl_host_coverage_rollout_envmajor(SmarlHostSession* s, const SmarlCoverageParams* p,
-                                                    const SmarlAccounting* acc, const uint8_t* starts_h,
-                                                    const uint8_t* actions_h, const double* lambdas_h, float* R_h,
-                                                    float* modR_h, int32_t* C_h, double* stats_h) {
-  SMARL_REQUIRE(s && p && acc, "null session / params");
-  SMARL_REQUIRE(s->kind == SMARL_ENV_COVERAGE && p->n_agents == s->A && acc->n_steps == s->T,
-                "session was created for kind=%d A=%d T=%d", s->kind, s->A, s->T);
-  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
-  SMARL_REQUIRE(p->lut_len >= 0 && p->lut_len <= 12287, "lut_len=%d outside 0..12287", p->lut_len);
-  SMARL_REQUIRE(starts_h && actions_h && R_h && modR_h && C_h, "null host buffer");
-  const int A = s->A, T = s->T, sl = stats_len(A, A);
-  const int64_t ld = s->ld, E = s->n_envs, chunk = s->chunk;
-  if (int rc = ensure_staging(s, (size_t)(T + 2) * A * chunk, (size_t)3 * A * chunk * 4)) return rc;
-  cudaStream_t s0 = s->streams[0];
-  if (p->lut_len) SMARL_CUDA(cudaMemcpyAsync(s->d_lut, p->lut, sizeof(float) * p->lut_len, cudaMemcpyHostToDevice, s0));
-  if (p->weights) SMARL_CUDA(cudaMemcpyAsync(s->d_weights, p->weights, sizeof(float) * A, cudaMemcpyHostToDevice, s0));
-  if (int rc = upload_small(s, lambdas_h, acc->thresholds, A)) return rc;
-  SmarlCoverageParams dp = *p;
-  dp.lut = s->d_lut;
-  dp.weights = p->weights ? s->d_weights : nullptr;
-  SmarlAccounting dacc = *acc;
-  dacc.thresholds = acc->thresholds ? s->d_thresholds : nullptr;
-  uint8_t* dx = static_cast<uint8_t*>(s->d_start_x);
-  uint8_t* dy = static_cast<uint8_t*>(s->d_start_y);
-  uint8_t* da = static_cast<uint8_t*>(s->d_actions);
-  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
-    uint8_t* st_in = s->d_stage_in[c.index & 1];
-    uint8_t* st_act = st_in + (size_t)2 * A * chunk;
-    // env-major host slabs of this chunk are contiguous per step: [e0, e0+n) x A
-    SMARL_CUDA(cudaMemcpyAsync(st_in, starts_h + c.e0 * 2 * A, (size_t)c.n * 2 * A, cudaMemcpyHostToDevice, c.st));
-    SMARL_CUDA(cudaMemcpy2DAsync(st_act, (size_t)chunk * A, actions_h + c.e0 * A, (size_t)E * A, (size_t)c.n * A, (size_t)T,
-                                 cudaMemcpyHostToDevice, c.st));
-    if (int rc = to_agent_major<uint8_t>(st_in, dx + c.e0, dy + c.e0, 2 * A, c.n, 1, 0, 0, ld, c.st)) return rc;
-    if (int rc = to_agent_major<uint8_t>(st_act, da + c.e0, nullptr, A, c.n, T, chunk * A, (int64_t)A * ld, ld, c.st)) return rc;
-    if (int rc = smarl_coverage_rollout(&dp, &dacc, dx + c.e0, dy + c.e0, da + c.e0, lambdas_h ? s->d_lambdas : nullptr,
-                                        nullptr, nullptr, s->d_R + c.e0, s->d_modR + c.e0, s->d_C + c.e0, nullptr,
-                                        nullptr, s->d_stats + (int64_t)c.index * sl,
-                                        s->d_scratch + (int64_t)c.index * s->scratch_per_chunk, c.n, ld, c.st))
-      return rc;
-    return download_env_major(s, c, A, A, R_h, modR_h, C_h);
-  });
-}
-
-extern "C" int smarl_host_congestion_rollout(SmarlHostSession* s, const SmarlCongestionParams* p,
-                                             const SmarlAccounting* acc, const uint8_t* start_x_h,
-                                             const uint8_t* start_y_h, const uint8_t* actions_h,
-                                             const uint8_t* moves_h, const double* lambdas_h, float* R_h,
-                                             float* modR_h, int32_t* C_h, double* stats_h) {
-  SMARL_REQUIRE(s && p && acc, "null session / params");
-  SMARL_REQUIRE(s->kind == SMARL_ENV_CONGESTION && p->n_agents == s->A && acc->n_steps == s->T,
-                "session was created for kind=%d A=%d T=%d", s->kind, s->A, s->T);
-  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
-  SMARL_REQUIRE(p->size >= 1 && p->size <= 254 && p->demand, "bad size or demand table");
-  SMARL_REQUIRE(start_x_h && start_y_h && actions_h && R_h && modR_h && C_h, "null host buffer");
-  SMARL_REQUIRE(p->noise_mode != 1 || moves_h, "noise_mode 1 needs the recorded moves");
-  const int A = s->A, T = s->T, sl = stats_len(A, 1), W = p->size + 1;
-  const int64_t ld = s->ld;
-  cudaStream_t s0 = s->streams[0];
-  SMARL_CUDA(cudaMemcpyAsync(s->d_demand, p->demand, sizeof(double) * W * W, cudaMemcpyHostToDevice, s0));
-  if (int rc = upload_small(s, lambdas_h, acc->thresholds, 1)) return rc;
-  if (moves_h && !s->d_moves) SMARL_CUDA(cudaMalloc(&s->d_moves, (size_t)T * A * ld));
-  SmarlCongestionParams dp = *p;
-  dp.episode_dev = nullptr;                 // host callers pass the episode by value
-  dp.demand = s->d_demand;
-  dp.wait_reward = nullptr;             // host callers pass the demand table only; the kernel divides
-  SmarlAccounting dacc = *acc;
-  dacc.thresholds = acc->thresholds ? s->d_thresholds : nullptr;
-  uint8_t* dx = static_cast<uint8_t*>(s->d_start_x);
-  uint8_t* dy = static_cast<uint8_t*>(s->d_start_y);
-  uint8_t* da = static_cast<uint8_t*>(s->d_actions);
-  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
-    if (int rc = copy_rows(dx, start_x_h, 1, A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = copy_rows(dy, start_y_h, 1, A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = copy_rows(da, actions_h, 1, (int64_t)T * A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (moves_h)
-      if (int rc = copy_rows(s->d_moves, moves_h, 1, (int64_t)T * A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    SmarlCongestionParams cp = dp;
-    cp.env_offset = dp.env_offset + c.e0;                 // Philox streams are keyed by the global env id
-    if (int rc = smarl_congestion_rollout(&cp, &dacc, dx + c.e0, dy + c.e0, da + c.e0, moves_h ? s->d_moves + c.e0 : nullptr,
-                                          lambdas_h ? s->d_lambdas : nullptr, nullptr, nullptr, s->d_R + c.e0,
-                                          s->d_modR + c.e0, s->d_C + c.e0, nullptr, nullptr,
-                                          s->d_stats + (int64_t)c.index * sl,
-                                          s->d_scratch + (int64_t)c.index * s->scratch_per_chunk, c.n, ld, c.st))
-      return rc;
-    if (int rc = copy_rows(R_h, s->d_R, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    if (int rc = copy_rows(modR_h, s->d_modR, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    return copy_rows(C_h, s->d_C, 4, 1, ld, c, cudaMemcpyDeviceToHost);
-  });
-}
-
-extern "C" int smarl_host_collision_rollout(SmarlHostSession* s, const SmarlCollisionParams* p,
-                                            const SmarlAccounting* acc, const double* start_x_h,
-                                            const double* start_y_h, const double* landmarks_h,
-                                            const float* actions_h, const double* lambdas_h, float* R_h,
-                                            float* modR_h, int32_t* C_h, int32_t* n_active_h, double* stats_h) {
-  SMARL_REQUIRE(s && p && acc, "null session / params");
-  SMARL_REQUIRE(s->kind == SMARL_ENV_COLLISION && p->n_agents == s->A && acc->n_steps == s->T &&
-                    p->n_landmarks == s->L, "session was created for kind=%d A=%d T=%d L=%d", s->kind, s->A, s->T, s->L);
-  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
-  SMARL_REQUIRE(start_x_h && start_y_h && landmarks_h && actions_h && R_h && modR_h && C_h, "null host buffer");
-  const int A = s->A, T = s->T, L = s->L, sl = stats_len(A, 1);
-  const int64_t ld = s->ld;
-  if (int rc = upload_small(s, lambdas_h, acc->thresholds, 1)) return rc;
-  SmarlAccounting dacc = *acc;
-  dacc.thresholds = acc->thresholds ? s->d_thresholds : nullptr;
-  double* dx = static_cast<double*>(s->d_start_x);
-  double* dy = static_cast<double*>(s->d_start_y);
-  float* da = static_cast<float*>(s->d_actions);
-  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
-    if (int rc = copy_rows(dx, start_x_h, 8, A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = copy_rows(dy, start_y_h, 8, A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = copy_rows(s->d_landmarks, landmarks_h, 8, 2 * L, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = copy_rows(da, actions_h, 4, (int64_t)T * 2 * A, ld, c, cudaMemcpyHostToDevice)) return rc;
-    if (int rc = smarl_collision_rollout(p, &dacc, dx + c.e0, dy + c.e0, s->d_landmarks + c.e0, da + c.e0,
-                                         lambdas_h ? s->d_lambdas : nullptr, nullptr, nullptr, nullptr,
-                                         s->d_n_active + c.e0, s->d_R + c.e0, s->d_modR + c.e0, s->d_C + c.e0, nullptr,
-                                         nullptr, s->d_stats + (int64_t)c.index * sl,
-                                         s->d_scratch + (int64_t)c.index * s->scratch_per_chunk, c.n, ld, c.st))
-      return rc;
-    if (int rc = copy_rows(R_h, s->d_R, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    if (int rc = copy_rows(modR_h, s->d_modR, 4, A, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    if (n_active_h)
-      if (int rc = copy_rows(n_active_h, s->d_n_active, 4, 1, ld, c, cudaMemcpyDeviceToHost)) return rc;
-    return copy_rows(C_h, s->d_C, 4, 1, ld, c, cudaMemcpyDeviceToHost);
-  });
-}
-
-extern "C" int smarl_host_congestion_rollout_envmajor(SmarlHostSession* s, const SmarlCongestionParams* p,
-                                                      const SmarlAccounting* acc, const uint8_t* starts_h,
-                                                      const uint8_t* actions_h, const uint8_t* moves_h,
-                                                      const double* lambdas_h, float* R_h, float* modR_h,
-                                                      int32_t* C_h, double* stats_h) {
-  SMARL_REQUIRE(s && p && acc, "null session / params");
-  SMARL_REQUIRE(s->kind == SMARL_ENV_CONGESTION && p->n_agents == s->A && acc->n_steps == s->T,
-                "session was created for kind=%d A=%d T=%d", s->kind, s->A, s->T);
-  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
-  SMARL_REQUIRE(p->size >= 1 && p->size <= 254 && p->demand, "bad size or demand table");
-  SMARL_REQUIRE(starts_h && actions_h && R_h && modR_h && C_h, "null host buffer");
-  SMARL_REQUIRE(p->noise_mode != 1 || moves_h, "noise_mode 1 needs the recorded moves");
-  const int A = s->A, T = s->T, sl = stats_len(A, 1), W = p->size + 1;
-  const int64_t ld = s->ld, E = s->n_envs, chunk = s->chunk;
-  if (int rc = ensure_staging(s, (size_t)(2 * T + 2) * A * chunk, (size_t)3 * A * chunk * 4)) return rc;
-  cudaStream_t s0 = s->streams[0];
-  SMARL_CUDA(cudaMemcpyAsync(s->d_demand, p->demand, sizeof(double) * W * W, cudaMemcpyHostToDevice, s0));
-  if (int rc = upload_small(s, lambdas_h, acc->thresholds, 1)) return rc;
-  if (moves_h && !s->d_moves) SMARL_CUDA(cudaMalloc(&s->d_moves, (size_t)T * A * ld));
-  SmarlCongestionParams dp = *p;
-  dp.episode_dev = nullptr;                 // host callers pass the episode by value
-  dp.demand = s->d_demand;
-  dp.wait_reward = nullptr;
-  SmarlAccounting dacc = *acc;
-  dacc.thresholds = acc->thresholds ? s->d_thresholds : nullptr;
-  uint8_t* dx = static_cast<uint8_t*>(s->d_start_x);
-  uint8_t* dy = static_cast<uint8_t*>(s->d_start_y);
-  uint8_t* da = static_cast<uint8_t*>(s->d_actions);
-  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
-    uint8_t* st_in = s->d_stage_in[c.index & 1];
-    uint8_t* st_act = st_in + (size_t)2 * A * chunk;
-    uint8_t* st_mov = st_act + (size_t)T * A * chunk;
-    SMARL_CUDA(cudaMemcpyAsync(st_in, starts_h + c.e0 * 2 * A, (size_t)c.n * 2 * A, cudaMemcpyHostToDevice, c.st));
-    SMARL_CUDA(cudaMemcpy2DAsync(st_act, (size_t)chunk * A, actions_h + c.e0 * A, (size_t)E * A, (size_t)c.n * A, (size_t)T,
-                                 cudaMemcpyHostToDevice, c.st));
-    if (int rc = to_agent_major<uint8_t>(st_in, dx + c.e0, dy + c.e0, 2 * A, c.n, 1, 0, 0, ld, c.st)) return rc;
-    if (int rc = to_agent_major<uint8_t>(st_act, da + c.e0, nullptr, A, c.n, T, chunk * A, (int64_t)A * ld, ld, c.st)) return rc;
-    if (moves_h) {
-      SMARL_CUDA(cudaMemcpy2DAsync(st_mov, (size_t)chunk * A, moves_h + c.e0 * A, (size_t)E * A, (size_t)c.n * A, (size_t)T,
-                                   cudaMemcpyHostToDevice, c.st));
-      if (int rc = to_agent_major<uint8_t>(st_mov, s->d_moves + c.e0, nullptr, A, c.n, T, chunk * A, (int64_t)A * ld, ld, c.st))
-        return rc;
-    }
-    SmarlCongestionParams cp = dp;
-    cp.env_offset = dp.env_offset + c.e0;                 // Philox streams are keyed by the global env id
-    if (int rc = smarl_congestion_rollout(&cp, &dacc, dx + c.e0, dy + c.e0, da + c.e0, moves_h ? s->d_moves + c.e0 : nullptr,
-                                          lambdas_h ? s->d_lambdas : nullptr, nullptr, nullptr, s->d_R + c.e0,
-                                          s->d_modR + c.e0, s->d_C + c.e0, nullptr, nullptr,
-                                          s->d_stats + (int64_t)c.index * sl,
-                                          s->d_scratch + (int64_t)c.index * s->scratch_per_chunk, c.n, ld, c.st))
-      return rc;
-    return download_env_major(s, c, A, 1, R_h, modR_h, C_h);
-  });
-}
-
-extern "C" int smarl_host_collision_rollout_envmajor(SmarlHostSession* s, const SmarlCollisionParams* p,
-                                                     const SmarlAccounting* acc, const double* starts_h,
-                                                     const double* landmarks_h, const float* actions_h,
-                                                     const double* lambdas_h, float* R_h, float* modR_h,
-                                                     int32_t* C_h, int32_t* n_active_h, double* stats_h) {
-  SMARL_REQUIRE(s && p && acc, "null session / params");
-  SMARL_REQUIRE(s->kind == SMARL_ENV_COLLISION && p->n_agents == s->A && acc->n_steps == s->T &&
-                    p->n_landmarks == s->L, "session was created for kind=%d A=%d T=%d L=%d", s->kind, s->A, s->T, s->L);
-  SMARL_REQUIRE(acc->g_mode == 0, "host rollout returns episode products only (g_mode 0)");
-  SMARL_REQUIRE(starts_h && landmarks_h && actions_h && R_h && modR_h && C_h, "null host buffer");
-  const int A = s->A, T = s->T, L = s->L, sl = stats_len(A, 1);
-  const int64_t ld = s->ld, E = s->n_envs, chunk = s->chunk;
-  const size_t start_b = (size_t)16 * A * chunk, lm_b = (size_t)16 * L * chunk, act_b = (size_t)T * 2 * A * 4 * chunk;
-  if (int rc = ensure_staging(s, start_b + lm_b + act_b, (size_t)3 * A * chunk * 4)) return rc;
-  if (int rc = upload_small(s, lambdas_h, acc->thresholds, 1)) return rc;
-  SmarlAccounting dacc = *acc;
-  dacc.thresholds = acc->thresholds ? s->d_thresholds : nullptr;
-  double* dx = static_cast<double*>(s->d_start_x);
-  double* dy = static_cast<double*>(s->d_start_y);
-  float* da = static_cast<float*>(s->d_actions);
-  return pipeline(s, stats_h, [&](const Chunk& c) -> int {
-    double* st_start = reinterpret_cast<double*>(s->d_stage_in[c.index & 1]);
-    double* st_lm = st_start + (size_t)2 * A * chunk;
-    float* st_act = reinterpret_cast<float*>(st_lm + (size_t)2 * L * chunk);
-    SMARL_CUDA(cudaMemcpyAsync(st_start, starts_h + c.e0 * 2 * A, (size_t)c.n * 2 * A * 8, cudaMemcpyHostToDevice, c.st));
-    SMARL_CUDA(cudaMemcpyAsync(st_lm, landmarks_h + c.e0 * 2 * L, (size_t)c.n * 2 * L * 8, cudaMemcpyHostToDevice, c.st));
-    SMARL_CUDA(cudaMemcpy2DAsync(st_act, (size_t)chunk * 2 * A * 4, actions_h + c.e0 * 2 * A, (size_t)E * 2 * A * 4,
-                                 (size_t)c.n * 2 * A * 4, (size_t)T, cudaMemcpyHostToDevice, c.st));
-    if (int rc = to_agent_major<double>(st_start, dx + c.e0, dy + c.e0, 2 * A, c.n, 1, 0, 0, ld, c.st)) return rc;
-    if (int rc = to_agent_major<double>(st_lm, s->d_landmarks + c.e0, nullptr, 2 * L, c.n, 1, 0, 0, ld, c.st)) return rc;
-    if (int rc = to_agent_major<float>(st_act, da + c.e0, nullptr, 2 * A, c.n, T, chunk * 2 * A, (int64_t)2 * A * ld, ld, c.st))
-      return rc;
-    if (int rc = smarl_collision_rollout(p, &dacc, dx + c.e0, dy + c.e0, s->d_landmarks + c.e0, da + c.e0,
-                                         lambdas_h ? s->d_lambdas : nullptr, nullptr, nullptr, nullptr,
-                                         s->d_n_active + c.e0, s->d_R + c.e0, s->d_modR + c.e0, s->d_C + c.e0, nullptr,
-                                         nullptr, s->d_stats + (int64_t)c.index * sl,
-                                         s->d_scratch + (int64_t)c.index * s->scratch_per_chunk, c.n, ld, c.st))
-      return rc;
-    if (n_active_h)
-      SMARL_CUDA(cudaMemcpyAsync(n_active_h + c.e0, s->d_n_active + c.e0, (size_t)c.n * 4, cudaMemcpyDeviceToHost, c.st));
-    return download_env_major(s, c, A, 1, R_h, modR_h, C_h);
-  });
 }

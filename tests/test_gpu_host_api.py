@@ -104,10 +104,12 @@ def test_host_collision_rollout_multi_chunk():
 
 def test_host_agent_major_entries_equal_env_major():
     """The padded agent-major entry points (what bench.py's e2e binds) and the env-major ones the numpy wrapper
-    uses must produce identical arrays, for Congestion (Philox noise and recorded moves) and Collision."""
+    uses must produce identical arrays, for Congestion (Philox noise and recorded moves), Collision and Coverage
+    (one byte per action and base-5 packed)."""
     import ctypes as C
     from safe_multiagent_rl_b200 import _lib
     from safe_multiagent_rl_b200.envs.congestion import keep_threshold
+    from safe_multiagent_rl_b200.envs.coverage import penalty_table
     from safe_multiagent_rl_b200.host import HostRollout, _am, _p
     rng = np.random.default_rng(5)
     # ---- Congestion
@@ -153,4 +155,84 @@ def test_host_agent_major_entries_equal_env_major():
     assert np.array_equal(R[:, :E].T, em["R"]) and np.array_equal(M[:, :E].T, em["modR"])
     assert np.array_equal(Cs[:, :E].T, em["C"]) and np.array_equal(na[0, :E], em["n_active"])
     assert np.array_equal(st, em["stats"])
+    h.close()
+    # ---- Coverage (3 chunks, ragged tail); base-5 packing as bench.py does it: rows padded to 3 * pitch5
+    size, A, E, T, gamma = 7, 4, 150_001, 6, 0.99
+    rng = np.random.default_rng(6)
+    starts = rng.integers(0, size, (E, A, 2))
+    actions = rng.integers(0, 5, (T, E, A))
+    w, lam, thr = np.array([1.0, 2.0, 3.0, 1.5], np.float32), np.linspace(0.1, 0.4, A), np.array([3.0] * A)
+    h = HostRollout("coverage", A, T, E)
+    ld, pitch5 = h.ld, int(h.lib.smarl_host_session_pitch5(h._sess))
+    em = h.coverage(size, starts, actions, weights=w, lambdas=lam, gamma=gamma, thresholds=thr)
+    lut = np.ascontiguousarray(penalty_table(size, A)[1], dtype=np.float32)
+    p = _lib.CoverageParams(size, A, len(lut), 0, _p(lut), _p(w))
+    acc = _lib.Accounting(gamma, T, 0, _p(thr))
+    sx, sy = _am(starts[:, :, 0], ld, np.uint8), _am(starts[:, :, 1], ld, np.uint8)
+    act = _am(actions, ld, np.uint8)                                                   # [T, A, ld]
+    pad = np.zeros((T, A, 3 * pitch5), np.uint8)
+    pad[:, :, :ld] = act
+    act5 = np.ascontiguousarray(pad[..., 0::3] + 5 * pad[..., 1::3] + 25 * pad[..., 2::3])   # [T, A, pitch5]
+    for fn, a in ((h.lib.smarl_host_coverage_rollout, act), (h.lib.smarl_host_coverage_rollout_packed5, act5)):
+        R, M = np.zeros((A, ld), np.float32), np.zeros((A, ld), np.float32)
+        Cs, st = np.zeros((A, ld), np.int32), np.zeros(h.lib.smarl_stats_len(A, A))
+        _lib.check(fn(h._sess, C.byref(p), C.byref(acc), _p(sx), _p(sy), _p(a), _p(lam), _p(R), _p(M), _p(Cs), _p(st)))
+        assert np.array_equal(R[:, :E].T, em["R"]) and np.array_equal(M[:, :E].T, em["modR"])
+        assert np.array_equal(Cs[:, :E].T, em["C"]) and np.array_equal(st, em["stats"])
+    h.close()
+
+
+def test_host_errors_leave_the_session_usable():
+    """Parameters that only the device entry point checks (Coverage size, every Collision field) fail with the
+    parameter named, an oversized Coverage table fails as unsupported, and after each failure the same session gives
+    what a fresh session gives."""
+    import ctypes as C
+    from safe_multiagent_rl_b200 import _lib
+    from safe_multiagent_rl_b200.envs.coverage import MAX_LUT, penalty_table
+    from safe_multiagent_rl_b200.host import HostRollout, _p
+    rng = np.random.default_rng(8)
+    # ---- Coverage
+    size, A, E, T, gamma = 6, 3, 140_000, 4, 0.99
+    starts = rng.integers(0, size, (E, A, 2)).astype(np.uint8)
+    actions = rng.integers(0, 5, (T, E, A)).astype(np.uint8)
+    w, lam, thr = np.array([1.0, 2.0, 3.0], np.float32), np.array([0.1, 0.2, 0.3]), np.array([2.0] * A)
+    kw = dict(weights=w, lambdas=lam, gamma=gamma, thresholds=thr)
+    fresh = HostRollout("coverage", A, T, E)
+    want = fresh.coverage(size, starts, actions, **kw)
+    fresh.close()
+    lut = np.ascontiguousarray(penalty_table(size, A)[1], dtype=np.float32)
+    acc = _lib.Accounting(gamma, T, 0, _p(thr))
+    h = HostRollout("coverage", A, T, E)
+    for bad_size, table, rc, name in ((200, lut, -1, "size"), (size, np.zeros(MAX_LUT + 1, np.float32), -3, "lut_len"),
+                                      (size, np.zeros(12288, np.float32), -3, "lut_len")):
+        p = _lib.CoverageParams(bad_size, A, len(table), 0, _p(table), _p(w))
+        R, M, Cs = np.zeros((E, A), np.float32), np.zeros((E, A), np.float32), np.zeros((E, A), np.int32)
+        st = np.zeros(h.lib.smarl_stats_len(A, A))
+        got = h.lib.smarl_host_coverage_rollout_envmajor(h._sess, C.byref(p), C.byref(acc), _p(starts), _p(actions),
+                                                         _p(lam), _p(R), _p(M), _p(Cs), _p(st))
+        assert got == rc and name in h.lib.smarl_last_error().decode(), (bad_size, len(table))
+        out = h.coverage(size, starts, actions, **kw)
+        for k in ("R", "modR", "C", "stats"):
+            assert np.array_equal(out[k], want[k]), k
+    h.close()
+    # ---- Collision
+    size, A, L, E, T = 5, 3, 2, 66_000, 4
+    starts, lm = rng.random((E, A, 2)) * size, rng.random((E, L, 2)) * size
+    actions = rng.normal(0, 0.5, (T, E, A, 2)).astype(np.float32)
+    kw = dict(lambdas=[0.5], gamma=gamma, thresholds=[1.0])
+    fresh = HostRollout("collision", A, T, E, n_landmarks=L)
+    want = fresh.collision(size, starts, lm, actions, **kw)
+    fresh.close()
+    h = HostRollout("collision", A, T, E, n_landmarks=L)
+    p = _lib.CollisionParams(size, A, L, 0, 0.0, 0, 0)                                  # agents_size = 0
+    thr1, lam1 = np.array([1.0]), np.array([0.5])
+    acc = _lib.Accounting(gamma, T, 0, _p(thr1))
+    R, M = np.zeros((E, A), np.float32), np.zeros((E, A), np.float32)
+    Cs, na, st = np.zeros(E, np.int32), np.zeros(E, np.int32), np.zeros(h.lib.smarl_stats_len(A, 1))
+    got = h.lib.smarl_host_collision_rollout_envmajor(h._sess, C.byref(p), C.byref(acc), _p(starts), _p(lm), _p(actions),
+                                                      _p(lam1), _p(R), _p(M), _p(Cs), _p(na), _p(st))
+    assert got == -1 and "agents_size" in h.lib.smarl_last_error().decode()
+    out = h.collision(size, starts, lm, actions, **kw)
+    for k in ("R", "modR", "C", "n_active", "stats"):
+        assert np.array_equal(out[k], want[k]), k
     h.close()
