@@ -410,6 +410,26 @@ typedef struct {
 int smarl_policy_act_gaussian(const SmarlGaussianPolicy* p, const float* obs, float* actions, float* logp, int32_t t,
                               int64_t n_envs, int64_t ld, smarl_stream_t stream);
 
+/* Whole ON-POLICY CollisionAvoidance episodes in one launch: main.py:28-57 with the policies inside, i.e. per step
+ * every agent's ContinuousPolicy (agent.py:48-76) on the current observation, the sample, CollisionAvoidance.step,
+ * MetaAgent.act, and Buffer.step + compute_returns as in smarl_collision_rollout.  Bit-identical to the closed loop
+ * reset + T x (smarl_policy_act_gaussian(t) + smarl_collision_step) on the same starts, weights and stream; actions
+ * and log-probabilities are sampled for every (t, agent, env), also for done agents and envs past their episode end.
+ *   p, acc, start_x .. lambdas and final_x .. stats_scratch as in smarl_collision_rollout (acc->g_mode 0..2)
+ *   pol: weights, seed, episode, episode_dev and env_offset as in smarl_policy_act_gaussian;
+ *        pol->state_size = 2A (+ 2L with p->obs_landmarks), hidden 16, 2 actions
+ *   obs_rec f32 [T][S][ld]  the observation the policy saw at step t      (NULL = skip)
+ *   actions f32 [T][2A][ld] the sampled rows dx0, dy0, dx1, ... (smarl_collision_rollout's layout; NULL = skip)
+ *   logp    f32 [T][A][ld]  log N(action; mu, sigma^2)                    (NULL = skip)
+ * A in 1..8 (one thread per env; A >= 9 returns SMARL_EUNSUPPORTED), T in 1..65536 (16 bits of the Philox counter). */
+int smarl_collision_policy_rollout(const SmarlCollisionParams* p, const SmarlGaussianPolicy* pol,
+                                   const SmarlAccounting* acc, const double* start_x, const double* start_y,
+                                   const double* landmarks, const double* lambdas, float* obs_rec, float* actions,
+                                   float* logp, double* final_x, double* final_y, uint8_t* final_done,
+                                   int32_t* n_active, float* R, float* modR, int32_t* C, float* G, float* g_scratch,
+                                   double* stats, double* stats_scratch, int64_t n_envs, int64_t ld,
+                                   smarl_stream_t stream);
+
 /* ------------------------------------------------------------------------------------
  * Multi-GPU: env instances are independent (envs/coverage.py:19, congestion.py:22,
  * collision_avoidance.py:60), so ranks own contiguous ranges of global env ids and the data path has no

@@ -26,9 +26,13 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
           "-I", INCLUDE]
 # Per-file extras.  collision.cu restates the reference's float64 arithmetic operation by
 # operation, so the compiler must not contract a*b+c into an FMA there.
-EXTRA = {"collision.cu": ["-fmad=false"], "collision_coop.cu": ["-fmad=false"], "coverage_float.cu": ["-fmad=false"]}
+EXTRA = {"collision.cu": ["-fmad=false"], "collision_coop.cu": ["-fmad=false"], "collision_policy.cu": ["-fmad=false"],
+         "coverage_float.cu": ["-fmad=false"]}
 # Heavy files (32 agent-count instantiations per kernel) are compiled as several translation units
 # in parallel: the file is built once per value of -DSMARL_TU=k (see the header of each file).
+# Sources that #include another .cu file: rebuilt when that file changes too (collision_policy.cu takes the env step
+# from collision.cu).
+CU_DEPS = {"collision_policy.cu": ["collision.cu"]}
 TU_SPLIT = {"coverage.cu": 3, "congestion.cu": 7, "collision.cu": 3, "collision_coop.cu": 2, "congestion_coop.cu": 6, "coverage_float.cu": 5}
 
 
@@ -64,7 +68,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
         for tu in range(n_tu):
             o = os.path.join(OBJ_DIR, src[:-3] + (f".tu{tu}" if n_tu > 1 else "") + ".o")
             objs.append(o)
-            if force or not os.path.exists(o) or os.path.getmtime(o) < max(os.path.getmtime(s), hm):
+            deps = [os.path.getmtime(os.path.join(CSRC, d)) for d in CU_DEPS.get(src, [])]
+            if force or not os.path.exists(o) or os.path.getmtime(o) < max([os.path.getmtime(s), hm] + deps):
                 cmd = [nvcc, *ARCH, *COMMON, *EXTRA.get(src, []), "-c", s, "-o", o]
                 if n_tu > 1:
                     cmd.insert(1, f"-DSMARL_TU={tu}")

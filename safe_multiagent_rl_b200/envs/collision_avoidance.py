@@ -127,3 +127,49 @@ class BatchedCollisionAvoidance(BatchedEnv):
             _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
         o["n_active"] = o["n_active_"][0, :E]
         return self._rollout_result(o)
+
+    def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
+                       out=None):
+        """Whole on-policy episode in one launch (smarl_collision_policy_rollout): every step samples
+        ``policy`` (a ``FusedGaussianPolicy``: its weights, seed and episode) on the current observation,
+        steps the env and accumulates what ``rollout`` returns -- the same bits as the closed loop
+        reset + T x (``policy.act(t=t)``, ``env.step``).  With ``record`` it adds views of the kernel-layout
+        slabs ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] (what ``rollout`` takes) and ``logp_`` [T, A, ld]:
+        ``obs`` [T, E, S], ``actions`` [T, A, E, 2] and ``logp`` [T, A, E], so that
+        ``policy.log_prob(out["obs"][t], out["actions"][t])`` is the learner's differentiable side.
+        With ``record=False`` the returned dict holds no records, also when ``out`` held some.
+        With ``out`` reused the call allocates nothing (CUDA-graph capturable)."""
+        from ..policy import FusedGaussianPolicy
+        if not isinstance(policy, FusedGaussianPolicy):
+            raise NotImplementedError("policy_rollout runs the reference's ContinuousPolicy: pass a FusedGaussianPolicy")
+        if self.n_agents > 8:
+            raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
+        T = int(n_steps)
+        A, E, S, dev = self.n_agents, self.n_envs, self.obs.shape[0], self.device
+        o = self._rollout_outputs(T, g_mode, out, 2 * T)
+        if "n_active_" not in o:
+            o["n_active_"] = self._alloc(1, torch.int32)
+        if record:
+            for name, rows in (("obs_", S), ("actions_", 2 * A), ("logp_", A)):
+                have = o.get(name)
+                if have is None or tuple(have.shape) != (T, rows, self.ld):
+                    o[name] = self._alloc(rows, torch.float32, (T,))
+            o["obs"] = o["obs_"][:, :, :E].permute(0, 2, 1)
+            o["actions"] = o["actions_"][:, :, :E].view(T, A, 2, E).permute(0, 1, 3, 2)
+            o["logp"] = o["logp_"][:, :, :E]
+        else:                                      # a reused dict must not hand back an earlier call's records
+            for name in ("obs_", "actions_", "logp_", "obs", "actions", "logp"):
+                o.pop(name, None)
+        rec = [o["obs_"], o["actions_"], o["logp_"]] if record else [None, None, None]
+        thr = device_thresholds(thresholds, dev, self.n_constraints)
+        acc = make_accounting(gamma, T, g_mode, thr)
+        pol = policy.c_params(self)
+        self._maybe_shuffle()
+        _lib.check(self.lib.smarl_collision_policy_rollout(
+            C.byref(self._params), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
+            _lib.ptr(self.landmarks), _lib.ptr(lambdas), *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x),
+            _lib.ptr(self.pos_y), _lib.ptr(self.agent_done), _lib.ptr(o["n_active_"]), _lib.ptr(o["R_"]),
+            _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]), _lib.ptr(o["stats_vec"]),
+            _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
+        o["n_active"] = o["n_active_"][0, :E]
+        return self._rollout_result(o)

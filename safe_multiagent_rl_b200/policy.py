@@ -157,19 +157,24 @@ class FusedGaussianPolicy(BatchedGaussianPolicy):
     def next_episode(self):
         self._episode_dev.add_(1)
 
+    def c_params(self, env):
+        """The ``SmarlGaussianPolicy`` of these weights and this sampling stream for ``env`` (its env_offset)."""
+        L = self._lib_mod
+        w = [t_.detach() for t_ in (self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias, self.fc2_.weight,
+                                    self.fc2_.bias)]
+        assert all(x.is_contiguous() and x.dtype == torch.float32 for x in w)
+        S = env.obs.shape[0]
+        assert S == env.state_space == self.fc1.weight.shape[1]
+        return L.GaussianPolicyParams(env.n_agents, S, 16, 2, 0, 0, *[L.ptr(x) for x in w], self.seed & (2 ** 64 - 1),
+                                      env.env_offset, L.ptr(self._episode_dev))
+
     @torch.no_grad()
     def act(self, obs=None, t=None):
         """Sample actions for step ``t`` into ``env.action_buffer``; returns (action_buffer, actions [A, E, 2] view,
         log_prob [A, E] view).  ``obs`` is ignored: the kernel reads ``env.obs``."""
         import ctypes as C
         env, L = self.env, self._lib_mod
-        w = [t_.detach() for t_ in (self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias, self.fc2_.weight,
-                                    self.fc2_.bias)]
-        assert all(x.is_contiguous() and x.dtype == torch.float32 for x in w)
-        S = env.obs.shape[0]
-        assert S == env.state_space == self.fc1.weight.shape[1]
-        p = L.GaussianPolicyParams(env.n_agents, S, 16, 2, 0, 0, *[L.ptr(x) for x in w], self.seed & (2 ** 64 - 1),
-                                   env.env_offset, L.ptr(self._episode_dev))
+        p = self.c_params(env)
         L.check(self.lib.smarl_policy_act_gaussian(C.byref(p), L.ptr(env.obs), L.ptr(env.action_buffer), L.ptr(self.logp),
                                                    int(env.t if t is None else t), env.n_envs, env.ld, L.stream_ptr()))
         A, E = env.n_agents, env.n_envs

@@ -1,0 +1,121 @@
+"""Time the on-policy CollisionAvoidance episode in one launch (BatchedCollisionAvoidance.policy_rollout,
+smarl_collision_policy_rollout) against the closed loop it replaces: T x (FusedGaussianPolicy.act + env.step) +
+the returns kernel, replayed from one CUDA graph exactly as bench.py's config2_collision_gaussian_graphed builds it.
+
+    python tools/time_policy_rollout.py [--iters 20] [--rounds 5] [--out FILE]
+
+Shapes: BASELINE configs[1] (5x5, 3 agents, 65 536 envs, T = 50, one landmark, lambda = 0.1, thresholds [2],
+reward-to-go G) and 2^20 envs at 3 and 8 agents.  The arms alternate within one process, each timed with CUDA
+events over --iters calls per round; the products of both paths are compared on the timed inputs.
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import statistics
+import subprocess
+import sys
+
+import numpy as np
+import torch
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+
+
+def event_ms(fn, iters):
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(iters):
+        fn()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / iters
+
+
+def gpu_info():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    return {"torch_name": torch.cuda.get_device_name(), "nvidia_smi": q.stdout.strip()}
+
+
+def shape(E, A, T, iters, rounds):
+    import safe_multiagent_rl_b200 as s
+    from safe_multiagent_rl_b200.policy import FusedGaussianPolicy
+    rng = np.random.default_rng(2)
+    starts, lms = rng.random((E, A, 2)) * 5, rng.random((E, 1, 2)) * 5
+    mk = lambda: s.BatchedCollisionAvoidance(5, A, n_envs=E, n_landmarks=1, starts=starts, landmarks=lms)
+    lam = torch.full((1,), 0.1, dtype=torch.float64, device="cuda")
+    thr = torch.tensor([2.0], dtype=torch.float64, device="cuda")
+    gamma = 0.999
+    env_c = mk()
+    pol_c = FusedGaussianPolicy(env_c, seed=7)                     # as bench.py builds config2_collision_gaussian_graphed
+    loop = s.GraphedClosedLoop(env_c, T, lambda obs, t: pol_c.act(t=t), lam, gamma, thresholds=[2.0])
+    env_p = mk()
+    pol_p = FusedGaussianPolicy(env_p, seed=7)
+    pol_p.load_state_dict(pol_c.state_dict())
+    kw = dict(lambdas=lam, gamma=gamma, thresholds=thr, g_mode=1)
+    out = env_p.policy_rollout(pol_p, T, **kw)
+    out_nr = env_p.policy_rollout(pol_p, T, record=False, **kw)
+    torch.cuda.synchronize()
+    graphs = {}
+    for tag, o, rec in (("fused_graphed", out, True), ("fused_graphed_no_record", out_nr, False)):
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            env_p.policy_rollout(pol_p, T, out=o, record=rec, **kw)
+        graphs[tag] = g
+    arms = {"closed_loop_graphed": loop.replay,
+            "fused_eager": lambda: env_p.policy_rollout(pol_p, T, out=out, **kw),
+            "fused_graphed": graphs["fused_graphed"].replay,
+            "fused_graphed_no_record": graphs["fused_graphed_no_record"].replay}
+    for fn in arms.values():
+        for _ in range(3):
+            fn()
+    torch.cuda.synchronize()
+    times = {k: [] for k in arms}
+    for _ in range(rounds):
+        for k, fn in arms.items():
+            times[k].append(event_ms(fn, iters))
+    # the products on the timed inputs: one more call of each path
+    ref = loop.replay()
+    graphs["fused_graphed"].replay()
+    torch.cuda.synchronize()
+    same = {k: bool(torch.equal(out[k], ref[k])) for k in ("R", "modR", "C", "G")}
+    same["n_active"] = bool(torch.equal(out["n_active"], env_c.episode_len[:E]))
+    same["final_state"] = all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                              ((env_p.pos_x, env_c.pos_x), (env_p.pos_y, env_c.pos_y), (env_p.agent_done, env_c.agent_done)))
+    same["last_step_actions"] = bool(torch.equal(out["actions_"][T - 1, :, :E], env_c.action_buffer[:, :E]))
+    same["last_step_logp"] = bool(torch.equal(out["logp_"][T - 1, :, :E], pol_c.logp[:, :E]))
+    sv, rv = out["stats_vec"], ref["stats"].vec
+    res = {"n_envs": E, "n_agents": A, "T": T, "iters": iters, "rounds": rounds,
+           "ms_per_batch": {k: {"min": min(v), "median": statistics.median(v), "all": v} for k, v in times.items()},
+           "identical": same, "stats_identical": bool(torch.equal(sv, rv)),
+           "stats_max_rel_diff": float(((sv - rv).abs() / rv.abs().clamp_min(1e-300)).max())}
+    c, f = res["ms_per_batch"]["closed_loop_graphed"]["median"], res["ms_per_batch"]["fused_graphed"]["median"]
+    res["speedup_fused_graphed_vs_closed_loop"] = c / f
+    del loop, graphs, out, out_nr
+    torch.cuda.empty_cache()
+    return res
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--rounds", type=int, default=5)
+    ap.add_argument("--shapes", default="65536x3,1048576x3,1048576x8", help="ExA list")
+    ap.add_argument("--out", default=None, help="also write the JSON lines here")
+    a = ap.parse_args()
+    lines = [json.dumps({"gpu": gpu_info(), "lib": os.path.basename(os.environ.get("SMARL_LIB", "libsmarl.so"))})]
+    print(lines[-1], flush=True)
+    for sh in a.shapes.split(","):
+        E, A = (int(x) for x in sh.split("x"))
+        lines.append(json.dumps(shape(E, A, 50, a.iters, a.rounds)))
+        print(lines[-1], flush=True)
+    if a.out:
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        with open(a.out, "w") as f:
+            f.write("\n".join(lines) + "\n")
+
+
+if __name__ == "__main__":
+    main()
