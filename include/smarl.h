@@ -430,6 +430,28 @@ int smarl_collision_policy_rollout(const SmarlCollisionParams* p, const SmarlGau
                                    double* stats, double* stats_scratch, int64_t n_envs, int64_t ld,
                                    smarl_stream_t stream);
 
+/* Whole ON-POLICY CoverageContinuous episodes in one launch: main.py:28-57 with the policies inside, i.e. per step
+ * every agent's ContinuousPolicy (agent.py:48-76) on the current observation (x0, y0, x1, ...: what the reset / step
+ * kernels write to env.obs), the sample, CoverageContinuous.step, MetaAgent.act, and Buffer.step + compute_returns as in
+ * smarl_coverage_float_rollout.  Records and final positions are bit-identical to the closed loop reset +
+ * T x (smarl_policy_act_gaussian(t) + smarl_coverage_float_step) on the same starts, weights and stream; the products
+ * are bit-identical to smarl_coverage_float_rollout fed the recorded actions (the closed loop's returns kernel sums the
+ * f32-rounded rewards, so its R, modR and C agree to ~1e-6 relative).
+ *   p (mode 0), acc, start_x .. lambdas and final_x .. stats_scratch as in smarl_coverage_float_rollout (acc->g_mode 0..2)
+ *   pol: weights, seed, episode, episode_dev and env_offset as in smarl_policy_act_gaussian;
+ *        pol->state_size = 2A, hidden 16, 2 actions
+ *   obs_rec f32 [T][2A][ld] the observation the policy saw at step t      (NULL = skip)
+ *   actions f32 [T][2A][ld] the sampled rows dx0, dy0, dx1, ... (smarl_coverage_float_rollout's layout; NULL = skip)
+ *   logp    f32 [T][A][ld]  log N(action; mu, sigma^2)                    (NULL = skip)
+ * A in 1..8 (one thread per env; A >= 9 or mode 1 returns SMARL_EUNSUPPORTED), T in 1..65536 (16 bits of the Philox
+ * counter). */
+int smarl_coverage_float_policy_rollout(const SmarlCoverageFloatParams* p, const SmarlGaussianPolicy* pol,
+                                        const SmarlAccounting* acc, const double* start_x, const double* start_y,
+                                        const double* lambdas, float* obs_rec, float* actions, float* logp,
+                                        double* final_x, double* final_y, float* R, float* modR, float* C, float* G,
+                                        float* g_scratch, double* stats, double* stats_scratch, int64_t n_envs,
+                                        int64_t ld, smarl_stream_t stream);
+
 /* ------------------------------------------------------------------------------------
  * Multi-GPU: env instances are independent (envs/coverage.py:19, congestion.py:22,
  * collision_avoidance.py:60), so ranks own contiguous ranges of global env ids and the data path has no

@@ -27,12 +27,12 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
 # Per-file extras.  collision.cu restates the reference's float64 arithmetic operation by
 # operation, so the compiler must not contract a*b+c into an FMA there.
 EXTRA = {"collision.cu": ["-fmad=false"], "collision_coop.cu": ["-fmad=false"], "collision_policy.cu": ["-fmad=false"],
-         "coverage_float.cu": ["-fmad=false"]}
+         "coverage_float.cu": ["-fmad=false"], "coverage_float_policy.cu": ["-fmad=false"]}
 # Heavy files (32 agent-count instantiations per kernel) are compiled as several translation units
 # in parallel: the file is built once per value of -DSMARL_TU=k (see the header of each file).
-# Sources that #include another .cu file: rebuilt when that file changes too (collision_policy.cu takes the env step
-# from collision.cu).
-CU_DEPS = {"collision_policy.cu": ["collision.cu"]}
+# Sources that #include another .cu file: rebuilt when that file changes too (the on-policy rollouts take the env step
+# from collision.cu / coverage_float.cu).
+CU_DEPS = {"collision_policy.cu": ["collision.cu"], "coverage_float_policy.cu": ["coverage_float.cu"]}
 TU_SPLIT = {"coverage.cu": 3, "congestion.cu": 7, "collision.cu": 3, "collision_coop.cu": 2, "congestion_coop.cu": 6, "coverage_float.cu": 5}
 
 

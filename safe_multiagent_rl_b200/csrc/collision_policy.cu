@@ -8,17 +8,13 @@
 // step the thread builds the f32 observation, evaluates the A networks, samples by Philox Box-Muller, steps the env
 // with the collision.cuh code the fused rollout uses and accumulates R / modR / C / G the way that kernel does.
 //
-// Bit-identity with the closed loop is the contract: the policy arithmetic keeps policy_gauss.cu's evaluation order
-// (h[u] = b1[u], then fma(x_k, w1[k][u], .) for k = 0..S-1; the heads from their bias over u = 0..15) and its Philox
-// counter.  This file is compiled with -fmad=false like collision.cu (the accounting relies on uncontracted f64 sums),
-// while policy_gauss.cu is compiled with contraction on: every multiply-add ptxas fuses there is written as an
-// explicit fmaf here.  Actions and log-probabilities are sampled for every (t, agent, env), including done agents and
+// Bit-identity with the closed loop is the contract: the policy code (gauss_policy.cuh, shared with
+// coverage_float_policy.cu) keeps policy_gauss.cu's evaluation order and its Philox counter.  This file is compiled with
+// -fmad=false like collision.cu (the accounting relies on uncontracted f64 sums), which gauss_policy.cuh's explicit
+// fmaf form expects.  Actions and log-probabilities are sampled for every (t, agent, env), including done agents and
 // envs past their episode end, as the policy kernel of the closed loop does.
-#include <math.h>
-
 #include "collision.cuh"
-#include "policy.cuh"
-#include "tc.cuh"
+#include "gauss_policy.cuh"
 
 // collision_env_step (the env step every one-thread CollisionAvoidance kernel runs) is defined in collision.cu; a
 // translation-unit index that selects none of that file's kernels brings in exactly the shared device code.
@@ -36,7 +32,6 @@ namespace smarl {
 #endif
 constexpr int kPolRollThreads = SMARL_POLICY_ROLLOUT_THREADS;
 constexpr int kPolRollMaxA = 8;                  // one thread per env: collision_coop_lanes returns 0 below A = 9
-constexpr int kHeadFloats = kPolHidden * 4 + 4;  // per agent: heads [u][mu0 mu1 v0 v1], then b_mu0 b_mu1 b_var0 b_var1
 
 struct CollisionPolicyArgs {
   CollisionRolloutArgs r;    // r.actions unused
@@ -68,66 +63,6 @@ constexpr size_t kPolRollStaticSmem = sizeof(double) * (kPolRollThreads / 32) +
 inline size_t policy_rollout_smem(int A, int S, int L, int obs_landmarks) {
   return sizeof(float) * ((size_t)A * (S * kPolHidden + kPolHidden + kHeadFloats) +
                           (obs_landmarks ? (size_t)2 * L * kPolRollThreads : 0));
-}
-
-// One agent's network on the observation (x: the 2A position inputs in registers, lobs: the landmark inputs), then
-// the Gaussian head: mu and sigma^2 = relu(fc2_) + 1e-4 (agent.py:60-67).
-template <int A>
-__device__ __forceinline__ void agent_heads(const float (&x)[2 * A], const float* __restrict__ lobs, int n_lobs,
-                                            const float* __restrict__ w1, const float* __restrict__ hd, float2& mu,
-                                            float& v0, float& v1) {
-  constexpr int H = kPolHidden;
-  const float* b1 = w1 + (2 * A + n_lobs) * H;
-  float2 h2[H / 2];
-#pragma unroll
-  for (int p = 0; p < H / 2; ++p) h2[p] = *reinterpret_cast<const float2*>(b1 + 2 * p);
-#pragma unroll
-  for (int k = 0; k < 2 * A; ++k) {
-    const float2 xx = make_float2(x[k], x[k]);
-    const float4* wr = reinterpret_cast<const float4*>(w1 + k * H);
-#pragma unroll
-    for (int v = 0; v < H / 4; ++v) {
-      const float4 w = wr[v];
-      h2[2 * v] = tc::ffma2(xx, make_float2(w.x, w.y), h2[2 * v]);
-      h2[2 * v + 1] = tc::ffma2(xx, make_float2(w.z, w.w), h2[2 * v + 1]);
-    }
-  }
-  for (int k = 0; k < n_lobs; ++k) {                  // shuffle=True: the landmark rows follow the positions
-    const float xk = lobs[k * kPolRollThreads];
-    const float2 xx = make_float2(xk, xk);
-    const float4* wr = reinterpret_cast<const float4*>(w1 + (2 * A + k) * H);
-#pragma unroll
-    for (int v = 0; v < H / 4; ++v) {
-      const float4 w = wr[v];
-      h2[2 * v] = tc::ffma2(xx, make_float2(w.x, w.y), h2[2 * v]);
-      h2[2 * v + 1] = tc::ffma2(xx, make_float2(w.z, w.w), h2[2 * v + 1]);
-    }
-  }
-  mu = make_float2(hd[H * 4 + 0], hd[H * 4 + 1]);
-  float2 var = make_float2(hd[H * 4 + 2], hd[H * 4 + 3]);
-#pragma unroll
-  for (int u = 0; u < H; ++u) {
-    const float r = fmaxf((u & 1) ? h2[u >> 1].y : h2[u >> 1].x, 0.f);
-    const float4 w = *reinterpret_cast<const float4*>(hd + 4 * u);
-    mu = tc::ffma2(make_float2(r, r), make_float2(w.x, w.y), mu);
-    var = tc::ffma2(make_float2(r, r), make_float2(w.z, w.w), var);
-  }
-  v0 = fmaxf(var.x, 0.f) + 1e-4f;
-  v1 = fmaxf(var.y, 0.f) + 1e-4f;
-}
-
-// Box-Muller sample and log N(action; mu, sigma^2) from two Philox words, policy_gauss.cu's arithmetic with its
-// contractions spelled out.
-__device__ __forceinline__ void gauss_sample(uint32_t wa, uint32_t wb, float2 mu, float v0, float v1, float& a0,
-                                             float& a1, float& lp) {
-  const float u0 = ((float)(wa >> 9) + 0.5f) * (1.0f / 8388608.0f), u1 = ((float)(wb >> 9) + 0.5f) * (1.0f / 8388608.0f);
-  const float rad = sqrtf(-2.0f * logf(u0));
-  float sn, cs;
-  sincospif(2.0f * u1, &sn, &cs);
-  a0 = fmaf(sqrtf(v0), rad * cs, mu.x);
-  a1 = fmaf(sqrtf(v1), rad * sn, mu.y);
-  const float d0 = a0 - mu.x, d1 = a1 - mu.y;
-  lp = fmaf(-0.5f, d0 * d0 / v0 + d1 * d1 / v1 + logf(v0) + logf(v1), -1.8378770664093453f);   // ln(2 pi)
 }
 
 template <int A>
@@ -206,7 +141,7 @@ __global__ void __launch_bounds__(kPolRollThreads) collision_policy_rollout_kern
         const int ag = 2 * j + h;
         float2 mu;
         float v0, v1, lp;
-        agent_heads<A>(x, lobs, n_lobs, s_w1 + ag * W1S, s_hd + ag * kHeadFloats, mu, v0, v1);
+        agent_heads<A, kPolRollThreads>(x, lobs, n_lobs, s_w1 + ag * W1S, s_hd + ag * kHeadFloats, mu, v0, v1);
         gauss_sample(h ? w.z : w.x, h ? w.w : w.y, mu, v0, v1, adx[ag], ady[ag], lp);
         if (live) {
           if (p.act_rec) {

@@ -35,7 +35,21 @@ constexpr int kCovFThreads = 128;
 
 int launch_coverage_float_step(int mode, int A, const CoverageFloatArgs& a, unsigned grid, cudaStream_t s);
 
-#if SMARL_TU_IS(0) || SMARL_TU_IS(1) || SMARL_TU_IS(3) || SMARL_TU_IS(4)
+// Host side of every entry point: the kernel's view of the env parameters, derived constants included.  The caller
+// sets the state, action and output pointers, n_envs and ld.
+inline void coverage_float_args(const SmarlCoverageFloatParams* p, CoverageFloatArgs& a) {
+  a = CoverageFloatArgs{};
+  a.weights = p->weights; a.size = (double)p->size; a.fieldview = p->fieldview; a.max_norm = p->max_norm;
+  a.zoom = p->zoom; a.hi = p->hi; a.cost_axis = p->cost_axis; a.cost_diag = p->cost_diag;
+  a.has_coarseness = p->has_coarseness;
+  const double m4 = (a.max_norm * a.max_norm) * (a.max_norm * a.max_norm);
+  a.m4_lo = m4 * (1.0 - 1e-9);
+  a.m4_hi = m4 * (1.0 + 1e-9);
+  a.rzoom = 1.0 / a.zoom;
+}
+
+// TU 99: coverage_float_policy.cu includes this file for the env step alone.
+#if SMARL_TU_IS(0) || SMARL_TU_IS(1) || SMARL_TU_IS(3) || SMARL_TU_IS(4) || SMARL_TU_IS(99)
 // x / zoom, correctly rounded, for the kernel-invariant divisor zoom with rzoom = RN(1 / zoom) from the host: a
 // multiply and two exact-residual corrections (5 instructions) instead of the ~45 of a float64 division, of which
 // CoverageDiscretized.transition needs two per agent-step (coverage.py:230).  q1 is a faithful quotient, and a faithful
@@ -48,24 +62,12 @@ __device__ __forceinline__ double div_by_zoom(double x, double zoom, double rzoo
   return __fma_rn(__fma_rn(-q1, zoom, x), rzoom, q1);
 }
 
-// One step of one env held in registers: moves every agent, returns the per-agent costs (f64) and the
-// unweighted env reward.  `act` points at this env's lane of step t's action rows.
+// One step of one env held in registers: moves every agent by the actions fa (mode 0: dx0, dy0, dx1, ...) or ma
+// (mode 1: 0..8), returns the per-agent costs (f64) and the unweighted env reward.
 template <int A, int MODE>
-__device__ __forceinline__ void coverage_float_env_step(double (&px)[A], double (&py)[A], const void* act, int64_t ld,
-                                                        const CoverageFloatArgs& a, double (&cost)[A], double& rew) {
-  // all action loads first: issued back to back with the caller's position loads, one memory latency per step
-  // instead of one per agent (ncu on the A = 3 step kernel: 6.9 of 13 stall cycles per issue were long_scoreboard)
-  float fa[MODE == 0 ? 2 * A : 1];
-  uint32_t ma[MODE == 1 ? A : 1];
-#pragma unroll
-  for (int i = 0; i < A; ++i) {
-    if (MODE == 0) {
-      fa[2 * i] = static_cast<const float*>(act)[(2 * i) * ld];
-      fa[2 * i + 1] = static_cast<const float*>(act)[(2 * i + 1) * ld];
-    } else {
-      ma[i] = static_cast<const uint8_t*>(act)[i * ld];
-    }
-  }
+__device__ __forceinline__ void coverage_float_env_step_regs(double (&px)[A], double (&py)[A],
+    const float (&fa)[MODE == 0 ? 2 * A : 1], const uint32_t (&ma)[MODE == 1 ? A : 1],
+    const CoverageFloatArgs& a, double (&cost)[A], double& rew) {
 #pragma unroll
   for (int i = 0; i < A; ++i) {
     if (MODE == 0) {                                   // CoverageContinuous.transition, coverage.py:54-74
@@ -107,6 +109,26 @@ __device__ __forceinline__ void coverage_float_env_step(double (&px)[A], double 
       if (gap > 0.0) rew = __dadd_rn(rew, -__dmul_rn(gap, gap));
     }
   }
+}
+
+// The same, the actions loaded from global memory: `act` points at this env's lane of step t's action rows.
+template <int A, int MODE>
+__device__ __forceinline__ void coverage_float_env_step(double (&px)[A], double (&py)[A], const void* act, int64_t ld,
+                                                        const CoverageFloatArgs& a, double (&cost)[A], double& rew) {
+  // all action loads first: issued back to back with the caller's position loads, one memory latency per step
+  // instead of one per agent (ncu on the A = 3 step kernel: 6.9 of 13 stall cycles per issue were long_scoreboard)
+  float fa[MODE == 0 ? 2 * A : 1];
+  uint32_t ma[MODE == 1 ? A : 1];
+#pragma unroll
+  for (int i = 0; i < A; ++i) {
+    if (MODE == 0) {
+      fa[2 * i] = static_cast<const float*>(act)[(2 * i) * ld];
+      fa[2 * i + 1] = static_cast<const float*>(act)[(2 * i + 1) * ld];
+    } else {
+      ma[i] = static_cast<const uint8_t*>(act)[i * ld];
+    }
+  }
+  coverage_float_env_step_regs<A, MODE>(px, py, fa, ma, a, cost, rew);
 }
 #endif
 
@@ -342,17 +364,9 @@ extern "C" int smarl_coverage_float_step(const SmarlCoverageFloatParams* p, doub
   SMARL_REQUIRE(pos_x && pos_y && actions && reward && cost, "null required pointer");
   SMARL_REQUIRE((lambdas == nullptr) == (penalty == nullptr), "lambdas and penalty go together");
   CoverageFloatArgs a;
+  coverage_float_args(p, a);
   a.pos_x = pos_x; a.pos_y = pos_y; a.actions = actions; a.obs = obs; a.reward = reward; a.cost = cost;
-  a.done = done; a.lambdas = lambdas; a.penalty = penalty; a.weights = p->weights; a.n_envs = n_envs;
-  a.ld = ld; a.size = (double)p->size; a.fieldview = p->fieldview; a.max_norm = p->max_norm;
-  a.zoom = p->zoom; a.hi = p->hi; a.cost_axis = p->cost_axis; a.cost_diag = p->cost_diag;
-  a.has_coarseness = p->has_coarseness;
-  {
-    const double m4 = (a.max_norm * a.max_norm) * (a.max_norm * a.max_norm);
-    a.m4_lo = m4 * (1.0 - 1e-9);
-    a.m4_hi = m4 * (1.0 + 1e-9);
-    a.rzoom = 1.0 / a.zoom;
-  }
+  a.done = done; a.lambdas = lambdas; a.penalty = penalty; a.n_envs = n_envs; a.ld = ld;
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
   return p->mode == 0 ? launch_coverage_float_step_m0(p->n_agents, a, grid, (cudaStream_t)stream)
                       : launch_coverage_float_step_m1(p->n_agents, a, grid, (cudaStream_t)stream);
@@ -375,17 +389,9 @@ extern "C" int smarl_coverage_float_rollout(const SmarlCoverageFloatParams* p, c
   SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   CoverageFloatRolloutArgs r;
   CoverageFloatArgs& a = r.env;
+  coverage_float_args(p, a);
   a.pos_x = const_cast<double*>(start_x); a.pos_y = const_cast<double*>(start_y); a.actions = actions;
-  a.obs = nullptr; a.reward = nullptr; a.cost = nullptr; a.done = nullptr; a.lambdas = lambdas; a.penalty = nullptr;
-  a.weights = p->weights; a.n_envs = n_envs; a.ld = ld; a.size = (double)p->size; a.fieldview = p->fieldview;
-  a.max_norm = p->max_norm; a.zoom = p->zoom; a.hi = p->hi; a.cost_axis = p->cost_axis; a.cost_diag = p->cost_diag;
-  a.has_coarseness = p->has_coarseness;
-  {
-    const double m4 = (a.max_norm * a.max_norm) * (a.max_norm * a.max_norm);
-    a.m4_lo = m4 * (1.0 - 1e-9);
-    a.m4_hi = m4 * (1.0 + 1e-9);
-    a.rzoom = 1.0 / a.zoom;
-  }
+  a.lambdas = lambdas; a.n_envs = n_envs; a.ld = ld;
   r.final_x = final_x; r.final_y = final_y; r.R = R; r.modR = modR; r.C = C; r.G = G; r.g_scratch = g_scratch;
   r.partials = stats_scratch; r.thresholds = acc->thresholds; r.gamma = acc->gamma; r.n_steps = acc->n_steps;
   r.g_mode = acc->g_mode;

@@ -164,6 +164,25 @@ class BatchedEnv:
             o["stats_scratch"] = torch.zeros(n_scratch, dtype=torch.float64, device=dev)
         return o
 
+    def _policy_records(self, o, T, S, record):
+        """The record slabs of an on-policy rollout in ``o``: ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] and
+        ``logp_`` [T, A, ld] (allocated unless ``o`` holds them in this shape), and their views ``obs`` [T, E, S],
+        ``actions`` [T, A, E, 2] and ``logp`` [T, A, E].  Returns the three slabs the kernel writes, or three
+        ``None`` with ``record=False``, which also drops the records ``o`` held from an earlier call."""
+        if not record:
+            for name in ("obs_", "actions_", "logp_", "obs", "actions", "logp"):
+                o.pop(name, None)
+            return [None, None, None]
+        A, E = self.n_agents, self.n_envs
+        for name, rows in (("obs_", S), ("actions_", 2 * A), ("logp_", A)):
+            have = o.get(name)
+            if have is None or tuple(have.shape) != (T, rows, self.ld):
+                o[name] = self._alloc(rows, torch.float32, (T,))
+        o["obs"] = o["obs_"][:, :, :E].permute(0, 2, 1)
+        o["actions"] = o["actions_"][:, :, :E].view(T, A, 2, E).permute(0, 1, 3, 2)
+        o["logp"] = o["logp_"][:, :, :E]
+        return [o["obs_"], o["actions_"], o["logp_"]]
+
     def _rollout_result(self, o):
         from ..rollout import Stats
         A, K, E = self.n_agents, self.n_constraints, self.n_envs

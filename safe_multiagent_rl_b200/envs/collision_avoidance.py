@@ -145,22 +145,11 @@ class BatchedCollisionAvoidance(BatchedEnv):
         if self.n_agents > 8:
             raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
         T = int(n_steps)
-        A, E, S, dev = self.n_agents, self.n_envs, self.obs.shape[0], self.device
+        E, S, dev = self.n_envs, self.obs.shape[0], self.device
         o = self._rollout_outputs(T, g_mode, out, 2 * T)
         if "n_active_" not in o:
             o["n_active_"] = self._alloc(1, torch.int32)
-        if record:
-            for name, rows in (("obs_", S), ("actions_", 2 * A), ("logp_", A)):
-                have = o.get(name)
-                if have is None or tuple(have.shape) != (T, rows, self.ld):
-                    o[name] = self._alloc(rows, torch.float32, (T,))
-            o["obs"] = o["obs_"][:, :, :E].permute(0, 2, 1)
-            o["actions"] = o["actions_"][:, :, :E].view(T, A, 2, E).permute(0, 1, 3, 2)
-            o["logp"] = o["logp_"][:, :, :E]
-        else:                                      # a reused dict must not hand back an earlier call's records
-            for name in ("obs_", "actions_", "logp_", "obs", "actions", "logp"):
-                o.pop(name, None)
-        rec = [o["obs_"], o["actions_"], o["logp_"]] if record else [None, None, None]
+        rec = self._policy_records(o, T, S, record)
         thr = device_thresholds(thresholds, dev, self.n_constraints)
         acc = make_accounting(gamma, T, g_mode, thr)
         pol = policy.c_params(self)

@@ -103,6 +103,37 @@ class BatchedCoverageContinuous(_CoverageFloat):
                                                 float(self.fieldview_size), max_norm, 0.0, 0.0, 0.0, 0.0,
                                                 _lib.ptr(self._weights))
 
+    def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
+                       out=None):
+        """Whole on-policy episode in one launch (smarl_coverage_float_policy_rollout): every step samples
+        ``policy`` (a ``FusedGaussianPolicy``: its weights, seed and episode) on the current observation,
+        steps the env and accumulates what ``rollout`` returns -- the records and final positions are the bits of
+        the closed loop reset + T x (``policy.act(t=t)``, ``env.step``), the products those of ``rollout`` fed the
+        recorded actions.  With ``record`` it adds views of the kernel-layout slabs ``obs_`` [T, 2A, ld],
+        ``actions_`` [T, 2A, ld] (what ``rollout`` takes) and ``logp_`` [T, A, ld]: ``obs`` [T, E, 2A],
+        ``actions`` [T, A, E, 2] and ``logp`` [T, A, E], so that ``policy.log_prob(out["obs"][t], out["actions"][t])``
+        is the learner's differentiable side.  With ``record=False`` the returned dict holds no records, also when
+        ``out`` held some.  With ``out`` reused the call allocates nothing (CUDA-graph capturable)."""
+        from ..policy import FusedGaussianPolicy
+        if not isinstance(policy, FusedGaussianPolicy):
+            raise NotImplementedError("policy_rollout runs the reference's ContinuousPolicy: pass a FusedGaussianPolicy")
+        if self.n_agents > 8:
+            raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
+        T = int(n_steps)
+        E, dev = self.n_envs, self.device
+        o = self._rollout_outputs(T, g_mode, out, 2 * T)
+        rec = self._policy_records(o, T, 2 * self.n_agents, record)
+        thr = device_thresholds(thresholds, dev, self.n_constraints)
+        acc = make_accounting(gamma, T, g_mode, thr)
+        pol = policy.c_params(self)
+        self._maybe_shuffle()
+        _lib.check(self.lib.smarl_coverage_float_policy_rollout(
+            C.byref(self._params), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
+            _lib.ptr(lambdas), *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x), _lib.ptr(self.pos_y),
+            _lib.ptr(o["R_"]), _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]),
+            _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
+        return self._rollout_result(o)
+
 
 class BatchedCoverageDiscretized(_CoverageFloat):
     """``CoverageDiscretized(size, n_agents, coarseness=20, shuffle, agents_size, fieldview_size, weights)``

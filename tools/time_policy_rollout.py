@@ -1,12 +1,14 @@
-"""Time the on-policy CollisionAvoidance episode in one launch (BatchedCollisionAvoidance.policy_rollout,
-smarl_collision_policy_rollout) against the closed loop it replaces: T x (FusedGaussianPolicy.act + env.step) +
-the returns kernel, replayed from one CUDA graph exactly as bench.py's config2_collision_gaussian_graphed builds it.
+"""Time the on-policy episode in one launch (``policy_rollout`` of BatchedCollisionAvoidance or
+BatchedCoverageContinuous) against the closed loop it replaces: T x (FusedGaussianPolicy.act + env.step) + the returns
+kernel, replayed from one CUDA graph (for CollisionAvoidance exactly as bench.py's config2_collision_gaussian_graphed
+builds it).
 
-    python tools/time_policy_rollout.py [--iters 20] [--rounds 5] [--out FILE]
+    python tools/time_policy_rollout.py [--env collision|coverage_continuous] [--iters 20] [--rounds 5] [--out FILE]
 
-Shapes: BASELINE configs[1] (5x5, 3 agents, 65 536 envs, T = 50, one landmark, lambda = 0.1, thresholds [2],
-reward-to-go G) and 2^20 envs at 3 and 8 agents.  The arms alternate within one process, each timed with CUDA
-events over --iters calls per round; the products of both paths are compared on the timed inputs.
+Shapes: 65 536 envs at 3 agents (BASELINE configs[1] for collision) and 2^20 envs at 3 and 8 agents, size 5, T = 50,
+lambda = 0.1, reward-to-go G.  collision: one landmark, thresholds [2].  coverage_continuous: lambda and threshold 25
+per agent, weights [1, 2, 3] at 3 agents.  The arms alternate within one process, each timed with CUDA events over
+--iters calls per round; the products of both paths are compared on the timed inputs.
 """
 from __future__ import annotations
 
@@ -98,8 +100,77 @@ def shape(E, A, T, iters, rounds):
     return res
 
 
+def shape_coverage(E, A, T, iters, rounds):
+    import safe_multiagent_rl_b200 as s
+    from safe_multiagent_rl_b200.policy import FusedGaussianPolicy
+    starts = np.random.default_rng(2).random((E, A, 2)) * 5
+    weights = [1.0, 2.0, 3.0] if A == 3 else None
+    mk = lambda: s.BatchedCoverageContinuous(5, A, n_envs=E, weights=weights, starts=starts)
+    lam = torch.full((A,), 0.1, dtype=torch.float64, device="cuda")
+    thr = torch.full((A,), 25.0, dtype=torch.float64, device="cuda")
+    gamma = 0.999
+    env_c = mk()
+    pol_c = FusedGaussianPolicy(env_c, seed=7)
+    loop = s.GraphedClosedLoop(env_c, T, lambda obs, t: pol_c.act(t=t), lam, gamma, thresholds=[25.0] * A)
+    env_p = mk()
+    pol_p = FusedGaussianPolicy(env_p, seed=7)
+    pol_p.load_state_dict(pol_c.state_dict())
+    kw = dict(lambdas=lam, gamma=gamma, thresholds=thr, g_mode=1)
+    out = env_p.policy_rollout(pol_p, T, **kw)
+    out_nr = env_p.policy_rollout(pol_p, T, record=False, **kw)
+    torch.cuda.synchronize()
+    graphs = {}
+    for tag, o, rec in (("fused_graphed", out, True), ("fused_graphed_no_record", out_nr, False)):
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            env_p.policy_rollout(pol_p, T, out=o, record=rec, **kw)
+        graphs[tag] = g
+    arms = {"closed_loop_graphed": loop.replay,
+            "fused_eager": lambda: env_p.policy_rollout(pol_p, T, out=out, **kw),
+            "fused_graphed": graphs["fused_graphed"].replay,
+            "fused_graphed_no_record": graphs["fused_graphed_no_record"].replay}
+    for fn in arms.values():
+        for _ in range(3):
+            fn()
+    torch.cuda.synchronize()
+    times = {k: [] for k in arms}
+    for _ in range(rounds):
+        for k, fn in arms.items():
+            times[k].append(event_ms(fn, iters))
+    # the products on the timed inputs: one more call of each path, then the open-loop rollout of the recorded actions
+    ref = loop.replay()
+    graphs["fused_graphed"].replay()
+    torch.cuda.synchronize()
+    same = {"final_state": all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                               ((env_p.pos_x, env_c.pos_x), (env_p.pos_y, env_c.pos_y))),
+            "last_step_actions": bool(torch.equal(out["actions_"][T - 1, :, :E], env_c.action_buffer[:, :E])),
+            "last_step_logp": bool(torch.equal(out["logp_"][T - 1, :, :E], pol_c.logp[:, :E]))}
+    fused = {k: out[k].clone() for k in ("R", "modR", "C", "G", "stats_vec")}
+    env_r = mk()
+    open_loop = env_r.rollout(out["actions_"], **kw)
+    torch.cuda.synchronize()
+    same_open = {k: bool(torch.equal(fused[k], open_loop[k])) for k in fused}
+    same_open["final_state"] = all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                                   ((env_p.pos_x, env_r.pos_x), (env_p.pos_y, env_r.pos_y)))
+
+    def rel(a, b):
+        a, b = a.double(), b.double()
+        return float(((a - b).abs() / b.abs().clamp_min(1e-300)).max())
+    res = {"env": "coverage_continuous", "n_envs": E, "n_agents": A, "T": T, "iters": iters, "rounds": rounds,
+           "ms_per_batch": {k: {"min": min(v), "median": statistics.median(v), "all": v} for k, v in times.items()},
+           "identical_to_closed_loop": same, "identical_to_open_loop_rollout": same_open,
+           "max_rel_diff_vs_closed_loop": {k: rel(fused[k], ref[k]) for k in ("R", "modR", "C")} |
+                                          {"stats": rel(fused["stats_vec"], ref["stats"].vec)}}
+    c, f = res["ms_per_batch"]["closed_loop_graphed"]["median"], res["ms_per_batch"]["fused_graphed"]["median"]
+    res["speedup_fused_graphed_vs_closed_loop"] = c / f
+    del loop, graphs, out, out_nr
+    torch.cuda.empty_cache()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--env", choices=("collision", "coverage_continuous"), default="collision")
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--shapes", default="65536x3,1048576x3,1048576x8", help="ExA list")
@@ -109,7 +180,8 @@ def main():
     print(lines[-1], flush=True)
     for sh in a.shapes.split(","):
         E, A = (int(x) for x in sh.split("x"))
-        lines.append(json.dumps(shape(E, A, 50, a.iters, a.rounds)))
+        run = shape if a.env == "collision" else shape_coverage
+        lines.append(json.dumps(run(E, A, 50, a.iters, a.rounds)))
         print(lines[-1], flush=True)
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
