@@ -2,9 +2,10 @@
 
     python -m safe_multiagent_rl_b200.build [--force] [--verbose]
 
-nvcc cross-compiles without a GPU.  Objects are rebuilt only when a source or header is
-newer.  The library lands in safe_multiagent_rl_b200/_lib/libsmarl.so (git-ignored, but it
-travels to the GPU box with the gpurun snapshot).
+nvcc cross-compiles without a GPU.  An object is rebuilt only when its own source or some header
+is newer, so code that several sources share lives in headers (.cuh): a source never includes
+another .cu file (tests/test_no_cu_includes.py checks this).  The library lands in
+safe_multiagent_rl_b200/_lib/libsmarl.so (git-ignored).
 """
 from __future__ import annotations
 
@@ -30,9 +31,6 @@ EXTRA = {"collision.cu": ["-fmad=false"], "collision_coop.cu": ["-fmad=false"], 
          "coverage_float.cu": ["-fmad=false"], "coverage_float_policy.cu": ["-fmad=false"]}
 # Heavy files (32 agent-count instantiations per kernel) are compiled as several translation units
 # in parallel: the file is built once per value of -DSMARL_TU=k (see the header of each file).
-# Sources that #include another .cu file: rebuilt when that file changes too (the on-policy rollouts take the env step
-# from collision.cu / coverage_float.cu).
-CU_DEPS = {"collision_policy.cu": ["collision.cu"], "coverage_float_policy.cu": ["coverage_float.cu"]}
 TU_SPLIT = {"coverage.cu": 3, "congestion.cu": 7, "collision.cu": 3, "collision_coop.cu": 2, "congestion_coop.cu": 6, "coverage_float.cu": 5}
 
 
@@ -68,8 +66,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
         for tu in range(n_tu):
             o = os.path.join(OBJ_DIR, src[:-3] + (f".tu{tu}" if n_tu > 1 else "") + ".o")
             objs.append(o)
-            deps = [os.path.getmtime(os.path.join(CSRC, d)) for d in CU_DEPS.get(src, [])]
-            if force or not os.path.exists(o) or os.path.getmtime(o) < max([os.path.getmtime(s), hm] + deps):
+            if force or not os.path.exists(o) or os.path.getmtime(o) < max(os.path.getmtime(s), hm):
                 cmd = [nvcc, *ARCH, *COMMON, *EXTRA.get(src, []), "-c", s, "-o", o]
                 if n_tu > 1:
                     cmd.insert(1, f"-DSMARL_TU={tu}")

@@ -17,112 +17,6 @@
 
 namespace smarl {
 
-constexpr int kPairPrefilterA = 12;   // agent count from which the pair loop is screened in f32
-
-// One CollisionAvoidance.step for one env held in registers.  Returns the env reward (same for
-// every agent) and the collision count; updates px/py/done_mask in place.
-// MOVED: the transition (collision_avoidance.py:103-121) was already applied by collision_transition_compact.
-template <int A, bool LM0>
-__device__ __forceinline__ void collision_env_step(double (&px)[A], double (&py)[A], uint32_t& done_mask,
-                                                   const double* __restrict__ lm, int64_t ld, int L,
-                                                   double lx0, double ly0, double size, double agents_size,
-                                                   double& reward, int& collisions) {
-  // landmark reach (:122-124) and per-agent min landmark distance (:158-161).  Both compare / minimise
-  // square roots; sqrt_rn is monotonic, so the reach test is decided on the squared norm outside a
-  // 1e-9 band around agents_size^2 and the minimum is taken over the squared distances, leaving ONE
-  // sqrt per agent (instead of two per agent and landmark).
-  double minq[A];
-  uint32_t reach = 0u;
-  const double as2 = agents_size * agents_size;
-  const double as2_lo = as2 * 0.999999999, as2_hi = as2 * 1.000000001;
-#pragma unroll
-  for (int i = 0; i < A; ++i) minq[i] = 1.0e300;
-  for (int l = 0; l < L; ++l) {
-    // LM0: landmark 0 was loaded by the caller together with the positions (the step kernel): loaded here, after the
-    // transition, its memory latency sat on every thread's critical path (A = 3 on 2^22 envs: 9.00 -> 8.16 ms closed
-    // loop).  The fused rollout keeps the load here (hoisted or held across the loop it measured 4-7 % slower).
-    const double lx = (LM0 && l == 0) ? lx0 : lm[(2 * l) * ld], ly = (LM0 && l == 0) ? ly0 : lm[(2 * l + 1) * ld];
-#pragma unroll
-    for (int i = 0; i < A; ++i) {
-      const double ax = __dadd_rn(px[i], -lx), ay = __dadd_rn(py[i], -ly);
-      const double axx = __dmul_rn(ax, ax);
-      // np.linalg.norm(state - land) = sqrt(ddot) = sqrt(fma(ay, ay, ax*ax))   [probed, OpenBLAS]
-      const double qn = __fma_rn(ay, ay, axx);
-      bool hit = qn < as2_lo;
-      if (!hit && qn < as2_hi) hit = sqrt_below(qn, agents_size);
-      reach |= hit ? (1u << i) : 0u;
-      // distance_matrix(states, landmarks): sqrt((lx-px)^2 + (ly-py)^2); (lx-px)^2 == (px-lx)^2 exactly
-      minq[i] = fmin(minq[i], __dadd_rn(axx, __dmul_rn(ay, ay)));
-    }
-  }
-  double mind[A];
-#pragma unroll
-  for (int i = 0; i < A; ++i) mind[i] = __dsqrt_rn(minq[i]);
-  done_mask |= reach & ~done_mask;   // only agents that moved this step are tested; done ones stay done
-  reward = -numpy_sum<A>(mind);      // :127-130, all agents incl. done ones
-  // collisions among agents not done after this step (:150-156)
-  int n = 0;
-  const double lim = 2.0 * agents_size;
-  const double lim2 = lim * lim;
-  const double lim2_lo = lim2 * 0.999999, lim2_hi = lim2 * 1.000001;
-  const uint32_t alive = ~done_mask;
-  if constexpr (A >= kPairPrefilterA) {
-    // Many agents: the A(A-1)/2 pair tests dominate and almost all pairs are far apart.  Screen them in f32
-    // (full-rate pipe, half the registers): coordinates <= 254 carry an absolute f32 error < 2e-5, so the f32
-    // squared distance of a pair with |d| ~ lim is off by < 1e-4 relative -- far inside the 1 % margin.  Only
-    // pairs that pass the screen are evaluated in f64, out of line, from a local-memory copy of the positions.
-    double cx[A], cy[A];
-    float fx[A], fy[A];
-#pragma unroll
-    for (int i = 0; i < A; ++i) {
-      cx[i] = px[i];
-      cy[i] = py[i];
-      fx[i] = (float)px[i];
-      fy[i] = (float)py[i];
-    }
-    const float screen = collision_screen_q(lim, size);
-#pragma unroll
-    for (int i = 0; i < A; ++i) {
-      uint32_t near = 0u;
-#pragma unroll
-      for (int j = i + 1; j < A; ++j) {
-        const float dx = fx[i] - fx[j], dy = fy[i] - fy[j];
-        near |= (fmaf(dy, dy, dx * dx) < screen) ? (1u << j) : 0u;
-      }
-      near &= ((alive >> i) & 1u) ? alive : 0u;
-      while (near) {
-        const int j = __ffs((int)near) - 1;
-        near &= near - 1u;
-        n += pair_collides(cx, cy, i, j, lim2_lo, lim2_hi, lim);
-      }
-    }
-  } else {
-    bool band = false;
-#pragma unroll
-    for (int i = 0; i < A; ++i) {
-#pragma unroll
-      for (int j = i + 1; j < A; ++j) {
-        const double dx = __dadd_rn(px[i], -px[j]), dy = __dadd_rn(py[i], -py[j]);
-        const double q = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
-        const bool below_lo = q < lim2_lo, below_hi = q < lim2_hi;
-        n += (below_lo && ((alive >> i) & (alive >> j) & 1u)) ? 1 : 0;
-        band |= below_lo != below_hi;
-      }
-    }
-    if (band) {
-      double cx[A], cy[A];
-#pragma unroll
-      for (int i = 0; i < A; ++i) {
-        cx[i] = px[i];
-        cy[i] = py[i];
-      }
-      n = collisions_exact(cx, cy, A, alive, lim);
-    }
-  }
-  collisions = n;
-}
-
-
 #if SMARL_TU_IS(0)
 // CAP: 64 registers (8 CTAs per SM) for A <= 4 on large batches, where occupancy pays (2^22 envs: closed loop +6.6 %,
 // fused +9 %); a one-wave batch like config 1 (65 536 envs) is latency-bound per thread and loses 3 % to the spills.
@@ -384,14 +278,6 @@ int collision_coop_lanes(int A, int L, int64_t ld, bool rollout) {
   return A <= 16 ? 2 : 4;
 }
 
-static int check_collision(const SmarlCollisionParams* p) {
-  SMARL_REQUIRE(p != nullptr, "params is NULL");
-  SMARL_REQUIRE(p->size >= 1, "size=%d must be >= 1", p->size);
-  SMARL_REQUIRE(p->n_landmarks >= 1 && p->n_landmarks <= 64, "n_landmarks=%d outside 1..64", p->n_landmarks);
-  SMARL_REQUIRE(p->agents_size > 0.0, "agents_size must be positive");
-  return SMARL_OK;
-}
-
 #endif
 
 }  // namespace smarl
@@ -450,13 +336,9 @@ extern "C" int smarl_collision_rollout(const SmarlCollisionParams* p, const Smar
                                        smarl_stream_t stream) {
   if (int rc = check_collision(p)) return rc;
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc != nullptr, "accounting params is NULL");
-  SMARL_REQUIRE(acc->n_steps >= 1, "n_steps=%d must be >= 1", acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 2, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, INT32_MAX, 2, G, stats, stats_scratch)) return rc;
   SMARL_REQUIRE(start_x && start_y && landmarks && actions && R && modR && C, "null required pointer");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
   SMARL_REQUIRE(acc->g_mode != 1 || g_scratch, "g_mode 1 needs g_scratch [2][T][ld]");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   CollisionRolloutArgs a;
   a.start_x = start_x; a.start_y = start_y; a.landmarks = landmarks; a.actions = actions;
   a.lambdas = lambdas; a.final_x = final_x; a.final_y = final_y; a.final_done = final_done;

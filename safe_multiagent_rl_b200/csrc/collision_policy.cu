@@ -6,21 +6,19 @@
 // One thread owns one env, as in collision_rollout_kernel (collision.cu): the f64 positions and the done mask stay in
 // registers for all T steps, every agent's weights sit in shared memory and are read as warp-wide broadcasts.  Per
 // step the thread builds the f32 observation, evaluates the A networks, samples by Philox Box-Muller, steps the env
-// with the collision.cuh code the fused rollout uses and accumulates R / modR / C / G the way that kernel does.
+// with the collision.cuh code the fused rollout uses (collision_transition_compact, collision_env_step) and accumulates
+// R / modR / C / G the way that kernel does.
 //
 // Bit-identity with the closed loop is the contract: the policy code (gauss_policy.cuh, shared with
 // coverage_float_policy.cu) keeps policy_gauss.cu's evaluation order and its Philox counter.  This file is compiled with
 // -fmad=false like collision.cu (the accounting relies on uncontracted f64 sums), which gauss_policy.cuh's explicit
 // fmaf form expects.  Actions and log-probabilities are sampled for every (t, agent, env), including done agents and
 // envs past their episode end, as the policy kernel of the closed loop does.
+//
+// The weight staging and the accounting are copies of coverage_float_policy.cu's and collision_rollout_kernel's (DESIGN.md
+// section 3.12 says why they are not shared).
 #include "collision.cuh"
 #include "gauss_policy.cuh"
-
-// collision_env_step (the env step every one-thread CollisionAvoidance kernel runs) is defined in collision.cu; a
-// translation-unit index that selects none of that file's kernels brings in exactly the shared device code.
-#define SMARL_TU 99
-#include "collision.cu"
-#undef SMARL_TU
 
 namespace smarl {
 
@@ -38,16 +36,7 @@ struct CollisionPolicyArgs {
   float* obs_rec;            // [T][S][ld]  or NULL
   float* act_rec;            // [T][2A][ld] or NULL
   float* logp_rec;           // [T][A][ld]  or NULL
-  const float* w1;           // [A][S][16]
-  const float* b1;           // [A][16]
-  const float* w_mu;         // [A][16][2]
-  const float* b_mu;         // [A][2]
-  const float* w_var;        // [A][16][2]
-  const float* b_var;        // [A][2]
-  uint64_t seed;
-  int64_t env_offset;
-  uint32_t episode;
-  const uint32_t* episode_dev;
+  GaussPolicyArgs pol;
   int32_t S;
   int32_t obs_landmarks;
   int32_t normalize;
@@ -77,17 +66,17 @@ __global__ void __launch_bounds__(kPolRollThreads) collision_policy_rollout_kern
   float* s_hd = s_w1 + A * W1S;                        // [A][kHeadFloats]
   float* s_lobs = s_hd + A * kHeadFloats;              // [n_lobs][kPolRollThreads]
   const int tid = threadIdx.x;
-  for (int i = tid; i < A * S * H; i += kPolRollThreads) s_w1[(i / (S * H)) * W1S + i % (S * H)] = __ldg(p.w1 + i);
-  for (int i = tid; i < A * H; i += kPolRollThreads) s_w1[(i / H) * W1S + S * H + i % H] = __ldg(p.b1 + i);
+  for (int i = tid; i < A * S * H; i += kPolRollThreads) s_w1[(i / (S * H)) * W1S + i % (S * H)] = __ldg(p.pol.w1 + i);
+  for (int i = tid; i < A * H; i += kPolRollThreads) s_w1[(i / H) * W1S + S * H + i % H] = __ldg(p.pol.b1 + i);
   for (int i = tid; i < A * kHeadFloats; i += kPolRollThreads) {
     const int ag = i / kHeadFloats, j = i % kHeadFloats;
     float v;
     if (j < H * 4) {
       const int u = j / 4, c = j % 4;
-      v = c < 2 ? __ldg(p.w_mu + (ag * H + u) * 2 + c) : __ldg(p.w_var + (ag * H + u) * 2 + (c - 2));
+      v = c < 2 ? __ldg(p.pol.w_mu + (ag * H + u) * 2 + c) : __ldg(p.pol.w_var + (ag * H + u) * 2 + (c - 2));
     } else {
       const int c = j - H * 4;
-      v = c < 2 ? __ldg(p.b_mu + ag * 2 + c) : __ldg(p.b_var + ag * 2 + (c - 2));
+      v = c < 2 ? __ldg(p.pol.b_mu + ag * 2 + c) : __ldg(p.pol.b_var + ag * 2 + (c - 2));
     }
     s_hd[i] = v;
   }
@@ -106,9 +95,9 @@ __global__ void __launch_bounds__(kPolRollThreads) collision_policy_rollout_kern
     px[i] = a.start_x[i * ld + e];
     py[i] = a.start_y[i * ld + e];
   }
-  const uint2 key = make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32) ^ 0x47415553u);   // "GAUS"
-  const uint32_t t_base = (p.episode << 16) + ((p.episode_dev ? __ldg(p.episode_dev) : 0u) << 16);
-  const uint64_t id = (uint64_t)(p.env_offset + e);
+  const uint2 key = make_uint2((uint32_t)p.pol.seed, (uint32_t)(p.pol.seed >> 32) ^ 0x47415553u);   // "GAUS"
+  const uint32_t t_base = (p.pol.episode << 16) + ((p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u) << 16);
+  const uint64_t id = (uint64_t)(p.pol.env_offset + e);
   __syncthreads();
 
   const uint32_t all = (1u << A) - 1u;
@@ -236,24 +225,13 @@ extern "C" int smarl_collision_policy_rollout(const SmarlCollisionParams* p, con
     set_error("the on-policy rollout runs one thread per env: n_agents=%d above %d", p->n_agents, kPolRollMaxA);
     return SMARL_EUNSUPPORTED;
   }
-  SMARL_REQUIRE(p->size >= 1, "size=%d must be >= 1", p->size);
-  SMARL_REQUIRE(p->n_landmarks >= 1 && p->n_landmarks <= 64, "n_landmarks=%d outside 1..64", p->n_landmarks);
-  SMARL_REQUIRE(p->agents_size > 0.0, "agents_size must be positive");
+  if (int rc = check_collision(p)) return rc;
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc->n_steps >= 1 && acc->n_steps <= 65536, "n_steps=%d outside 1..65536 (16 bits of the Philox counter)",
-                acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 2, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, 65536, 2, G, stats, stats_scratch)) return rc;   // 16 bits of the Philox counter
   const int A = p->n_agents, S = 2 * A + (p->obs_landmarks ? 2 * p->n_landmarks : 0);
-  SMARL_REQUIRE(pol->n_agents == A, "policy has %d agents, the env %d", pol->n_agents, A);
-  SMARL_REQUIRE(pol->state_size == S, "state_size=%d, the env's observation has %d rows", pol->state_size, S);
-  SMARL_REQUIRE(pol->hidden == kPolHidden && pol->n_actions == 2,
-                "only the reference's ContinuousPolicy shape (hidden 16, 2 actions) is built (got %d, %d)", pol->hidden,
-                pol->n_actions);
-  SMARL_REQUIRE(pol->w1 && pol->b1 && pol->w_mu && pol->b_mu && pol->w_var && pol->b_var, "null policy weight");
+  if (int rc = check_gaussian_policy(pol, A, S)) return rc;
   SMARL_REQUIRE(start_x && start_y && landmarks && R && modR && C, "null required pointer");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
   SMARL_REQUIRE(acc->g_mode != 1 || g_scratch, "g_mode 1 needs g_scratch [2][T][ld]");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   CollisionPolicyArgs k;
   CollisionRolloutArgs& a = k.r;
   a.start_x = start_x; a.start_y = start_y; a.landmarks = landmarks; a.actions = nullptr;
@@ -262,9 +240,7 @@ extern "C" int smarl_collision_policy_rollout(const SmarlCollisionParams* p, con
   a.partials = stats_scratch; a.thresholds = acc->thresholds; a.gamma = acc->gamma; a.n_envs = n_envs;
   a.ld = ld; a.size = (double)p->size; a.agents_size = p->agents_size; a.L = p->n_landmarks;
   a.n_steps = acc->n_steps; a.g_mode = acc->g_mode;
-  k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
-  k.w1 = pol->w1; k.b1 = pol->b1; k.w_mu = pol->w_mu; k.b_mu = pol->b_mu; k.w_var = pol->w_var; k.b_var = pol->b_var;
-  k.seed = pol->seed; k.env_offset = pol->env_offset; k.episode = pol->episode; k.episode_dev = pol->episode_dev;
+  k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp; k.pol = gauss_policy_args(pol);
   k.S = S; k.obs_landmarks = p->obs_landmarks; k.normalize = p->normalize_state;
   const size_t smem = policy_rollout_smem(A, S, p->n_landmarks, p->obs_landmarks);
   const unsigned grid = (unsigned)((n_envs + kPolRollThreads - 1) / kPolRollThreads);

@@ -43,6 +43,11 @@ bool pdl_enabled();
 // Checks the shared layout contract of smarl.h for one call.
 int check_layout(int64_t n_envs, int64_t ld);
 
+// Checks the accounting arguments every fused rollout and returns entry point takes: acc present,
+// 1 <= n_steps <= max_steps, 0 <= g_mode <= max_g_mode, G present unless g_mode is 0, stats and stats_scratch together.
+int check_accounting(const SmarlAccounting* acc, int max_steps, int max_g_mode, const float* G, const double* stats,
+                     const double* stats_scratch);
+
 // Dispatch a compile-time agent count 1..32.
 #define SMARL_CASE_A(N, ...) \
   case N: {                  \

@@ -406,14 +406,10 @@ extern "C" int smarl_congestion_rollout(const SmarlCongestionParams* p, const Sm
                                         int64_t ld, smarl_stream_t stream) {
   if (int rc = check_congestion(p)) return rc;
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc != nullptr, "accounting params is NULL");
-  SMARL_REQUIRE(acc->n_steps >= 1, "n_steps=%d must be >= 1", acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 2, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, INT32_MAX, 2, G, stats, stats_scratch)) return rc;
   SMARL_REQUIRE(start_x && start_y && actions && R && modR && C, "null required pointer");
   SMARL_REQUIRE(p->noise_mode != 1 || moves, "noise_mode 1 needs the recorded moves [T][A][ld]");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
   SMARL_REQUIRE(acc->g_mode != 1 || g_scratch, "g_mode 1 needs g_scratch");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   SMARL_REQUIRE((int64_t)p->n_agents * ld < (1ll << 32), "A*ld = %lld exceeds 32-bit element offsets; split the env batch",
                 (long long)((int64_t)p->n_agents * ld));
   SMARL_REQUIRE(aligned16(start_x) && aligned16(start_y) && aligned16(actions) && aligned16(moves) &&

@@ -459,14 +459,9 @@ extern "C" int smarl_coverage_rollout(const SmarlCoverageParams* p, const SmarlA
                                       smarl_stream_t stream) {
   if (int rc = check_coverage(p)) return rc;
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc != nullptr, "accounting params is NULL");
-  SMARL_REQUIRE(acc->n_steps >= 1 && acc->n_steps <= 255, "fused rollout needs 1 <= n_steps <= 255 (got %d)",
-                acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 2, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, 255, 2, G, stats, stats_scratch)) return rc;
   SMARL_REQUIRE(start_x && start_y && actions && R && modR && C, "null required pointer");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
   SMARL_REQUIRE(acc->g_mode != 1 || g_scratch, "g_mode 1 needs g_scratch [2][T][ld]");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   SMARL_REQUIRE(aligned16(start_x) && aligned16(start_y) && aligned16(actions) && aligned16(final_x) &&
                     aligned16(final_y) && aligned16(R) && aligned16(modR) && aligned16(C) &&
                     aligned16(G) && aligned16(g_scratch), "pointers must be 16-byte aligned");

@@ -7,18 +7,14 @@
 // registers for all T steps, every agent's weights sit in shared memory and are read as warp-wide broadcasts.  Per step
 // the thread builds the f32 observation (x_i, y_i: what the reset / step kernels write to env.obs), evaluates the A
 // networks and samples them with gauss_policy.cuh (policy_gauss.cu's arithmetic and Philox counter), steps the env with
-// coverage_float_env_step_regs from coverage_float.cu and accumulates R / modR / C / G / stats exactly as
+// coverage_float_env_step_regs from coverage_float.cuh and accumulates R / modR / C / G / stats exactly as
 // coverage_float_rollout_kernel does.  Compiled with -fmad=false like coverage_float.cu.
 //
 // The weight staging and the accounting are copies of collision_policy.cu's and coverage_float_rollout_kernel's:
 // moving either into a shared function changed the SASS of the kernel it came from (DESIGN.md section 3.12).
+#include "coverage_float.cuh"
 #include "gauss_policy.cuh"
-
-// The env step is defined in coverage_float.cu; a translation-unit index that selects none of that file's kernels brings
-// in exactly the shared device code.
-#define SMARL_TU 99
-#include "coverage_float.cu"
-#undef SMARL_TU
+#include "stats.cuh"
 
 namespace smarl {
 
@@ -29,16 +25,7 @@ struct CoverageFloatPolicyArgs {
   float* obs_rec;                   // [T][2A][ld] or NULL
   float* act_rec;                   // [T][2A][ld] or NULL
   float* logp_rec;                  // [T][A][ld]  or NULL
-  const float* w1;                  // [A][2A][16]
-  const float* b1;                  // [A][16]
-  const float* w_mu;                // [A][16][2]
-  const float* b_mu;                // [A][2]
-  const float* w_var;               // [A][16][2]
-  const float* b_var;               // [A][2]
-  uint64_t seed;
-  int64_t env_offset;
-  uint32_t episode;
-  const uint32_t* episode_dev;
+  GaussPolicyArgs pol;              // S = 2A
 };
 
 // kCovFThreads threads per CTA keep coverage_float_rollout_kernel's summation tree of the stats partials (one row per
@@ -53,17 +40,17 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_float_policy_rollout_ke
   const CoverageFloatRolloutArgs& r = p.r;
   const CoverageFloatArgs& a = r.env;
   const int tid = threadIdx.x;
-  for (int i = tid; i < A * S * H; i += kCovFThreads) s_w1[(i / (S * H)) * W1S + i % (S * H)] = __ldg(p.w1 + i);
-  for (int i = tid; i < A * H; i += kCovFThreads) s_w1[(i / H) * W1S + S * H + i % H] = __ldg(p.b1 + i);
+  for (int i = tid; i < A * S * H; i += kCovFThreads) s_w1[(i / (S * H)) * W1S + i % (S * H)] = __ldg(p.pol.w1 + i);
+  for (int i = tid; i < A * H; i += kCovFThreads) s_w1[(i / H) * W1S + S * H + i % H] = __ldg(p.pol.b1 + i);
   for (int i = tid; i < A * kHeadFloats; i += kCovFThreads) {
     const int ag = i / kHeadFloats, j = i % kHeadFloats;
     float v;
     if (j < H * 4) {
       const int u = j / 4, c = j % 4;
-      v = c < 2 ? __ldg(p.w_mu + (ag * H + u) * 2 + c) : __ldg(p.w_var + (ag * H + u) * 2 + (c - 2));
+      v = c < 2 ? __ldg(p.pol.w_mu + (ag * H + u) * 2 + c) : __ldg(p.pol.w_var + (ag * H + u) * 2 + (c - 2));
     } else {
       const int c = j - H * 4;
-      v = c < 2 ? __ldg(p.b_mu + ag * 2 + c) : __ldg(p.b_var + ag * 2 + (c - 2));
+      v = c < 2 ? __ldg(p.pol.b_mu + ag * 2 + c) : __ldg(p.pol.b_var + ag * 2 + (c - 2));
     }
     s_hd[i] = v;
   }
@@ -81,9 +68,9 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_float_policy_rollout_ke
     csum[i] = 0.0;
     lam[i] = a.lambdas ? __ldg(a.lambdas + i) : 0.0;
   }
-  const uint2 key = make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32) ^ 0x47415553u);   // "GAUS"
-  const uint32_t t_base = (p.episode << 16) + ((p.episode_dev ? __ldg(p.episode_dev) : 0u) << 16);
-  const uint64_t id = (uint64_t)(p.env_offset + e);
+  const uint2 key = make_uint2((uint32_t)p.pol.seed, (uint32_t)(p.pol.seed >> 32) ^ 0x47415553u);   // "GAUS"
+  const uint32_t t_base = (p.pol.episode << 16) + ((p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u) << 16);
+  const uint64_t id = (uint64_t)(p.pol.env_offset + e);
   __syncthreads();
 
   double s_rew = 0.0, s_pen = 0.0, disc = 1.0;
@@ -214,20 +201,11 @@ extern "C" int smarl_coverage_float_policy_rollout(const SmarlCoverageFloatParam
   }
   SMARL_REQUIRE(p->size >= 1, "size=%d must be >= 1", p->size);
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc->n_steps >= 1 && acc->n_steps <= 65536, "n_steps=%d outside 1..65536 (16 bits of the Philox counter)",
-                acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 2, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, 65536, 2, G, stats, stats_scratch)) return rc;   // 16 bits of the Philox counter
   const int A = p->n_agents;
-  SMARL_REQUIRE(pol->n_agents == A, "policy has %d agents, the env %d", pol->n_agents, A);
-  SMARL_REQUIRE(pol->state_size == 2 * A, "state_size=%d, the env's observation has %d rows", pol->state_size, 2 * A);
-  SMARL_REQUIRE(pol->hidden == kPolHidden && pol->n_actions == 2,
-                "only the reference's ContinuousPolicy shape (hidden 16, 2 actions) is built (got %d, %d)", pol->hidden,
-                pol->n_actions);
-  SMARL_REQUIRE(pol->w1 && pol->b1 && pol->w_mu && pol->b_mu && pol->w_var && pol->b_var, "null policy weight");
+  if (int rc = check_gaussian_policy(pol, A, 2 * A)) return rc;
   SMARL_REQUIRE(start_x && start_y && R && modR && C, "null required pointer");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
   SMARL_REQUIRE(acc->g_mode != 1 || g_scratch, "g_mode 1 needs g_scratch [2][T][ld]");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   CoverageFloatPolicyArgs k;
   CoverageFloatRolloutArgs& r = k.r;
   coverage_float_args(p, r.env);
@@ -236,9 +214,7 @@ extern "C" int smarl_coverage_float_policy_rollout(const SmarlCoverageFloatParam
   r.final_x = final_x; r.final_y = final_y; r.R = R; r.modR = modR; r.C = C; r.G = G; r.g_scratch = g_scratch;
   r.partials = stats_scratch; r.thresholds = acc->thresholds; r.gamma = acc->gamma; r.n_steps = acc->n_steps;
   r.g_mode = acc->g_mode;
-  k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
-  k.w1 = pol->w1; k.b1 = pol->b1; k.w_mu = pol->w_mu; k.b_mu = pol->b_mu; k.w_var = pol->w_var; k.b_var = pol->b_var;
-  k.seed = pol->seed; k.env_offset = pol->env_offset; k.episode = pol->episode; k.episode_dev = pol->episode_dev;
+  k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp; k.pol = gauss_policy_args(pol);
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
   cudaStream_t st = (cudaStream_t)stream;
   switch (A) {

@@ -1,6 +1,6 @@
 // The reference's ContinuousPolicy (agent.py:48-76) evaluated by one thread for one env, with every agent's weights
 // in shared memory: the network, the Gaussian head and the Philox Box-Muller sample of the on-policy rollouts
-// (collision_policy.cu, coverage_float_policy.cu).
+// (collision_policy.cu, coverage_float_policy.cu), and the host side of their policy arguments.
 //
 // Bit-identity with smarl_policy_act_gaussian is the contract: the arithmetic keeps policy_gauss.cu's evaluation order
 // (h[u] = b1[u], then fma(x_k, w1[k][u], .) for k = 0..S-1; the heads from their bias over u = 0..15).  policy_gauss.cu
@@ -16,6 +16,38 @@
 namespace smarl {
 
 constexpr int kHeadFloats = kPolHidden * 4 + 4;  // per agent: heads [u][mu0 mu1 v0 v1], then b_mu0 b_mu1 b_var0 b_var1
+
+// The policy part of the on-policy rollout kernels' arguments: every agent's weights and the sampling stream.
+struct GaussPolicyArgs {
+  const float* w1;           // [A][S][16]
+  const float* b1;           // [A][16]
+  const float* w_mu;         // [A][16][2]
+  const float* b_mu;         // [A][2]
+  const float* w_var;        // [A][16][2]
+  const float* b_var;        // [A][2]
+  uint64_t seed;
+  int64_t env_offset;
+  uint32_t episode;
+  const uint32_t* episode_dev;
+};
+
+inline GaussPolicyArgs gauss_policy_args(const SmarlGaussianPolicy* pol) {
+  GaussPolicyArgs g;
+  g.w1 = pol->w1; g.b1 = pol->b1; g.w_mu = pol->w_mu; g.b_mu = pol->b_mu; g.w_var = pol->w_var; g.b_var = pol->b_var;
+  g.seed = pol->seed; g.env_offset = pol->env_offset; g.episode = pol->episode; g.episode_dev = pol->episode_dev;
+  return g;
+}
+
+// A policy for an env of A agents whose observation has S rows, in the one shape the on-policy rollouts build.
+inline int check_gaussian_policy(const SmarlGaussianPolicy* pol, int A, int S) {
+  SMARL_REQUIRE(pol->n_agents == A, "policy has %d agents, the env %d", pol->n_agents, A);
+  SMARL_REQUIRE(pol->state_size == S, "state_size=%d, the env's observation has %d rows", pol->state_size, S);
+  SMARL_REQUIRE(pol->hidden == kPolHidden && pol->n_actions == 2,
+                "only the reference's ContinuousPolicy shape (hidden 16, 2 actions) is built (got %d, %d)", pol->hidden,
+                pol->n_actions);
+  SMARL_REQUIRE(pol->w1 && pol->b1 && pol->w_mu && pol->b_mu && pol->w_var && pol->b_var, "null policy weight");
+  return SMARL_OK;
+}
 
 // One agent's network on the observation (x: the 2A position inputs in registers, lobs: n_lobs further inputs, one
 // every LSTRIDE floats), then the Gaussian head: mu and sigma^2 = relu(fc2_) + 1e-4 (agent.py:60-67).

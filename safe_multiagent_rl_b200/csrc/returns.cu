@@ -40,6 +40,16 @@ int check_layout(int64_t n_envs, int64_t ld) {
   return SMARL_OK;
 }
 
+int check_accounting(const SmarlAccounting* acc, int max_steps, int max_g_mode, const float* G, const double* stats,
+                     const double* stats_scratch) {
+  SMARL_REQUIRE(acc != nullptr, "accounting params is NULL");
+  SMARL_REQUIRE(acc->n_steps >= 1 && acc->n_steps <= max_steps, "n_steps=%d outside 1..%d", acc->n_steps, max_steps);
+  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= max_g_mode, "bad g_mode %d", acc->g_mode);
+  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
+  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
+  return SMARL_OK;
+}
+
 constexpr int kAccThreads = 128;
 constexpr int kReturnsThreads = 128;   // default CTA size of returns_kernel (>= 64: stats scratch rows are sized for 64)
 constexpr int kReturnsStages = 6;      // returns_kernel's ring depth: up to kReturnsStages - 1 steps in flight per CTA
@@ -621,15 +631,11 @@ extern "C" int smarl_rollout_returns(const SmarlAccounting* acc, const float* re
                                      int32_t n_agents, int32_t n_constraints, int64_t n_envs,
                                      int64_t ld, smarl_stream_t stream) {
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc != nullptr, "accounting params is NULL");
-  SMARL_REQUIRE(acc->n_steps >= 1, "n_steps=%d must be >= 1", acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 3, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, INT32_MAX, 3, G, stats, stats_scratch)) return rc;
   SMARL_REQUIRE(n_agents >= 1 && n_agents <= SMARL_MAX_AGENTS, "n_agents=%d outside 1..32", n_agents);
   SMARL_REQUIRE(n_constraints >= 1 && n_constraints <= SMARL_MAX_AGENTS, "n_constraints=%d outside 1..32",
                 n_constraints);
   SMARL_REQUIRE(reward && cost && R && modR && C, "null required pointer");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   SMARL_REQUIRE(aligned16(reward) && aligned16(cost) && aligned16(penalty) && aligned16(R) &&
                     aligned16(modR) && aligned16(C) && aligned16(G), "pointers must be 16-byte aligned");
   ReturnsArgs a;
@@ -674,15 +680,11 @@ extern "C" int smarl_rollout_returns_shared(const SmarlAccounting* acc, const fl
                                             int32_t n_constraints, int64_t n_envs, int64_t ld,
                                             smarl_stream_t stream) {
   if (int rc = check_layout(n_envs, ld)) return rc;
-  SMARL_REQUIRE(acc != nullptr, "accounting params is NULL");
-  SMARL_REQUIRE(acc->n_steps >= 1, "n_steps=%d must be >= 1", acc->n_steps);
-  SMARL_REQUIRE(acc->g_mode >= 0 && acc->g_mode <= 3, "bad g_mode %d", acc->g_mode);
+  if (int rc = check_accounting(acc, INT32_MAX, 3, G, stats, stats_scratch)) return rc;
   SMARL_REQUIRE(n_agents >= 1 && n_agents <= SMARL_MAX_AGENTS, "n_agents=%d outside 1..32", n_agents);
   SMARL_REQUIRE(n_constraints >= 1 && n_constraints <= SMARL_MAX_AGENTS, "n_constraints=%d outside 1..32",
                 n_constraints);
   SMARL_REQUIRE(reward_env && cost && R && modR && C, "null required pointer");
-  SMARL_REQUIRE(acc->g_mode == 0 || G, "g_mode != 0 needs G");
-  SMARL_REQUIRE((stats == nullptr) == (stats_scratch == nullptr), "stats and stats_scratch go together");
   SMARL_REQUIRE(aligned16(reward_env) && aligned16(cost) && aligned16(penalty) && aligned16(R) && aligned16(modR) &&
                     aligned16(C) && aligned16(G), "pointers must be 16-byte aligned");
   ReturnsArgs a;

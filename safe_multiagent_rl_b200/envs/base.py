@@ -1,5 +1,6 @@
 """Shared host logic of the batched envs: buffers in the agent-major SoA layout, action ingest,
-reference-oriented views, closed-loop rollout helper and the single-env list adaptor."""
+reference-oriented views, closed-loop and fused rollout helpers, the on-policy rollout of the
+Gaussian-policy envs and the single-env list adaptor."""
 from __future__ import annotations
 
 import numpy as np
@@ -7,7 +8,7 @@ import torch
 
 from .. import _lib
 from ..layout import alloc, env_major, pad_ld, require_cuda
-from ..rollout import G_REWARD_TO_GO, RolloutBuffer
+from ..rollout import G_NONE, G_REWARD_TO_GO, RolloutBuffer, device_thresholds, make_accounting
 
 
 class BatchedEnv:
@@ -164,6 +165,15 @@ class BatchedEnv:
             o["stats_scratch"] = torch.zeros(n_scratch, dtype=torch.float64, device=dev)
         return o
 
+    def _begin_rollout(self, T, g_mode, out, g_scratch_rows, gamma, thresholds):
+        """What every fused rollout does before its launch: the product buffers (``_rollout_outputs``), the
+        accounting block and, with shuffle=True, this episode's start draw.  Returns (o, acc)."""
+        o = self._rollout_outputs(T, g_mode, out, g_scratch_rows)
+        thr = device_thresholds(thresholds, self.device, self.n_constraints)
+        acc = make_accounting(gamma, T, g_mode, thr)
+        self._maybe_shuffle()
+        return o, acc
+
     def _policy_records(self, o, T, S, record):
         """The record slabs of an on-policy rollout in ``o``: ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] and
         ``logp_`` [T, A, ld] (allocated unless ``o`` holds them in this shape), and their views ``obs`` [T, E, S],
@@ -218,6 +228,35 @@ class BatchedEnv:
         out = buf.finish(gamma, thresholds, g_mode, n_active=getattr(self, "episode_len", None))
         out["buffer"] = buf
         return out
+
+
+class GaussianPolicyRollout:
+    """``policy_rollout`` of the envs whose reference policy is the ContinuousPolicy (BatchedEnv subclasses).  The env
+    supplies ``_policy_rollout_impl(pol, acc, lambdas, rec, o)``, its C entry point's call."""
+
+    def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
+                       out=None):
+        """Whole on-policy episode in one launch: every step samples ``policy`` (a ``FusedGaussianPolicy``: its
+        weights, seed and episode) on the current observation, steps the env and accumulates what ``rollout``
+        returns (CollisionAvoidance's ``n_active`` included).  The records and the final state are the bits of the closed loop reset + T x (``policy.act(t=t)``,
+        ``env.step``), the products those of ``rollout`` fed the recorded actions.  With ``record`` it adds views of
+        the kernel-layout slabs ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] (what ``rollout`` takes) and ``logp_``
+        [T, A, ld]: ``obs`` [T, E, S], ``actions`` [T, A, E, 2] and ``logp`` [T, A, E], so that
+        ``policy.log_prob(out["obs"][t], out["actions"][t])`` is the learner's differentiable side.  With
+        ``record=False`` the returned dict holds no records, also when ``out`` held some.  With ``out`` reused the
+        call allocates nothing (CUDA-graph capturable)."""
+        from ..policy import FusedGaussianPolicy
+        if not isinstance(policy, FusedGaussianPolicy):
+            raise NotImplementedError("policy_rollout runs the reference's ContinuousPolicy: pass a FusedGaussianPolicy")
+        if self.n_agents > 8:
+            raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
+        T = int(n_steps)
+        o = out if out is not None else {}
+        rec = self._policy_records(o, T, self.obs.shape[0], record)
+        pol = policy.c_params(self)
+        o, acc = self._begin_rollout(T, g_mode, o, 2 * T, gamma, thresholds)
+        self._policy_rollout_impl(pol, acc, lambdas, rec, o)
+        return self._rollout_result(o)
 
 
 class SingleEnvAdapter:

@@ -10,8 +10,8 @@ import torch
 
 from .. import _lib
 from ..layout import env_major
-from ..rollout import G_NONE, device_thresholds, make_accounting
-from .base import BatchedEnv
+from ..rollout import G_NONE
+from .base import BatchedEnv, GaussianPolicyRollout
 
 
 def default_starts(size, n_agents, n_envs, n_landmarks=1):
@@ -22,7 +22,7 @@ def default_starts(size, n_agents, n_envs, n_landmarks=1):
     return draws[:, :n_agents], draws[:, n_agents:]
 
 
-class BatchedCollisionAvoidance(BatchedEnv):
+class BatchedCollisionAvoidance(GaussianPolicyRollout, BatchedEnv):
     """Constructor mirrors ``CollisionAvoidance(size, n_agents, n_landmarks, shuffle, agents_size,
     normalize_state)`` (collision_avoidance.py:49) plus ``n_envs`` / ``device``.
 
@@ -107,18 +107,20 @@ class BatchedCollisionAvoidance(BatchedEnv):
             _lib.ptr(done), _lib.ptr(self.episode_len), _lib.ptr(lambdas), _lib.ptr(penalty), self.n_envs, self.ld,
             _lib.stream_ptr()))
 
+    def _rollout_outputs(self, T, g_mode, out, g_scratch_rows):
+        # both fused rollouts also return the episode lengths, n_active
+        o = super()._rollout_outputs(T, g_mode, out, g_scratch_rows)
+        if "n_active_" not in o:
+            o["n_active_"] = self._alloc(1, torch.int32)
+        return o
+
     def rollout(self, actions, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, out=None):
         """Open-loop fused episode (one launch).  actions ``[T, 2*n_agents, ld]`` float32 (kernel layout,
         rows dx0, dy0, dx1, ...).  Adds ``n_active`` [E]: the episode length T' (main.py:51)."""
         T = int(actions.shape[0])
-        A, E, dev = self.n_agents, self.n_envs, self.device
+        A, E = self.n_agents, self.n_envs
         assert actions.dtype == torch.float32 and tuple(actions.shape) == (T, 2 * A, self.ld) and actions.is_contiguous()
-        o = self._rollout_outputs(T, g_mode, out, 2 * T)
-        if "n_active_" not in o:
-            o["n_active_"] = self._alloc(1, torch.int32)
-        thr = device_thresholds(thresholds, dev, self.n_constraints)
-        acc = make_accounting(gamma, T, g_mode, thr)
-        self._maybe_shuffle()
+        o, acc = self._begin_rollout(T, g_mode, out, 2 * T, gamma, thresholds)
         _lib.check(self.lib.smarl_collision_rollout(
             C.byref(self._params), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
             _lib.ptr(self.landmarks), _lib.ptr(actions), _lib.ptr(lambdas), _lib.ptr(self.pos_x), _lib.ptr(self.pos_y),
@@ -128,37 +130,11 @@ class BatchedCollisionAvoidance(BatchedEnv):
         o["n_active"] = o["n_active_"][0, :E]
         return self._rollout_result(o)
 
-    def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
-                       out=None):
-        """Whole on-policy episode in one launch (smarl_collision_policy_rollout): every step samples
-        ``policy`` (a ``FusedGaussianPolicy``: its weights, seed and episode) on the current observation,
-        steps the env and accumulates what ``rollout`` returns -- the same bits as the closed loop
-        reset + T x (``policy.act(t=t)``, ``env.step``).  With ``record`` it adds views of the kernel-layout
-        slabs ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] (what ``rollout`` takes) and ``logp_`` [T, A, ld]:
-        ``obs`` [T, E, S], ``actions`` [T, A, E, 2] and ``logp`` [T, A, E], so that
-        ``policy.log_prob(out["obs"][t], out["actions"][t])`` is the learner's differentiable side.
-        With ``record=False`` the returned dict holds no records, also when ``out`` held some.
-        With ``out`` reused the call allocates nothing (CUDA-graph capturable)."""
-        from ..policy import FusedGaussianPolicy
-        if not isinstance(policy, FusedGaussianPolicy):
-            raise NotImplementedError("policy_rollout runs the reference's ContinuousPolicy: pass a FusedGaussianPolicy")
-        if self.n_agents > 8:
-            raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
-        T = int(n_steps)
-        E, S, dev = self.n_envs, self.obs.shape[0], self.device
-        o = self._rollout_outputs(T, g_mode, out, 2 * T)
-        if "n_active_" not in o:
-            o["n_active_"] = self._alloc(1, torch.int32)
-        rec = self._policy_records(o, T, S, record)
-        thr = device_thresholds(thresholds, dev, self.n_constraints)
-        acc = make_accounting(gamma, T, g_mode, thr)
-        pol = policy.c_params(self)
-        self._maybe_shuffle()
+    def _policy_rollout_impl(self, pol, acc, lambdas, rec, o):
         _lib.check(self.lib.smarl_collision_policy_rollout(
             C.byref(self._params), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
             _lib.ptr(self.landmarks), _lib.ptr(lambdas), *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x),
             _lib.ptr(self.pos_y), _lib.ptr(self.agent_done), _lib.ptr(o["n_active_"]), _lib.ptr(o["R_"]),
             _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]), _lib.ptr(o["stats_vec"]),
-            _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
-        o["n_active"] = o["n_active_"][0, :E]
-        return self._rollout_result(o)
+            _lib.ptr(o["stats_scratch"]), self.n_envs, self.ld, _lib.stream_ptr()))
+        o["n_active"] = o["n_active_"][0, :self.n_envs]

@@ -10,7 +10,7 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..rollout import G_NONE, device_thresholds, make_accounting
+from ..rollout import G_NONE
 from .base import BatchedEnv
 
 # congestion.py:28 -- the reference's hard-coded table (only valid for size <= 3)
@@ -161,16 +161,13 @@ class BatchedCongestion(BatchedEnv):
         ``moves`` of the same shape replays recorded effective moves, otherwise noise comes from the
         Philox stream (same stream as T calls of ``step``)."""
         T = int(actions.shape[0])
-        A, E, dev = self.n_agents, self.n_envs, self.device
+        A, E = self.n_agents, self.n_envs
         assert actions.dtype == torch.uint8 and tuple(actions.shape) == (T, A, self.ld) and actions.is_contiguous()
         if moves is not None:
             assert moves.dtype == torch.uint8 and tuple(moves.shape) == (T, A, self.ld) and moves.is_contiguous()
         mode = NOISE_RECORDED if moves is not None else (NOISE_PHILOX if self.noise > 0 else NOISE_NONE)
-        o = self._rollout_outputs(T, g_mode, out, T)
-        thr = device_thresholds(thresholds, dev, self.n_constraints)
-        acc = make_accounting(gamma, T, g_mode, thr)
+        o, acc = self._begin_rollout(T, g_mode, out, T, gamma, thresholds)
         p = self._params(mode)
-        self._maybe_shuffle()
         self._next_noise_episode()
         _lib.check(self.lib.smarl_congestion_rollout(
             C.byref(p), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y), _lib.ptr(actions),

@@ -8,7 +8,7 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..rollout import G_NONE, device_thresholds, make_accounting
+from ..rollout import G_NONE
 from .base import BatchedEnv
 
 
@@ -134,12 +134,9 @@ class BatchedCoverageDiscrete(BatchedEnv):
         R/modR [E,A], C [E,A] i32, G [T,E,A] or None, final positions, stats.
         """
         T = int(actions.shape[0])
-        A, E, dev = self.n_agents, self.n_envs, self.device
+        A, E = self.n_agents, self.n_envs
         assert actions.dtype == torch.uint8 and tuple(actions.shape) == (T, A, self.ld) and actions.is_contiguous()
-        o = self._rollout_outputs(T, g_mode, out, 2 * T)
-        thr = device_thresholds(thresholds, dev, self.n_constraints)
-        acc = make_accounting(gamma, T, g_mode, thr)
-        self._maybe_shuffle()
+        o, acc = self._begin_rollout(T, g_mode, out, 2 * T, gamma, thresholds)
         _lib.check(self.lib.smarl_coverage_rollout(
             C.byref(self._params), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
             _lib.ptr(actions), _lib.ptr(lambdas), _lib.ptr(self.pos_x), _lib.ptr(self.pos_y), _lib.ptr(o["R_"]),

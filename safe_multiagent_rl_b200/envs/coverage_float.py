@@ -8,8 +8,8 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..rollout import G_NONE, device_thresholds, make_accounting
-from .base import BatchedEnv
+from ..rollout import G_NONE
+from .base import BatchedEnv, GaussianPolicyRollout
 
 
 class _CoverageFloat(BatchedEnv):
@@ -64,18 +64,14 @@ class _CoverageFloat(BatchedEnv):
         """Open-loop fused episode (one launch).  actions in the kernel layout: float32 ``[T, 2*n_agents, ld]``
         (Continuous) or uint8 ``[T, n_agents, ld]`` (Discretized).  ``C`` holds float cost sums."""
         T = int(actions.shape[0])
-        A, E, dev = self.n_agents, self.n_envs, self.device
         assert actions.dtype == self.action_dtype and tuple(actions.shape) == (T, self.action_rows, self.ld) \
             and actions.is_contiguous()
-        o = self._rollout_outputs(T, g_mode, out, 2 * T)
-        thr = device_thresholds(thresholds, dev, self.n_constraints)
-        acc = make_accounting(gamma, T, g_mode, thr)
-        self._maybe_shuffle()
+        o, acc = self._begin_rollout(T, g_mode, out, 2 * T, gamma, thresholds)
         _lib.check(self.lib.smarl_coverage_float_rollout(
             C.byref(self._params), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y), _lib.ptr(actions),
             _lib.ptr(lambdas), _lib.ptr(self.pos_x), _lib.ptr(self.pos_y), _lib.ptr(o["R_"]), _lib.ptr(o["modR_"]),
             _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]), _lib.ptr(o["stats_vec"]),
-            _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
+            _lib.ptr(o["stats_scratch"]), self.n_envs, self.ld, _lib.stream_ptr()))
         return self._rollout_result(o)
 
     def _draw_starts(self, episode):
@@ -83,7 +79,7 @@ class _CoverageFloat(BatchedEnv):
         self._draw_float_starts(episode, 3 if zoom is not None else 2, zoom or 0.0)
 
 
-class BatchedCoverageContinuous(_CoverageFloat):
+class BatchedCoverageContinuous(GaussianPolicyRollout, _CoverageFloat):
     """``CoverageContinuous(size, n_agents, shuffle, agents_size, fieldview_size, weights, coarseness)``
     (coverage.py:11) + ``n_envs``/``device``.  Actions are ``[n_envs, n_agents, 2]`` float32."""
 
@@ -103,36 +99,12 @@ class BatchedCoverageContinuous(_CoverageFloat):
                                                 float(self.fieldview_size), max_norm, 0.0, 0.0, 0.0, 0.0,
                                                 _lib.ptr(self._weights))
 
-    def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
-                       out=None):
-        """Whole on-policy episode in one launch (smarl_coverage_float_policy_rollout): every step samples
-        ``policy`` (a ``FusedGaussianPolicy``: its weights, seed and episode) on the current observation,
-        steps the env and accumulates what ``rollout`` returns -- the records and final positions are the bits of
-        the closed loop reset + T x (``policy.act(t=t)``, ``env.step``), the products those of ``rollout`` fed the
-        recorded actions.  With ``record`` it adds views of the kernel-layout slabs ``obs_`` [T, 2A, ld],
-        ``actions_`` [T, 2A, ld] (what ``rollout`` takes) and ``logp_`` [T, A, ld]: ``obs`` [T, E, 2A],
-        ``actions`` [T, A, E, 2] and ``logp`` [T, A, E], so that ``policy.log_prob(out["obs"][t], out["actions"][t])``
-        is the learner's differentiable side.  With ``record=False`` the returned dict holds no records, also when
-        ``out`` held some.  With ``out`` reused the call allocates nothing (CUDA-graph capturable)."""
-        from ..policy import FusedGaussianPolicy
-        if not isinstance(policy, FusedGaussianPolicy):
-            raise NotImplementedError("policy_rollout runs the reference's ContinuousPolicy: pass a FusedGaussianPolicy")
-        if self.n_agents > 8:
-            raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
-        T = int(n_steps)
-        E, dev = self.n_envs, self.device
-        o = self._rollout_outputs(T, g_mode, out, 2 * T)
-        rec = self._policy_records(o, T, 2 * self.n_agents, record)
-        thr = device_thresholds(thresholds, dev, self.n_constraints)
-        acc = make_accounting(gamma, T, g_mode, thr)
-        pol = policy.c_params(self)
-        self._maybe_shuffle()
+    def _policy_rollout_impl(self, pol, acc, lambdas, rec, o):
         _lib.check(self.lib.smarl_coverage_float_policy_rollout(
             C.byref(self._params), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
             _lib.ptr(lambdas), *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x), _lib.ptr(self.pos_y),
             _lib.ptr(o["R_"]), _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]),
-            _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
-        return self._rollout_result(o)
+            _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), self.n_envs, self.ld, _lib.stream_ptr()))
 
 
 class BatchedCoverageDiscretized(_CoverageFloat):

@@ -66,6 +66,42 @@ def test_validation_errors_before_any_cuda_work(lib):
     assert rc == -1 and b"aligned" in lib.smarl_last_error()
     with pytest.raises(_lib.SmarlError):
         _lib.check(rc)
+    # The accounting arguments of the open-loop rollouts and the returns entry points: each call below fails on them
+    f = fake
+    cov = _lib.CoverageParams(5, 3, 0, 0, None, None)
+    cong = _lib.CongestionParams(5, 3, f, 0, 0, 0, 0, 0, None, None)
+    coll = _lib.CollisionParams(5, 3, 1, 0, 0.25, 0, 0)
+    covf = _lib.CoverageFloatParams(5, 3, 0, 0, 2.0, 0.0, 0.0, 0.0, 0.0, 0.0, None)
+
+    def acc(n_steps=4, g_mode=0):
+        return C.byref(_lib.Accounting(0.9, n_steps, g_mode, None))
+    entry_points = [   # (call(acc, G, g_scratch, stats, stats_scratch), longest episode, largest g_mode, takes g_scratch)
+        (lambda a, G, gs, s, ss: lib.smarl_coverage_rollout(C.byref(cov), a, f, f, f, None, f, f, f, f, f, G, gs, s, ss,
+                                                            16, 16, None), 255, 2, True),
+        (lambda a, G, gs, s, ss: lib.smarl_congestion_rollout(C.byref(cong), a, f, f, f, None, None, f, f, f, f, f, G, gs,
+                                                              s, ss, 16, 16, None), 2 ** 31 - 1, 2, True),
+        (lambda a, G, gs, s, ss: lib.smarl_collision_rollout(C.byref(coll), a, f, f, f, f, None, f, f, f, f, f, f, f, G,
+                                                             gs, s, ss, 16, 16, None), 2 ** 31 - 1, 2, True),
+        (lambda a, G, gs, s, ss: lib.smarl_coverage_float_rollout(C.byref(covf), a, f, f, f, None, f, f, f, f, f, G, gs,
+                                                                  s, ss, 16, 16, None), 2 ** 31 - 1, 2, True),
+        (lambda a, G, gs, s, ss: lib.smarl_rollout_returns(a, f, f, 0, f, None, f, f, f, G, s, ss, 3, 3, 16, 16, None),
+         2 ** 31 - 1, 3, False),
+        (lambda a, G, gs, s, ss: lib.smarl_rollout_returns_shared(a, f, f, f, 0, f, None, f, f, f, G, s, ss, 3, 3, 16, 16,
+                                                                  None), 2 ** 31 - 1, 3, False),
+    ]
+    for call, max_steps, max_g, takes_gs in entry_points:
+        cases = [((None, f, f, None, None), b"accounting params is NULL"),
+                 ((acc(n_steps=0), f, f, None, None), b"n_steps=0 outside"),
+                 ((acc(g_mode=-1), f, f, None, None), b"bad g_mode -1"),
+                 ((acc(g_mode=max_g + 1), f, f, None, None), b"bad g_mode %d" % (max_g + 1)),
+                 ((acc(g_mode=2), None, f, None, None), b"needs G"),
+                 ((acc(), f, f, f, None), b"stats and stats_scratch go together")]
+        if max_steps < 2 ** 31 - 1:
+            cases.append(((acc(n_steps=max_steps + 1), f, f, None, None), b"outside 1..%d" % max_steps))
+        if takes_gs:
+            cases.append(((acc(g_mode=1), f, None, None, None), b"needs g_scratch"))
+        for args, needle in cases:
+            assert call(*args) == -1 and needle in lib.smarl_last_error(), (needle, lib.smarl_last_error())
     assert lib.smarl_stats_len(16, 16) == 65
     assert lib.smarl_stats_scratch_len(3, 3, 50) == 26      # one row of partials per 32 envs
 

@@ -242,7 +242,7 @@ def test_rejected_inputs_queue_no_work():
     st = torch.cuda.current_stream().cuda_stream
 
     def call(A, S=None, pol_agents=None, hidden=16, n_actions=2, g_mode=0, mode=0, n_steps=T, null_start=False,
-             null_weight=False, null_g=False, null_gs=False):
+             null_weight=False, null_g=False, null_gs=False, stats_only=False):
         S = 2 * A if S is None else S
         big = torch.zeros(4096, ld, dtype=torch.float64, device="cuda")
         out = torch.full((4096, ld), 5.0, dtype=torch.float32, device="cuda")
@@ -253,7 +253,7 @@ def test_rejected_inputs_queue_no_work():
         rc = lib.smarl_coverage_float_policy_rollout(
             C.byref(kp), C.byref(pol), C.byref(acc), None if null_start else P(big), P(big), None, P(out), P(out),
             P(out), P(big), P(big), P(out), P(out), P(out), None if null_g else P(out), None if null_gs else P(out),
-            None, None, E, ld, st)
+            P(big) if stats_only else None, None, E, ld, st)
         torch.cuda.synchronize()
         assert bool((out == 5.0).all()) and not bool(big.any())       # nothing ran
         return rc
@@ -271,6 +271,7 @@ def test_rejected_inputs_queue_no_work():
     assert call(3, g_mode=2, null_g=True) == -1
     assert call(3, g_mode=1, null_gs=True) == -1
     assert call(3, pol_agents=2) == -1
+    assert call(3, stats_only=True) == -1
     import safe_multiagent_rl_b200 as s
     from safe_multiagent_rl_b200.policy import BatchedGaussianPolicy, FusedGaussianPolicy
     env = s.BatchedCoverageContinuous(6, 3, n_envs=E)

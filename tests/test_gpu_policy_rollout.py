@@ -241,15 +241,19 @@ def test_rejected_inputs_queue_no_work():
     P = _lib.ptr
     st = torch.cuda.current_stream().cuda_stream
 
-    def call(A, S, hidden=16, g_mode=0, null_start=False):
+    def call(A, S, hidden=16, g_mode=0, n_steps=T, null_start=False, null_weight=False, null_g=False, null_gs=False,
+             stats_only=False):
         big = torch.zeros(4096, ld, dtype=torch.float64, device="cuda")
         out = torch.full((4096, ld), 5.0, dtype=torch.float32, device="cuda")
         kp = _lib.CollisionParams(6, A, 1, 0, 0.25, 0, 0)
-        pol = _lib.GaussianPolicyParams(A, S, hidden, 2, 0, 0, P(out), P(out), P(out), P(out), P(out), P(out), 1, 0, None)
-        acc = _lib.Accounting(0.9, T, g_mode, None)
+        pol = _lib.GaussianPolicyParams(A, S, hidden, 2, 0, 0, None if null_weight else P(out), P(out), P(out), P(out),
+                                        P(out), P(out), 1, 0, None)
+        acc = _lib.Accounting(0.9, n_steps, g_mode, None)
         rc = lib.smarl_collision_policy_rollout(C.byref(kp), C.byref(pol), C.byref(acc), None if null_start else P(big),
                                                 P(big), P(big), None, P(out), P(out), P(out), P(big), P(big), P(big),
-                                                P(big), P(out), P(out), P(big), P(out), P(out), None, None, E, ld, st)
+                                                P(big), P(out), P(out), P(big), None if null_g else P(out),
+                                                None if null_gs else P(out), P(big) if stats_only else None, None, E, ld,
+                                                st)
         torch.cuda.synchronize()
         assert bool((out == 5.0).all()) and not bool(big.any())       # nothing ran
         return rc
@@ -258,6 +262,12 @@ def test_rejected_inputs_queue_no_work():
     assert call(3, 8) == -1
     assert call(3, 6, hidden=8) == -1
     assert call(3, 6, null_start=True) == -1
+    assert call(3, 6, n_steps=0) == -1
+    assert call(3, 6, n_steps=65537) == -1
+    assert call(3, 6, null_weight=True) == -1
+    assert call(3, 6, g_mode=2, null_g=True) == -1
+    assert call(3, 6, g_mode=1, null_gs=True) == -1
+    assert call(3, 6, stats_only=True) == -1
     import safe_multiagent_rl_b200 as s
     from safe_multiagent_rl_b200.policy import BatchedGaussianPolicy, FusedGaussianPolicy
     env = s.BatchedCollisionAvoidance(6, 3, n_envs=E)
