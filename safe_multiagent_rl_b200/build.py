@@ -6,10 +6,16 @@ nvcc cross-compiles without a GPU.  An object is rebuilt only when its own sourc
 is newer, so code that several sources share lives in headers (.cuh): a source never includes
 another .cu file (tests/test_no_cu_includes.py checks this).  The library lands in
 safe_multiagent_rl_b200/_lib/libsmarl.so (git-ignored).
+
+A heavy source (32 agent-count instantiations per kernel) is compiled as several translation units in parallel, once
+per -DSMARL_TU=k.  Its `#if SMARL_TU_IS(k)` guards say what each unit holds, and its unit count is 1 + the largest k
+it names (1 for a source that names none).  The library is linked with --no-undefined, so a unit or an explicit
+instantiation that goes missing fails here rather than when the library is loaded.
 """
 from __future__ import annotations
 
 import os
+import re
 import shutil
 import subprocess
 import sys
@@ -29,9 +35,7 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
 # operation, so the compiler must not contract a*b+c into an FMA there.
 EXTRA = {"collision.cu": ["-fmad=false"], "collision_coop.cu": ["-fmad=false"], "collision_policy.cu": ["-fmad=false"],
          "coverage_float.cu": ["-fmad=false"], "coverage_float_policy.cu": ["-fmad=false"]}
-# Heavy files (32 agent-count instantiations per kernel) are compiled as several translation units
-# in parallel: the file is built once per value of -DSMARL_TU=k (see the header of each file).
-TU_SPLIT = {"coverage.cu": 3, "congestion.cu": 7, "collision.cu": 3, "collision_coop.cu": 2, "congestion_coop.cu": 6, "coverage_float.cu": 5}
+TU_INDEX = re.compile(r"\bSMARL_TU_IS\((\d+)\)")
 
 
 def _nvcc() -> str:
@@ -43,6 +47,12 @@ def _nvcc() -> str:
 
 def sources():
     return sorted(f for f in os.listdir(CSRC) if f.endswith(".cu"))
+
+
+def tu_count(src: str) -> int:
+    """Translation units of csrc/<src>: 1 + the largest k it names in SMARL_TU_IS(k), or 1."""
+    with open(os.path.join(CSRC, src)) as f:
+        return 1 + max((int(k) for k in TU_INDEX.findall(f.read())), default=0)
 
 
 def _headers_mtime() -> float:
@@ -62,7 +72,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     objs = []
     for src in sources():
         s = os.path.join(CSRC, src)
-        n_tu = TU_SPLIT.get(src, 1)
+        n_tu = tu_count(src)
         for tu in range(n_tu):
             o = os.path.join(OBJ_DIR, src[:-3] + (f".tu{tu}" if n_tu > 1 else "") + ".o")
             objs.append(o)
@@ -85,7 +95,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
             if r.returncode != 0:
                 raise RuntimeError(f"nvcc failed for {cmd[-3]}: " + r.stderr[-2000:])
     if jobs or not os.path.exists(LIB_PATH):
-        cmd = [nvcc, *ARCH, "-shared", "-o", LIB_PATH, *objs, "-ldl"]
+        cmd = [nvcc, *ARCH, "-shared", "-Xlinker", "--no-undefined", "-o", LIB_PATH, *objs, "-ldl"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             sys.stderr.write(r.stdout + r.stderr)

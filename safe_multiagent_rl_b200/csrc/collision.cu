@@ -10,10 +10,6 @@
 
 // Built as three translation units (build.py compiles this file once per SMARL_TU value):
 //   0 step kernel   1 fused rollout kernel   2 reset kernel + C entry points
-#ifndef SMARL_TU
-#define SMARL_TU -1   // single-TU build: everything
-#endif
-#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
 
 namespace smarl {
 
@@ -104,18 +100,17 @@ __global__ void __launch_bounds__(kCollThreads, (CAP ? 8 : 0)) collision_step_ke
 }
 
 int launch_collision_step(int A, const CollisionStepArgs& a, unsigned grid, cudaStream_t s) {
-  if (A <= 4 && a.n_envs >= kCollCapMinEnvs) {
-    switch (A) {
-      case 1: SMARL_CUDA(launch_pdl(collision_step_kernel<1, true>, grid, kCollThreads, 0, s, a)); break;
-      case 2: SMARL_CUDA(launch_pdl(collision_step_kernel<2, true>, grid, kCollThreads, 0, s, a)); break;
-      case 3: SMARL_CUDA(launch_pdl(collision_step_kernel<3, true>, grid, kCollThreads, 0, s, a)); break;
-      default: SMARL_CUDA(launch_pdl(collision_step_kernel<4, true>, grid, kCollThreads, 0, s, a)); break;
-    }
-  } else {
-    SMARL_DISPATCH_A(A, SMARL_CUDA(launch_pdl(collision_step_kernel<kA, false>, grid, kCollThreads, 0, s, a)));
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  if (A <= 4 && a.n_envs >= kCollCapMinEnvs)
+    return dispatch<1, 4>(A, [&](auto kA) {
+      SMARL_CUDA(launch_pdl(collision_step_kernel<kA, true>, grid, kCollThreads, 0, s, a));
+      SMARL_CUDA(cudaGetLastError());
+      return SMARL_OK;
+    });
+  return dispatch<1, 32>(A, [&](auto kA) {
+    SMARL_CUDA(launch_pdl(collision_step_kernel<kA, false>, grid, kCollThreads, 0, s, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
 }
 #endif
 
@@ -227,18 +222,17 @@ __global__ void __launch_bounds__(kCollThreads, (CAP ? 8 : (A >= 5 && A <= 8 ? 5
 }
 
 int launch_collision_rollout(int A, const CollisionRolloutArgs& a, unsigned grid, cudaStream_t s) {
-  if (A <= 4 && a.n_envs >= kCollCapMinEnvs) {
-    switch (A) {
-      case 1: collision_rollout_kernel<1, true><<<grid, kCollThreads, 0, s>>>(a); break;
-      case 2: collision_rollout_kernel<2, true><<<grid, kCollThreads, 0, s>>>(a); break;
-      case 3: collision_rollout_kernel<3, true><<<grid, kCollThreads, 0, s>>>(a); break;
-      default: collision_rollout_kernel<4, true><<<grid, kCollThreads, 0, s>>>(a); break;
-    }
-  } else {
-    SMARL_DISPATCH_A(A, collision_rollout_kernel<kA, false><<<grid, kCollThreads, 0, s>>>(a));
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  if (A <= 4 && a.n_envs >= kCollCapMinEnvs)
+    return dispatch<1, 4>(A, [&](auto kA) {
+      collision_rollout_kernel<kA, true><<<grid, kCollThreads, 0, s>>>(a);
+      SMARL_CUDA(cudaGetLastError());
+      return SMARL_OK;
+    });
+  return dispatch<1, 32>(A, [&](auto kA) {
+    collision_rollout_kernel<kA, false><<<grid, kCollThreads, 0, s>>>(a);
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
 }
 #endif
 

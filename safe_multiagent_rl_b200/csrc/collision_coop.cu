@@ -25,16 +25,10 @@
 #include "collision.cuh"
 
 // Built as two translation units (build.py compiles this file once per SMARL_TU value): 0 step, 1 rollout.
-#ifndef SMARL_TU
-#define SMARL_TU -1
-#endif
-#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
 
 namespace smarl {
 
 constexpr int kCoopThreads = 128;
-constexpr int kCoopMinA = 9;          // smallest agent count the cooperative kernels are instantiated for
-
 
 template <int A, int S>
 struct CollCoop {
@@ -355,28 +349,16 @@ __global__ void __launch_bounds__(kCoopThreads, 5) collision_coop_step_kernel(co
 
 template <int S, bool COMPACT>
 static int launch_step_s(int A, const CollisionStepArgs& a, cudaStream_t st) {
-  switch (A) {
-#define SMARL_COOP_CASE(N)                                                                              \
-  case N: {                                                                                             \
-    using C = CollCoop<N, S>;                                                                           \
-    auto kern = collision_coop_step_kernel<N, S, COMPACT>;                                                     \
-    if (C::kSmem > 48 * 1024)                                                                           \
-      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmem)); \
-    const unsigned grid = (unsigned)((a.n_envs + C::EPC - 1) / C::EPC);                                 \
-    SMARL_CUDA(launch_pdl(kern, grid, kCoopThreads, C::kSmem, st, a));                                                      \
-  } break;
-    SMARL_COOP_CASE(9) SMARL_COOP_CASE(10) SMARL_COOP_CASE(11) SMARL_COOP_CASE(12) SMARL_COOP_CASE(13)
-    SMARL_COOP_CASE(14) SMARL_COOP_CASE(15) SMARL_COOP_CASE(16) SMARL_COOP_CASE(17) SMARL_COOP_CASE(18)
-    SMARL_COOP_CASE(19) SMARL_COOP_CASE(20) SMARL_COOP_CASE(21) SMARL_COOP_CASE(22) SMARL_COOP_CASE(23)
-    SMARL_COOP_CASE(24) SMARL_COOP_CASE(25) SMARL_COOP_CASE(26) SMARL_COOP_CASE(27) SMARL_COOP_CASE(28)
-    SMARL_COOP_CASE(29) SMARL_COOP_CASE(30) SMARL_COOP_CASE(31) SMARL_COOP_CASE(32)
-#undef SMARL_COOP_CASE
-    default:
-      set_error("cooperative Collision kernels cover n_agents %d..32 (got %d)", kCoopMinA, A);
-      return SMARL_EUNSUPPORTED;
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  return dispatch<9, 32>(A, [&](auto kA) {
+    using C = CollCoop<kA, S>;
+    auto kern = collision_coop_step_kernel<kA, S, COMPACT>;
+    if (C::kSmem > 48 * 1024)
+      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmem));
+    const unsigned grid = (unsigned)((a.n_envs + C::EPC - 1) / C::EPC);
+    SMARL_CUDA(launch_pdl(kern, grid, kCoopThreads, C::kSmem, st, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  }, "cooperative Collision kernels cover n_agents 9..32 (got %d)");
 }
 
 int launch_collision_coop_step(int A, int S, const CollisionStepArgs& a, cudaStream_t st) {
@@ -510,28 +492,16 @@ __global__ void __launch_bounds__(kCoopThreads, 5) collision_coop_rollout_kernel
 
 template <int S, bool COMPACT>
 static int launch_rollout_s(int A, const CollisionRolloutArgs& a, cudaStream_t st) {
-  switch (A) {
-#define SMARL_COOP_CASE(N)                                                                              \
-  case N: {                                                                                             \
-    using C = CollCoop<N, S>;                                                                           \
-    auto kern = collision_coop_rollout_kernel<N, S, COMPACT>;                                                  \
-    if (C::kSmem + 64 > 48 * 1024)                                                                      \
-      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmem)); \
-    const unsigned grid = (unsigned)((a.n_envs + C::EPC - 1) / C::EPC);                                 \
-    kern<<<grid, kCoopThreads, C::kSmem, st>>>(a);                                                      \
-  } break;
-    SMARL_COOP_CASE(9) SMARL_COOP_CASE(10) SMARL_COOP_CASE(11) SMARL_COOP_CASE(12) SMARL_COOP_CASE(13)
-    SMARL_COOP_CASE(14) SMARL_COOP_CASE(15) SMARL_COOP_CASE(16) SMARL_COOP_CASE(17) SMARL_COOP_CASE(18)
-    SMARL_COOP_CASE(19) SMARL_COOP_CASE(20) SMARL_COOP_CASE(21) SMARL_COOP_CASE(22) SMARL_COOP_CASE(23)
-    SMARL_COOP_CASE(24) SMARL_COOP_CASE(25) SMARL_COOP_CASE(26) SMARL_COOP_CASE(27) SMARL_COOP_CASE(28)
-    SMARL_COOP_CASE(29) SMARL_COOP_CASE(30) SMARL_COOP_CASE(31) SMARL_COOP_CASE(32)
-#undef SMARL_COOP_CASE
-    default:
-      set_error("cooperative Collision kernels cover n_agents %d..32 (got %d)", kCoopMinA, A);
-      return SMARL_EUNSUPPORTED;
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  return dispatch<9, 32>(A, [&](auto kA) {
+    using C = CollCoop<kA, S>;
+    auto kern = collision_coop_rollout_kernel<kA, S, COMPACT>;
+    if (C::kSmem + 64 > 48 * 1024)
+      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmem));
+    const unsigned grid = (unsigned)((a.n_envs + C::EPC - 1) / C::EPC);
+    kern<<<grid, kCoopThreads, C::kSmem, st>>>(a);
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  }, "cooperative Collision kernels cover n_agents 9..32 (got %d)");
 }
 
 int launch_collision_coop_rollout(int A, int S, const CollisionRolloutArgs& a, cudaStream_t st) {

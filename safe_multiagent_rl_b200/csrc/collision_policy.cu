@@ -245,20 +245,15 @@ extern "C" int smarl_collision_policy_rollout(const SmarlCollisionParams* p, con
   const size_t smem = policy_rollout_smem(A, S, p->n_landmarks, p->obs_landmarks);
   const unsigned grid = (unsigned)((n_envs + kPolRollThreads - 1) / kPolRollThreads);
   cudaStream_t st = (cudaStream_t)stream;
-  switch (A) {
-#define SMARL_POLICY_ROLLOUT_CASE(N)                                                                           \
-  case N: {                                                                                                    \
-    auto kern = collision_policy_rollout_kernel<N>;                                                            \
-    if (smem + kPolRollStaticSmem > 48 * 1024)                                                                 \
-      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));          \
-    kern<<<grid, kPolRollThreads, smem, st>>>(k);                                                              \
-  } break;
-    SMARL_POLICY_ROLLOUT_CASE(1) SMARL_POLICY_ROLLOUT_CASE(2) SMARL_POLICY_ROLLOUT_CASE(3)
-    SMARL_POLICY_ROLLOUT_CASE(4) SMARL_POLICY_ROLLOUT_CASE(5) SMARL_POLICY_ROLLOUT_CASE(6)
-    SMARL_POLICY_ROLLOUT_CASE(7) SMARL_POLICY_ROLLOUT_CASE(8)
-#undef SMARL_POLICY_ROLLOUT_CASE
-  }
-  SMARL_CUDA(cudaGetLastError());
+  if (int rc = dispatch<1, 8>(A, [&](auto kA) {
+        auto kern = collision_policy_rollout_kernel<kA>;
+        if (smem + kPolRollStaticSmem > 48 * 1024)
+          SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<grid, kPolRollThreads, smem, st>>>(k);
+        SMARL_CUDA(cudaGetLastError());
+        return SMARL_OK;
+      }))
+    return rc;
   if (stats) return launch_stats_finalize(stats_scratch, grid, A, 1, n_envs, stats, st);
   return SMARL_OK;
 }

@@ -5,6 +5,9 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <type_traits>
+#include <utility>
+
 #include "../../include/smarl.h"
 
 namespace smarl {
@@ -48,29 +51,25 @@ int check_layout(int64_t n_envs, int64_t ld);
 int check_accounting(const SmarlAccounting* acc, int max_steps, int max_g_mode, const float* G, const double* stats,
                      const double* stats_scratch);
 
-// Dispatch a compile-time agent count 1..32.
-#define SMARL_CASE_A(N, ...) \
-  case N: {                  \
-    constexpr int kA = N;    \
-    __VA_ARGS__;             \
-  } break;
-#define SMARL_DISPATCH_A(value, ...)                                                         \
-  switch (value) {                                                                           \
-    SMARL_CASE_A(1, __VA_ARGS__) SMARL_CASE_A(2, __VA_ARGS__) SMARL_CASE_A(3, __VA_ARGS__)   \
-    SMARL_CASE_A(4, __VA_ARGS__) SMARL_CASE_A(5, __VA_ARGS__) SMARL_CASE_A(6, __VA_ARGS__)   \
-    SMARL_CASE_A(7, __VA_ARGS__) SMARL_CASE_A(8, __VA_ARGS__) SMARL_CASE_A(9, __VA_ARGS__)   \
-    SMARL_CASE_A(10, __VA_ARGS__) SMARL_CASE_A(11, __VA_ARGS__) SMARL_CASE_A(12, __VA_ARGS__) \
-    SMARL_CASE_A(13, __VA_ARGS__) SMARL_CASE_A(14, __VA_ARGS__) SMARL_CASE_A(15, __VA_ARGS__) \
-    SMARL_CASE_A(16, __VA_ARGS__) SMARL_CASE_A(17, __VA_ARGS__) SMARL_CASE_A(18, __VA_ARGS__) \
-    SMARL_CASE_A(19, __VA_ARGS__) SMARL_CASE_A(20, __VA_ARGS__) SMARL_CASE_A(21, __VA_ARGS__) \
-    SMARL_CASE_A(22, __VA_ARGS__) SMARL_CASE_A(23, __VA_ARGS__) SMARL_CASE_A(24, __VA_ARGS__) \
-    SMARL_CASE_A(25, __VA_ARGS__) SMARL_CASE_A(26, __VA_ARGS__) SMARL_CASE_A(27, __VA_ARGS__) \
-    SMARL_CASE_A(28, __VA_ARGS__) SMARL_CASE_A(29, __VA_ARGS__) SMARL_CASE_A(30, __VA_ARGS__) \
-    SMARL_CASE_A(31, __VA_ARGS__) SMARL_CASE_A(32, __VA_ARGS__)                               \
-    default:                                                                                 \
-      ::smarl::set_error("n_agents=%d outside 1..32", (int)(value));                         \
-      return SMARL_EUNSUPPORTED;                                                             \
-  }
+// Selects a compile-time value: calls f(std::integral_constant<int, N>{}) for the N in Lo..Hi that equals n and returns
+// its result.  Outside Lo..Hi it sets the error from fmt (one %d, given n) and returns SMARL_EUNSUPPORTED.
+template <int Lo, typename F, int... I>
+int dispatch_seq(int n, F& f, const char* fmt, std::integer_sequence<int, I...>) {
+  int rc = SMARL_EUNSUPPORTED;
+  if (!((n == Lo + I && (rc = f(std::integral_constant<int, Lo + I>{}), true)) || ...)) set_error(fmt, n);
+  return rc;
+}
+template <int Lo, int Hi, typename F>
+int dispatch(int n, F&& f, const char* fmt = "n_agents=%d outside 1..32") {
+  return dispatch_seq<Lo>(n, f, fmt, std::make_integer_sequence<int, Hi - Lo + 1>{});
+}
+
+// Which translation unit of a split source this compile is (build.py builds a source once per -DSMARL_TU=k, k from 0
+// to the largest k the source names in SMARL_TU_IS(k); -1, the default, builds everything).
+#ifndef SMARL_TU
+#define SMARL_TU -1
+#endif
+#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
 
 #ifdef __CUDACC__
 // ---------------------------------------------------------------------------------------

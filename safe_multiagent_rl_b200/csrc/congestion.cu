@@ -6,10 +6,6 @@
 // Built as several translation units (build.py compiles this file once per SMARL_TU value) so the
 // 32 agent-count instantiations of each kernel compile in parallel:
 //   0,1,2 step kernel noise mode 0/1/2   3,4,5 rollout kernel mode 0/1/2   6 C entry points
-#ifndef SMARL_TU
-#define SMARL_TU -1   // single-TU build: everything
-#endif
-#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
 
 namespace smarl {
 
@@ -46,13 +42,6 @@ __device__ __forceinline__ void congestion_transition(uint32_t (&xw)[A], uint32_
 // (CongestionRolloutArgs lives in congestion.cuh: the cooperative rollout kernel of congestion_coop.cu shares it)
 
 constexpr int kCongRollThreads = 64;
-
-int launch_congestion_step_m0(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s);
-int launch_congestion_step_m1(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s);
-int launch_congestion_step_m2(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s);
-int launch_congestion_rollout_m0(int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s);
-int launch_congestion_rollout_m1(int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s);
-int launch_congestion_rollout_m2(int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s);
 
 #if SMARL_TU_IS(0) || SMARL_TU_IS(1) || SMARL_TU_IS(2)
 template <int A, int MODE>
@@ -123,21 +112,23 @@ __global__ void __launch_bounds__(kCongThreads, cong_step_min_blocks(A)) congest
   }
 }
 
-#define SMARL_DEFINE_CONG_STEP(M)                                                                       \
-  int launch_congestion_step_m##M(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s) {  \
-    SMARL_DISPATCH_A(A, SMARL_CUDA(launch_pdl(congestion_step_kernel<kA, M>, grid, kCongThreads, 0, s, a)));                \
-    SMARL_CUDA(cudaGetLastError());                                                                     \
-    return SMARL_OK;                                                                                    \
-  }
+template <int M>
+int launch_congestion_step(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s) {
+  return dispatch<1, 32>(A, [&](auto kA) {
+    SMARL_CUDA(launch_pdl(congestion_step_kernel<kA, M>, grid, kCongThreads, 0, s, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
+}
+#endif
 #if SMARL_TU_IS(0)
-SMARL_DEFINE_CONG_STEP(0)
+template int launch_congestion_step<0>(int, const CongestionStepArgs&, unsigned, cudaStream_t);
 #endif
 #if SMARL_TU_IS(1)
-SMARL_DEFINE_CONG_STEP(1)
+template int launch_congestion_step<1>(int, const CongestionStepArgs&, unsigned, cudaStream_t);
 #endif
 #if SMARL_TU_IS(2)
-SMARL_DEFINE_CONG_STEP(2)
-#endif
+template int launch_congestion_step<2>(int, const CongestionStepArgs&, unsigned, cudaStream_t);
 #endif
 
 #if SMARL_TU_IS(3) || SMARL_TU_IS(4) || SMARL_TU_IS(5)
@@ -298,39 +289,30 @@ __global__ void __launch_bounds__(kCongRollThreads, cong_min_blocks(A)) congesti
   }
 }
 
-#define SMARL_DEFINE_CONG_ROLLOUT(M)                                                                         \
-  int launch_congestion_rollout_m##M(int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s) { \
-    const size_t smem = sizeof(double) * 4 * kCongRollThreads * (size_t)A;                                   \
-    SMARL_DISPATCH_A(A, {                                                                                    \
-      auto kern = congestion_rollout_kernel<kA, M>;                                                          \
-      if (smem + 64 > 48 * 1024)   /* + the static reduction buffer */                                       \
-        SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));      \
-      kern<<<grid, kCongRollThreads, smem, s>>>(a);                                                          \
-    });                                                                                                      \
-    SMARL_CUDA(cudaGetLastError());                                                                          \
-    return SMARL_OK;                                                                                         \
-  }
+template <int M>
+int launch_congestion_rollout(int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s) {
+  const size_t smem = sizeof(double) * 4 * kCongRollThreads * (size_t)A;
+  return dispatch<1, 32>(A, [&](auto kA) {
+    auto kern = congestion_rollout_kernel<kA, M>;
+    if (smem + 64 > 48 * 1024)   // + the static reduction buffer
+      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, kCongRollThreads, smem, s>>>(a);
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
+}
+#endif
 #if SMARL_TU_IS(3)
-SMARL_DEFINE_CONG_ROLLOUT(0)
+template int launch_congestion_rollout<0>(int, const CongestionRolloutArgs&, unsigned, cudaStream_t);
 #endif
 #if SMARL_TU_IS(4)
-SMARL_DEFINE_CONG_ROLLOUT(1)
+template int launch_congestion_rollout<1>(int, const CongestionRolloutArgs&, unsigned, cudaStream_t);
 #endif
 #if SMARL_TU_IS(5)
-SMARL_DEFINE_CONG_ROLLOUT(2)
-#endif
+template int launch_congestion_rollout<2>(int, const CongestionRolloutArgs&, unsigned, cudaStream_t);
 #endif
 
 #if SMARL_TU_IS(6)
-static int launch_congestion_step(int mode, int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s) {
-  return mode == 0 ? launch_congestion_step_m0(A, a, grid, s)
-       : mode == 1 ? launch_congestion_step_m1(A, a, grid, s) : launch_congestion_step_m2(A, a, grid, s);
-}
-static int launch_congestion_rollout(int mode, int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s) {
-  return mode == 0 ? launch_congestion_rollout_m0(A, a, grid, s)
-       : mode == 1 ? launch_congestion_rollout_m1(A, a, grid, s) : launch_congestion_rollout_m2(A, a, grid, s);
-}
-
 // Lanes per env quad of the step kernel: 0 = one thread per four envs (this file), 2 / 4 = lane-cooperative
 // scan kernel (congestion_coop.cu).  Crossover measured on B200 (profiles/r02); smarl_set_kernel_variant overrides.
 static int congestion_coop_lanes(int A) {
@@ -388,13 +370,10 @@ extern "C" int smarl_congestion_step(const SmarlCongestionParams* p, uint8_t* po
   a.episode = p->episode; a.episode_dev = p->episode_dev;
   const unsigned grid = (unsigned)((a.n_groups + kCongThreads - 1) / kCongThreads);
   cudaStream_t s = (cudaStream_t)stream;
-  if (const int lanes = congestion_coop_lanes(p->n_agents)) {
-    return p->noise_mode == 0 ? launch_congestion_coop_step_m0(p->n_agents, lanes, a, s)
-         : p->noise_mode == 1 ? launch_congestion_coop_step_m1(p->n_agents, lanes, a, s)
-                              : launch_congestion_coop_step_m2(p->n_agents, lanes, a, s);
-  }
-  if (int rc = launch_congestion_step(p->noise_mode, p->n_agents, a, grid, s)) return rc;
-  return SMARL_OK;
+  const int lanes = congestion_coop_lanes(p->n_agents);
+  return dispatch<0, 2>(p->noise_mode, [&](auto m) {
+    return lanes ? launch_congestion_coop_step<m>(p->n_agents, lanes, a, s) : launch_congestion_step<m>(p->n_agents, a, grid, s);
+  }, "bad noise_mode %d");
 }
 
 extern "C" int smarl_congestion_rollout(const SmarlCongestionParams* p, const SmarlAccounting* acc,
@@ -426,18 +405,15 @@ extern "C" int smarl_congestion_rollout(const SmarlCongestionParams* p, const Sm
   a.episode = p->episode; a.episode_dev = p->episode_dev;
   const unsigned grid = (unsigned)((a.n_groups + kCongRollThreads - 1) / kCongRollThreads);
   cudaStream_t s = (cudaStream_t)stream;
-  if (congestion_coop_rollout_lanes(p->n_agents)) {
-    unsigned coop_grid = 0;
-    if (int rc = p->noise_mode == 0 ? launch_congestion_coop_rollout_m0(p->n_agents, a, &coop_grid, s)
-               : p->noise_mode == 1 ? launch_congestion_coop_rollout_m1(p->n_agents, a, &coop_grid, s)
-                                    : launch_congestion_coop_rollout_m2(p->n_agents, a, &coop_grid, s))
-      return rc;
-    if (stats) return launch_stats_finalize(stats_scratch, coop_grid, p->n_agents, 1, n_envs, stats, s);
-    return SMARL_OK;
-  }
-  if (int rc = launch_congestion_rollout(p->noise_mode, p->n_agents, a, grid, s)) return rc;
+  const bool coop = congestion_coop_rollout_lanes(p->n_agents) != 0;
+  unsigned rows = grid;                                 // CTAs launched = rows of stats partials
+  if (int rc = dispatch<0, 2>(p->noise_mode, [&](auto m) {
+        return coop ? launch_congestion_coop_rollout<m>(p->n_agents, a, &rows, s)
+                    : launch_congestion_rollout<m>(p->n_agents, a, grid, s);
+      }, "bad noise_mode %d"))
+    return rc;
   if (stats)
-    return launch_stats_finalize(stats_scratch, grid, p->n_agents, 1, n_envs, stats, s);
+    return launch_stats_finalize(stats_scratch, rows, p->n_agents, 1, n_envs, stats, s);
   return SMARL_OK;
 }
 #endif

@@ -221,13 +221,12 @@ struct CongestionRolloutArgs {
   const uint32_t* episode_dev;
 };
 
-int launch_congestion_coop_step_m0(int A, int S, const CongestionStepArgs& a, cudaStream_t st);
-int launch_congestion_coop_step_m1(int A, int S, const CongestionStepArgs& a, cudaStream_t st);
-int launch_congestion_coop_step_m2(int A, int S, const CongestionStepArgs& a, cudaStream_t st);
+// Launchers of noise mode M = 0..2 (congestion.cu, congestion_coop.cu), each mode instantiated in its own translation unit
+template <int M> int launch_congestion_step(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s);
+template <int M> int launch_congestion_rollout(int A, const CongestionRolloutArgs& a, unsigned grid, cudaStream_t s);
+template <int M> int launch_congestion_coop_step(int A, int S, const CongestionStepArgs& a, cudaStream_t st);
 // fused rollout, four lanes per env quad (congestion_coop.cu); *grid returns the CTA count (= rows of stats partials)
-int launch_congestion_coop_rollout_m0(int A, const CongestionRolloutArgs& a, unsigned* grid, cudaStream_t st);
-int launch_congestion_coop_rollout_m1(int A, const CongestionRolloutArgs& a, unsigned* grid, cudaStream_t st);
-int launch_congestion_coop_rollout_m2(int A, const CongestionRolloutArgs& a, unsigned* grid, cudaStream_t st);
+template <int M> int launch_congestion_coop_rollout(int A, const CongestionRolloutArgs& a, unsigned* grid, cudaStream_t st);
 
 // Waiting-branch reward in f64, the reference's operation order (congestion.py:86-87).
 __device__ __forceinline__ double congestion_reward_f64(uint32_t con, uint32_t nx, uint32_t ny,

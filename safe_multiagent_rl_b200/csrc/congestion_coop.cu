@@ -24,10 +24,6 @@
 
 // Built as six translation units (build.py passes -DSMARL_TU=k): step kernels of noise mode k = 0..2, fused rollout
 // kernels of noise mode k - 3 = 0..2.
-#ifndef SMARL_TU
-#define SMARL_TU -1
-#endif
-#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
 
 namespace smarl {
 
@@ -517,85 +513,58 @@ __global__ void __launch_bounds__(kCongCoopThreads, 3) congestion_coop_rollout_k
 }
 
 template <int MODE>
-static int launch_roll(int A, const CongestionRolloutArgs& a, unsigned* grid_out, cudaStream_t st) {
-  switch (A) {
-#define SMARL_COOP_CASE(N)                                                                              \
-  case N: {                                                                                             \
-    using C = CongCoop<N, 4>;                                                                           \
-    auto kern = congestion_coop_rollout_kernel<N, 4, MODE>;                                             \
-    const size_t smem = CongCoopRoll<N, 4>::kSmem;                                                      \
-    if (smem + 256 > 48 * 1024)                                                                         \
-      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-    const unsigned grid = (unsigned)((a.n_groups + C::EPC - 1) / C::EPC);                               \
-    kern<<<grid, kCongCoopThreads, smem, st>>>(a);                                                      \
-    *grid_out = grid;                                                                                   \
-  } break;
-    SMARL_COOP_CASE(9) SMARL_COOP_CASE(10) SMARL_COOP_CASE(11) SMARL_COOP_CASE(12) SMARL_COOP_CASE(13)
-    SMARL_COOP_CASE(14) SMARL_COOP_CASE(15) SMARL_COOP_CASE(16) SMARL_COOP_CASE(17) SMARL_COOP_CASE(18)
-    SMARL_COOP_CASE(19) SMARL_COOP_CASE(20) SMARL_COOP_CASE(21) SMARL_COOP_CASE(22) SMARL_COOP_CASE(23)
-    SMARL_COOP_CASE(24) SMARL_COOP_CASE(25) SMARL_COOP_CASE(26) SMARL_COOP_CASE(27) SMARL_COOP_CASE(28)
-    SMARL_COOP_CASE(29) SMARL_COOP_CASE(30) SMARL_COOP_CASE(31) SMARL_COOP_CASE(32)
-#undef SMARL_COOP_CASE
-    default:
-      set_error("cooperative Congestion kernels cover n_agents 9..32 (got %d)", A);
-      return SMARL_EUNSUPPORTED;
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+int launch_congestion_coop_rollout(int A, const CongestionRolloutArgs& a, unsigned* grid_out, cudaStream_t st) {
+  return dispatch<9, 32>(A, [&](auto kA) {
+    using C = CongCoop<kA, 4>;
+    auto kern = congestion_coop_rollout_kernel<kA, 4, MODE>;
+    const size_t smem = CongCoopRoll<kA, 4>::kSmem;
+    if (smem + 256 > 48 * 1024)
+      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned grid = (unsigned)((a.n_groups + C::EPC - 1) / C::EPC);
+    kern<<<grid, kCongCoopThreads, smem, st>>>(a);
+    *grid_out = grid;
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  }, "cooperative Congestion kernels cover n_agents 9..32 (got %d)");
 }
 
 template <int S, int MODE>
 static int launch_sm(int A, const CongestionStepArgs& a, cudaStream_t st) {
-  switch (A) {
-#define SMARL_COOP_CASE(N)                                                                              \
-  case N: {                                                                                             \
-    using C = CongCoop<N, S>;                                                                           \
-    auto kern = congestion_coop_step_kernel<N, S, MODE>;                                                \
-    const size_t smem = C::kSmem;                                                                       \
-    if (smem > 48 * 1024)                                                                               \
-      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-    const unsigned grid = (unsigned)((a.n_groups + C::EPC - 1) / C::EPC);                               \
-    SMARL_CUDA(launch_pdl(kern, grid, kCongCoopThreads, smem, st, a));                                                      \
-  } break;
-    SMARL_COOP_CASE(9) SMARL_COOP_CASE(10) SMARL_COOP_CASE(11) SMARL_COOP_CASE(12) SMARL_COOP_CASE(13)
-    SMARL_COOP_CASE(14) SMARL_COOP_CASE(15) SMARL_COOP_CASE(16) SMARL_COOP_CASE(17) SMARL_COOP_CASE(18)
-    SMARL_COOP_CASE(19) SMARL_COOP_CASE(20) SMARL_COOP_CASE(21) SMARL_COOP_CASE(22) SMARL_COOP_CASE(23)
-    SMARL_COOP_CASE(24) SMARL_COOP_CASE(25) SMARL_COOP_CASE(26) SMARL_COOP_CASE(27) SMARL_COOP_CASE(28)
-    SMARL_COOP_CASE(29) SMARL_COOP_CASE(30) SMARL_COOP_CASE(31) SMARL_COOP_CASE(32)
-#undef SMARL_COOP_CASE
-    default:
-      set_error("cooperative Congestion kernels cover n_agents 9..32 (got %d)", A);
-      return SMARL_EUNSUPPORTED;
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  return dispatch<9, 32>(A, [&](auto kA) {
+    using C = CongCoop<kA, S>;
+    auto kern = congestion_coop_step_kernel<kA, S, MODE>;
+    const size_t smem = C::kSmem;
+    if (smem > 48 * 1024)
+      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned grid = (unsigned)((a.n_groups + C::EPC - 1) / C::EPC);
+    SMARL_CUDA(launch_pdl(kern, grid, kCongCoopThreads, smem, st, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  }, "cooperative Congestion kernels cover n_agents 9..32 (got %d)");
 }
 
-#define SMARL_DEFINE_CONG_COOP(M)                                                                          \
-  int launch_congestion_coop_step_m##M(int A, int S, const CongestionStepArgs& a, cudaStream_t st) {      \
-    return S == 2 ? launch_sm<2, M>(A, a, st) : launch_sm<4, M>(A, a, st);                                 \
-  }
+template <int MODE>
+int launch_congestion_coop_step(int A, int S, const CongestionStepArgs& a, cudaStream_t st) {
+  return S == 2 ? launch_sm<2, MODE>(A, a, st) : launch_sm<4, MODE>(A, a, st);
+}
+
 #if SMARL_TU_IS(0)
-SMARL_DEFINE_CONG_COOP(0)
+template int launch_congestion_coop_step<0>(int, int, const CongestionStepArgs&, cudaStream_t);
 #endif
 #if SMARL_TU_IS(1)
-SMARL_DEFINE_CONG_COOP(1)
+template int launch_congestion_coop_step<1>(int, int, const CongestionStepArgs&, cudaStream_t);
 #endif
 #if SMARL_TU_IS(2)
-SMARL_DEFINE_CONG_COOP(2)
+template int launch_congestion_coop_step<2>(int, int, const CongestionStepArgs&, cudaStream_t);
 #endif
-#define SMARL_DEFINE_CONG_COOP_ROLL(M)                                                                         \
-  int launch_congestion_coop_rollout_m##M(int A, const CongestionRolloutArgs& a, unsigned* grid, cudaStream_t st) { \
-    return launch_roll<M>(A, a, grid, st);                                                                     \
-  }
 #if SMARL_TU_IS(3)
-SMARL_DEFINE_CONG_COOP_ROLL(0)
+template int launch_congestion_coop_rollout<0>(int, const CongestionRolloutArgs&, unsigned*, cudaStream_t);
 #endif
 #if SMARL_TU_IS(4)
-SMARL_DEFINE_CONG_COOP_ROLL(1)
+template int launch_congestion_coop_rollout<1>(int, const CongestionRolloutArgs&, unsigned*, cudaStream_t);
 #endif
 #if SMARL_TU_IS(5)
-SMARL_DEFINE_CONG_COOP_ROLL(2)
+template int launch_congestion_coop_rollout<2>(int, const CongestionRolloutArgs&, unsigned*, cudaStream_t);
 #endif
 
 }  // namespace smarl

@@ -13,10 +13,6 @@
 
 // Built as three translation units (build.py compiles this file once per SMARL_TU value):
 //   0 step kernel   1 fused rollout kernel   2 reset kernel + C entry points
-#ifndef SMARL_TU
-#define SMARL_TU -1   // single-TU build: everything
-#endif
-#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
 
 namespace smarl {
 
@@ -174,13 +170,17 @@ __global__ void __launch_bounds__(kStepThreads) coverage_step_kernel(const Cover
 
 int launch_coverage_step(int A, const CoverageStepArgs& a, unsigned grid, cudaStream_t s) {
   const size_t smem = (size_t)(a.lut_len + 1) * sizeof(float);
-  if (a.keep_pos) {
-    SMARL_DISPATCH_A(A, SMARL_CUDA(launch_pdl(coverage_step_kernel<kA, true>, grid, kStepThreads, smem, s, a)));
-  } else {
-    SMARL_DISPATCH_A(A, SMARL_CUDA(launch_pdl(coverage_step_kernel<kA, false>, grid, kStepThreads, smem, s, a)));
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  if (a.keep_pos)
+    return dispatch<1, 32>(A, [&](auto kA) {
+      SMARL_CUDA(launch_pdl(coverage_step_kernel<kA, true>, grid, kStepThreads, smem, s, a));
+      SMARL_CUDA(cudaGetLastError());
+      return SMARL_OK;
+    });
+  return dispatch<1, 32>(A, [&](auto kA) {
+    SMARL_CUDA(launch_pdl(coverage_step_kernel<kA, false>, grid, kStepThreads, smem, s, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
 }
 #endif
 
@@ -345,9 +345,11 @@ __global__ void __launch_bounds__(kRolloutThreads, (A <= 4 ? 8 : 0)) coverage_ro
 
 int launch_coverage_rollout(int A, const CoverageRolloutArgs& a, unsigned grid, cudaStream_t s) {
   const size_t smem = (size_t)(a.lut_len + 1) * sizeof(float);
-  SMARL_DISPATCH_A(A, coverage_rollout_kernel<kA><<<grid, kRolloutThreads, smem, s>>>(a));
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  return dispatch<1, 32>(A, [&](auto kA) {
+    coverage_rollout_kernel<kA><<<grid, kRolloutThreads, smem, s>>>(a);
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
 }
 #endif
 

@@ -183,29 +183,17 @@ __global__ void __launch_bounds__(kCovCoopThreads, 4) coverage_coop_step_kernel(
 
 template <int S>
 static int launch_s(int A, const CoverageCoopArgs& a, cudaStream_t st) {
-  switch (A) {
-#define SMARL_COOP_CASE(N)                                                                                 \
-  case N: {                                                                                                \
-    using C = CovCoop<N, S>;                                                                               \
-    auto kern = coverage_coop_step_kernel<N, S>;                                                           \
-    const size_t smem = (size_t)((a.lut_len + 1 + 3) & ~3) * sizeof(float) + C::kPosWords * sizeof(uint32_t); \
-    if (smem > 48 * 1024)                                                                                  \
-      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));      \
-    const unsigned grid = (unsigned)((a.n_groups + C::EPC - 1) / C::EPC);                                  \
-    SMARL_CUDA(launch_pdl(kern, grid, kCovCoopThreads, smem, st, a));                                                          \
-  } break;
-    SMARL_COOP_CASE(9) SMARL_COOP_CASE(10) SMARL_COOP_CASE(11) SMARL_COOP_CASE(12) SMARL_COOP_CASE(13)
-    SMARL_COOP_CASE(14) SMARL_COOP_CASE(15) SMARL_COOP_CASE(16) SMARL_COOP_CASE(17) SMARL_COOP_CASE(18)
-    SMARL_COOP_CASE(19) SMARL_COOP_CASE(20) SMARL_COOP_CASE(21) SMARL_COOP_CASE(22) SMARL_COOP_CASE(23)
-    SMARL_COOP_CASE(24) SMARL_COOP_CASE(25) SMARL_COOP_CASE(26) SMARL_COOP_CASE(27) SMARL_COOP_CASE(28)
-    SMARL_COOP_CASE(29) SMARL_COOP_CASE(30) SMARL_COOP_CASE(31) SMARL_COOP_CASE(32)
-#undef SMARL_COOP_CASE
-    default:
-      set_error("cooperative Coverage kernels cover n_agents 9..32 (got %d)", A);
-      return SMARL_EUNSUPPORTED;
-  }
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
+  return dispatch<9, 32>(A, [&](auto kA) {
+    using C = CovCoop<kA, S>;
+    auto kern = coverage_coop_step_kernel<kA, S>;
+    const size_t smem = (size_t)((a.lut_len + 1 + 3) & ~3) * sizeof(float) + C::kPosWords * sizeof(uint32_t);
+    if (smem > 48 * 1024)
+      SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned grid = (unsigned)((a.n_groups + C::EPC - 1) / C::EPC);
+    SMARL_CUDA(launch_pdl(kern, grid, kCovCoopThreads, smem, st, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  }, "cooperative Coverage kernels cover n_agents 9..32 (got %d)");
 }
 
 // Entry used by smarl_coverage_step (coverage.cu).

@@ -5,11 +5,6 @@
 #include "coverage_float.cuh"
 #include "stats.cuh"
 
-#ifndef SMARL_TU
-#define SMARL_TU -1
-#endif
-#define SMARL_TU_IS(k) (SMARL_TU == -1 || SMARL_TU == (k))
-
 namespace smarl {
 
 #if SMARL_TU_IS(0) || SMARL_TU_IS(1)
@@ -46,18 +41,20 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_float_step_kernel(const
   if (a.penalty) a.penalty[e] = (float)pen;
 }
 
-#define SMARL_DEFINE_COVF_STEP(M)                                                                        \
-  int launch_coverage_float_step_m##M(int A, const CoverageFloatArgs& a, unsigned grid, cudaStream_t s) { \
-    SMARL_DISPATCH_A(A, SMARL_CUDA(launch_pdl(coverage_float_step_kernel<kA, M>, grid, kCovFThreads, 0, s, a)));             \
-    SMARL_CUDA(cudaGetLastError());                                                                      \
-    return SMARL_OK;                                                                                     \
-  }
+template <int M>
+int launch_coverage_float_step(int A, const CoverageFloatArgs& a, unsigned grid, cudaStream_t s) {
+  return dispatch<1, 32>(A, [&](auto kA) {
+    SMARL_CUDA(launch_pdl(coverage_float_step_kernel<kA, M>, grid, kCovFThreads, 0, s, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
+}
 #endif
 #if SMARL_TU_IS(0)
-SMARL_DEFINE_COVF_STEP(0)
+template int launch_coverage_float_step<0>(int, const CoverageFloatArgs&, unsigned, cudaStream_t);
 #endif
 #if SMARL_TU_IS(1)
-SMARL_DEFINE_COVF_STEP(1)
+template int launch_coverage_float_step<1>(int, const CoverageFloatArgs&, unsigned, cudaStream_t);
 #endif
 
 #if SMARL_TU_IS(3) || SMARL_TU_IS(4)
@@ -154,27 +151,26 @@ __global__ void __launch_bounds__(kCovFThreads, (CAP ? 8 : 0)) coverage_float_ro
     }
   }
 }
-#define SMARL_DEFINE_COVF_ROLLOUT(M)                                                                              \
-  int launch_coverage_float_rollout_m##M(int A, const CoverageFloatRolloutArgs& a, unsigned grid, cudaStream_t s) { \
-    if (A <= 4 && a.env.n_envs >= (1 << 18)) {                                                                      \
-      switch (A) {                                                                                                  \
-        case 1: coverage_float_rollout_kernel<1, M, true><<<grid, kCovFThreads, 0, s>>>(a); break;                  \
-        case 2: coverage_float_rollout_kernel<2, M, true><<<grid, kCovFThreads, 0, s>>>(a); break;                  \
-        case 3: coverage_float_rollout_kernel<3, M, true><<<grid, kCovFThreads, 0, s>>>(a); break;                  \
-        default: coverage_float_rollout_kernel<4, M, true><<<grid, kCovFThreads, 0, s>>>(a); break;                 \
-      }                                                                                                             \
-    } else {                                                                                                        \
-      SMARL_DISPATCH_A(A, coverage_float_rollout_kernel<kA, M, false><<<grid, kCovFThreads, 0, s>>>(a));            \
-    }                                                                                                               \
-    SMARL_CUDA(cudaGetLastError());                                                                               \
-    return SMARL_OK;                                                                                              \
-  }
+template <int M>
+int launch_coverage_float_rollout(int A, const CoverageFloatRolloutArgs& a, unsigned grid, cudaStream_t s) {
+  if (A <= 4 && a.env.n_envs >= (1 << 18))
+    return dispatch<1, 4>(A, [&](auto kA) {
+      coverage_float_rollout_kernel<kA, M, true><<<grid, kCovFThreads, 0, s>>>(a);
+      SMARL_CUDA(cudaGetLastError());
+      return SMARL_OK;
+    });
+  return dispatch<1, 32>(A, [&](auto kA) {
+    coverage_float_rollout_kernel<kA, M, false><<<grid, kCovFThreads, 0, s>>>(a);
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
+  });
+}
 #endif
 #if SMARL_TU_IS(3)
-SMARL_DEFINE_COVF_ROLLOUT(0)
+template int launch_coverage_float_rollout<0>(int, const CoverageFloatRolloutArgs&, unsigned, cudaStream_t);
 #endif
 #if SMARL_TU_IS(4)
-SMARL_DEFINE_COVF_ROLLOUT(1)
+template int launch_coverage_float_rollout<1>(int, const CoverageFloatRolloutArgs&, unsigned, cudaStream_t);
 #endif
 
 #if SMARL_TU_IS(2)
@@ -228,8 +224,8 @@ extern "C" int smarl_coverage_float_step(const SmarlCoverageFloatParams* p, doub
   a.pos_x = pos_x; a.pos_y = pos_y; a.actions = actions; a.obs = obs; a.reward = reward; a.cost = cost;
   a.done = done; a.lambdas = lambdas; a.penalty = penalty; a.n_envs = n_envs; a.ld = ld;
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
-  return p->mode == 0 ? launch_coverage_float_step_m0(p->n_agents, a, grid, (cudaStream_t)stream)
-                      : launch_coverage_float_step_m1(p->n_agents, a, grid, (cudaStream_t)stream);
+  return dispatch<0, 1>(p->mode, [&](auto m) { return launch_coverage_float_step<m>(p->n_agents, a, grid, (cudaStream_t)stream); },
+                        "bad mode %d");
 }
 
 extern "C" int smarl_coverage_float_rollout(const SmarlCoverageFloatParams* p, const SmarlAccounting* acc,
@@ -255,8 +251,8 @@ extern "C" int smarl_coverage_float_rollout(const SmarlCoverageFloatParams* p, c
   r.g_mode = acc->g_mode;
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
   cudaStream_t st = (cudaStream_t)stream;
-  if (int rc = p->mode == 0 ? launch_coverage_float_rollout_m0(p->n_agents, r, grid, st)
-                            : launch_coverage_float_rollout_m1(p->n_agents, r, grid, st))
+  if (int rc = dispatch<0, 1>(p->mode, [&](auto m) { return launch_coverage_float_rollout<m>(p->n_agents, r, grid, st); },
+                              "bad mode %d"))
     return rc;
   if (stats) return launch_stats_finalize(stats_scratch, grid, p->n_agents, p->n_agents, n_envs, stats, st);
   return SMARL_OK;

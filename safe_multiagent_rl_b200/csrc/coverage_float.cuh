@@ -137,9 +137,8 @@ struct CoverageFloatRolloutArgs {
   int32_t g_mode;
 };
 
-int launch_coverage_float_step_m0(int A, const CoverageFloatArgs& a, unsigned grid, cudaStream_t s);
-int launch_coverage_float_step_m1(int A, const CoverageFloatArgs& a, unsigned grid, cudaStream_t s);
-int launch_coverage_float_rollout_m0(int A, const CoverageFloatRolloutArgs& a, unsigned grid, cudaStream_t s);
-int launch_coverage_float_rollout_m1(int A, const CoverageFloatRolloutArgs& a, unsigned grid, cudaStream_t s);
+// Launchers of mode M (0 = Continuous, 1 = Discretized), in coverage_float.cu
+template <int M> int launch_coverage_float_step(int A, const CoverageFloatArgs& a, unsigned grid, cudaStream_t s);
+template <int M> int launch_coverage_float_rollout(int A, const CoverageFloatRolloutArgs& a, unsigned grid, cudaStream_t s);
 
 }  // namespace smarl

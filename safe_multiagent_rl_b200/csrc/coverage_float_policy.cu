@@ -217,14 +217,12 @@ extern "C" int smarl_coverage_float_policy_rollout(const SmarlCoverageFloatParam
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp; k.pol = gauss_policy_args(pol);
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
   cudaStream_t st = (cudaStream_t)stream;
-  switch (A) {
-#define SMARL_COVF_POLICY_CASE(N) \
-  case N: coverage_float_policy_rollout_kernel<N><<<grid, kCovFThreads, 0, st>>>(k); break;
-    SMARL_COVF_POLICY_CASE(1) SMARL_COVF_POLICY_CASE(2) SMARL_COVF_POLICY_CASE(3) SMARL_COVF_POLICY_CASE(4)
-    SMARL_COVF_POLICY_CASE(5) SMARL_COVF_POLICY_CASE(6) SMARL_COVF_POLICY_CASE(7) SMARL_COVF_POLICY_CASE(8)
-#undef SMARL_COVF_POLICY_CASE
-  }
-  SMARL_CUDA(cudaGetLastError());
+  if (int rc = dispatch<1, 8>(A, [&](auto kA) {
+        coverage_float_policy_rollout_kernel<kA><<<grid, kCovFThreads, 0, st>>>(k);
+        SMARL_CUDA(cudaGetLastError());
+        return SMARL_OK;
+      }))
+    return rc;
   if (stats) return launch_stats_finalize(stats_scratch, grid, A, A, n_envs, stats, st);
   return SMARL_OK;
 }

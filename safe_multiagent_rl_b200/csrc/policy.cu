@@ -160,12 +160,12 @@ extern "C" int smarl_policy_act_discrete(const SmarlDiscretePolicy* p, const uin
   // two env tiles per CTA iteration, 1 = groups of up to 16 agents and one tile
   const int variant = kernel_variant(SMARL_KERNEL_POLICY);
   if (variant != 0) return launch_policy_tc(a, p->n_agents, variant == 1 ? 16 : 8, sms, st);
-  SMARL_DISPATCH_A(p->n_agents, {
+  return dispatch<1, 32>(p->n_agents, [&](auto kA) {
     using C = PolCfg<kA>;
     auto kern = policy_act_discrete_kernel<kA>;
     const size_t smem = C::kSmemFloats * sizeof(float);
     if (smem > 227 * 1024) {
-      set_error("policy weights of %d agents need %zu bytes of shared memory", kA, smem);
+      set_error("policy weights of %d agents need %zu bytes of shared memory", (int)kA, smem);
       return SMARL_EUNSUPPORTED;
     }
     if (smem > 48 * 1024) SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -174,7 +174,7 @@ extern "C" int smarl_policy_act_discrete(const SmarlDiscretePolicy* p, const uin
     a.n_tiles = (ld + C::TE - 1) / C::TE;
     const int64_t grid = a.n_tiles < (int64_t)sms * per_sm ? a.n_tiles : (int64_t)sms * per_sm;
     SMARL_CUDA(launch_pdl(kern, (unsigned)grid, C::THREADS, smem, st, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
   });
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
 }

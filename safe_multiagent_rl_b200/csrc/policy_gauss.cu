@@ -180,12 +180,12 @@ extern "C" int smarl_policy_act_gaussian(const SmarlGaussianPolicy* p, const flo
   SMARL_CUDA(cudaGetDevice(&dev));
   SMARL_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   cudaStream_t st = (cudaStream_t)stream;
-  SMARL_DISPATCH_A(p->n_agents, {
+  return dispatch<1, 32>(p->n_agents, [&](auto kA) {
     using C = GaussCfg<kA>;
     auto kern = policy_act_gaussian_kernel<kA>;
     const size_t smem = C::smem_floats(a.S) * sizeof(float);
     if (smem > 227 * 1024) {
-      set_error("policy weights of %d agents with %d inputs need %zu bytes of shared memory", kA, a.S, smem);
+      set_error("policy weights of %d agents with %d inputs need %zu bytes of shared memory", (int)kA, a.S, smem);
       return SMARL_EUNSUPPORTED;
     }
     if (smem > 48 * 1024) SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -195,7 +195,7 @@ extern "C" int smarl_policy_act_gaussian(const SmarlGaussianPolicy* p, const flo
     a.n_tiles = (ld + C::TE - 1) / C::TE;
     const int64_t grid = a.n_tiles < (int64_t)sms * per_sm ? a.n_tiles : (int64_t)sms * per_sm;
     SMARL_CUDA(launch_pdl(kern, (unsigned)grid, C::THREADS, smem, st, a));
+    SMARL_CUDA(cudaGetLastError());
+    return SMARL_OK;
   });
-  SMARL_CUDA(cudaGetLastError());
-  return SMARL_OK;
 }

@@ -385,8 +385,7 @@ static int launch_tc_any(const PolicyArgs& a, int group_max, int sms, cudaStream
 }
 
 int launch_policy_tc(const PolicyArgs& a, int n_agents, int group_max, int sms, cudaStream_t st) {
-  SMARL_DISPATCH_A(n_agents, return launch_tc_any<kA>(a, group_max, sms, st));
-  return SMARL_OK;
+  return dispatch<1, 32>(n_agents, [&](auto kA) { return launch_tc_any<kA>(a, group_max, sms, st); });
 }
 
 }  // namespace smarl

@@ -51,6 +51,37 @@ def test_abi_struct_sizes():
     assert C.sizeof(_lib.CollisionParams) == 32
 
 
+def agent_count_call(lib, env, kind, n_agents, n_envs):
+    """One open-loop step or rollout of `env` with `n_agents` agents over n_envs = ld envs, every other argument valid.
+    The state pointers are fake: the call must be rejected before it touches them."""
+    from safe_multiagent_rl_b200 import _lib
+    f = C.c_void_p(0x1000)
+    acc = C.byref(_lib.Accounting(0.9, 4, 0, None))
+    if env == "coverage":
+        p = C.byref(_lib.CoverageParams(5, n_agents, 0, 0, None, None))
+        if kind == "step":
+            return lib.smarl_coverage_step(p, f, f, f, None, f, f, None, None, None, n_envs, n_envs, None)
+        return lib.smarl_coverage_rollout(p, acc, f, f, f, None, f, f, f, f, f, None, None, None, None, n_envs, n_envs,
+                                          None)
+    if env == "congestion":
+        p = C.byref(_lib.CongestionParams(5, n_agents, f, 0, 0, 0, 0, 0, None, None))
+        if kind == "step":
+            return lib.smarl_congestion_step(p, f, f, f, None, None, f, f, None, None, None, 0, n_envs, n_envs, None)
+        return lib.smarl_congestion_rollout(p, acc, f, f, f, None, None, f, f, f, f, f, None, None, None, None, n_envs,
+                                            n_envs, None)
+    if env == "collision":
+        p = C.byref(_lib.CollisionParams(5, n_agents, 3, 0, 0.25, 0, 0))
+        if kind == "step":
+            return lib.smarl_collision_step(p, f, f, f, f, f, None, f, f, None, None, None, None, n_envs, n_envs, None)
+        return lib.smarl_collision_rollout(p, acc, f, f, f, f, None, f, f, f, f, f, f, f, None, None, None, None, n_envs,
+                                           n_envs, None)
+    p = C.byref(_lib.CoverageFloatParams(5, n_agents, 0, 0, 2.0, 0.0, 0.0, 0.0, 0.0, 0.0, None))
+    if kind == "step":
+        return lib.smarl_coverage_float_step(p, f, f, f, None, f, f, None, None, None, n_envs, n_envs, None)
+    return lib.smarl_coverage_float_rollout(p, acc, f, f, f, None, f, f, f, f, f, None, None, None, None, n_envs, n_envs,
+                                            None)
+
+
 def test_validation_errors_before_any_cuda_work(lib):
     from safe_multiagent_rl_b200 import _lib
     p = _lib.CoverageParams(5, 3, 0, 0, None, None)
@@ -102,8 +133,30 @@ def test_validation_errors_before_any_cuda_work(lib):
             cases.append(((acc(g_mode=1), f, None, None, None), b"needs g_scratch"))
         for args, needle in cases:
             assert call(*args) == -1 and needle in lib.smarl_last_error(), (needle, lib.smarl_last_error())
+    # Agent counts no kernel is built for: the open-loop steps and rollouts leave them to the launchers' dispatch
+    for env in ("coverage", "congestion", "collision", "coverage_float"):
+        for kind in ("step", "rollout"):
+            rc = agent_count_call(lib, env, kind, 0, 16)
+            assert rc == -3 and b"n_agents=0 outside 1..32" in lib.smarl_last_error(), (env, kind)
+    coop = b"cooperative %s kernels cover n_agents 9..32 (got 33)"
+    for env, kind, needle in [("coverage", "step", coop % b"Coverage"), ("coverage", "rollout", b"n_agents=33 outside 1..32"),
+                              ("congestion", "step", coop % b"Congestion"), ("congestion", "rollout", coop % b"Congestion"),
+                              ("collision", "step", coop % b"Collision"), ("collision", "rollout", coop % b"Collision"),
+                              ("coverage_float", "step", b"n_agents=33 outside 1..32"),
+                              ("coverage_float", "rollout", b"n_agents=33 outside 1..32")]:
+        rc = agent_count_call(lib, env, kind, 33, 16)
+        assert rc == -3 and needle in lib.smarl_last_error(), (env, kind, rc, lib.smarl_last_error())
     assert lib.smarl_stats_len(16, 16) == 65
     assert lib.smarl_stats_scratch_len(3, 3, 50) == 26      # one row of partials per 32 envs
+
+
+def test_register_capped_launchers_reject_bad_agent_counts(lib):
+    """From 2^18 envs the A <= 4 kernels of these entry points run register-capped; a count below 1 must still be
+    rejected before any launch, not run through the A = 4 kernel."""
+    for env, kind in [("collision", "step"), ("collision", "rollout"), ("coverage_float", "rollout")]:
+        for A in (0, -1):
+            rc = agent_count_call(lib, env, kind, A, 1 << 18)
+            assert rc == -3 and b"n_agents=%d outside 1..32" % A in lib.smarl_last_error(), (env, kind, A, rc)
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
