@@ -38,40 +38,6 @@ struct CoverageStepArgs {
 
 constexpr int kStepThreads = 128;
 
-// ---------------------------------------------------------------------------------------
-// Fused open-loop episode: positions, cost counters and discounted sums never leave
-// registers for the whole horizon; per step a thread reads A action words (1 B / agent-step).
-// Replaces main.py:28-57 (minus the policy nets) + buffer.py:30-39 + meta_agent.py:18-30 +
-// agent.py:129-132 / :200-206 for four envs per thread.
-// ---------------------------------------------------------------------------------------
-struct CoverageRolloutArgs {
-  const uint8_t* start_x;
-  const uint8_t* start_y;
-  const uint8_t* actions;   // [T][A][ld]
-  const double* lambdas;
-  uint8_t* final_x;
-  uint8_t* final_y;
-  float* R;
-  float* modR;
-  int32_t* C;
-  float* G;                 // [T][A][ld]
-  float* g_scratch;         // [2][T][ld]
-  double* partials;         // [gridDim.x][stats_len]
-  const double* thresholds;
-  const float* lut;
-  const float* weights;
-  double gamma;
-  int64_t n_groups;
-  int64_t n_envs;
-  int64_t ld;
-  int32_t size;
-  int32_t lut_len;
-  int32_t n_steps;
-  int32_t g_mode;
-};
-
-constexpr int kRolloutThreads = 128;
-
 int launch_coverage_step(int A, const CoverageStepArgs& a, unsigned grid, cudaStream_t s);
 int launch_coverage_coop_step(int A, int S, uint8_t* pos_x, uint8_t* pos_y, const uint8_t* actions, float* obs,
                               float* reward, uint8_t* cost, uint8_t* done, const double* lambdas, float* penalty,
@@ -380,17 +346,6 @@ static int coverage_coop_lanes(int A) {
   const int forced = kernel_variant(SMARL_ENV_COVERAGE);
   if (forced >= 0) return forced;
   return A >= 22 ? 2 : 0;       // A = 20: 0.76 vs 0.75 (tie), A = 24: 0.66 -> 0.71, A = 32: 0.58 -> 0.65 of the HBM peak, closed loop
-}
-
-static int check_coverage(const SmarlCoverageParams* p) {
-  SMARL_REQUIRE(p != nullptr, "params is NULL");
-  SMARL_REQUIRE(p->size >= 1 && p->size <= 127, "size=%d outside 1..127", p->size);
-  SMARL_REQUIRE(p->lut_len >= 0 && (p->lut_len == 0 || p->lut != nullptr), "bad penalty table");
-  if (p->lut_len > kCoverageMaxLut) {
-    set_error("lut_len=%d exceeds the shared-memory table limit %d", p->lut_len, kCoverageMaxLut);
-    return SMARL_EUNSUPPORTED;
-  }
-  return SMARL_OK;
 }
 
 #endif

@@ -9,6 +9,51 @@ namespace smarl {
 // (the fused rollout kernel keeps a 32-byte static reduction buffer beside the table: (12279 + 1) * 4 + 32 = 48 KB)
 constexpr int kCoverageMaxLut = 12279;
 
+// ---------------------------------------------------------------------------------------
+// Fused open-loop episode: positions, cost counters and discounted sums never leave
+// registers for the whole horizon; per step a thread reads A action words (1 B / agent-step).
+// Replaces main.py:28-57 (minus the policy nets) + buffer.py:30-39 + meta_agent.py:18-30 +
+// agent.py:129-132 / :200-206 for four envs per thread.
+// ---------------------------------------------------------------------------------------
+struct CoverageRolloutArgs {
+  const uint8_t* start_x;
+  const uint8_t* start_y;
+  const uint8_t* actions;   // [T][A][ld]
+  const double* lambdas;
+  uint8_t* final_x;
+  uint8_t* final_y;
+  float* R;
+  float* modR;
+  int32_t* C;
+  float* G;                 // [T][A][ld]
+  float* g_scratch;         // [2][T][ld]
+  double* partials;         // [gridDim.x][stats_len]
+  const double* thresholds;
+  const float* lut;
+  const float* weights;
+  double gamma;
+  int64_t n_groups;
+  int64_t n_envs;
+  int64_t ld;
+  int32_t size;
+  int32_t lut_len;
+  int32_t n_steps;
+  int32_t g_mode;
+};
+
+constexpr int kRolloutThreads = 128;
+
+inline int check_coverage(const SmarlCoverageParams* p) {
+  SMARL_REQUIRE(p != nullptr, "params is NULL");
+  SMARL_REQUIRE(p->size >= 1 && p->size <= 127, "size=%d outside 1..127", p->size);
+  SMARL_REQUIRE(p->lut_len >= 0 && (p->lut_len == 0 || p->lut != nullptr), "bad penalty table");
+  if (p->lut_len > kCoverageMaxLut) {
+    set_error("lut_len=%d exceeds the shared-memory table limit %d", p->lut_len, kCoverageMaxLut);
+    return SMARL_EUNSUPPORTED;
+  }
+  return SMARL_OK;
+}
+
 // Agents of env lane k packed for the pair loop: p[a] = (2x | 2y << 8), upper bytes zero.
 // One PRMT gathers (x_k, y_k) and zero-fills bytes 2,3 by replicating the (clear) sign bit of
 // x_k -- coordinates are <= 127 -- and one add doubles both bytes without carry.

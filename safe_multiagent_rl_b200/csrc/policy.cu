@@ -142,10 +142,8 @@ extern "C" int smarl_policy_act_discrete(const SmarlDiscretePolicy* p, const uin
   SMARL_REQUIRE(p != nullptr, "policy params is NULL");
   if (int rc = check_layout(n_envs, ld)) return rc;
   SMARL_REQUIRE(p->n_agents >= 1 && p->n_agents <= SMARL_MAX_AGENTS, "n_agents=%d outside 1..32", p->n_agents);
-  SMARL_REQUIRE(p->hidden == kPolHidden && p->n_actions == kPolActions,
-                "only the reference's DiscretePolicy shape (hidden 16, 5 actions) is built (got %d, %d)", p->hidden,
-                p->n_actions);
-  SMARL_REQUIRE(p->w1 && p->b1 && p->w2 && p->b2 && pos_x && pos_y && actions, "null pointer");
+  if (int rc = check_discrete_policy(p, p->n_agents)) return rc;
+  SMARL_REQUIRE(pos_x && pos_y && actions, "null pointer");
   SMARL_REQUIRE(t >= 0 && t < 65536, "t=%d outside 0..65535", t);
   SMARL_REQUIRE(aligned16(pos_x) && aligned16(pos_y) && aligned16(actions) && aligned16(logp), "pointers must be 16-byte aligned");
   PolicyArgs a;

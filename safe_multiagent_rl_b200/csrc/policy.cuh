@@ -31,6 +31,16 @@ struct PolicyArgs {
 // tensor-core build (policy_tc.cu); SMARL_EUNSUPPORTED when the shape does not fit it
 int launch_policy_tc(const PolicyArgs& a, int n_agents, int group_max, int sms, cudaStream_t st);
 
+// The policy checks of the entry points that run the DiscretePolicy (p not NULL) for an env of A agents.
+inline int check_discrete_policy(const SmarlDiscretePolicy* p, int A) {
+  SMARL_REQUIRE(p->n_agents == A, "policy has %d agents, the env %d", p->n_agents, A);
+  SMARL_REQUIRE(p->hidden == kPolHidden && p->n_actions == kPolActions,
+                "only the reference's DiscretePolicy shape (hidden 16, 5 actions) is built (got %d, %d)", p->hidden,
+                p->n_actions);
+  SMARL_REQUIRE(p->w1 && p->b1 && p->w2 && p->b2, "null pointer");
+  return SMARL_OK;
+}
+
 #ifdef __CUDACC__
 __device__ __forceinline__ uint2 policy_key(uint64_t seed) {
   return make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ 0x504C4359u);   // "PLCY"

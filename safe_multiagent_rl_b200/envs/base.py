@@ -1,6 +1,6 @@
 """Shared host logic of the batched envs: buffers in the agent-major SoA layout, action ingest,
-reference-oriented views, closed-loop and fused rollout helpers, the on-policy rollout of the
-Gaussian-policy envs and the single-env list adaptor."""
+reference-oriented views, closed-loop and fused rollout helpers, the one-launch on-policy rollout
+and the single-env list adaptor."""
 from __future__ import annotations
 
 import numpy as np
@@ -175,21 +175,25 @@ class BatchedEnv:
         return o, acc
 
     def _policy_records(self, o, T, S, record):
-        """The record slabs of an on-policy rollout in ``o``: ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] and
-        ``logp_`` [T, A, ld] (allocated unless ``o`` holds them in this shape), and their views ``obs`` [T, E, S],
-        ``actions`` [T, A, E, 2] and ``logp`` [T, A, E].  Returns the three slabs the kernel writes, or three
-        ``None`` with ``record=False``, which also drops the records ``o`` held from an earlier call."""
+        """The record slabs of an on-policy rollout in ``o``: ``obs_`` [T, S, ld], ``actions_`` [T, action_rows, ld]
+        of ``action_dtype`` and ``logp_`` [T, A, ld] (allocated unless ``o`` holds them in this shape and dtype), and
+        their views ``obs`` [T, E, S], ``actions`` [T, A, E, 2] (continuous actions) or [T, A, E] (discrete) and
+        ``logp`` [T, A, E].  Returns the three slabs the kernel writes, or three ``None`` with ``record=False``, which
+        also drops the records ``o`` held from an earlier call."""
         if not record:
             for name in ("obs_", "actions_", "logp_", "obs", "actions", "logp"):
                 o.pop(name, None)
             return [None, None, None]
         A, E = self.n_agents, self.n_envs
-        for name, rows in (("obs_", S), ("actions_", 2 * A), ("logp_", A)):
+        for name, rows, dtype in (("obs_", S, torch.float32), ("actions_", self.action_rows, self.action_dtype),
+                                  ("logp_", A, torch.float32)):
             have = o.get(name)
-            if have is None or tuple(have.shape) != (T, rows, self.ld):
-                o[name] = self._alloc(rows, torch.float32, (T,))
+            if have is None or tuple(have.shape) != (T, rows, self.ld) or have.dtype != dtype:
+                o[name] = self._alloc(rows, dtype, (T,))
         o["obs"] = o["obs_"][:, :, :E].permute(0, 2, 1)
-        o["actions"] = o["actions_"][:, :, :E].view(T, A, 2, E).permute(0, 1, 3, 2)
+        o["actions"] = o["actions_"][:, :, :E]
+        if self.action_rows != A:                                        # rows dx0, dy0, dx1, ...
+            o["actions"] = o["actions"].view(T, A, 2, E).permute(0, 1, 3, 2)
         o["logp"] = o["logp_"][:, :, :E]
         return [o["obs_"], o["actions_"], o["logp_"]]
 
@@ -230,30 +234,37 @@ class BatchedEnv:
         return out
 
 
-class GaussianPolicyRollout:
-    """``policy_rollout`` of the envs whose reference policy is the ContinuousPolicy (BatchedEnv subclasses).  The env
-    supplies ``_policy_rollout_impl(pol, acc, lambdas, rec, o)``, its C entry point's call."""
+class PolicyRollout:
+    """``policy_rollout`` of the envs that run a whole on-policy episode in one launch (BatchedEnv subclasses).  The env
+    supplies ``rollout_policy`` (the name of the fused policy class it samples, in ``policy.py``),
+    ``reference_policy`` (the reference's policy that class implements), ``rollout_threads`` (how its kernel maps
+    envs to threads, up to 8 agents) and ``_policy_rollout_impl(pol, acc, lambdas, rec, o)``, its C entry point's
+    call."""
 
     def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
                        out=None):
-        """Whole on-policy episode in one launch: every step samples ``policy`` (a ``FusedGaussianPolicy``: its
-        weights, seed and episode) on the current observation, steps the env and accumulates what ``rollout``
-        returns (CollisionAvoidance's ``n_active`` included).  The records and the final state are the bits of the closed loop reset + T x (``policy.act(t=t)``,
-        ``env.step``), the products those of ``rollout`` fed the recorded actions.  With ``record`` it adds views of
-        the kernel-layout slabs ``obs_`` [T, S, ld], ``actions_`` [T, 2A, ld] (what ``rollout`` takes) and ``logp_``
-        [T, A, ld]: ``obs`` [T, E, S], ``actions`` [T, A, E, 2] and ``logp`` [T, A, E], so that
-        ``policy.log_prob(out["obs"][t], out["actions"][t])`` is the learner's differentiable side.  With
-        ``record=False`` the returned dict holds no records, also when ``out`` held some.  With ``out`` reused the
-        call allocates nothing (CUDA-graph capturable)."""
-        from ..policy import FusedGaussianPolicy
-        if not isinstance(policy, FusedGaussianPolicy):
-            raise NotImplementedError("policy_rollout runs the reference's ContinuousPolicy: pass a FusedGaussianPolicy")
+        """Whole on-policy episode in one launch: every step samples ``policy`` (a ``FusedGaussianPolicy`` for the
+        continuous envs, a ``FusedDiscretePolicy`` for CoverageDiscrete: its weights, seed and episode) on the current
+        observation, steps the env and accumulates what ``rollout`` returns (CollisionAvoidance's ``n_active``
+        included).  The records and the final state are the bits of the closed loop reset + T x (``policy.act(t=t)``,
+        ``env.step``) (for CoverageDiscrete with the FP32-pipe policy build,
+        ``_lib.kernel_variant(_lib.KERNEL_POLICY, 0)``), the products those of ``rollout`` fed the recorded actions.
+        The episode index of ``policy`` is not advanced: call ``policy.next_episode()`` for fresh samples.  With
+        ``record`` it adds views of the kernel-layout slabs ``obs_`` [T, S, ld], ``actions_`` [T, action_rows, ld]
+        (what ``rollout`` takes) and ``logp_`` [T, A, ld]: ``obs`` [T, E, S], ``actions`` [T, A, E, 2] (continuous)
+        or [T, A, E] (discrete) and ``logp`` [T, A, E], so that ``policy.log_prob(out["obs"][t], out["actions"][t])``
+        is the learner's differentiable side.  With ``record=False`` the returned dict holds no records, also when
+        ``out`` held some.  With ``out`` reused the call allocates nothing (CUDA-graph capturable)."""
+        from .. import policy as policies
+        if not isinstance(policy, getattr(policies, self.rollout_policy)):
+            raise NotImplementedError(f"policy_rollout runs the reference's {self.reference_policy}: pass a "
+                                      f"{self.rollout_policy}")
         if self.n_agents > 8:
-            raise NotImplementedError("policy_rollout runs one thread per env, for n_agents up to 8")
+            raise NotImplementedError(f"policy_rollout runs {self.rollout_threads}, for n_agents up to 8")
+        pol = policy.c_params(self)
         T = int(n_steps)
         o = out if out is not None else {}
         rec = self._policy_records(o, T, self.obs.shape[0], record)
-        pol = policy.c_params(self)
         o, acc = self._begin_rollout(T, g_mode, o, 2 * T, gamma, thresholds)
         self._policy_rollout_impl(pol, acc, lambdas, rec, o)
         return self._rollout_result(o)

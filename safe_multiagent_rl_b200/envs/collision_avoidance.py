@@ -11,7 +11,7 @@ import torch
 from .. import _lib
 from ..layout import env_major
 from ..rollout import G_NONE
-from .base import BatchedEnv, GaussianPolicyRollout
+from .base import BatchedEnv, PolicyRollout
 
 
 def default_starts(size, n_agents, n_envs, n_landmarks=1):
@@ -22,7 +22,7 @@ def default_starts(size, n_agents, n_envs, n_landmarks=1):
     return draws[:, :n_agents], draws[:, n_agents:]
 
 
-class BatchedCollisionAvoidance(GaussianPolicyRollout, BatchedEnv):
+class BatchedCollisionAvoidance(PolicyRollout, BatchedEnv):
     """Constructor mirrors ``CollisionAvoidance(size, n_agents, n_landmarks, shuffle, agents_size,
     normalize_state)`` (collision_avoidance.py:49) plus ``n_envs`` / ``device``.
 
@@ -35,6 +35,7 @@ class BatchedCollisionAvoidance(GaussianPolicyRollout, BatchedEnv):
     cost_dtype = torch.int32
     action_dtype = torch.float32
     supports_lean = True       # the reward is one value shared by all agents (collision_avoidance.py:129-130)
+    rollout_policy, reference_policy, rollout_threads = "FusedGaussianPolicy", "ContinuousPolicy", "one thread per env"
 
     def __init__(self, size, n_agents, n_envs=1, n_landmarks=1, shuffle=False, agents_size=0.25,
                  normalize_state=False, device="cuda", starts=None, landmarks=None, env_offset=0, seed=0):

@@ -9,7 +9,7 @@ import torch
 
 from .. import _lib
 from ..rollout import G_NONE
-from .base import BatchedEnv
+from .base import BatchedEnv, PolicyRollout
 
 
 MAX_LUT = 12279      # kCoverageMaxLut (csrc/coverage.cuh): the table + the rollout kernel's reduction buffer fill 48 KB
@@ -42,7 +42,7 @@ def default_starts(size, n_agents, n_envs):
     return np.floor(draws[:, n_agents:, :] * size)
 
 
-class BatchedCoverageDiscrete(BatchedEnv):
+class BatchedCoverageDiscrete(PolicyRollout, BatchedEnv):
     """Constructor mirrors ``CoverageDiscrete(size, n_agents, shuffle, agents_size, fieldview_size,
     weights)`` (coverage.py:167) plus ``n_envs`` / ``device``.
 
@@ -57,6 +57,7 @@ class BatchedCoverageDiscrete(BatchedEnv):
     action_dtype = torch.uint8
     never_done = True          # check_done is all-False (coverage.py:97-98)
     supports_lean = True       # reward_a = w_a * rew: one env-reward row is enough (DESIGN.md section 3.6)
+    rollout_policy, reference_policy, rollout_threads = "FusedDiscretePolicy", "DiscretePolicy", "one thread per four envs"
 
     def __init__(self, size, n_agents, n_envs=1, shuffle=False, agents_size=0.5, fieldview_size=None,
                  weights=None, device="cuda", starts=None, env_offset=0, seed=0):
@@ -143,3 +144,10 @@ class BatchedCoverageDiscrete(BatchedEnv):
             _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]),
             _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
         return self._rollout_result(o)
+
+    def _policy_rollout_impl(self, pol, acc, lambdas, rec, o):
+        _lib.check(self.lib.smarl_coverage_policy_rollout(
+            C.byref(self._params), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
+            _lib.ptr(lambdas), *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x), _lib.ptr(self.pos_y),
+            _lib.ptr(o["R_"]), _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]),
+            _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), self.n_envs, self.ld, _lib.stream_ptr()))

@@ -9,7 +9,7 @@ import torch
 
 from .. import _lib
 from ..rollout import G_NONE
-from .base import BatchedEnv, GaussianPolicyRollout
+from .base import BatchedEnv, PolicyRollout
 
 
 class _CoverageFloat(BatchedEnv):
@@ -79,12 +79,13 @@ class _CoverageFloat(BatchedEnv):
         self._draw_float_starts(episode, 3 if zoom is not None else 2, zoom or 0.0)
 
 
-class BatchedCoverageContinuous(GaussianPolicyRollout, _CoverageFloat):
+class BatchedCoverageContinuous(PolicyRollout, _CoverageFloat):
     """``CoverageContinuous(size, n_agents, shuffle, agents_size, fieldview_size, weights, coarseness)``
     (coverage.py:11) + ``n_envs``/``device``.  Actions are ``[n_envs, n_agents, 2]`` float32."""
 
     action_space = 2
     action_dtype = torch.float32
+    rollout_policy, reference_policy, rollout_threads = "FusedGaussianPolicy", "ContinuousPolicy", "one thread per env"
 
     def __init__(self, size, n_agents, n_envs=1, shuffle=False, agents_size=0.5, fieldview_size=None, weights=None,
                  coarseness=None, device="cuda", starts=None, env_offset=0, seed=0):

@@ -85,6 +85,20 @@ class FusedDiscretePolicy(BatchedDiscretePolicy):
         """Advance the sampling stream's episode index (a device-side increment: CUDA-graph capturable)."""
         self._episode_dev.add_(1)
 
+    def c_params(self, env):
+        """The ``SmarlDiscretePolicy`` of these weights and this sampling stream for ``env`` (its env_offset).  Raises
+        ValueError when the weights are not those of ``env``'s agent count: the kernels read ``env.n_agents`` agents'
+        networks of ``env.state_space`` inputs."""
+        L = self._lib_mod
+        w = [t_.detach() for t_ in (self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias)]
+        assert all(x.is_contiguous() and x.dtype == torch.float32 for x in w)
+        A, S = self.fc1.weight.shape[:2]
+        if (A, S) != (env.n_agents, env.state_space):
+            raise ValueError(f"the policy holds {A} agents' networks of {S} inputs; the env has {env.n_agents} agents "
+                             f"and {env.state_space} inputs")
+        return L.DiscretePolicyParams(A, 16, 5, 0, L.ptr(w[0]), L.ptr(w[1]), L.ptr(w[2]), L.ptr(w[3]),
+                                      self.seed & (2 ** 64 - 1), env.env_offset, L.ptr(self._episode_dev))
+
     @torch.no_grad()
     def act(self, obs=None, t=None):
         """Sample actions for step ``t`` (default: the env's step counter) into ``env.action_buffer``; returns
@@ -92,10 +106,7 @@ class FusedDiscretePolicy(BatchedDiscretePolicy):
         ``env.pos_x`` / ``env.pos_y``."""
         import ctypes as C
         env, L = self.env, self._lib_mod
-        w = [t_.detach() for t_ in (self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias)]
-        assert all(x.is_contiguous() and x.dtype == torch.float32 for x in w)
-        p = L.DiscretePolicyParams(env.n_agents, 16, 5, 0, L.ptr(w[0]), L.ptr(w[1]), L.ptr(w[2]), L.ptr(w[3]),
-                                   self.seed & (2 ** 64 - 1), env.env_offset, L.ptr(self._episode_dev))
+        p = self.c_params(env)
         L.check(self.lib.smarl_policy_act_discrete(C.byref(p), L.ptr(env.pos_x), L.ptr(env.pos_y),
                                                    L.ptr(env.action_buffer), L.ptr(self.logp),
                                                    int(env.t if t is None else t), env.n_envs, env.ld, L.stream_ptr()))

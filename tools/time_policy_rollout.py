@@ -1,19 +1,24 @@
-"""Time the on-policy episode in one launch (``policy_rollout`` of BatchedCollisionAvoidance or
-BatchedCoverageContinuous) against the closed loop it replaces: T x (FusedGaussianPolicy.act + env.step) + the returns
+"""Time the on-policy episode in one launch (``policy_rollout`` of BatchedCollisionAvoidance, BatchedCoverageContinuous
+or BatchedCoverageDiscrete) against the closed loop it replaces: T x (fused policy act + env.step) + the returns
 kernel, replayed from one CUDA graph (for CollisionAvoidance exactly as bench.py's config2_collision_gaussian_graphed
-builds it).
+builds it, for CoverageDiscrete as its config1_graphed.fused).
 
-    python tools/time_policy_rollout.py [--env collision|coverage_continuous] [--iters 20] [--rounds 5] [--out FILE]
+    python tools/time_policy_rollout.py [--env collision|coverage_continuous|coverage_discrete] [--iters 20]
+                                        [--rounds 5] [--out FILE]
 
 Shapes: 65 536 envs at 3 agents (BASELINE configs[1] for collision) and 2^20 envs at 3 and 8 agents, size 5, T = 50,
 lambda = 0.1, reward-to-go G.  collision: one landmark, thresholds [2].  coverage_continuous: lambda and threshold 25
-per agent, weights [1, 2, 3] at 3 agents.  The arms alternate within one process, each timed with CUDA events over
---iters calls per round; the products of both paths are compared on the timed inputs.
+per agent, weights [1, 2, 3] at 3 agents.  coverage_discrete: BASELINE configs[0] (50 envs x 3 agents) and the same
+setup at 65 536 x 3, 2^20 x 3 and 2^20 x 8; there --iters rises per shape until every timed window lasts at least
+--min-window-ms (150 ms).
+The arms alternate within one process, each timed with CUDA events over --iters calls per round; the products of the
+paths are compared on the timed inputs.
 """
 from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import statistics
 import subprocess
@@ -168,20 +173,116 @@ def shape_coverage(E, A, T, iters, rounds):
     return res
 
 
+def shape_coverage_discrete(E, A, T, iters, rounds, min_window_ms):
+    """BASELINE configs[0] at every batch size: size 5, weights [1, 2, 3] at 3 agents, lambda 0.1, thresholds 25,
+    gamma 0.999, reward-to-go G.  Closed loops with FusedDiscretePolicy in its default (tensor-core) build, as bench.py
+    builds config1_graphed.fused, and in its FP32-pipe build, whose samples the one launch reproduces bit for bit."""
+    import safe_multiagent_rl_b200 as s
+    from safe_multiagent_rl_b200 import _lib
+    from safe_multiagent_rl_b200.policy import FusedDiscretePolicy
+    starts = np.random.default_rng(1).integers(0, 5, (E, A, 2))
+    weights = [1.0, 2.0, 3.0] if A == 3 else None
+    mk = lambda: s.BatchedCoverageDiscrete(5, A, n_envs=E, weights=weights, starts=starts)
+    lam = torch.full((A,), 0.1, dtype=torch.float64, device="cuda")
+    thr = torch.full((A,), 25.0, dtype=torch.float64, device="cuda")
+    gamma = 0.999
+    env_tc = mk()
+    pol_tc = FusedDiscretePolicy(env_tc, seed=7)
+    loop_tc = s.GraphedClosedLoop(env_tc, T, lambda obs, t: pol_tc.act(t=t), lam, gamma, thresholds=[25.0] * A)
+    env_c = mk()
+    pol_c = FusedDiscretePolicy(env_c, seed=7)
+    pol_c.load_state_dict(pol_tc.state_dict())
+    with _lib.kernel_variant(_lib.KERNEL_POLICY, 0):       # the kernel is chosen when the graph is captured
+        loop_c = s.GraphedClosedLoop(env_c, T, lambda obs, t: pol_c.act(t=t), lam, gamma, thresholds=[25.0] * A)
+    env_p = mk()
+    pol_p = FusedDiscretePolicy(env_p, seed=7)
+    pol_p.load_state_dict(pol_tc.state_dict())
+    kw = dict(lambdas=lam, gamma=gamma, thresholds=thr, g_mode=1)
+    out = env_p.policy_rollout(pol_p, T, **kw)
+    out_nr = env_p.policy_rollout(pol_p, T, record=False, **kw)
+    torch.cuda.synchronize()
+    graphs = {}
+    for tag, o, rec in (("fused_graphed", out, True), ("fused_graphed_no_record", out_nr, False)):
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            env_p.policy_rollout(pol_p, T, out=o, record=rec, **kw)
+        graphs[tag] = g
+    arms = {"closed_loop_graphed": loop_tc.replay,
+            "closed_loop_graphed_fp32_policy": loop_c.replay,
+            "fused_eager": lambda: env_p.policy_rollout(pol_p, T, out=out, **kw),
+            "fused_graphed": graphs["fused_graphed"].replay,
+            "fused_graphed_no_record": graphs["fused_graphed_no_record"].replay}
+    for fn in arms.values():
+        for _ in range(3):
+            fn()
+    torch.cuda.synchronize()
+    # enough calls per window that even the fastest arm's window lasts min_window_ms
+    iters = max(iters, math.ceil(min_window_ms / min(event_ms(fn, 5) for fn in arms.values())))
+    times = {k: [] for k in arms}
+    for _ in range(rounds):
+        for k, fn in arms.items():
+            times[k].append(event_ms(fn, iters))
+    # the products on the timed inputs: one more call of each path, then the open-loop rollout of the recorded actions
+    ref = loop_c.replay()
+    graphs["fused_graphed"].replay()
+    torch.cuda.synchronize()
+    same = {"final_state": all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                               ((env_p.pos_x, env_c.pos_x), (env_p.pos_y, env_c.pos_y))),
+            "last_step_actions": bool(torch.equal(out["actions_"][T - 1, :, :E], env_c.action_buffer[:, :E])),
+            "last_step_logp": bool(torch.equal(out["logp_"][T - 1, :, :E], pol_c.logp[:, :E])),
+            "C": bool(torch.equal(out["C"].long(), ref["C"].long()))}
+    fused = {k: out[k].clone() for k in ("R", "modR", "C", "G", "stats_vec")}
+    env_r = mk()
+    open_loop = env_r.rollout(out["actions_"], **kw)
+    torch.cuda.synchronize()
+    same_open = {k: bool(torch.equal(fused[k], open_loop[k])) for k in fused}
+    same_open["final_state"] = all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                                   ((env_p.pos_x, env_r.pos_x), (env_p.pos_y, env_r.pos_y)))
+    # the default build at t = 0 (same observation): share of equal samples, log-prob gap where they agree
+    env_tc.reset()
+    _, a0, lp0 = pol_tc.act(t=0)
+    agree = a0 == out["actions"][0]
+    tc = {"actions_agree": float(agree.float().mean()),
+          "max_logp_diff_where_equal": float((lp0 - out["logp"][0]).abs()[agree].max())}
+
+    def rel(a, b):
+        a, b = a.double(), b.double()
+        return float(((a - b).abs() / b.abs().clamp_min(1e-300)).max())
+    res = {"env": "coverage_discrete", "n_envs": E, "n_agents": A, "T": T, "iters": iters, "rounds": rounds,
+           "ms_per_batch": {k: {"min": min(v), "median": statistics.median(v), "all": v} for k, v in times.items()},
+           "identical_to_fp32_closed_loop": same, "identical_to_open_loop_rollout": same_open,
+           "max_rel_diff_vs_fp32_closed_loop": {k: rel(fused[k], ref[k]) for k in ("R", "modR")} |
+                                               {"stats": rel(fused["stats_vec"], ref["stats"].vec)},
+           "tensor_core_build_t0": tc}
+    m = {k: v["median"] for k, v in res["ms_per_batch"].items()}
+    res["speedup_fused_graphed_vs_closed_loop"] = m["closed_loop_graphed"] / m["fused_graphed"]
+    res["speedup_fused_graphed_vs_fp32_closed_loop"] = m["closed_loop_graphed_fp32_policy"] / m["fused_graphed"]
+    del loop_tc, loop_c, graphs, out, out_nr
+    torch.cuda.empty_cache()
+    return res
+
+
+SHAPES = {"collision": "65536x3,1048576x3,1048576x8", "coverage_continuous": "65536x3,1048576x3,1048576x8",
+          "coverage_discrete": "50x3,65536x3,1048576x3,1048576x8"}
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--env", choices=("collision", "coverage_continuous"), default="collision")
-    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--env", choices=tuple(SHAPES), default="collision")
+    ap.add_argument("--iters", type=int, default=20, help="calls per timed window (coverage_discrete: at least)")
+    ap.add_argument("--min-window-ms", type=float, default=150.0,
+                    help="coverage_discrete: raise the calls per window until the fastest arm's window lasts this long")
     ap.add_argument("--rounds", type=int, default=5)
-    ap.add_argument("--shapes", default="65536x3,1048576x3,1048576x8", help="ExA list")
+    ap.add_argument("--shapes", default=None, help="ExA list (default: per env)")
     ap.add_argument("--out", default=None, help="also write the JSON lines here")
     a = ap.parse_args()
     lines = [json.dumps({"gpu": gpu_info(), "lib": os.path.basename(os.environ.get("SMARL_LIB", "libsmarl.so"))})]
     print(lines[-1], flush=True)
-    for sh in a.shapes.split(","):
+    run = {"collision": shape, "coverage_continuous": shape_coverage, "coverage_discrete": shape_coverage_discrete}[a.env]
+    for sh in (a.shapes or SHAPES[a.env]).split(","):
         E, A = (int(x) for x in sh.split("x"))
-        run = shape if a.env == "collision" else shape_coverage
-        lines.append(json.dumps(run(E, A, 50, a.iters, a.rounds)))
+        extra = (a.min_window_ms,) if a.env == "coverage_discrete" else ()
+        lines.append(json.dumps(run(E, A, 50, a.iters, a.rounds, *extra)))
         print(lines[-1], flush=True)
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
