@@ -475,6 +475,32 @@ int smarl_coverage_policy_rollout(const SmarlCoverageParams* p, const SmarlDiscr
                                   float* g_scratch, double* stats, double* stats_scratch, int64_t n_envs, int64_t ld,
                                   smarl_stream_t stream);
 
+/* Whole ON-POLICY Congestion episodes in one launch: main.py:28-57 with the policies inside, i.e. per step every agent's
+ * DiscretePolicy (agent.py:23-47) on the joint state (x0, y0, x1, ...: what the reset / step kernels write to env.obs),
+ * the sample, Congestion.step with its action noise, MetaAgent.act, and Buffer.step + compute_returns as in
+ * smarl_congestion_rollout.  Records and final positions are bit-identical to the closed loop reset +
+ * T x (smarl_policy_act_discrete(t) + smarl_congestion_step(t)) on the same starts, weights, policy stream and noise
+ * episode with the FP32-pipe policy build (smarl_set_kernel_variant(SMARL_KERNEL_POLICY, 0)); the default tensor-core
+ * build agrees on all but a few samples in 10^4, and an episode diverges from the step where one sample differs.  The
+ * products are bit-identical to smarl_congestion_rollout fed the recorded actions with the same noise episode (the
+ * closed loop's returns kernel sums the f32-rounded rewards, so its R, modR and stats agree to 1e-5 relative and C is
+ * equal).
+ *   p (noise_mode 0 or 2), acc, start_x .. lambdas and final_x .. stats_scratch as in smarl_congestion_rollout
+ *   (acc->g_mode 0..2; g_scratch [T][ld] with g_mode 1)
+ *   pol: weights, seed, episode, episode_dev and env_offset as in smarl_policy_act_discrete;
+ *        pol->n_agents = p->n_agents, hidden 16, 5 actions
+ *   obs_rec f32 [T][2A][ld] the observation the policy saw at step t      (NULL = skip)
+ *   actions u8  [T][A][ld]  the sampled actions (smarl_congestion_rollout's layout; NULL = skip)
+ *   logp    f32 [T][A][ld]  log-probability of the sampled action        (NULL = skip)
+ * A in 1..8 (one thread per four envs; A >= 9 or noise_mode 1 returns SMARL_EUNSUPPORTED), T in 1..65536 (16 bits of
+ * the Philox counter). */
+int smarl_congestion_policy_rollout(const SmarlCongestionParams* p, const SmarlDiscretePolicy* pol,
+                                    const SmarlAccounting* acc, const uint8_t* start_x, const uint8_t* start_y,
+                                    const double* lambdas, float* obs_rec, uint8_t* actions, float* logp,
+                                    uint8_t* final_x, uint8_t* final_y, float* R, float* modR, int32_t* C, float* G,
+                                    float* g_scratch, double* stats, double* stats_scratch, int64_t n_envs, int64_t ld,
+                                    smarl_stream_t stream);
+
 /* ------------------------------------------------------------------------------------
  * Multi-GPU: env instances are independent (envs/coverage.py:19, congestion.py:22,
  * collision_avoidance.py:60), so ranks own contiguous ranges of global env ids and the data path has no

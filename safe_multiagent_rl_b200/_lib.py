@@ -106,6 +106,9 @@ PROTOTYPES = {
     "smarl_coverage_policy_rollout": (C.c_int, [P(CoverageParams), P(DiscretePolicyParams), P(Accounting), c_ptr, c_ptr,
                                                 c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                                 c_ptr, c_ptr, c_ptr, i64, i64, c_ptr]),
+    "smarl_congestion_policy_rollout": (C.c_int, [P(CongestionParams), P(DiscretePolicyParams), P(Accounting), c_ptr,
+                                                  c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                                  c_ptr, c_ptr, c_ptr, c_ptr, i64, i64, c_ptr]),
     "smarl_comm_get_unique_id": (C.c_int, [c_ptr]),
     "smarl_comm_init_from_unique_id": (C.c_int, [P(c_ptr), c_ptr, i32, i32]),
     "smarl_comm_destroy": (None, [c_ptr]),

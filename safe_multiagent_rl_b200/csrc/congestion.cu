@@ -18,21 +18,6 @@ constexpr int kCongThreads = 128;
 constexpr int cong_step_min_blocks(int A) { return A <= 8 ? 6 : 0; }   // 0 = unspecified (1 would lift the register heuristic to 255)
 constexpr int cong_min_blocks(int A) { return A <= 8 ? 8 : (A <= 12 ? 5 : 0); }   // A = 9..12: 168 registers (A = 12 fused +9 %)
 
-// One Congestion transition for four envs (congestion.py:49-75): applies the effective moves,
-// leaves the new positions in xw/yw and the displacement codes in dcw.
-template <int A>
-__device__ __forceinline__ void congestion_transition(uint32_t (&xw)[A], uint32_t (&yw)[A],
-                                                      const uint32_t (&mw)[A], uint32_t (&dcw)[A],
-                                                      uint32_t size4) {
-  const uint32_t k1 = 0x01010101u;
-#pragma unroll
-  for (int i = 0; i < A; ++i) {
-    const uint32_t ox = xw[i], oy = yw[i];
-    grid_move4(xw[i], yw[i], mw[i], size4);
-    dcw[i] = ((xw[i] + k1) - ox) | (((yw[i] + k1) - oy) << 2);
-  }
-}
-
 // ---------------------------------------------------------------------------------------
 // Fused open-loop episode (main.py:28-57 minus the policy nets, buffer.py:30-39,
 // meta_agent.py:18-30, agent.py:129-132 / :200-206).  Positions stay in registers; the
@@ -40,8 +25,6 @@ __device__ __forceinline__ void congestion_transition(uint32_t (&xw)[A], uint32_
 // [agent][env lane][thread] so that every access is conflict-free.
 // ---------------------------------------------------------------------------------------
 // (CongestionRolloutArgs lives in congestion.cuh: the cooperative rollout kernel of congestion_coop.cu shares it)
-
-constexpr int kCongRollThreads = 64;
 
 #if SMARL_TU_IS(0) || SMARL_TU_IS(1) || SMARL_TU_IS(2)
 template <int A, int MODE>
@@ -329,15 +312,6 @@ static int congestion_coop_rollout_lanes(int A) {
   const int forced = kernel_variant(SMARL_ENV_CONGESTION);
   if (forced >= 0) return forced ? 4 : 0;
   return A >= 12 ? 4 : 0;       // fused ms per 2^20 envs x T = 20: A = 12 1.12 -> 1.09, 16 1.75 -> 1.55, 24 3.90 -> 3.01, 32 9.33 -> 4.80
-}
-
-static int check_congestion(const SmarlCongestionParams* p) {
-  SMARL_REQUIRE(p != nullptr, "params is NULL");
-  SMARL_REQUIRE(p->size >= 1 && p->size <= 254, "size=%d outside 1..254", p->size);
-  SMARL_REQUIRE(p->demand != nullptr, "demand table is NULL");
-  SMARL_REQUIRE(p->noise_mode >= 0 && p->noise_mode <= 2, "bad noise_mode %d", p->noise_mode);
-  SMARL_REQUIRE(p->keep_threshold <= (1ull << 32), "keep_threshold must be <= 2^32");
-  return SMARL_OK;
 }
 
 #endif

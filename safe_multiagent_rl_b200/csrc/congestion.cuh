@@ -44,6 +44,21 @@ __device__ __forceinline__ void congestion_noise_moves(const uint32_t (&aw)[A], 
   }
 }
 
+// One Congestion transition for four envs (congestion.py:49-75): applies the effective moves,
+// leaves the new positions in xw/yw and the displacement codes in dcw.
+template <int A>
+__device__ __forceinline__ void congestion_transition(uint32_t (&xw)[A], uint32_t (&yw)[A],
+                                                      const uint32_t (&mw)[A], uint32_t (&dcw)[A],
+                                                      uint32_t size4) {
+  const uint32_t k1 = 0x01010101u;
+#pragma unroll
+  for (int i = 0; i < A; ++i) {
+    const uint32_t ox = xw[i], oy = yw[i];
+    grid_move4(xw[i], yw[i], mw[i], size4);
+    dcw[i] = ((xw[i] + k1) - ox) | (((yw[i] + k1) - oy) << 2);
+  }
+}
+
 // 0x01 in every byte of v that is zero (carry-free: the low 7 bits are tested by an add that cannot leave the byte).
 __device__ __forceinline__ uint32_t zero_bytes01(uint32_t v) {
   const uint32_t k7f = 0x7F7F7F7Fu;
@@ -220,6 +235,19 @@ struct CongestionRolloutArgs {
   uint32_t episode;
   const uint32_t* episode_dev;
 };
+
+// CTA size of the fused rollouts that keep the per-agent sums in shared memory (congestion_rollout_kernel and
+// congestion_policy_rollout_kernel): the block summation tree of their stats partials depends on it.
+constexpr int kCongRollThreads = 64;
+
+inline int check_congestion(const SmarlCongestionParams* p) {
+  SMARL_REQUIRE(p != nullptr, "params is NULL");
+  SMARL_REQUIRE(p->size >= 1 && p->size <= 254, "size=%d outside 1..254", p->size);
+  SMARL_REQUIRE(p->demand != nullptr, "demand table is NULL");
+  SMARL_REQUIRE(p->noise_mode >= 0 && p->noise_mode <= 2, "bad noise_mode %d", p->noise_mode);
+  SMARL_REQUIRE(p->keep_threshold <= (1ull << 32), "keep_threshold must be <= 2^32");
+  return SMARL_OK;
+}
 
 // Launchers of noise mode M = 0..2 (congestion.cu, congestion_coop.cu), each mode instantiated in its own translation unit
 template <int M> int launch_congestion_step(int A, const CongestionStepArgs& a, unsigned grid, cudaStream_t s);

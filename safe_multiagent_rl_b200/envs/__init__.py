@@ -1,8 +1,8 @@
 from .base import BatchedEnv, SingleEnvAdapter
 from .collision_avoidance import BatchedCollisionAvoidance
-from .congestion import BatchedCongestion
+from .congestion import BatchedCongestion, BatchedCongestionOnPolicy
 from .coverage import BatchedCoverageDiscrete
 from .coverage_float import BatchedCoverageContinuous, BatchedCoverageDiscretized
 
-__all__ = ["BatchedEnv", "SingleEnvAdapter", "BatchedCoverageDiscrete", "BatchedCongestion",
+__all__ = ["BatchedEnv", "SingleEnvAdapter", "BatchedCoverageDiscrete", "BatchedCongestion", "BatchedCongestionOnPolicy",
            "BatchedCollisionAvoidance", "BatchedCoverageContinuous", "BatchedCoverageDiscretized"]

@@ -244,11 +244,13 @@ class PolicyRollout:
     def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
                        out=None):
         """Whole on-policy episode in one launch: every step samples ``policy`` (a ``FusedGaussianPolicy`` for the
-        continuous envs, a ``FusedDiscretePolicy`` for CoverageDiscrete: its weights, seed and episode) on the current
-        observation, steps the env and accumulates what ``rollout`` returns (CollisionAvoidance's ``n_active``
-        included).  The records and the final state are the bits of the closed loop reset + T x (``policy.act(t=t)``,
-        ``env.step``) (for CoverageDiscrete with the FP32-pipe policy build,
+        continuous envs, a ``FusedDiscretePolicy`` for CoverageDiscrete and Congestion (``BatchedCongestionOnPolicy``):
+        its weights, seed and episode) on the current observation, steps the env and accumulates what ``rollout``
+        returns (CollisionAvoidance's ``n_active`` included).  The records and the final state are the bits of the closed loop reset + T x
+        (``policy.act(t=t)``, ``env.step``) (for the discrete envs with the FP32-pipe policy build,
         ``_lib.kernel_variant(_lib.KERNEL_POLICY, 0)``), the products those of ``rollout`` fed the recorded actions.
+        Congestion draws its action noise as the closed loop does: the call advances the noise episode like ``reset``
+        and ``rollout``, so after ``set_noise_episode(n)`` both draw the noise of episode ``n``.
         The episode index of ``policy`` is not advanced: call ``policy.next_episode()`` for fresh samples.  With
         ``record`` it adds views of the kernel-layout slabs ``obs_`` [T, S, ld], ``actions_`` [T, action_rows, ld]
         (what ``rollout`` takes) and ``logp_`` [T, A, ld]: ``obs`` [T, E, S], ``actions`` [T, A, E, 2] (continuous)

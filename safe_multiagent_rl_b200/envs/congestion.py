@@ -11,7 +11,7 @@ import torch
 
 from .. import _lib
 from ..rollout import G_NONE
-from .base import BatchedEnv
+from .base import BatchedEnv, PolicyRollout
 
 # congestion.py:28 -- the reference's hard-coded table (only valid for size <= 3)
 REFERENCE_DEMAND = np.array([[2, 2, 4, 4], [3, 6, 10, 5], [3, 8, 3, 4], [4, 6, 7, 8]], dtype=np.float64)
@@ -176,3 +176,20 @@ class BatchedCongestion(BatchedEnv):
             _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), E, self.ld, _lib.stream_ptr()))
         self.t = T
         return self._rollout_result(o)
+
+
+class BatchedCongestionOnPolicy(PolicyRollout, BatchedCongestion):
+    """``BatchedCongestion`` that also runs whole on-policy episodes in one launch: ``policy_rollout(policy, T, ...)``
+    with a ``FusedDiscretePolicy`` (``PolicyRollout``, DESIGN.md section 3.14).  Constructor, state, ``reset`` / ``step`` /
+    ``rollout`` and the noise stream are those of ``BatchedCongestion``, whose own interface stays as it was."""
+
+    rollout_policy, reference_policy, rollout_threads = "FusedDiscretePolicy", "DiscretePolicy", "one thread per four envs"
+
+    def _policy_rollout_impl(self, pol, acc, lambdas, rec, o):
+        p = self._params(NOISE_PHILOX if self.noise > 0 else NOISE_NONE)
+        self._next_noise_episode()                 # as rollout(): the same noise as the closed loop after its reset
+        _lib.check(self.lib.smarl_congestion_policy_rollout(
+            C.byref(p), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y), _lib.ptr(lambdas),
+            *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x), _lib.ptr(self.pos_y), _lib.ptr(o["R_"]),
+            _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]), _lib.ptr(o["stats_vec"]),
+            _lib.ptr(o["stats_scratch"]), self.n_envs, self.ld, _lib.stream_ptr()))
