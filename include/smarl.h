@@ -60,7 +60,8 @@ int smarl_device_info(int* sm_count, int* cc_major, int* cc_minor);
  * env_kind is SMARL_ENV_COVERAGE / _CONGESTION / _COLLISION.  With env_kind = SMARL_KERNEL_POLICY the knob picks the
  * build of smarl_policy_act_discrete: -1 = automatic (tensor cores), 0 = FP32 pipes only (packed FFMA2), 1 = fc1 on
  * the tensor cores (tcgen05.mma, accumulators in tensor memory) with groups of up to 16 agents per CTA, 2 = the same
- * with groups of up to 8.  Process-wide; returns the previous setting. */
+ * with groups of up to 8.  smarl_policy_act_discretized has one build (FP32 pipes) and ignores the knob.
+ * Process-wide; returns the previous setting. */
 int smarl_set_kernel_variant(int32_t env_kind, int32_t lanes);
 
 /* Programmatic dependent launch of the per-step kernels (the *_step and policy_act_* entry points): the next step's
@@ -410,6 +411,19 @@ typedef struct {
 int smarl_policy_act_gaussian(const SmarlGaussianPolicy* p, const float* obs, float* actions, float* logp, int32_t t,
                               int64_t n_envs, int64_t ld, smarl_stream_t stream);
 
+/* The DiscretePolicy (agent.py:23-47) of CoverageDiscretized (9 actions, coverage.py:210-241), whose positions are f64
+ * multiples of 1 / zoom rather than u8 cells: the kernel reads the f32 observation rows the reset / step kernels
+ * maintain (as smarl_policy_act_gaussian) and writes the u8 action row the step consumes plus the log-probabilities.
+ *   w1 f32 [A][2A][16] ([in][out]), b1 [A][16], w2 f32 [A][16][9], b2 [A][9]: DEVICE
+ *   obs f32 [2A][ld] in    actions u8 [A][ld] out    logp f32 [A][ld] out (NULL to skip)
+ *   p->n_agents in 1..32, hidden 16, n_actions 9; t in 0..65535; obs, actions and logp 16-byte aligned
+ * Sampling: smarl_policy_act_discrete's Philox stream and inverse-CDF head over the 9 actions
+ * (action = #{c < 8 : sum_{c' <= c} e_c' <= u * sum e}).  One build, all multiply-adds on the FP32 pipes
+ * (smarl_set_kernel_variant(SMARL_KERNEL_POLICY, ...) does not apply): h = b1, then fma(x_k, w1[k], h) for
+ * k = 0..2A-1; logits2 = log2(e) b2, then fma(relu(h_u), log2(e) w2[u], logits2) for u = 0..15. */
+int smarl_policy_act_discretized(const SmarlDiscretePolicy* p, const float* obs, uint8_t* actions, float* logp,
+                                 int32_t t, int64_t n_envs, int64_t ld, smarl_stream_t stream);
+
 /* Whole ON-POLICY CollisionAvoidance episodes in one launch: main.py:28-57 with the policies inside, i.e. per step
  * every agent's ContinuousPolicy (agent.py:48-76) on the current observation, the sample, CollisionAvoidance.step,
  * MetaAgent.act, and Buffer.step + compute_returns as in smarl_collision_rollout.  Bit-identical to the closed loop
@@ -500,6 +514,28 @@ int smarl_congestion_policy_rollout(const SmarlCongestionParams* p, const SmarlD
                                     uint8_t* final_x, uint8_t* final_y, float* R, float* modR, int32_t* C, float* G,
                                     float* g_scratch, double* stats, double* stats_scratch, int64_t n_envs, int64_t ld,
                                     smarl_stream_t stream);
+
+/* Whole ON-POLICY CoverageDiscretized episodes in one launch: main.py:28-57 with the policies inside, i.e. per step
+ * every agent's DiscretePolicy (agent.py:23-47, 9 actions) on the current observation (x0, y0, x1, ...: what the
+ * reset / step kernels write to env.obs), the sample, CoverageDiscretized.step, MetaAgent.act, and Buffer.step +
+ * compute_returns as in smarl_coverage_float_rollout.  Records and final positions are bit-identical to the closed loop
+ * reset + T x (smarl_policy_act_discretized(t) + smarl_coverage_float_step) on the same starts, weights and stream; the
+ * products are bit-identical to smarl_coverage_float_rollout fed the recorded actions (the closed loop's returns kernel
+ * sums the f32-rounded rewards, so its R, modR and stats agree to 1e-5 relative and C is equal).
+ *   p (mode 1), acc, start_x .. lambdas and final_x .. stats_scratch as in smarl_coverage_float_rollout (acc->g_mode 0..2)
+ *   pol: weights, seed, episode, episode_dev and env_offset as in smarl_policy_act_discretized;
+ *        pol->n_agents = p->n_agents, hidden 16, 9 actions
+ *   obs_rec f32 [T][2A][ld] the observation the policy saw at step t      (NULL = skip)
+ *   actions u8  [T][A][ld]  the sampled actions (smarl_coverage_float_rollout's layout; NULL = skip)
+ *   logp    f32 [T][A][ld]  log-probability of the sampled action        (NULL = skip)
+ * A in 1..8 (one thread per env; A >= 9 or mode 0 returns SMARL_EUNSUPPORTED: smarl_coverage_float_policy_rollout
+ * runs mode 0), T in 1..65536 (16 bits of the Philox counter). */
+int smarl_coverage_discretized_policy_rollout(const SmarlCoverageFloatParams* p, const SmarlDiscretePolicy* pol,
+                                              const SmarlAccounting* acc, const double* start_x, const double* start_y,
+                                              const double* lambdas, float* obs_rec, uint8_t* actions, float* logp,
+                                              double* final_x, double* final_y, float* R, float* modR, float* C,
+                                              float* G, float* g_scratch, double* stats, double* stats_scratch,
+                                              int64_t n_envs, int64_t ld, smarl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
  * Multi-GPU: env instances are independent (envs/coverage.py:19, congestion.py:22,

@@ -97,6 +97,7 @@ PROTOTYPES = {
     "smarl_lambda_update": (C.c_int, [c_ptr, c_ptr, c_ptr, f64, i32, i32, c_ptr]),
     "smarl_policy_act_discrete": (C.c_int, [P(DiscretePolicyParams), c_ptr, c_ptr, c_ptr, c_ptr, i32, i64, i64, c_ptr]),
     "smarl_policy_act_gaussian": (C.c_int, [P(GaussianPolicyParams), c_ptr, c_ptr, c_ptr, i32, i64, i64, c_ptr]),
+    "smarl_policy_act_discretized": (C.c_int, [P(DiscretePolicyParams), c_ptr, c_ptr, c_ptr, i32, i64, i64, c_ptr]),
     "smarl_collision_policy_rollout": (C.c_int, [P(CollisionParams), P(GaussianPolicyParams), P(Accounting), c_ptr,
                                                  c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                                  c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, i64, i64, c_ptr]),
@@ -109,6 +110,10 @@ PROTOTYPES = {
     "smarl_congestion_policy_rollout": (C.c_int, [P(CongestionParams), P(DiscretePolicyParams), P(Accounting), c_ptr,
                                                   c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                                   c_ptr, c_ptr, c_ptr, c_ptr, i64, i64, c_ptr]),
+    "smarl_coverage_discretized_policy_rollout": (C.c_int, [P(CoverageFloatParams), P(DiscretePolicyParams),
+                                                            P(Accounting), c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                                            c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                                            c_ptr, i64, i64, c_ptr]),
     "smarl_comm_get_unique_id": (C.c_int, [c_ptr]),
     "smarl_comm_init_from_unique_id": (C.c_int, [P(c_ptr), c_ptr, i32, i32]),
     "smarl_comm_destroy": (None, [c_ptr]),

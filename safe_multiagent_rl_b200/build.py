@@ -34,7 +34,8 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
 # Per-file extras.  collision.cu restates the reference's float64 arithmetic operation by
 # operation, so the compiler must not contract a*b+c into an FMA there.
 EXTRA = {"collision.cu": ["-fmad=false"], "collision_coop.cu": ["-fmad=false"], "collision_policy.cu": ["-fmad=false"],
-         "coverage_float.cu": ["-fmad=false"], "coverage_float_policy.cu": ["-fmad=false"]}
+         "coverage_float.cu": ["-fmad=false"], "coverage_float_policy.cu": ["-fmad=false"],
+         "coverage_discretized_policy.cu": ["-fmad=false"]}
 TU_INDEX = re.compile(r"\bSMARL_TU_IS\((\d+)\)")
 
 

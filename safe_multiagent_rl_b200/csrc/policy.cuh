@@ -31,12 +31,18 @@ struct PolicyArgs {
 // tensor-core build (policy_tc.cu); SMARL_EUNSUPPORTED when the shape does not fit it
 int launch_policy_tc(const PolicyArgs& a, int n_agents, int group_max, int sms, cudaStream_t st);
 
-// The policy checks of the entry points that run the DiscretePolicy (p not NULL) for an env of A agents.
-inline int check_discrete_policy(const SmarlDiscretePolicy* p, int A) {
+// The policy checks of the entry points that run the DiscretePolicy (p not NULL) for an env of A agents and n_actions
+// actions: 5 on the grid envs, 9 on CoverageDiscretized (policy_discretized.cu).
+inline int check_discrete_policy(const SmarlDiscretePolicy* p, int A, int n_actions = kPolActions) {
   SMARL_REQUIRE(p->n_agents == A, "policy has %d agents, the env %d", p->n_agents, A);
-  SMARL_REQUIRE(p->hidden == kPolHidden && p->n_actions == kPolActions,
-                "only the reference's DiscretePolicy shape (hidden 16, 5 actions) is built (got %d, %d)", p->hidden,
-                p->n_actions);
+  if (n_actions == kPolActions)
+    SMARL_REQUIRE(p->hidden == kPolHidden && p->n_actions == kPolActions,
+                  "only the reference's DiscretePolicy shape (hidden 16, 5 actions) is built (got %d, %d)", p->hidden,
+                  p->n_actions);
+  else
+    SMARL_REQUIRE(p->hidden == kPolHidden && p->n_actions == n_actions,
+                  "CoverageDiscretized runs the reference's DiscretePolicy of hidden 16 and %d actions (got %d, %d)",
+                  n_actions, p->hidden, p->n_actions);
   SMARL_REQUIRE(p->w1 && p->b1 && p->w2 && p->b2, "null pointer");
   return SMARL_OK;
 }
@@ -65,17 +71,19 @@ __device__ __forceinline__ float lg2_ftz(float x) {
   return y;
 }
 
-// softmax (agent.py:35), Categorical sample by inverse CDF and log_prob (:44-46) of one agent and env.  The logits
+// softmax (agent.py:35), Categorical sample by inverse CDF and log_prob (:44-46) of one agent and env over NA actions
+// (5 on the grid envs, 9 on CoverageDiscretized; deduced from the logits array).  The logits
 // arrive in log2 units, l2_c = log2(e) * logit_c (both builds scale their shared-memory copies of fc2 by log2(e)), so
 // e_c = exp(logit_c - max) is one subtraction and one MUFU.EX2:
-// u = ((word >> 8) + 0.5) * 2^-24; action = #{c < 4 : sum_{c' <= c} e_c' <= u * sum e}.
-__device__ __forceinline__ void policy_head(const float (&l2)[kPolActions], uint32_t word, int& pick, float& logp) {
+// u = ((word >> 8) + 0.5) * 2^-24; action = #{c < NA - 1 : sum_{c' <= c} e_c' <= u * sum e}.
+template <int NA>
+__device__ __forceinline__ void policy_head(const float (&l2)[NA], uint32_t word, int& pick, float& logp) {
   float m = l2[0];
 #pragma unroll
-  for (int c = 1; c < kPolActions; ++c) m = fmaxf(m, l2[c]);
-  float ex[kPolActions], sum = 0.f;
+  for (int c = 1; c < NA; ++c) m = fmaxf(m, l2[c]);
+  float ex[NA], sum = 0.f;
 #pragma unroll
-  for (int c = 0; c < kPolActions; ++c) {
+  for (int c = 0; c < NA; ++c) {
     ex[c] = ex2_ftz(l2[c] - m);
     sum += ex[c];
   }
@@ -83,7 +91,7 @@ __device__ __forceinline__ void policy_head(const float (&l2)[kPolActions], uint
   float cum = 0.f, l_pick = l2[0];
   pick = 0;
 #pragma unroll
-  for (int c = 0; c < kPolActions - 1; ++c) {
+  for (int c = 0; c < NA - 1; ++c) {
     cum += ex[c];
     if (cum <= target) {
       pick = c + 1;

@@ -244,8 +244,9 @@ class PolicyRollout:
     def policy_rollout(self, policy, n_steps, lambdas=None, gamma=0.99, thresholds=None, g_mode=G_NONE, record=True,
                        out=None):
         """Whole on-policy episode in one launch: every step samples ``policy`` (a ``FusedGaussianPolicy`` for the
-        continuous envs, a ``FusedDiscretePolicy`` for CoverageDiscrete and Congestion (``BatchedCongestionOnPolicy``):
-        its weights, seed and episode) on the current observation, steps the env and accumulates what ``rollout``
+        continuous envs, a ``FusedDiscretePolicy`` for CoverageDiscrete and Congestion (``BatchedCongestionOnPolicy``),
+        a ``FusedDiscretizedPolicy`` for CoverageDiscretized (``BatchedCoverageDiscretizedOnPolicy``): its weights,
+        seed and episode) on the current observation, steps the env and accumulates what ``rollout``
         returns (CollisionAvoidance's ``n_active`` included).  The records and the final state are the bits of the closed loop reset + T x
         (``policy.act(t=t)``, ``env.step``) (for the discrete envs with the FP32-pipe policy build,
         ``_lib.kernel_variant(_lib.KERNEL_POLICY, 0)``), the products those of ``rollout`` fed the recorded actions.

@@ -130,3 +130,19 @@ class BatchedCoverageDiscretized(_CoverageFloat):
         self._params = _lib.CoverageFloatParams(self.size, self.n_agents, 1, 0, float(self.fieldview_size), 0.0,
                                                 float(self.zoom_fac), float(self.size * self.zoom_fac),
                                                 float(table[0]), float(table[1]), _lib.ptr(self._weights))
+
+
+class BatchedCoverageDiscretizedOnPolicy(PolicyRollout, BatchedCoverageDiscretized):
+    """``BatchedCoverageDiscretized`` that also runs whole on-policy episodes in one launch: ``policy_rollout(policy, T,
+    ...)`` with a ``FusedDiscretizedPolicy`` (``PolicyRollout``, DESIGN.md section 3.15).  Constructor, state,
+    ``reset`` / ``step`` / ``rollout`` are those of ``BatchedCoverageDiscretized``, whose own interface stays as it
+    was."""
+
+    rollout_policy, reference_policy, rollout_threads = "FusedDiscretizedPolicy", "DiscretePolicy", "one thread per env"
+
+    def _policy_rollout_impl(self, pol, acc, lambdas, rec, o):
+        _lib.check(self.lib.smarl_coverage_discretized_policy_rollout(
+            C.byref(self._params), C.byref(pol), C.byref(acc), _lib.ptr(self.start_x), _lib.ptr(self.start_y),
+            _lib.ptr(lambdas), *[_lib.ptr(x) for x in rec], _lib.ptr(self.pos_x), _lib.ptr(self.pos_y),
+            _lib.ptr(o["R_"]), _lib.ptr(o["modR_"]), _lib.ptr(o["C_"]), _lib.ptr(o["G_"]), _lib.ptr(o["gs_"]),
+            _lib.ptr(o["stats_vec"]), _lib.ptr(o["stats_scratch"]), self.n_envs, self.ld, _lib.stream_ptr()))

@@ -59,21 +59,14 @@ class BatchedDiscretePolicy(nn.Module):
         return self.dist(obs).log_prob(actions)
 
 
-class FusedDiscretePolicy(BatchedDiscretePolicy):
-    """``BatchedDiscretePolicy`` whose ``act`` is ONE libsmarl kernel (smarl_policy_act_discrete): it reads the env's u8
-    position rows (not the float observation: the env may run with ``emit_obs = False``), evaluates every agent's
-    2A -> 16 -> 5 MLP -- fc1 as tcgen05 tensor-core GEMMs over 256-env tiles with f32-grade accuracy (exact bf16
-    positions x three bf16 pieces per fp32 weight, f32 accumulators in tensor memory), the rest on the FP32 pipes out of
-    tensor memory -- samples the Categorical with a Philox stream keyed by (global env id, episode, step, agent) and
-    writes ``env.action_buffer`` and the log-probabilities: about 7 bytes of HBM traffic per agent-step instead of the
-    [A, E, 16] / [A, E, 5] intermediates of the PyTorch forward.  ``_lib.kernel_variant(_lib.KERNEL_POLICY, 0)`` forces
-    the FP32-pipe build of the kernel.
-    ``log_prob`` / ``dist`` (the differentiable path the learners train through) stay the parent's."""
+class _FusedDiscreteSampler(BatchedDiscretePolicy):
+    """What the fused DiscretePolicy kernels share: the Philox sampling stream (``seed`` and a device episode index),
+    the log-probability row and the ``SmarlDiscretePolicy`` block of the weights.  Subclasses set ``n_actions``, the
+    action count their kernel is built for."""
+
+    n_actions = None
 
     def __init__(self, env, hidden_size=16, seed=0):
-        if hidden_size != 16 or env.action_space != 5 or env.state_space != 2 * env.n_agents:
-            raise NotImplementedError("the fused kernel is built for the reference's DiscretePolicy on the grid envs: "
-                                      "state_space = 2 n_agents, hidden 16, 5 actions")
         super().__init__(env, hidden_size)
         from . import _lib
         self._lib_mod, self.lib = _lib, _lib.load()
@@ -96,8 +89,28 @@ class FusedDiscretePolicy(BatchedDiscretePolicy):
         if (A, S) != (env.n_agents, env.state_space):
             raise ValueError(f"the policy holds {A} agents' networks of {S} inputs; the env has {env.n_agents} agents "
                              f"and {env.state_space} inputs")
-        return L.DiscretePolicyParams(A, 16, 5, 0, L.ptr(w[0]), L.ptr(w[1]), L.ptr(w[2]), L.ptr(w[3]),
+        return L.DiscretePolicyParams(A, 16, self.n_actions, 0, L.ptr(w[0]), L.ptr(w[1]), L.ptr(w[2]), L.ptr(w[3]),
                                       self.seed & (2 ** 64 - 1), env.env_offset, L.ptr(self._episode_dev))
+
+
+class FusedDiscretePolicy(_FusedDiscreteSampler):
+    """``BatchedDiscretePolicy`` whose ``act`` is ONE libsmarl kernel (smarl_policy_act_discrete): it reads the env's u8
+    position rows (not the float observation: the env may run with ``emit_obs = False``), evaluates every agent's
+    2A -> 16 -> 5 MLP -- fc1 as tcgen05 tensor-core GEMMs over 256-env tiles with f32-grade accuracy (exact bf16
+    positions x three bf16 pieces per fp32 weight, f32 accumulators in tensor memory), the rest on the FP32 pipes out of
+    tensor memory -- samples the Categorical with a Philox stream keyed by (global env id, episode, step, agent) and
+    writes ``env.action_buffer`` and the log-probabilities: about 7 bytes of HBM traffic per agent-step instead of the
+    [A, E, 16] / [A, E, 5] intermediates of the PyTorch forward.  ``_lib.kernel_variant(_lib.KERNEL_POLICY, 0)`` forces
+    the FP32-pipe build of the kernel.
+    ``log_prob`` / ``dist`` (the differentiable path the learners train through) stay the parent's."""
+
+    n_actions = 5
+
+    def __init__(self, env, hidden_size=16, seed=0):
+        if hidden_size != 16 or env.action_space != 5 or env.state_space != 2 * env.n_agents:
+            raise NotImplementedError("the fused kernel is built for the reference's DiscretePolicy on the grid envs: "
+                                      "state_space = 2 n_agents, hidden 16, 5 actions")
+        super().__init__(env, hidden_size, seed)
 
     @torch.no_grad()
     def act(self, obs=None, t=None):
@@ -110,6 +123,40 @@ class FusedDiscretePolicy(BatchedDiscretePolicy):
         L.check(self.lib.smarl_policy_act_discrete(C.byref(p), L.ptr(env.pos_x), L.ptr(env.pos_y),
                                                    L.ptr(env.action_buffer), L.ptr(self.logp),
                                                    int(env.t if t is None else t), env.n_envs, env.ld, L.stream_ptr()))
+        E = env.n_envs
+        return env.action_buffer, env.action_buffer[:, :E], self.logp[:, :E]
+
+
+class FusedDiscretizedPolicy(_FusedDiscreteSampler):
+    """``BatchedDiscretePolicy`` on CoverageDiscretized (9 actions) whose ``act`` is ONE libsmarl kernel
+    (smarl_policy_act_discretized): it reads the env's f32 observation rows ``env.obs`` (the positions are float64
+    multiples of 1 / zoom, not u8 cells), evaluates every agent's 2A -> 16 -> 9 MLP on the FP32 pipes with the weights in
+    shared memory, samples the Categorical from ``FusedDiscretePolicy``'s Philox stream (global env id, episode, step,
+    agent) and writes ``env.action_buffer`` and the log-probabilities.  A sibling of ``FusedDiscretePolicy``, not a
+    subclass: each env's ``policy_rollout`` takes exactly one of the two.
+    ``log_prob`` / ``dist`` (the differentiable path the learners train through) stay the parent's."""
+
+    n_actions = 9
+
+    def __init__(self, env, hidden_size=16, seed=0):
+        if (hidden_size != 16 or env.action_space != 9 or env.state_space != 2 * env.n_agents
+                or getattr(env, "obs", None) is None or env.obs.dtype != torch.float32):
+            raise NotImplementedError("the fused kernel is built for the reference's DiscretePolicy on "
+                                      "CoverageDiscretized: state_space = 2 n_agents, hidden 16, 9 actions, f32 "
+                                      "observation rows")
+        super().__init__(env, hidden_size, seed)
+
+    @torch.no_grad()
+    def act(self, obs=None, t=None):
+        """Sample actions for step ``t`` (default: the env's step counter) into ``env.action_buffer``; returns
+        (action_buffer, actions [A, E] uint8 view, log_prob [A, E] view).  ``obs`` is ignored: the kernel reads
+        ``env.obs``."""
+        import ctypes as C
+        env, L = self.env, self._lib_mod
+        p = self.c_params(env)
+        L.check(self.lib.smarl_policy_act_discretized(C.byref(p), L.ptr(env.obs), L.ptr(env.action_buffer),
+                                                      L.ptr(self.logp), int(env.t if t is None else t), env.n_envs,
+                                                      env.ld, L.stream_ptr()))
         E = env.n_envs
         return env.action_buffer, env.action_buffer[:, :E], self.logp[:, :E]
 

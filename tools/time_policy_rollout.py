@@ -1,10 +1,10 @@
 """Time the on-policy episode in one launch (``policy_rollout`` of BatchedCollisionAvoidance, BatchedCoverageContinuous,
-BatchedCoverageDiscrete or BatchedCongestionOnPolicy) against the closed loop it replaces: T x (fused policy act + env.step) + the returns
+BatchedCoverageDiscrete, BatchedCongestionOnPolicy or BatchedCoverageDiscretizedOnPolicy) against the closed loop it replaces: T x (fused policy act + env.step) + the returns
 kernel, replayed from one CUDA graph (for CollisionAvoidance exactly as bench.py's config2_collision_gaussian_graphed
 builds it, for CoverageDiscrete as its config1_graphed.fused).
 
-    python tools/time_policy_rollout.py [--env collision|coverage_continuous|coverage_discrete|congestion] [--iters 20]
-                                        [--rounds 5] [--out FILE]
+    python tools/time_policy_rollout.py [--env collision|coverage_continuous|coverage_discrete|congestion|
+                                               coverage_discretized] [--iters 20] [--rounds 5] [--out FILE]
 
 Shapes: 65 536 envs at 3 agents (BASELINE configs[1] for collision) and 2^20 envs at 3 and 8 agents, size 5, T = 50,
 lambda = 0.1, reward-to-go G.  collision: one landmark, thresholds [2].  coverage_continuous: lambda and threshold 25
@@ -13,6 +13,9 @@ setup at 65 536 x 3, 2^20 x 3 and 2^20 x 8; there --iters rises per shape until 
 --min-window-ms (150 ms).  congestion: the paper's setup (size 3, the reference's demand table, noise 0.1, lambda 0.1,
 threshold 1.5, gamma 0.9, T = 10, reward-to-go G) at 50 x 3, 65 536 x 3 and 2^20 x 3, and bench.py's
 c3_congestion_1M_T100 shape (size 10, 2^20 x 8, T = 100, its seeded demand table); the windows rise as for
+coverage_discrete.  coverage_discretized: the paper's runs (size 5, coarseness 6, lambda 0.1, threshold 25 per agent,
+weights [1, 2, 3] at 3 agents, T = 50, reward-to-go G) at 50 x 3, 65 536 x 3, 2^20 x 3 and 2^20 x 8, the closed loop
+graphed with the PyTorch BatchedDiscretePolicy and with FusedDiscretizedPolicy; the windows rise as for
 coverage_discrete.  A --shapes entry is E x A, or E x A x T x size for congestion.
 The arms alternate within one process, each timed with CUDA events over --iters calls per round; the products of the
 paths are compared on the timed inputs.
@@ -362,17 +365,105 @@ def shape_congestion(E, A, T, size, iters, rounds, min_window_ms):
     return res
 
 
+def shape_coverage_discretized(E, A, T, iters, rounds, min_window_ms):
+    """The paper's CoverageDiscretized runs (size 5, coarseness 6, as tools/sweep.py): weights [1, 2, 3] at 3 agents,
+    lambda 0.1, threshold 25 per agent, gamma 0.999, reward-to-go G.  Closed loops with the PyTorch glue
+    BatchedDiscretePolicy (sampled by torch; its own stream) and with FusedDiscretizedPolicy, whose samples the one
+    launch reproduces bit for bit; the one launch eager, graphed, and graphed without records."""
+    import safe_multiagent_rl_b200 as s
+    from safe_multiagent_rl_b200.policy import BatchedDiscretePolicy, FusedDiscretizedPolicy
+    size, coarseness = 5, 6
+    zoom = coarseness / size
+    starts = np.floor(np.random.default_rng(1).random((E, A, 2)) * size * zoom) / zoom
+    weights = [1.0, 2.0, 3.0] if A == 3 else None
+    mk = lambda cls=s.BatchedCoverageDiscretized: cls(size, A, n_envs=E, coarseness=coarseness, weights=weights,
+                                                      starts=starts)
+    lam = torch.full((A,), 0.1, dtype=torch.float64, device="cuda")
+    thr = torch.full((A,), 25.0, dtype=torch.float64, device="cuda")
+    gamma = 0.999
+    env_g = mk()
+    pol_g = BatchedDiscretePolicy(env_g)
+    loop_g = s.GraphedClosedLoop(env_g, T, lambda obs, t: pol_g.act(obs), lam, gamma, thresholds=[25.0] * A)
+    env_c = mk()
+    pol_c = FusedDiscretizedPolicy(env_c, seed=7)
+    pol_c.load_state_dict(pol_g.state_dict())
+    loop_c = s.GraphedClosedLoop(env_c, T, lambda obs, t: pol_c.act(t=t), lam, gamma, thresholds=[25.0] * A)
+    env_p = mk(s.BatchedCoverageDiscretizedOnPolicy)
+    pol_p = FusedDiscretizedPolicy(env_p, seed=7)
+    pol_p.load_state_dict(pol_g.state_dict())
+    kw = dict(lambdas=lam, gamma=gamma, thresholds=thr, g_mode=1)
+    out = env_p.policy_rollout(pol_p, T, **kw)
+    out_nr = env_p.policy_rollout(pol_p, T, record=False, **kw)
+    torch.cuda.synchronize()
+    graphs = {}
+    for tag, o, rec in (("fused_graphed", out, True), ("fused_graphed_no_record", out_nr, False)):
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            env_p.policy_rollout(pol_p, T, out=o, record=rec, **kw)
+        graphs[tag] = g
+    arms = {"closed_loop_graphed_pytorch_policy": loop_g.replay,
+            "closed_loop_graphed": loop_c.replay,
+            "fused_eager": lambda: env_p.policy_rollout(pol_p, T, out=out, **kw),
+            "fused_graphed": graphs["fused_graphed"].replay,
+            "fused_graphed_no_record": graphs["fused_graphed_no_record"].replay}
+    for fn in arms.values():
+        for _ in range(3):
+            fn()
+    torch.cuda.synchronize()
+    # enough calls per window that even the fastest arm's window lasts min_window_ms
+    iters = max(iters, math.ceil(min_window_ms / min(event_ms(fn, 5) for fn in arms.values())))
+    times = {k: [] for k in arms}
+    for _ in range(rounds):
+        for k, fn in arms.items():
+            times[k].append(event_ms(fn, iters))
+    # the products on the timed inputs: one more call of each path, then the open-loop rollout of the recorded actions
+    ref = loop_c.replay()
+    graphs["fused_graphed"].replay()
+    torch.cuda.synchronize()
+    same = {"final_state": all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                               ((env_p.pos_x, env_c.pos_x), (env_p.pos_y, env_c.pos_y))),
+            "last_step_actions": bool(torch.equal(out["actions_"][T - 1, :, :E], env_c.action_buffer[:, :E])),
+            "last_step_logp": bool(torch.equal(out["logp_"][T - 1, :, :E], pol_c.logp[:, :E])),
+            "C": bool(torch.equal(out["C"], ref["C"]))}
+    fused = {k: out[k].clone() for k in ("R", "modR", "C", "G", "stats_vec")}
+    env_r = mk()
+    open_loop = env_r.rollout(out["actions_"], **kw)
+    torch.cuda.synchronize()
+    same_open = {k: bool(torch.equal(fused[k], open_loop[k])) for k in fused}
+    same_open["final_state"] = all(bool(torch.equal(a[:, :E], b[:, :E])) for a, b in
+                                   ((env_p.pos_x, env_r.pos_x), (env_p.pos_y, env_r.pos_y)))
+
+    def rel(a, b):
+        a, b = a.double(), b.double()
+        return float(((a - b).abs() / b.abs().clamp_min(1e-300)).max())
+    res = {"env": "coverage_discretized", "n_envs": E, "n_agents": A, "T": T, "size": size, "coarseness": coarseness,
+           "iters": iters, "rounds": rounds,
+           "ms_per_batch": {k: {"min": min(v), "median": statistics.median(v), "all": v} for k, v in times.items()},
+           "identical_to_closed_loop": same, "identical_to_open_loop_rollout": same_open,
+           "max_rel_diff_vs_closed_loop": {k: rel(fused[k], ref[k]) for k in ("R", "modR")} |
+                                          {"stats": rel(fused["stats_vec"], ref["stats"].vec)}}
+    m = {k: v["median"] for k, v in res["ms_per_batch"].items()}
+    res["speedup_fused_graphed_vs_pytorch_closed_loop"] = m["closed_loop_graphed_pytorch_policy"] / m["fused_graphed"]
+    res["speedup_fused_graphed_vs_closed_loop"] = m["closed_loop_graphed"] / m["fused_graphed"]
+    del loop_g, loop_c, graphs, out, out_nr
+    torch.cuda.empty_cache()
+    return res
+
+
 SHAPES = {"collision": "65536x3,1048576x3,1048576x8", "coverage_continuous": "65536x3,1048576x3,1048576x8",
           "coverage_discrete": "50x3,65536x3,1048576x3,1048576x8",
+          "coverage_discretized": "50x3,65536x3,1048576x3,1048576x8",
           "congestion": "50x3x10x3,65536x3x10x3,1048576x3x10x3,1048576x8x100x10"}
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--env", choices=tuple(SHAPES), default="collision")
-    ap.add_argument("--iters", type=int, default=20, help="calls per timed window (coverage_discrete, congestion: at least)")
+    ap.add_argument("--iters", type=int, default=20,
+                    help="calls per timed window (coverage_discrete, coverage_discretized, congestion: at least)")
     ap.add_argument("--min-window-ms", type=float, default=150.0,
-                    help="coverage_discrete, congestion: raise the calls per window until the fastest arm's window lasts this long")
+                    help="coverage_discrete, coverage_discretized, congestion: raise the calls per window until the "
+                         "fastest arm's window lasts this long")
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--shapes", default=None, help="ExA list (default: per env)")
     ap.add_argument("--out", default=None, help="also write the JSON lines here")
@@ -380,7 +471,7 @@ def main():
     lines = [json.dumps({"gpu": gpu_info(), "lib": os.path.basename(os.environ.get("SMARL_LIB", "libsmarl.so"))})]
     print(lines[-1], flush=True)
     run = {"collision": shape, "coverage_continuous": shape_coverage, "coverage_discrete": shape_coverage_discrete,
-           "congestion": shape_congestion}[a.env]
+           "coverage_discretized": shape_coverage_discretized, "congestion": shape_congestion}[a.env]
     for sh in (a.shapes or SHAPES[a.env]).split(","):
         dims = [int(x) for x in sh.split("x")]
         if a.env == "congestion":
@@ -388,7 +479,7 @@ def main():
             lines.append(json.dumps(run(E, A, T, size, a.iters, a.rounds, a.min_window_ms)))
         else:
             E, A = dims
-            extra = (a.min_window_ms,) if a.env == "coverage_discrete" else ()
+            extra = (a.min_window_ms,) if a.env in ("coverage_discrete", "coverage_discretized") else ()
             lines.append(json.dumps(run(E, A, 50, a.iters, a.rounds, *extra)))
         print(lines[-1], flush=True)
     if a.out:
