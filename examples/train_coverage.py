@@ -11,7 +11,10 @@ lambda update from the (all-reduced) cost statistics (meta_agent.py:32-39).
 
 --fused: the batch is ONE launch instead (env.policy_rollout with a FusedDiscretePolicy: policies, sampling, steps
 and accounting in one kernel, DESIGN.md section 3.13); the same loss is computed from its records, and
-policy.next_episode() moves the sampling stream on so that the next batch draws fresh samples."""
+policy.next_episode() moves the sampling stream on so that the next batch draws fresh samples.
+
+--fused_grad (with --fused): the loss and its gradients come from ONE kernel too (policy.policy_gradient_loss on the
+records, DESIGN.md section 3.16) instead of T log_prob forwards and an autograd backward; Adam stays torch.optim."""
 import argparse
 import os
 import sys
@@ -23,7 +26,7 @@ import safe_multiagent_rl_b200 as smarl  # noqa: E402
 from safe_multiagent_rl_b200.policy import BatchedDiscretePolicy, FusedDiscretePolicy  # noqa: E402
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--size", type=int, default=5)
     ap.add_argument("--n_agents", type=int, default=3)
@@ -37,7 +40,16 @@ def main():
     ap.add_argument("--thresholds", type=float, nargs="*", default=[25.0, 25.0, 25.0])
     ap.add_argument("--weights", type=float, nargs="*", default=[1.0, 2.0, 3.0])
     ap.add_argument("--fused", action="store_true", help="one launch per batch (env.policy_rollout)")
-    a = ap.parse_args()
+    ap.add_argument("--fused_grad", action="store_true",
+                    help="with --fused: loss and gradients in one launch (policy.policy_gradient_loss)")
+    a = ap.parse_args(argv)
+    if a.fused_grad and not a.fused:
+        ap.error("--fused_grad needs --fused")
+    return a
+
+
+def train(a):
+    """The training loop; returns the policy."""
     torch.manual_seed(0)
     A, E, T = a.n_agents, a.n_envs, a.max_t
     env = smarl.BatchedCoverageDiscrete(a.size, A, n_envs=E, weights=a.weights, shuffle=True, seed=0)
@@ -68,8 +80,11 @@ def main():
             meta.step(out["stats"])
             G = out["G"].permute(0, 2, 1)                                   # [T, A, E] reward-to-go of r - <lambda, c>
             adv = (G - G.mean(dim=2, keepdim=True)) / (G.std(dim=2, keepdim=True) + 1e-6)
-            logp = torch.stack([policy.log_prob(obs_log[t], act_log[t]) for t in range(T)])
-            loss = -(logp * adv).mean()
+            if a.fused_grad:
+                loss = policy.policy_gradient_loss(out, adv)
+            else:
+                logp = torch.stack([policy.log_prob(obs_log[t], act_log[t]) for t in range(T)])
+                loss = -(logp * adv).mean()
             opt.zero_grad()
             loss.backward()
             opt.step()
@@ -81,7 +96,8 @@ def main():
         s, ms, viol = hist.mean_score(n=E)
         print(f"meta {mc}: score {s.round(2)}  cost - thr {[round(float(v), 2) for v in viol]}  "
               f"lambda {meta.lambdas.cpu().numpy().round(3)}")
+    return policy
 
 
 if __name__ == "__main__":
-    main()
+    train(parse_args())

@@ -424,6 +424,34 @@ int smarl_policy_act_gaussian(const SmarlGaussianPolicy* p, const float* obs, fl
 int smarl_policy_act_discretized(const SmarlDiscretePolicy* p, const float* obs, uint8_t* actions, float* logp,
                                  int32_t t, int64_t n_envs, int64_t ld, smarl_stream_t stream);
 
+/* REINFORCE / actor loss of the DiscretePolicy (agent.py:23-47, loss agent.py:134-157) over recorded episodes, and
+ * its gradients with respect to every agent's fc1 / fc2, in one kernel.  For every agent a, step t < n_steps and env
+ * e < n_envs, with x = obs_rec[t][:, e] (2A floats), c = actions[t][a][e] and psi = psi[t][a][e]:
+ *   h = b1 + W1^T x,  r = relu(h),  l = b2 + W2^T r,  p = softmax(l)
+ *   loss += -scale psi log p_c
+ *   g_l = -scale psi (onehot(c) - p);   dW2 += r (x) g_l,  db2 += g_l
+ *   g_h = (W2 g_l) * [h > 0];           dW1 += x (x) g_h,  db1 += g_h   (zero gradient at h == 0, as torch's relu)
+ *   p: n_agents 1..32, hidden 16, n_actions 5 or 9, weights w1 [A][2A][16], b1 [A][16], w2 [A][16][NA], b2 [A][NA]
+ *      (DEVICE; seed, episode, episode_dev and env_offset are ignored)
+ *   obs_rec f32 [T][2A][ld], actions u8 [T][A][ld], psi f32 [T][A][ld]: what the on-policy rollouts record; 16-byte
+ *      aligned.  Only env columns e < n_envs are read.  An action >= NA is a caller error: its sample's contribution is
+ *      unspecified, but nothing is read or written out of bounds.
+ *   dw1, db1, dw2, db2 f32 out, the layouts of the weights (overwritten, not accumulated); loss f64 [1] out (NULL = skip)
+ *   scratch f64 [smarl_policy_grad_scratch_len(A, NA, T, n_envs)], DEVICE, caller-owned (its contents are overwritten)
+ * Deterministic: no floating-point atomics; tile partials are f32 over at most 256 samples, the sums across tiles and
+ * CTAs are f64 in a fixed order, and the number of partials depends on (A, T, n_envs) only, so the result bits depend
+ * on the inputs and the shape, not on the device, the stream or earlier launches.  Computed in f32 with exact expf /
+ * logf; scale is applied in f64 at the end.  A 132-byte memset of the scratch's counters precedes the kernel (both are
+ * stream-ordered and CUDA-graph capturable).  Scratch is 64 + A * P * (32A + 17 NA + 17) doubles with
+ * P = min(T * ceil(n_envs / 256), max(1, 1184 / A)): 11.3 MB at A = 32, NA = 9, T = 50, 2^20 envs.
+ * smarl_policy_grad_scratch_len returns -1 for arguments the entry point rejects (n_agents, n_actions, n_steps,
+ * n_envs < 1). */
+int64_t smarl_policy_grad_scratch_len(int32_t n_agents, int32_t n_actions, int32_t n_steps, int64_t n_envs);
+int smarl_policy_grad_discrete(const SmarlDiscretePolicy* p, const float* obs_rec, const uint8_t* actions,
+                               const float* psi, int32_t n_steps, double scale, float* dw1, float* db1, float* dw2,
+                               float* db2, double* loss, double* scratch, int64_t n_envs, int64_t ld,
+                               smarl_stream_t stream);
+
 /* Whole ON-POLICY CollisionAvoidance episodes in one launch: main.py:28-57 with the policies inside, i.e. per step
  * every agent's ContinuousPolicy (agent.py:48-76) on the current observation, the sample, CollisionAvoidance.step,
  * MetaAgent.act, and Buffer.step + compute_returns as in smarl_collision_rollout.  Bit-identical to the closed loop

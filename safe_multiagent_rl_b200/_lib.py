@@ -98,6 +98,9 @@ PROTOTYPES = {
     "smarl_policy_act_discrete": (C.c_int, [P(DiscretePolicyParams), c_ptr, c_ptr, c_ptr, c_ptr, i32, i64, i64, c_ptr]),
     "smarl_policy_act_gaussian": (C.c_int, [P(GaussianPolicyParams), c_ptr, c_ptr, c_ptr, i32, i64, i64, c_ptr]),
     "smarl_policy_act_discretized": (C.c_int, [P(DiscretePolicyParams), c_ptr, c_ptr, c_ptr, i32, i64, i64, c_ptr]),
+    "smarl_policy_grad_scratch_len": (i64, [i32, i32, i32, i64]),
+    "smarl_policy_grad_discrete": (C.c_int, [P(DiscretePolicyParams), c_ptr, c_ptr, c_ptr, i32, f64, c_ptr, c_ptr,
+                                             c_ptr, c_ptr, c_ptr, c_ptr, i64, i64, c_ptr]),
     "smarl_collision_policy_rollout": (C.c_int, [P(CollisionParams), P(GaussianPolicyParams), P(Accounting), c_ptr,
                                                  c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                                  c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, i64, i64, c_ptr]),

@@ -59,6 +59,29 @@ class BatchedDiscretePolicy(nn.Module):
         return self.dist(obs).log_prob(actions)
 
 
+class _PolicyGradLoss(torch.autograd.Function):
+    """The loss of ``_FusedDiscreteSampler.policy_gradient_loss``: the forward makes the one launch and keeps the
+    gradients, the backward scales them by ``grad_output``."""
+
+    @staticmethod
+    def forward(ctx, w1, b1, w2, b2, call):
+        import ctypes as C
+        pol, obs_, act_, psi, T, scale, scratch = call
+        env, L = pol.env, pol._lib_mod
+        p = pol.c_params(env)
+        grads = [torch.empty_like(w) for w in (w1, b1, w2, b2)]
+        loss = torch.empty((), dtype=torch.float64, device=env.device)
+        L.check(pol.lib.smarl_policy_grad_discrete(C.byref(p), L.ptr(obs_), L.ptr(act_), L.ptr(psi), T, scale,
+                                                   *[L.ptr(g) for g in grads], L.ptr(loss), L.ptr(scratch),
+                                                   env.n_envs, env.ld, L.stream_ptr()))
+        ctx.save_for_backward(*grads)
+        return loss.float()
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        return (*[grad_output * g for g in ctx.saved_tensors], None)
+
+
 class _FusedDiscreteSampler(BatchedDiscretePolicy):
     """What the fused DiscretePolicy kernels share: the Philox sampling stream (``seed`` and a device episode index),
     the log-probability row and the ``SmarlDiscretePolicy`` block of the weights.  Subclasses set ``n_actions``, the
@@ -91,6 +114,49 @@ class _FusedDiscreteSampler(BatchedDiscretePolicy):
                              f"and {env.state_space} inputs")
         return L.DiscretePolicyParams(A, 16, self.n_actions, 0, L.ptr(w[0]), L.ptr(w[1]), L.ptr(w[2]), L.ptr(w[3]),
                                       self.seed & (2 ** 64 - 1), env.env_offset, L.ptr(self._episode_dev))
+
+    def policy_gradient_loss(self, records, psi, scale=None):
+        """The REINFORCE / actor loss ``-(psi * log pi(a|s)).sum() * scale`` (agent.py:134-157) of the episodes a
+        ``policy_rollout`` recorded, as ONE libsmarl kernel (smarl_policy_grad_discrete) that reads the record slabs
+        ``records["obs_"]`` / ``records["actions_"]`` and computes the loss and its gradients with respect to fc1 / fc2
+        at once.  ``psi`` [T, A, E] float32 is the constant advantage (no gradient flows into it); the
+        ``[:, :, :E]`` view of a contiguous [T, A, ld] slab is read in place, anything else is copied into one.
+        ``scale`` defaults to 1 / (T A E), i.e. ``.mean()``.  Returns a 0-dim float32 loss whose ``backward()``
+        accumulates ``grad_output x`` the kernel's gradients into ``fc1`` / ``fc2``'s ``.grad`` as the PyTorch loss
+        does."""
+        env = self.env
+        self.c_params(env)                                # the weights are this env's agent count and input width
+        A, E, ld = env.n_agents, env.n_envs, env.ld
+        obs_, act_ = records.get("obs_"), records.get("actions_")
+        if obs_ is None or act_ is None:
+            raise ValueError("records hold no obs_ / actions_ slabs: call policy_rollout with record=True")
+        T = obs_.shape[0]
+        if (tuple(obs_.shape) != (T, 2 * A, ld) or tuple(act_.shape) != (T, A, ld) or obs_.dtype != torch.float32
+                or act_.dtype != torch.uint8 or not obs_.is_contiguous() or not act_.is_contiguous()):
+            raise ValueError(f"records of shape {tuple(obs_.shape)} / {tuple(act_.shape)} are not those of this env "
+                             f"({A} agents, ld {ld})")
+        if not isinstance(psi, torch.Tensor) or tuple(psi.shape) != (T, A, E) or psi.dtype != torch.float32:
+            raise ValueError(f"psi must be a float32 tensor of shape {(T, A, E)}")
+        if psi.requires_grad:
+            raise ValueError("psi requires grad: it is a constant advantage and the kernel has no gradient for it; "
+                             "pass psi.detach()")
+        if psi.device != env.device:
+            raise ValueError(f"psi is on {psi.device}, the records on {env.device}")
+        if psi.stride() != (A * ld, ld, 1) or psi.data_ptr() % 16:
+            slab = self.__dict__.get("_psi_slab")
+            if slab is None or tuple(slab.shape) != (T, A, ld):
+                slab = self._psi_slab = torch.zeros(T, A, ld, dtype=torch.float32, device=env.device)
+            slab[:, :, :E].copy_(psi)
+            psi = slab
+        scale = 1.0 / (T * A * E) if scale is None else float(scale)
+        n = int(self.lib.smarl_policy_grad_scratch_len(A, self.n_actions, T, E))
+        if n < 0:
+            raise ValueError(f"no policy gradient for {A} agents, {self.n_actions} actions, T = {T}, E = {E}")
+        scratch = self.__dict__.get("_grad_scratch")
+        if scratch is None or scratch.numel() < n:
+            scratch = self._grad_scratch = torch.empty(n, dtype=torch.float64, device=env.device)
+        return _PolicyGradLoss.apply(self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias,
+                                     (self, obs_, act_, psi, T, scale, scratch))
 
 
 class FusedDiscretePolicy(_FusedDiscreteSampler):
