@@ -356,8 +356,10 @@ int smarl_lambda_update(double* lambdas, const double* stats, const double* thre
  * the step consumes plus the f32 log-probability of the sampled action.
  *   w1 f32 [A][2A][16] (fc1.weight transposed: [in][out]), b1 f32 [A][16], w2 f32 [A][16][5], b2 f32 [A][5]: DEVICE
  *   pos_x,pos_y u8 [A][ld] in    actions u8 [A][ld] out    logp f32 [A][ld] out (NULL to skip)
- * Sampling: Philox4x32-10, counter (global env id lo, hi, t | episode << 16, agent >> 2), key seed ^ "PLCY" (hi word):
- * one block serves four consecutive agents, agent a takes word w[a & 3]; u = ((w >> 8) + 0.5) * 2^-24;
+ * Sampling: Philox4x32-10, counter (global env id lo, hi, t | episode << 16, agent >> 2 | (episode >> 16) << 3), key
+ * seed ^ "PLCY" (hi word), episode = p->episode + *p->episode_dev: one block serves four consecutive agents, agent a
+ * takes word w[a & 3]; u = min(fl32((w >> 8) + 0.5) * 2^-24, 1 - 2^-24) (the float32 sum rounds to 2^24 for the top
+ * word; the clamp keeps u * sum below sum, so an action of probability 0 is never drawn);
  * action = #{c < 4 : sum_{c' <= c} e_c' <= u * sum e}, e_c = exp(logit_c - max).
  * Streams depend on the global env id, not on sharding or on the kernel build.  t in 0..65535.
  * Two builds (smarl_set_kernel_variant(SMARL_KERNEL_POLICY, ...)): all multiply-adds on the FP32 pipes, or fc1 as one
@@ -368,7 +370,7 @@ typedef struct {
   int32_t n_agents;        /* A; the observation has 2A components                                   */
   int32_t hidden;          /* 16 (agent.py:24)                                                       */
   int32_t n_actions;       /* 5  (env.action_space of the grid envs)                                 */
-  uint32_t episode;        /* mixed into the Philox counter so that episodes draw independent samples */
+  uint32_t episode;        /* mixed into the Philox counter (all 32 bits) so that episodes draw independent samples */
   const float* w1;
   const float* b1;
   const float* w2;
@@ -387,8 +389,8 @@ int smarl_policy_act_discrete(const SmarlDiscretePolicy* p, const uint8_t* pos_x
  * step / reset kernels maintain and writes the f32 action rows the step consumes plus the log-probabilities.
  *   w1 f32 [A][S][16] ([in][out]), b1 [A][16], w_mu / w_var f32 [A][16][2], b_mu / b_var [A][2]: DEVICE
  *   obs f32 [S][ld] in    actions f32 [2A][ld] out (rows dx0, dy0, dx1, ...)    logp f32 [A][ld] out (NULL to skip)
- * Sampling: Philox4x32-10, counter (global env id lo, hi, t | episode << 16, agent >> 1), key seed ^ "GAUS" (hi word):
- * one block serves two agents, agent a takes w[2 (a & 1)], w[2 (a & 1) + 1]; u_k = ((w_k >> 9) + 0.5) * 2^-23;
+ * Sampling: Philox4x32-10, counter (global env id lo, hi, t | episode << 16, agent >> 1 | (episode >> 16) << 4), key
+ * seed ^ "GAUS" (hi word), episode = p->episode + *p->episode_dev (all 32 bits): one block serves two agents, agent a takes w[2 (a & 1)], w[2 (a & 1) + 1]; u_k = ((w_k >> 9) + 0.5) * 2^-23;
  * Box-Muller r = sqrt(-2 ln u_0), z = (r cos 2 pi u_1, r sin 2 pi u_1); action_k = mu_k + sigma_k z_k;
  * log_prob = -1/2 sum_k ((action_k - mu_k)^2 / sigma_k^2 + ln sigma_k^2) - ln 2 pi.  t in 0..65535. */
 typedef struct {

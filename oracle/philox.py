@@ -104,17 +104,40 @@ def random_starts(kind, size, seed, env_ids, episode, n_rows, zoom=None, row_off
     return xy
 
 
-def policy_uniforms(seed, env_ids, t, n_agents, episode=0):
-    """u [E, A] of smarl_policy_act_discrete: Philox counter (env id lo, hi, t | episode << 16, agent >> 2), key
-    (seed lo, seed hi ^ "PLCY"); agent a takes word a & 3 of its block; u = ((w >> 8) + 0.5) * 2**-24 (the kernel forms
-    it in float32, where k + 0.5 rounds to even for k >= 2**23: off by 2**-25 there, below the margin the tests allow)."""
+def policy_words(seed, env_ids, t, n_agents, episode=0):
+    """uint32 word w [E, A] of the discrete policy stream: Philox counter (env id lo, hi, t | episode << 16,
+    agent >> 2 | (episode >> 16) << 3), key (seed lo, seed hi ^ "PLCY"); agent a takes word a & 3 of its block.  The
+    episode's bits above 16 sit above the agent quad (at most 8 quads for 32 agents), so episode 65 536 does not repeat
+    the stream of episode 0."""
     env_ids = np.asarray(env_ids, dtype=np.uint64)
-    tw = (int(t) | (int(episode) << 16)) & 0xFFFFFFFF
+    episode = int(episode)
+    tw = (int(t) | (episode << 16)) & 0xFFFFFFFF
+    ag = np.arange(n_agents, dtype=np.uint64)
+    c3 = (ag >> np.uint64(2)) | np.uint64(((episode >> 16) << 3) & 0xFFFFFFFF)
     o = philox4x32_10((env_ids & MASK)[:, None], (env_ids >> np.uint64(32))[:, None], np.full((1, 1), tw, dtype=np.uint64),
-                      (np.arange(n_agents, dtype=np.uint64) >> np.uint64(2))[None, :], seed & 0xFFFFFFFF,
-                      ((seed >> 32) & 0xFFFFFFFF) ^ 0x504C4359)
-    w = np.stack(o, axis=0)[np.arange(n_agents) & 3, :, np.arange(n_agents)].T          # [E, A]: word a & 3
-    return ((w >> np.uint32(8)).astype(np.float64) + 0.5) / 16777216.0
+                      c3[None, :], seed & 0xFFFFFFFF, ((seed >> 32) & 0xFFFFFFFF) ^ 0x504C4359)
+    return np.stack(o, axis=0)[np.arange(n_agents) & 3, :, np.arange(n_agents)].T             # [E, A]: word a & 3
+
+
+def policy_uniforms(seed, env_ids, t, n_agents, episode=0):
+    """u [E, A] of smarl_policy_act_discrete in float64: u = ((w >> 8) + 0.5) * 2**-24 of the words of policy_words.
+    The kernel forms u in float32 (policy_uniforms_f32), where k + 0.5 rounds to even for k = w >> 8 >= 2**23: off by
+    2**-25 there, below the margin the tests allow, except at k = 2**24 - 1, where the kernel's u is 1 - 2**-24."""
+    k = policy_words(seed, env_ids, t, n_agents, episode) >> np.uint32(8)
+    return (k.astype(np.float64) + 0.5) / 16777216.0
+
+
+def policy_uniforms_f32(seed, env_ids, t, n_agents, episode=0):
+    """u [E, A] exactly as the kernel's float32 arithmetic forms it: fl(k + 0.5) * 2**-24 (k = w >> 8; k + 0.5 rounds
+    to even for k >= 2**23 and to 2**24 at k = 2**24 - 1), clamped to at most 1 - 2**-24 so that u * sum stays below
+    sum and a zero-probability last action is never drawn."""
+    return policy_u_f32(policy_words(seed, env_ids, t, n_agents, episode) >> np.uint32(8))
+
+
+def policy_u_f32(k):
+    """The kernel's float32 uniform of k = w >> 8 (policy_uniforms_f32)."""
+    u = (np.asarray(k).astype(np.float32) + np.float32(0.5)) * np.float32(2.0 ** -24)
+    return np.minimum(u, np.float32(1.0 - 2.0 ** -24))
 
 
 def policy_sample(logits, u):
@@ -134,22 +157,33 @@ def policy_sample(logits, u):
     return a, logp, margin
 
 
-def gaussian_normals(seed, env_ids, t, n_agents, episode=0):
-    """z [E, A, 2] of smarl_policy_act_gaussian: Philox counter (env id lo, hi, t | episode << 16, agent >> 1), key
-    (seed lo, seed hi ^ "GAUS"); agent a takes words 2 (a & 1), 2 (a & 1) + 1; u = ((w >> 9) + 0.5) * 2**-23 (23 bits:
-    exactly representable in float32, never 0 or 1);
-    Box-Muller r = sqrt(-2 ln u0), z = (r cos 2 pi u1, r sin 2 pi u1) (float64 here)."""
+def gaussian_words(seed, env_ids, t, n_agents, episode=0):
+    """uint32 words (wa, wb), each [E, A], of the Gaussian policy stream: Philox counter (env id lo, hi,
+    t | episode << 16, agent >> 1 | (episode >> 16) << 4), key (seed lo, seed hi ^ "GAUS"); agent a takes words
+    2 (a & 1) and 2 (a & 1) + 1.  The episode's bits above 16 sit above the agent pair (at most 16 pairs for 32 agents),
+    so episode 65 536 does not repeat the stream of episode 0."""
     env_ids = np.asarray(env_ids, dtype=np.uint64)
-    tw = (int(t) | (int(episode) << 16)) & 0xFFFFFFFF
+    episode = int(episode)
+    tw = (int(t) | (episode << 16)) & 0xFFFFFFFF
     ag = np.arange(n_agents)
+    c3 = (ag.astype(np.uint64) >> np.uint64(1)) | np.uint64(((episode >> 16) << 4) & 0xFFFFFFFF)
     o = philox4x32_10((env_ids & MASK)[:, None], (env_ids >> np.uint64(32))[:, None], np.full((1, 1), tw, dtype=np.uint64),
-                      (ag.astype(np.uint64) >> np.uint64(1))[None, :], seed & 0xFFFFFFFF,
-                      ((seed >> 32) & 0xFFFFFFFF) ^ 0x47415553)
+                      c3[None, :], seed & 0xFFFFFFFF, ((seed >> 32) & 0xFFFFFFFF) ^ 0x47415553)
     w = np.stack(o, axis=0)                                                              # [4, E, A]
-    wa = w[2 * (ag & 1), :, ag].T                                                        # [E, A]
-    wb = w[2 * (ag & 1) + 1, :, ag].T
-    u0 = ((wa >> np.uint32(9)).astype(np.float64) + 0.5) / 8388608.0
-    u1 = ((wb >> np.uint32(9)).astype(np.float64) + 0.5) / 8388608.0
+    return w[2 * (ag & 1), :, ag].T, w[2 * (ag & 1) + 1, :, ag].T
+
+
+def gaussian_uniforms(seed, env_ids, t, n_agents, episode=0):
+    """(u0, u1), each [E, A]: u = ((w >> 9) + 0.5) * 2**-23 of the words of gaussian_words (24 significant bits:
+    exact in float32, so the kernel forms the same values; never 0 or 1)."""
+    wa, wb = gaussian_words(seed, env_ids, t, n_agents, episode)
+    return tuple(((w >> np.uint32(9)).astype(np.float64) + 0.5) / 8388608.0 for w in (wa, wb))
+
+
+def gaussian_normals(seed, env_ids, t, n_agents, episode=0):
+    """z [E, A, 2] of smarl_policy_act_gaussian from the uniforms of gaussian_uniforms;
+    Box-Muller r = sqrt(-2 ln u0), z = (r cos 2 pi u1, r sin 2 pi u1) (float64 here)."""
+    u0, u1 = gaussian_uniforms(seed, env_ids, t, n_agents, episode)
     r = np.sqrt(-2.0 * np.log(u0))
     return np.stack([r * np.cos(2.0 * np.pi * u1), r * np.sin(2.0 * np.pi * u1)], axis=-1)
 
@@ -160,3 +194,25 @@ def gaussian_sample(mu, var, z):
     a = mu + np.sqrt(var) * z
     logp = -0.5 * (((a - mu) ** 2 / var) + np.log(var)).sum(axis=-1) - np.log(2.0 * np.pi)
     return a, logp
+
+
+# Global env ids whose policy words sit at the extremes of the uniforms, for seed EDGE_SEED and episode 0, found by a
+# search over the first 2**25 ids (tests/test_policy_sampling_draws.py re-derives every entry; the GPU tests place them
+# inside batches through env_offset).  Entries are (env id, agent, t).
+EDGE_SEED = 77
+# discrete stream (policy_words, 8 agents: both agent quads, every word slot): k = w >> 8
+DISCRETE_TOP = [(14399409, 0, 0), (5068164, 1, 0), (13308236, 2, 0), (11493987, 4, 0), (12665387, 5, 0),
+                (2342586, 7, 0), (16214439, 0, 1), (1484137, 3, 1), (14008471, 5, 1), (28475229, 6, 1)]   # k = 2**24 - 1
+DISCRETE_BOTTOM = [(28550453, 0, 0), (11866442, 2, 0), (2229929, 4, 0), (4043212, 7, 0), (11228756, 1, 1),
+                   (13522544, 3, 1), (7472350, 5, 1), (7714371, 6, 1)]                                     # k = 0
+# (env id, agent, t, j): k = 2**24 - j, the top of the CDF where an action of probability ~1e-6 is drawn
+DISCRETE_NEAR_TOP = [(3983378, 6, 0, 2), (1278034, 7, 1, 4), (179760, 1, 0, 6), (2403015, 2, 1, 8), (2811240, 0, 0, 10),
+                     (6355444, 3, 1, 12), (4532832, 4, 0, 14), (8541136, 5, 1, 17), (1388300, 0, 0, 20),
+                     (1982424, 7, 1, 26), (805129, 5, 0, 32), (169398, 5, 1, 38)]
+# Gaussian stream (gaussian_words, 4 agents: both agent pairs), keyed by the uniform and w >> 9: 0 or 2**23 - 1
+GAUSS_EDGES = {
+    ("u0", 0): [(125380, 0, 0), (2698502, 1, 0), (3012936, 2, 0), (7978842, 3, 0), (7030430, 0, 1), (2871920, 1, 1)],
+    ("u0", 2 ** 23 - 1): [(1246992, 0, 0), (2289924, 1, 0), (12656889, 2, 0), (3390058, 3, 0), (2160676, 3, 1)],
+    ("u1", 0): [(208835, 0, 0), (415691, 1, 0), (16037746, 2, 0), (3081717, 3, 0), (7881140, 0, 1)],
+    ("u1", 2 ** 23 - 1): [(209714, 0, 0), (4525523, 2, 0), (9812806, 3, 0), (8933202, 1, 1)],
+}

@@ -33,7 +33,7 @@ struct CongestionPolicyArgs {
   const float* b2;                      // [A][5]
   uint64_t pol_seed;
   int64_t pol_env_offset;
-  uint32_t pol_t_base;                  // policy episode << 16; *pol_episode_dev << 16 is added on the device
+  uint32_t pol_episode;                 // policy episode; *pol_episode_dev is added on the device
   const uint32_t* pol_episode_dev;
 };
 
@@ -92,7 +92,8 @@ __global__ void __launch_bounds__(kCongRollThreads) congestion_policy_rollout_ke
   for (int k = 0; k < 4; ++k) s_pen[k * kCongRollThreads + tid] = 0.0;
   __syncthreads();                                            // the weights
   const uint2 key = policy_key(p.pol_seed);
-  const uint32_t t_base = p.pol_t_base + ((p.pol_episode_dev ? __ldg(p.pol_episode_dev) : 0u) << 16);
+  const uint32_t pol_episode = p.pol_episode + (p.pol_episode_dev ? __ldg(p.pol_episode_dev) : 0u);
+  const uint32_t t_base = pol_episode << 16, ep_hi = policy_episode_hi(pol_episode);
   const uint64_t id0 = (uint64_t)(p.pol_env_offset + e0);
   int csum[4] = {0, 0, 0, 0};
   double disc = 1.0;
@@ -114,7 +115,7 @@ __global__ void __launch_bounds__(kCongRollThreads) congestion_policy_rollout_ke
     for (int ag = 0; ag < A; ++ag) {
       if ((ag & 3) == 0) {
 #pragma unroll
-        for (int k = 0; k < 4; ++k) words[k] = policy_words(id0 + k, t_word, ag >> 2, key);
+        for (int k = 0; k < 4; ++k) words[k] = policy_words(id0 + k, t_word, ep_hi, ag >> 2, key);
       }
       const float* w1 = s_w1 + ag * Cfg::W1S;
       const float* w2 = s_w2 + ag * Cfg::W2S;
@@ -364,7 +365,7 @@ extern "C" int smarl_congestion_policy_rollout(const SmarlCongestionParams* p, c
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
   k.w1 = pol->w1; k.b1 = pol->b1; k.w2 = pol->w2; k.b2 = pol->b2;
   k.pol_seed = pol->seed; k.pol_env_offset = pol->env_offset;
-  k.pol_t_base = pol->episode << 16; k.pol_episode_dev = pol->episode_dev;
+  k.pol_episode = pol->episode; k.pol_episode_dev = pol->episode_dev;
   const unsigned grid = (unsigned)((r.n_groups + kCongRollThreads - 1) / kCongRollThreads);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = p->noise_mode == 2 ? launch_congestion_policy_rollout<2>(A, k, grid, st)

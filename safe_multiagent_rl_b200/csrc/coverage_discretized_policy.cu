@@ -36,7 +36,7 @@ struct CoverageDiscretizedPolicyArgs {
   const float* b2;                  // [A][9]
   uint64_t seed;
   int64_t env_offset;
-  uint32_t t_base;                  // episode << 16; *episode_dev << 16 is added on the device
+  uint32_t episode;                 // policy episode; *episode_dev is added on the device
   const uint32_t* episode_dev;
 };
 
@@ -72,7 +72,8 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_discretized_policy_roll
     lam[i] = a.lambdas ? __ldg(a.lambdas + i) : 0.0;
   }
   const uint2 key = policy_key(p.seed);
-  const uint32_t t_base = p.t_base + ((p.episode_dev ? __ldg(p.episode_dev) : 0u) << 16);
+  const uint32_t episode = p.episode + (p.episode_dev ? __ldg(p.episode_dev) : 0u);
+  const uint32_t t_base = episode << 16, ep_hi = policy_episode_hi(episode);
   const uint64_t id = (uint64_t)(p.env_offset + e);
   __syncthreads();
 
@@ -96,7 +97,7 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_discretized_policy_roll
     uint4 words;
 #pragma unroll
     for (int ag = 0; ag < A; ++ag) {
-      if ((ag & 3) == 0) words = policy_words(id, t_word, ag >> 2, key);
+      if ((ag & 3) == 0) words = policy_words(id, t_word, ep_hi, ag >> 2, key);
       const float* w1 = s_w1 + ag * W1S;
       const float* w2 = s_w2 + ag * W2S;
       float2 h2[H / 2];
@@ -241,7 +242,7 @@ extern "C" int smarl_coverage_discretized_policy_rollout(const SmarlCoverageFloa
   r.g_mode = acc->g_mode;
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
   k.w1 = pol->w1; k.b1 = pol->b1; k.w2 = pol->w2; k.b2 = pol->b2; k.seed = pol->seed; k.env_offset = pol->env_offset;
-  k.t_base = pol->episode << 16; k.episode_dev = pol->episode_dev;
+  k.episode = pol->episode; k.episode_dev = pol->episode_dev;
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = dispatch<1, kCovDzPolMaxA>(A, [&](auto kA) {

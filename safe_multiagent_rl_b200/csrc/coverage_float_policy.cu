@@ -69,7 +69,8 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_float_policy_rollout_ke
     lam[i] = a.lambdas ? __ldg(a.lambdas + i) : 0.0;
   }
   const uint2 key = make_uint2((uint32_t)p.pol.seed, (uint32_t)(p.pol.seed >> 32) ^ 0x47415553u);   // "GAUS"
-  const uint32_t t_base = (p.pol.episode << 16) + ((p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u) << 16);
+  const uint32_t episode = p.pol.episode + (p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u);
+  const uint32_t t_base = episode << 16, ep_hi = gauss_episode_hi(episode);
   const uint64_t id = (uint64_t)(p.pol.env_offset + e);
   __syncthreads();
 
@@ -92,7 +93,7 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_float_policy_rollout_ke
     const uint32_t t_word = t_base + (uint32_t)t;
 #pragma unroll
     for (int j = 0; j < (A + 1) / 2; ++j) {
-      const uint4 w = philox4x32_10(make_uint4((uint32_t)id, (uint32_t)(id >> 32), t_word, (uint32_t)j), key);
+      const uint4 w = philox4x32_10(make_uint4((uint32_t)id, (uint32_t)(id >> 32), t_word, ep_hi | (uint32_t)j), key);
 #pragma unroll
       for (int h = 0; h < 2 && 2 * j + h < A; ++h) {
         const int ag = 2 * j + h;

@@ -32,7 +32,7 @@ struct CoveragePolicyArgs {
   const float* b2;                      // [A][5]
   uint64_t seed;
   int64_t env_offset;
-  uint32_t t_base;                      // episode << 16; *episode_dev << 16 is added on the device
+  uint32_t episode;                     // policy episode; *episode_dev is added on the device
   const uint32_t* episode_dev;
 };
 
@@ -79,7 +79,8 @@ __global__ void __launch_bounds__(kRolloutThreads) coverage_policy_rollout_kerne
   }
   const uint32_t ge_bias = (uint32_t)(128 - a.size) * 0x01010101u;
   const uint2 key = policy_key(p.seed);
-  const uint32_t t_base = p.t_base + ((p.episode_dev ? __ldg(p.episode_dev) : 0u) << 16);
+  const uint32_t episode = p.episode + (p.episode_dev ? __ldg(p.episode_dev) : 0u);
+  const uint32_t t_base = episode << 16, ep_hi = policy_episode_hi(episode);
   const uint64_t id0 = (uint64_t)(p.env_offset + e0);
   double s_rew[4] = {0, 0, 0, 0}, s_pen[4] = {0, 0, 0, 0};
   double disc = 1.0;
@@ -101,7 +102,7 @@ __global__ void __launch_bounds__(kRolloutThreads) coverage_policy_rollout_kerne
     for (int ag = 0; ag < A; ++ag) {
       if ((ag & 3) == 0) {
 #pragma unroll
-        for (int k = 0; k < 4; ++k) words[k] = policy_words(id0 + k, t_word, ag >> 2, key);
+        for (int k = 0; k < 4; ++k) words[k] = policy_words(id0 + k, t_word, ep_hi, ag >> 2, key);
       }
       const float* w1 = s_w1 + ag * Cfg::W1S;
       const float* w2 = s_w2 + ag * Cfg::W2S;
@@ -321,7 +322,7 @@ extern "C" int smarl_coverage_policy_rollout(const SmarlCoverageParams* p, const
   r.lut_len = p->lut_len; r.n_steps = acc->n_steps; r.g_mode = acc->g_mode;
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
   k.w1 = pol->w1; k.b1 = pol->b1; k.w2 = pol->w2; k.b2 = pol->b2; k.seed = pol->seed; k.env_offset = pol->env_offset;
-  k.t_base = pol->episode << 16; k.episode_dev = pol->episode_dev;
+  k.episode = pol->episode; k.episode_dev = pol->episode_dev;
   const unsigned grid = (unsigned)((r.n_groups + kRolloutThreads - 1) / kRolloutThreads);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = dispatch<1, kCovDiscPolMaxA>(A, [&](auto kA) {

@@ -20,8 +20,8 @@
 // (both conflict-free broadcasts) against 64 FFMA.
 //
 // Sampling (policy.cuh, shared with the tensor-core build): Philox4x32-10 with counter (global env id lo, hi,
-// t | episode << 16, agent >> 2) and key seed ^ "PLCY"; agent a takes word a & 3, u = ((w >> 8) + 0.5) * 2^-24; the
-// action is the inverse CDF of the softmax, a = #{c : sum_{c' <= c} e_c' <= u * sum_c e_c}.  Streams do not depend
+// t | episode << 16, agent >> 2 | (episode >> 16) << 3) and key seed ^ "PLCY"; agent a takes word a & 3,
+// u = min(((w >> 8) + 0.5) * 2^-24, 1 - 2^-24) in float32; the action is the inverse CDF of the softmax, a = #{c : sum_{c' <= c} e_c' <= u * sum_c e_c}.  Streams do not depend
 // on sharding, nor on which of the two builds runs.
 //
 // This file is the FP32-pipe build (all 592 multiply-adds as packed FFMA2, two per issue slot); policy_tc.cu puts fc1
@@ -65,7 +65,8 @@ __global__ void __launch_bounds__(PolCfg<A>::THREADS) policy_act_discrete_kernel
   for (int i = tid; i < A * NA; i += C::THREADS) s_b2[(i / NA) * 8 + i % NA] = __ldg(a.b2 + i) * kLog2e;
   const int ag = tid / QPT, quad = tid % QPT;
   const uint2 key = policy_key(a.seed);
-  const uint32_t t_word = a.t_word + ((a.episode_dev ? __ldg(a.episode_dev) : 0u) << 16);
+  const uint32_t episode = a.episode + (a.episode_dev ? __ldg(a.episode_dev) : 0u);
+  const uint32_t t_word = a.t | episode << 16, ep_hi = policy_episode_hi(episode);
   const float* w1 = s_w1 + ag * C::W1S;
   const float* w2 = s_w2 + ag * C::W2S;
 
@@ -120,7 +121,7 @@ __global__ void __launch_bounds__(PolCfg<A>::THREADS) policy_act_discrete_kernel
         for (int c = 0; c < NA; ++c) l[c] = fmaf(r, w2[u * NA + c], l[c]);
       }
       const uint64_t id = (uint64_t)(a.env_offset + e0 + k);
-      const uint4 o = policy_words(id, t_word, ag >> 2, key);
+      const uint4 o = policy_words(id, t_word, ep_hi, ag >> 2, key);
       int pick;
       policy_head(l, word_of(o, ag & 3), pick, lp[k]);
       act4 |= (uint32_t)pick << (8 * k);
@@ -149,7 +150,7 @@ extern "C" int smarl_policy_act_discrete(const SmarlDiscretePolicy* p, const uin
   PolicyArgs a;
   a.pos_x = pos_x; a.pos_y = pos_y; a.actions = actions; a.logp = logp; a.w1 = p->w1; a.b1 = p->b1; a.w2 = p->w2;
   a.b2 = p->b2; a.seed = p->seed; a.env_offset = p->env_offset; a.n_envs = n_envs; a.ld = ld;
-  a.t_word = (uint32_t)t | (p->episode << 16); a.episode_dev = p->episode_dev;
+  a.t = (uint32_t)t; a.episode = p->episode; a.episode_dev = p->episode_dev;
   int dev = 0, sms = 148;
   SMARL_CUDA(cudaGetDevice(&dev));
   SMARL_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));

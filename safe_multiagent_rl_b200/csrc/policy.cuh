@@ -24,7 +24,8 @@ struct PolicyArgs {
   int64_t n_envs;
   int64_t ld;
   int64_t n_tiles;
-  uint32_t t_word;     // t | episode << 16
+  uint32_t t;
+  uint32_t episode;    // *episode_dev is added on the device
   const uint32_t* episode_dev;
 };
 
@@ -52,10 +53,17 @@ __device__ __forceinline__ uint2 policy_key(uint64_t seed) {
   return make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ 0x504C4359u);   // "PLCY"
 }
 // One Philox block serves four consecutive agents of one env and step: counter (env id lo, hi, t | episode << 16,
-// agent >> 2), agent a uses word a & 3 (oracle/philox.policy_uniforms restates it).
-__device__ __forceinline__ uint4 policy_words(uint64_t env_id, uint32_t t_word, int agent_quad, uint2 key) {
-  return philox4x32_10(make_uint4((uint32_t)env_id, (uint32_t)(env_id >> 32), t_word, (uint32_t)agent_quad), key);
+// agent >> 2 | (episode >> 16) << 3), agent a uses word a & 3 (oracle/philox.policy_words restates it).  The episode's
+// bits above the 16 of the step word sit above the agent quad (8 quads for 32 agents), so the streams of episodes
+// 65 536 apart differ; ep_hi is policy_episode_hi(episode).
+__device__ __forceinline__ uint32_t policy_episode_hi(uint32_t episode) { return (episode >> 16) << 3; }
+__device__ __forceinline__ uint4 policy_words(uint64_t env_id, uint32_t t_word, uint32_t ep_hi, int agent_quad,
+                                              uint2 key) {
+  return philox4x32_10(make_uint4((uint32_t)env_id, (uint32_t)(env_id >> 32), t_word, ep_hi | (uint32_t)agent_quad),
+                       key);
 }
+// The Gaussian stream's counter (policy_gauss.cu) carries the same episode bits above its agent pair (16 pairs).
+__device__ __forceinline__ uint32_t gauss_episode_hi(uint32_t episode) { return (episode >> 16) << 4; }
 __device__ __forceinline__ uint32_t word_of(const uint4& o, int i) {
   return i == 0 ? o.x : (i == 1 ? o.y : (i == 2 ? o.z : o.w));
 }
@@ -75,7 +83,10 @@ __device__ __forceinline__ float lg2_ftz(float x) {
 // (5 on the grid envs, 9 on CoverageDiscretized; deduced from the logits array).  The logits
 // arrive in log2 units, l2_c = log2(e) * logit_c (both builds scale their shared-memory copies of fc2 by log2(e)), so
 // e_c = exp(logit_c - max) is one subtraction and one MUFU.EX2:
-// u = ((word >> 8) + 0.5) * 2^-24; action = #{c < NA - 1 : sum_{c' <= c} e_c' <= u * sum e}.
+// u = min(((word >> 8) + 0.5) * 2^-24, 1 - 2^-24); action = #{c < NA - 1 : sum_{c' <= c} e_c' <= u * sum e}.
+// In float32, (word >> 8) + 0.5 rounds to 2^24 for the top word, so u would be 1 and u * sum == sum would pick the last
+// action whatever its probability; below 1, fl(u * sum) < sum for every sum >= 1, and an action of probability 0
+// (its e_c flushed to 0) is never drawn.
 template <int NA>
 __device__ __forceinline__ void policy_head(const float (&l2)[NA], uint32_t word, int& pick, float& logp) {
   float m = l2[0];
@@ -87,7 +98,7 @@ __device__ __forceinline__ void policy_head(const float (&l2)[NA], uint32_t word
     ex[c] = ex2_ftz(l2[c] - m);
     sum += ex[c];
   }
-  const float target = ((float)(word >> 8) + 0.5f) * (1.0f / 16777216.0f) * sum;
+  const float target = fminf(((float)(word >> 8) + 0.5f) * (1.0f / 16777216.0f), 0x1.fffffep-1f) * sum;
   float cum = 0.f, l_pick = l2[0];
   pick = 0;
 #pragma unroll

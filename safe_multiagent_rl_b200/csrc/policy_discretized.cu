@@ -22,8 +22,9 @@
 // fc2 / b2 are scaled by log2(e) once when they are staged (the logits in log2 units, as policy.cu).
 //
 // Sampling: policy.cu's discrete stream unchanged -- Philox4x32-10, counter (global env id lo, hi, t | episode << 16,
-// agent >> 2), key seed ^ "PLCY", agent a takes word a & 3, u = ((w >> 8) + 0.5) * 2^-24, action = #{c < 8 :
-// sum_{c' <= c} e_c' <= u * sum e} (oracle/philox.policy_uniforms / policy_sample restate it).
+// agent >> 2 | (episode >> 16) << 3), key seed ^ "PLCY", agent a takes word a & 3, u = min(((w >> 8) + 0.5) * 2^-24,
+// 1 - 2^-24) in float32, action = #{c < 8 : sum_{c' <= c} e_c' <= u * sum e} (oracle/philox.policy_uniforms_f32 /
+// policy_sample restate it).
 //
 // One build, the FP32 pipes: a tensor-core fc1 on f32 observations would need a 3 x 3 bf16 piece split, which does not
 // pay at these agent counts (policy_gauss.cu), so smarl_set_kernel_variant(SMARL_KERNEL_POLICY, ...) does not apply.
@@ -49,7 +50,8 @@ struct DiscretizedPolicyArgs {
   int64_t n_envs;
   int64_t ld;
   int64_t n_tiles;
-  uint32_t t_word;     // t | episode << 16
+  uint32_t t;
+  uint32_t episode;    // *episode_dev is added on the device
   const uint32_t* episode_dev;
 };
 
@@ -85,7 +87,8 @@ __global__ void __launch_bounds__(DzCfg<A>::THREADS) policy_act_discretized_kern
   for (int i = tid; i < A * NA; i += C::THREADS) s_b2[(i / NA) * C::B2S + i % NA] = __ldg(a.b2 + i) * kLog2e;
   const int ag = tid / QPT, quad = tid % QPT;
   const uint2 key = policy_key(a.seed);
-  const uint32_t t_word = a.t_word + ((a.episode_dev ? __ldg(a.episode_dev) : 0u) << 16);
+  const uint32_t episode = a.episode + (a.episode_dev ? __ldg(a.episode_dev) : 0u);
+  const uint32_t t_word = a.t | episode << 16, ep_hi = policy_episode_hi(episode);
   const float* w1 = s_w1 + ag * C::W1S;
   const float* w2 = s_w2 + ag * C::W2S;
 
@@ -138,7 +141,7 @@ __global__ void __launch_bounds__(DzCfg<A>::THREADS) policy_act_discretized_kern
         for (int c = 0; c < NA; ++c) l[c] = fmaf(r, w2[u * NA + c], l[c]);
       }
       const uint64_t id = (uint64_t)(a.env_offset + e0 + k);
-      const uint4 o = policy_words(id, t_word, ag >> 2, key);
+      const uint4 o = policy_words(id, t_word, ep_hi, ag >> 2, key);
       int pick;
       policy_head(l, word_of(o, ag & 3), pick, lp[k]);
       act4 |= (uint32_t)pick << (8 * k);
@@ -167,7 +170,7 @@ extern "C" int smarl_policy_act_discretized(const SmarlDiscretePolicy* p, const 
   DiscretizedPolicyArgs a;
   a.obs = obs; a.actions = actions; a.logp = logp; a.w1 = p->w1; a.b1 = p->b1; a.w2 = p->w2; a.b2 = p->b2;
   a.seed = p->seed; a.env_offset = p->env_offset; a.n_envs = n_envs; a.ld = ld;
-  a.t_word = (uint32_t)t | (p->episode << 16); a.episode_dev = p->episode_dev;
+  a.t = (uint32_t)t; a.episode = p->episode; a.episode_dev = p->episode_dev;
   int dev = 0, sms = 148;
   SMARL_CUDA(cudaGetDevice(&dev));
   SMARL_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));

@@ -15,7 +15,8 @@
 // tensor cores, policy_tc.cu, because u8 grid positions are exact in bf16; f32 observations would need a 3 x 3 piece
 // split, and at the agent counts of the continuous envs' configs -- 3 to 8 -- the kernel is not fc1-bound.)
 //
-// Sampling: Philox4x32-10, counter (global env id lo, hi, t | episode << 16, agent >> 1), key seed ^ "GAUS" (hi word):
+// Sampling: Philox4x32-10, counter (global env id lo, hi, t | episode << 16,
+// agent >> 1 | (episode >> 16) << 4), key seed ^ "GAUS" (hi word):
 // one block serves two agents, agent a takes words w[2 (a & 1)], w[2 (a & 1) + 1];  u_k = ((w_k >> 9) + 0.5) * 2^-23
 // (23 bits: exact in f32, never 0 or 1),
 // Box-Muller  r = sqrt(-2 ln u_0), z = (r cos(2 pi u_1), r sin(2 pi u_1)),  action_k = mu_k + sqrt(sigma_k^2) z_k,
@@ -45,7 +46,8 @@ struct GaussArgs {
   int64_t n_envs;
   int64_t ld;
   int64_t n_tiles;
-  uint32_t t_word;
+  uint32_t t;
+  uint32_t episode;    // *episode_dev is added on the device
   const uint32_t* episode_dev;
   int32_t S;
 };
@@ -83,7 +85,8 @@ __global__ void __launch_bounds__(GaussCfg<A>::THREADS) policy_act_gaussian_kern
   for (int i = tid; i < A * 4; i += C::THREADS) s_bh[i] = (i & 3) < 2 ? __ldg(a.b_mu + (i >> 2) * 2 + (i & 3)) : __ldg(a.b_var + (i >> 2) * 2 + (i & 3) - 2);
   const int ag = tid / QPT, quad = tid % QPT;
   const uint2 key = make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32) ^ 0x47415553u);   // "GAUS"
-  const uint32_t t_word = a.t_word + ((a.episode_dev ? __ldg(a.episode_dev) : 0u) << 16);
+  const uint32_t episode = a.episode + (a.episode_dev ? __ldg(a.episode_dev) : 0u);
+  const uint32_t t_word = a.t | episode << 16, ep_hi = gauss_episode_hi(episode);
   const float* w1 = s_w1 + ag * W1S;
   const float* hd = s_hd + ag * C::HS;
 
@@ -135,7 +138,7 @@ __global__ void __launch_bounds__(GaussCfg<A>::THREADS) policy_act_gaussian_kern
       }
       const float v0 = fmaxf(var.x, 0.f) + 1e-4f, v1 = fmaxf(var.y, 0.f) + 1e-4f;      // relu(fc2_) + 1e-4 (:67)
       const uint64_t id = (uint64_t)(a.env_offset + e0 + k);
-      const uint4 o = philox4x32_10(make_uint4((uint32_t)id, (uint32_t)(id >> 32), t_word, (uint32_t)(ag >> 1)), key);
+      const uint4 o = philox4x32_10(make_uint4((uint32_t)id, (uint32_t)(id >> 32), t_word, ep_hi | (uint32_t)(ag >> 1)), key);
       const uint32_t wa = (ag & 1) ? o.z : o.x, wb = (ag & 1) ? o.w : o.y;
       const float u0 = ((float)(wa >> 9) + 0.5f) * (1.0f / 8388608.0f), u1 = ((float)(wb >> 9) + 0.5f) * (1.0f / 8388608.0f);   // exact in f32, in (0, 1)
       const float rad = sqrtf(-2.0f * logf(u0));
@@ -175,7 +178,7 @@ extern "C" int smarl_policy_act_gaussian(const SmarlGaussianPolicy* p, const flo
   GaussArgs a;
   a.obs = obs; a.actions = actions; a.logp = logp; a.w1 = p->w1; a.b1 = p->b1; a.w_mu = p->w_mu; a.b_mu = p->b_mu;
   a.w_var = p->w_var; a.b_var = p->b_var; a.seed = p->seed; a.env_offset = p->env_offset; a.n_envs = n_envs; a.ld = ld;
-  a.t_word = (uint32_t)t | (p->episode << 16); a.episode_dev = p->episode_dev; a.S = p->state_size;
+  a.t = (uint32_t)t; a.episode = p->episode; a.episode_dev = p->episode_dev; a.S = p->state_size;
   int dev = 0, sms = 148;
   SMARL_CUDA(cudaGetDevice(&dev));
   SMARL_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));

@@ -161,7 +161,8 @@ __global__ void __launch_bounds__(TcCfg<A, GMAX, R, RT>::THREADS, TcCfg<A, GMAX,
   const int r_lo = ((tid >> 7) / NWG) * RT;                         // first of this thread's RT tiles
   const uint32_t t_lane = tmem + ((uint32_t)(row & ~31) << 16);     // this warp's 32 TMEM lanes
   const uint2 key = policy_key(a.seed);
-  const uint32_t t_word = a.t_word + ((a.episode_dev ? __ldg(a.episode_dev) : 0u) << 16);
+  const uint32_t episode = a.episode + (a.episode_dev ? __ldg(a.episode_dev) : 0u);
+  const uint32_t t_word = a.t | episode << 16, ep_hi = policy_episode_hi(episode);
   const uint32_t idesc = tc::idesc_bf16_f32(128, N);
   const uint32_t sa_addr = tc::smem_u32(s_a), sb_addr = tc::smem_u32(s_b);
   const int j_lo = wg * AW;                                         // first local agent of this warpgroup
@@ -246,7 +247,8 @@ __global__ void __launch_bounds__(TcCfg<A, GMAX, R, RT>::THREADS, TcCfg<A, GMAX,
     for (int g4 = 0; g4 < (AW + 3) / 4; ++g4)
 #pragma unroll
       for (int r = 0; r < RT; ++r)
-        rnd_all[g4][r] = policy_words((uint64_t)(a.env_offset + e0 + 128 * r), t_word, (a0 + j_lo + 4 * g4) >> 2, key);
+        rnd_all[g4][r] = policy_words((uint64_t)(a.env_offset + e0 + 128 * r), t_word, ep_hi,
+                                       (a0 + j_lo + 4 * g4) >> 2, key);
     tc::mbar_wait(s_bar, phase);
     phase ^= 1u;
     tc::fence_after_sync();
