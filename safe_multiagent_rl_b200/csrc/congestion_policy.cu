@@ -6,17 +6,15 @@
 // One thread owns four consecutive envs, as in congestion_rollout_kernel: the packed u8 positions stay in registers for
 // all T steps, the per-agent f64 discounted sums in the [A][4][threads] shared-memory array, and the CTA has
 // kCongRollThreads threads, so the stats partials come out of the same block summation tree.  Every agent's weights sit
-// in dynamic shared memory after the sums and are read as warp-wide broadcasts.  Per step the thread evaluates the A
-// networks on the joint observation (x0, y0, x1, ...: what the reset / step kernels write to env.obs) in exactly
-// policy_act_discrete_kernel's operation order, as coverage_policy_rollout_kernel does: fc1 as packed FFMA2 from b1,
-// relu, fc2 from log2(e) b2 as packed FFMA2 over env pairs, then policy_head with the same Philox word.  So the actions
-// and log-probabilities are the bits of the FP32-pipe build of smarl_policy_act_discrete.  The env step (noise modes 0
-// and 2) and the accounting are copies of congestion_rollout_kernel's (DESIGN.md section 3.14), compiled with the same
-// flags (contraction on), so the products are the bits of smarl_congestion_rollout fed the recorded actions.
+// in dynamic shared memory after the sums and are read as warp-wide broadcasts.  The policy part is policy.cuh's:
+// stage_discrete_policy, then per step discrete_policy_step4 on the joint observation
+// (x0, y0, x1, ...: what the reset / step kernels write to env.obs), so the actions and log-probabilities are the bits
+// of the FP32-pipe build of smarl_policy_act_discrete.  The env step (noise modes 0 and 2) and the accounting are copies
+// of congestion_rollout_kernel's (DESIGN.md section 3.14), compiled with the same flags (contraction on), so the
+// products are the bits of smarl_congestion_rollout fed the recorded actions.
 #include "congestion.cuh"
 #include "policy.cuh"
 #include "stats.cuh"
-#include "tc.cuh"
 
 namespace smarl {
 
@@ -27,26 +25,16 @@ struct CongestionPolicyArgs {
   float* obs_rec;                       // [T][2A][ld] or NULL
   uint8_t* act_rec;                     // [T][A][ld]  or NULL
   float* logp_rec;                      // [T][A][ld]  or NULL
-  const float* w1;                      // [A][2A][16]
-  const float* b1;                      // [A][16]
-  const float* w2;                      // [A][16][5]
-  const float* b2;                      // [A][5]
-  uint64_t pol_seed;
-  int64_t pol_env_offset;
-  uint32_t pol_episode;                 // policy episode; *pol_episode_dev is added on the device
-  const uint32_t* pol_episode_dev;
+  DiscretePolicyArgs pol;
 };
 
 // Dynamic shared memory: the reward sums [A][4][kCongRollThreads] and penalty sums [4][kCongRollThreads] in f64, then
-// the weights as policy.cu stages them (per-agent strides padded by 4 floats).  The penalty sums live in shared memory
-// too: kept in registers across the policy part they made A = 7 spill.
+// the weights (stage_discrete_policy).  The penalty sums live in shared memory too: kept in registers across the policy
+// part they made A = 7 spill.
 template <int A>
 struct CongPolCfg {
-  static constexpr int IN = 2 * A;
-  static constexpr int W1S = IN * kPolHidden + 4;
-  static constexpr int W2S = kPolHidden * kPolActions + 4;
-  static constexpr int kWeightFloats = A * W1S + A * W2S + A * kPolHidden + A * 8;
-  static constexpr size_t kSmem = sizeof(double) * 4 * kCongRollThreads * (A + 1) + sizeof(float) * kWeightFloats;
+  static constexpr size_t kSmem =
+      sizeof(double) * 4 * kCongRollThreads * (A + 1) + sizeof(float) * PolCfg<A, kPolActions>::kWeightFloats;
 };
 
 // Launcher of noise mode M (0 or 2), each mode instantiated in its own translation unit
@@ -55,21 +43,14 @@ template <int M> int launch_congestion_policy_rollout(int A, const CongestionPol
 #if SMARL_TU_IS(0) || SMARL_TU_IS(1)
 template <int A, int MODE>
 __global__ void __launch_bounds__(kCongRollThreads) congestion_policy_rollout_kernel(const CongestionPolicyArgs p) {
-  using Cfg = CongPolCfg<A>;
-  constexpr int IN = Cfg::IN, H = kPolHidden, NA = kPolActions;
+  constexpr int IN = 2 * A;
   extern __shared__ __align__(16) double s_acc[];             // [A][4][kCongRollThreads]
   __shared__ double s_red[kCongRollThreads / 32];
   double* s_pen = s_acc + 4 * kCongRollThreads * A;           // [4][kCongRollThreads]
-  float* s_w1 = reinterpret_cast<float*>(s_pen + 4 * kCongRollThreads);       // [A][W1S]  w1[a][k][u]
-  float* s_w2 = s_w1 + A * Cfg::W1S;                          // [A][W2S]  log2(e) w2[a][u][c]
-  float* s_b1 = s_w2 + A * Cfg::W2S;                          // [A][16]
-  float* s_b2 = s_b1 + A * H;                                 // [A][8]    log2(e) b2[a][c]
+  float* s_w = reinterpret_cast<float*>(s_pen + 4 * kCongRollThreads);
   const CongestionRolloutArgs& a = p.r;
   const int tid = threadIdx.x;
-  for (int i = tid; i < A * IN * H; i += kCongRollThreads) s_w1[(i / (IN * H)) * Cfg::W1S + i % (IN * H)] = __ldg(p.w1 + i);
-  for (int i = tid; i < A * H * NA; i += kCongRollThreads) s_w2[(i / (H * NA)) * Cfg::W2S + i % (H * NA)] = __ldg(p.w2 + i) * kLog2e;
-  for (int i = tid; i < A * H; i += kCongRollThreads) s_b1[i] = __ldg(p.b1 + i);
-  for (int i = tid; i < A * NA; i += kCongRollThreads) s_b2[(i / NA) * 8 + i % NA] = __ldg(p.b2 + i) * kLog2e;
+  stage_discrete_policy<A, kPolActions, kCongRollThreads>(s_w, p.pol, tid);
   const int64_t g = (int64_t)blockIdx.x * kCongRollThreads + tid;
   const bool live = g < a.n_groups;
   const int64_t e0 = (live ? g : 0) * 4;
@@ -91,10 +72,10 @@ __global__ void __launch_bounds__(kCongRollThreads) congestion_policy_rollout_ke
 #pragma unroll
   for (int k = 0; k < 4; ++k) s_pen[k * kCongRollThreads + tid] = 0.0;
   __syncthreads();                                            // the weights
-  const uint2 key = policy_key(p.pol_seed);
-  const uint32_t pol_episode = p.pol_episode + (p.pol_episode_dev ? __ldg(p.pol_episode_dev) : 0u);
-  const uint32_t t_base = pol_episode << 16, ep_hi = policy_episode_hi(pol_episode);
-  const uint64_t id0 = (uint64_t)(p.pol_env_offset + e0);
+  const uint2 key = policy_key(p.pol.seed);
+  const uint32_t policy_episode = p.pol.episode + (p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u);
+  const uint32_t t_base = policy_episode << 16, ep_hi = policy_episode_hi(policy_episode);
+  const uint64_t id0 = (uint64_t)(p.pol.env_offset + e0);
   int csum[4] = {0, 0, 0, 0};
   double disc = 1.0;
 
@@ -107,73 +88,10 @@ __global__ void __launch_bounds__(kCongRollThreads) congestion_policy_rollout_ke
         st_stream_f4(o + (2 * i + 1) * ld, bytes_to_float4(yw[i]));
       }
     }
-    // every agent's policy (agent.py:33-46); one Philox block serves four consecutive agents of an env
-    const uint32_t t_word = t_base + (uint32_t)t;
+    // every agent's policy (agent.py:33-46)
     uint32_t aw[A];
-    uint4 words[4];
-#pragma unroll
-    for (int ag = 0; ag < A; ++ag) {
-      if ((ag & 3) == 0) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) words[k] = policy_words(id0 + k, t_word, ep_hi, ag >> 2, key);
-      }
-      const float* w1 = s_w1 + ag * Cfg::W1S;
-      const float* w2 = s_w2 + ag * Cfg::W2S;
-      float2 h2[4][H / 2];
-#pragma unroll
-      for (int q = 0; q < H / 2; ++q) {
-        const float2 b = *reinterpret_cast<const float2*>(s_b1 + ag * H + 2 * q);
-        h2[0][q] = h2[1][q] = h2[2][q] = h2[3][q] = b;
-      }
-#pragma unroll
-      for (int k = 0; k < IN; ++k) {
-        const float4 x = bytes_to_float4((k & 1) ? yw[k >> 1] : xw[k >> 1]);
-        const float2 xx[4] = {make_float2(x.x, x.x), make_float2(x.y, x.y), make_float2(x.z, x.z), make_float2(x.w, x.w)};
-        const float4* wr = reinterpret_cast<const float4*>(w1 + k * H);
-#pragma unroll
-        for (int v = 0; v < H / 4; ++v) {
-          const float4 w = wr[v];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            h2[e][2 * v] = tc::ffma2(xx[e], make_float2(w.x, w.y), h2[e][2 * v]);
-            h2[e][2 * v + 1] = tc::ffma2(xx[e], make_float2(w.z, w.w), h2[e][2 * v + 1]);
-          }
-        }
-      }
-      // fc2 as packed FFMA2 over the env pairs (0, 1) and (2, 3): per env the fmaf chain over u = 0..15 of policy.cu
-      float2 l2[2][NA];
-#pragma unroll
-      for (int c = 0; c < NA; ++c) l2[0][c] = l2[1][c] = make_float2(s_b2[ag * 8 + c], s_b2[ag * 8 + c]);
-#pragma unroll
-      for (int u = 0; u < H; ++u) {
-        float r[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) r[e] = fmaxf((u & 1) ? h2[e][u >> 1].y : h2[e][u >> 1].x, 0.f);
-        const float2 r01 = make_float2(r[0], r[1]), r23 = make_float2(r[2], r[3]);
-#pragma unroll
-        for (int c = 0; c < NA; ++c) {
-          const float w = w2[u * NA + c];
-          l2[0][c] = tc::ffma2(r01, make_float2(w, w), l2[0][c]);
-          l2[1][c] = tc::ffma2(r23, make_float2(w, w), l2[1][c]);
-        }
-      }
-      uint32_t act4 = 0u;
-      float lp[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        float l[NA];
-#pragma unroll
-        for (int c = 0; c < NA; ++c) l[c] = (k & 1) ? l2[k >> 1][c].y : l2[k >> 1][c].x;
-        int pick;
-        policy_head(l, word_of(words[k], ag & 3), pick, lp[k]);
-        act4 |= (uint32_t)pick << (8 * k);
-      }
-      aw[ag] = act4;
-      if (live) {
-        if (p.act_rec) st_stream_u32(p.act_rec + ((int64_t)t * A + ag) * ld + e0, act4);
-        if (p.logp_rec) st_stream_f4(p.logp_rec + ((int64_t)t * A + ag) * ld + e0, make_float4(lp[0], lp[1], lp[2], lp[3]));
-      }
-    }
+    discrete_policy_step4<A>(xw, yw, s_w, key, id0, t_base + (uint32_t)t, ep_hi, aw, p.act_rec, p.logp_rec, live, t, ld,
+                             e0);
     // the env step and the accounting, exactly as congestion_rollout_kernel
     uint32_t mw[A];
     if (MODE == 0) {
@@ -363,9 +281,7 @@ extern "C" int smarl_congestion_policy_rollout(const SmarlCongestionParams* p, c
   r.size = p->size; r.n_steps = acc->n_steps; r.g_mode = acc->g_mode;
   r.episode = p->episode; r.episode_dev = p->episode_dev;
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
-  k.w1 = pol->w1; k.b1 = pol->b1; k.w2 = pol->w2; k.b2 = pol->b2;
-  k.pol_seed = pol->seed; k.pol_env_offset = pol->env_offset;
-  k.pol_episode = pol->episode; k.pol_episode_dev = pol->episode_dev;
+  k.pol = discrete_policy_args(pol);
   const unsigned grid = (unsigned)((r.n_groups + kCongRollThreads - 1) / kCongRollThreads);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = p->noise_mode == 2 ? launch_congestion_policy_rollout<2>(A, k, grid, st)

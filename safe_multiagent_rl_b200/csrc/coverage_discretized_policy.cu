@@ -7,14 +7,15 @@
 // One thread owns one env, as in coverage_float_rollout_kernel: the f64 positions, cost sums and discounted sums stay in
 // registers for all T steps, every agent's weights sit in static shared memory and are read as warp-wide broadcasts.
 // Per step the thread builds the f32 observation (x_i, y_i: what the reset / step kernels write to env.obs), evaluates
-// the A networks in policy_discretized.cu's operation order (fc1 as packed FFMA2 from b1 over k = 0..2A-1, relu, fc2 as
-// an fmaf chain over u = 0..15 from log2(e) b2), samples each with policy_head<9> on the shared Philox word, steps the
-// env with coverage_float_env_step_regs<A, 1> and accumulates R / modR / C / G / stats exactly as
-// coverage_float_rollout_kernel does.  Compiled with -fmad=false like coverage_float.cu: every multiply-add the
-// contraction-on policy kernel fuses is an explicit fmaf / ffma2 here.
+// the A networks in the operation order of policy.cuh's policy_act_discrete_kernel<A, 9> (fc1 as packed FFMA2 from b1
+// over k = 0..2A-1, relu, fc2 as an fmaf chain over u = 0..15 from log2(e) b2), samples each with policy_head<9> on the
+// shared Philox word, steps the env with coverage_float_env_step_regs<A, 1> and accumulates R / modR / C / G / stats
+// exactly as coverage_float_rollout_kernel does.  Compiled with -fmad=false like coverage_float.cu: every multiply-add
+// the contraction-on policy kernel fuses is an explicit fmaf / ffma2 here.
 //
-// The accounting is a copy of coverage_float_rollout_kernel's (as in coverage_float_policy.cu): moving it into a shared
-// function changed the SASS of the kernel it came from (DESIGN.md section 3.12).
+// Only the policy arguments (DiscretePolicyArgs) are shared with the other on-policy rollouts; the one-env network is
+// this kernel's own, and the accounting is a copy of coverage_float_rollout_kernel's (as in coverage_float_policy.cu):
+// moving it into a shared function changed the SASS of the kernel it came from (DESIGN.md section 3.12).
 #include "coverage_float.cuh"
 #include "policy.cuh"
 #include "stats.cuh"
@@ -23,21 +24,13 @@
 namespace smarl {
 
 constexpr int kCovDzPolMaxA = 8;    // one thread per env: the A networks' registers
-constexpr int kDzActions = 9;
 
 struct CoverageDiscretizedPolicyArgs {
   CoverageFloatRolloutArgs r;       // r.env.pos_x / pos_y = start positions, r.env.actions unused
   float* obs_rec;                   // [T][2A][ld] or NULL
   uint8_t* act_rec;                 // [T][A][ld]  or NULL
   float* logp_rec;                  // [T][A][ld]  or NULL
-  const float* w1;                  // [A][2A][16]
-  const float* b1;                  // [A][16]
-  const float* w2;                  // [A][16][9]
-  const float* b2;                  // [A][9]
-  uint64_t seed;
-  int64_t env_offset;
-  uint32_t episode;                 // policy episode; *episode_dev is added on the device
-  const uint32_t* episode_dev;
+  DiscretePolicyArgs pol;
 };
 
 // kCovFThreads threads per CTA keep coverage_float_rollout_kernel's summation tree of the stats partials (one row per
@@ -46,17 +39,17 @@ struct CoverageDiscretizedPolicyArgs {
 template <int A>
 __global__ void __launch_bounds__(kCovFThreads) coverage_discretized_policy_rollout_kernel(
     const CoverageDiscretizedPolicyArgs p) {
-  constexpr int S = 2 * A, H = kPolHidden, NA = kDzActions, W1S = S * H + H, W2S = H * NA + NA;
+  constexpr int S = 2 * A, H = kPolHidden, NA = kDiscretizedActions, W1S = S * H + H, W2S = H * NA + NA;
   __shared__ __align__(16) float s_w1[A * W1S];        // [A][W1S]: w1[a][k][u], then b1[a][u]
   __shared__ float s_w2[A * W2S];                      // [A][W2S]: log2(e) w2[a][u][c], then log2(e) b2[a][c]
   __shared__ double s_red[kCovFThreads / 32];
   const CoverageFloatRolloutArgs& r = p.r;
   const CoverageFloatArgs& a = r.env;
   const int tid = threadIdx.x;
-  for (int i = tid; i < A * S * H; i += kCovFThreads) s_w1[(i / (S * H)) * W1S + i % (S * H)] = __ldg(p.w1 + i);
-  for (int i = tid; i < A * H; i += kCovFThreads) s_w1[(i / H) * W1S + S * H + i % H] = __ldg(p.b1 + i);
-  for (int i = tid; i < A * H * NA; i += kCovFThreads) s_w2[(i / (H * NA)) * W2S + i % (H * NA)] = __ldg(p.w2 + i) * kLog2e;
-  for (int i = tid; i < A * NA; i += kCovFThreads) s_w2[(i / NA) * W2S + H * NA + i % NA] = __ldg(p.b2 + i) * kLog2e;
+  for (int i = tid; i < A * S * H; i += kCovFThreads) s_w1[(i / (S * H)) * W1S + i % (S * H)] = __ldg(p.pol.w1 + i);
+  for (int i = tid; i < A * H; i += kCovFThreads) s_w1[(i / H) * W1S + S * H + i % H] = __ldg(p.pol.b1 + i);
+  for (int i = tid; i < A * H * NA; i += kCovFThreads) s_w2[(i / (H * NA)) * W2S + i % (H * NA)] = __ldg(p.pol.w2 + i) * kLog2e;
+  for (int i = tid; i < A * NA; i += kCovFThreads) s_w2[(i / NA) * W2S + H * NA + i % NA] = __ldg(p.pol.b2 + i) * kLog2e;
 
   const int64_t eg = (int64_t)blockIdx.x * kCovFThreads + tid;
   const bool live = eg < a.n_envs;                     // lanes past n_envs replay env 0 and store nothing
@@ -71,10 +64,10 @@ __global__ void __launch_bounds__(kCovFThreads) coverage_discretized_policy_roll
     csum[i] = 0.0;
     lam[i] = a.lambdas ? __ldg(a.lambdas + i) : 0.0;
   }
-  const uint2 key = policy_key(p.seed);
-  const uint32_t episode = p.episode + (p.episode_dev ? __ldg(p.episode_dev) : 0u);
+  const uint2 key = policy_key(p.pol.seed);
+  const uint32_t episode = p.pol.episode + (p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u);
   const uint32_t t_base = episode << 16, ep_hi = policy_episode_hi(episode);
-  const uint64_t id = (uint64_t)(p.env_offset + e);
+  const uint64_t id = (uint64_t)(p.pol.env_offset + e);
   __syncthreads();
 
   double s_rew = 0.0, s_pen = 0.0, disc = 1.0;
@@ -229,7 +222,7 @@ extern "C" int smarl_coverage_discretized_policy_rollout(const SmarlCoverageFloa
   if (int rc = check_layout(n_envs, ld)) return rc;
   if (int rc = check_accounting(acc, 65536, 2, G, stats, stats_scratch)) return rc;   // 16 bits of the Philox counter
   const int A = p->n_agents;
-  if (int rc = check_discrete_policy(pol, A, kDzActions)) return rc;
+  if (int rc = check_discrete_policy(pol, A, kDiscretizedActions)) return rc;
   SMARL_REQUIRE(start_x && start_y && R && modR && C, "null required pointer");
   SMARL_REQUIRE(acc->g_mode != 1 || g_scratch, "g_mode 1 needs g_scratch [2][T][ld]");
   CoverageDiscretizedPolicyArgs k;
@@ -241,8 +234,7 @@ extern "C" int smarl_coverage_discretized_policy_rollout(const SmarlCoverageFloa
   r.partials = stats_scratch; r.thresholds = acc->thresholds; r.gamma = acc->gamma; r.n_steps = acc->n_steps;
   r.g_mode = acc->g_mode;
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
-  k.w1 = pol->w1; k.b1 = pol->b1; k.w2 = pol->w2; k.b2 = pol->b2; k.seed = pol->seed; k.env_offset = pol->env_offset;
-  k.episode = pol->episode; k.episode_dev = pol->episode_dev;
+  k.pol = discrete_policy_args(pol);
   const unsigned grid = (unsigned)((n_envs + kCovFThreads - 1) / kCovFThreads);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = dispatch<1, kCovDzPolMaxA>(A, [&](auto kA) {

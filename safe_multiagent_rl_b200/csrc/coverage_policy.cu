@@ -5,13 +5,16 @@
 //
 // One thread owns four consecutive envs, as in coverage_rollout_kernel: the packed u8 positions, the byte cost counters
 // and the discounted sums stay in registers for all T steps.  Every agent's weights sit in shared memory beside the
-// penalty table and are read as warp-wide broadcasts.  Per step the thread evaluates the A networks on the joint
-// observation (x0, y0, x1, ...: what the reset / step kernels write to env.obs) in exactly policy_act_discrete_kernel's
-// operation order: fc1 as packed FFMA2 from b1 over the inputs k = 0..2A-1, relu, fc2 from log2(e) b2 over the 16
-// hidden units (packed FFMA2 over env pairs: per env policy.cu's fmaf chain), then policy_head with the same Philox
-// word.  So the actions and log-probabilities are the bits of the FP32-pipe build of smarl_policy_act_discrete.  The
-// env step and the accounting are copies of coverage_rollout_kernel's (DESIGN.md section 3.13), compiled with the same
-// flags (contraction on), so the products are the bits of smarl_coverage_rollout fed the recorded actions.
+// penalty table and are read as warp-wide broadcasts; they are staged by policy.cuh's stage_discrete_policy.  Per step the
+// thread evaluates the A networks on the joint observation (x0, y0, x1, ...: what the reset / step kernels write to
+// env.obs) in exactly policy_act_discrete_kernel's operation order: fc1 as packed FFMA2 from b1 over the inputs
+// k = 0..2A-1, relu, fc2 from log2(e) b2 over the 16 hidden units (packed FFMA2 over env pairs: per env policy.cu's fmaf
+// chain), then policy_head with the same Philox word.  So the actions and log-probabilities are the bits of the
+// FP32-pipe build of smarl_policy_act_discrete.  That per-step loop is a copy of policy.cuh's discrete_policy_step4,
+// which congestion_policy.cu calls: calling it here made the one launch without records 4.7 % slower on a B200 at
+// 50 envs x 3 agents (DESIGN.md section 3.13).  The env step and the accounting are copies of coverage_rollout_kernel's,
+// compiled with the same flags (contraction on), so the products are the bits of smarl_coverage_rollout fed the recorded
+// actions.
 #include "coverage.cuh"
 #include "policy.cuh"
 #include "stats.cuh"
@@ -26,41 +29,22 @@ struct CoveragePolicyArgs {
   float* obs_rec;                       // [T][2A][ld] or NULL
   uint8_t* act_rec;                     // [T][A][ld]  or NULL
   float* logp_rec;                      // [T][A][ld]  or NULL
-  const float* w1;                      // [A][2A][16]
-  const float* b1;                      // [A][16]
-  const float* w2;                      // [A][16][5]
-  const float* b2;                      // [A][5]
-  uint64_t seed;
-  int64_t env_offset;
-  uint32_t episode;                     // policy episode; *episode_dev is added on the device
-  const uint32_t* episode_dev;
-};
-
-// Dynamic shared memory: the weights as policy.cu stages them (per-agent strides padded by 4 floats), then the table.
-template <int A>
-struct CovPolCfg {
-  static constexpr int IN = 2 * A;
-  static constexpr int W1S = IN * kPolHidden + 4;
-  static constexpr int W2S = kPolHidden * kPolActions + 4;
-  static constexpr int kWeightFloats = A * W1S + A * W2S + A * kPolHidden + A * 8;
+  DiscretePolicyArgs pol;
 };
 
 template <int A>
 __global__ void __launch_bounds__(kRolloutThreads) coverage_policy_rollout_kernel(const CoveragePolicyArgs p) {
-  using Cfg = CovPolCfg<A>;
+  using Cfg = PolCfg<A, kPolActions>;
   constexpr int IN = Cfg::IN, H = kPolHidden, NA = kPolActions;
   extern __shared__ __align__(16) float s_mem[];
-  float* s_w1 = s_mem;                               // [A][W1S]  w1[a][k][u]
-  float* s_w2 = s_w1 + A * Cfg::W1S;                 // [A][W2S]  log2(e) w2[a][u][c]
-  float* s_b1 = s_w2 + A * Cfg::W2S;                 // [A][16]
-  float* s_b2 = s_b1 + A * H;                        // [A][8]    log2(e) b2[a][c]
-  float* s_lut = s_b2 + A * 8;
+  const float* s_w1 = s_mem;                         // [A][W1S]  w1[a][k][u]
+  const float* s_w2 = s_w1 + A * Cfg::W1S;           // [A][W2S]  log2(e) w2[a][u][c]
+  const float* s_b1 = s_w2 + A * Cfg::W2S;           // [A][16]
+  const float* s_b2 = s_b1 + A * H;                  // [A][8]    log2(e) b2[a][c]
+  float* s_lut = s_mem + Cfg::kWeightFloats;
   const CoverageRolloutArgs& a = p.r;
   const int tid = threadIdx.x;
-  for (int i = tid; i < A * IN * H; i += kRolloutThreads) s_w1[(i / (IN * H)) * Cfg::W1S + i % (IN * H)] = __ldg(p.w1 + i);
-  for (int i = tid; i < A * H * NA; i += kRolloutThreads) s_w2[(i / (H * NA)) * Cfg::W2S + i % (H * NA)] = __ldg(p.w2 + i) * kLog2e;
-  for (int i = tid; i < A * H; i += kRolloutThreads) s_b1[i] = __ldg(p.b1 + i);
-  for (int i = tid; i < A * NA; i += kRolloutThreads) s_b2[(i / NA) * 8 + i % NA] = __ldg(p.b2 + i) * kLog2e;
+  stage_discrete_policy<A, kPolActions, kRolloutThreads>(s_mem, p.pol, tid);
   coverage_load_lut(s_lut, a.lut, a.lut_len);       // its barrier also covers the weights
   const int64_t g = (int64_t)blockIdx.x * kRolloutThreads + tid;
   const bool live = g < a.n_groups;
@@ -78,10 +62,10 @@ __global__ void __launch_bounds__(kRolloutThreads) coverage_policy_rollout_kerne
     lam[i] = a.lambdas ? __ldg(a.lambdas + i) : 0.0;
   }
   const uint32_t ge_bias = (uint32_t)(128 - a.size) * 0x01010101u;
-  const uint2 key = policy_key(p.seed);
-  const uint32_t episode = p.episode + (p.episode_dev ? __ldg(p.episode_dev) : 0u);
+  const uint2 key = policy_key(p.pol.seed);
+  const uint32_t episode = p.pol.episode + (p.pol.episode_dev ? __ldg(p.pol.episode_dev) : 0u);
   const uint32_t t_base = episode << 16, ep_hi = policy_episode_hi(episode);
-  const uint64_t id0 = (uint64_t)(p.env_offset + e0);
+  const uint64_t id0 = (uint64_t)(p.pol.env_offset + e0);
   double s_rew[4] = {0, 0, 0, 0}, s_pen[4] = {0, 0, 0, 0};
   double disc = 1.0;
 
@@ -321,13 +305,12 @@ extern "C" int smarl_coverage_policy_rollout(const SmarlCoverageParams* p, const
   r.n_groups = (n_envs + 3) / 4; r.n_envs = n_envs; r.ld = ld; r.size = p->size;
   r.lut_len = p->lut_len; r.n_steps = acc->n_steps; r.g_mode = acc->g_mode;
   k.obs_rec = obs_rec; k.act_rec = actions; k.logp_rec = logp;
-  k.w1 = pol->w1; k.b1 = pol->b1; k.w2 = pol->w2; k.b2 = pol->b2; k.seed = pol->seed; k.env_offset = pol->env_offset;
-  k.episode = pol->episode; k.episode_dev = pol->episode_dev;
+  k.pol = discrete_policy_args(pol);
   const unsigned grid = (unsigned)((r.n_groups + kRolloutThreads - 1) / kRolloutThreads);
   cudaStream_t st = (cudaStream_t)stream;
   if (int rc = dispatch<1, kCovDiscPolMaxA>(A, [&](auto kA) {
         auto kern = coverage_policy_rollout_kernel<kA>;
-        const size_t smem = (size_t)(CovPolCfg<kA>::kWeightFloats + p->lut_len + 1) * sizeof(float);
+        const size_t smem = (size_t)(PolCfg<kA, kPolActions>::kWeightFloats + p->lut_len + 1) * sizeof(float);
         if (smem > 48 * 1024) SMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<grid, kRolloutThreads, smem, st>>>(k);
         SMARL_CUDA(cudaGetLastError());
