@@ -312,9 +312,9 @@ __device__ __forceinline__ void collision_env_step(double (&px)[A], double (&py)
   const uint32_t alive = ~done_mask;
   if constexpr (A >= kPairPrefilterA) {
     // Many agents: the A(A-1)/2 pair tests dominate and almost all pairs are far apart.  Screen them in f32
-    // (full-rate pipe, half the registers): coordinates <= 254 carry an absolute f32 error < 2e-5, so the f32
-    // squared distance of a pair with |d| ~ lim is off by < 1e-4 relative -- far inside the 1 % margin.  Only
-    // pairs that pass the screen are evaluated in f64, out of line, from a local-memory copy of the positions.
+    // (full-rate pipe, half the registers) against collision_screen_q, whose margin covers the f32 rounding of
+    // coordinates up to size on any field.  Only pairs of two alive agents that pass the screen are evaluated in
+    // f64, out of line, from a local-memory copy of the positions.
     double cx[A], cy[A];
     float fx[A], fy[A];
 #pragma unroll
@@ -372,6 +372,11 @@ inline int check_collision(const SmarlCollisionParams* p) {
   SMARL_REQUIRE(p->size >= 1, "size=%d must be >= 1", p->size);
   SMARL_REQUIRE(p->n_landmarks >= 1 && p->n_landmarks <= 64, "n_landmarks=%d outside 1..64", p->n_landmarks);
   SMARL_REQUIRE(p->agents_size > 0.0, "agents_size must be positive");
+  // The reach and pair tests compare squared distances with agents_size^2 (1 -+ 1e-9) and (2 agents_size)^2 (1 -+ 1e-6)
+  // and take the square root only inside those bands.  Below 2^-511 the square is subnormal or zero, the bands collapse
+  // to nothing and the squared test alone would decide wrong (an agent exactly on its landmark: 0 < 0 is false).
+  SMARL_REQUIRE(p->agents_size >= 0x1p-511, "agents_size=%g below 2^-511: its square is not a normal double",
+                p->agents_size);
   return SMARL_OK;
 }
 

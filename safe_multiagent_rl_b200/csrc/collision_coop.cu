@@ -183,23 +183,26 @@ __device__ __forceinline__ void collision_coop_env_step(double (&px)[CollCoop<A,
   // error by 28 * 2^-24 size^2 < size^2 * 2^-19; the threshold adds twice that to the coordinate-rounding margin
   // of collision_screen_q, so no pair inside the exact test's reach is ever screened out.
   const float T = (float)((double)collision_screen_q(lim, size) + size * size * (1.0 / 262144.0)) * 1.000001f;
+  const float inf = __int_as_float(0x7f800000);
   float mx2[B], my2[B], thr[B];
 #pragma unroll
   for (int j = 0; j < B; ++j) {
     const int i = j * S + s;
     const bool alive = !((done_bits >> j) & 1u);
-    // done (and padding) agents never collide: as partners they sit on distinct far-away sentinels, as owners
-    // their threshold is -inf
+    // done (and padding) agents never collide (:150-156 counts agents not done): as partners they publish a squared
+    // norm of +inf, which makes every screen value they enter +inf (the two products are finite), on any field; as
+    // owners their threshold is -inf.  (Their f32 coordinates stay parked at (4096 (i + 1), 0), which was the whole
+    // exclusion once and missed partners near that point on fields >= 4096; they no longer decide anything.)
     const float fx = alive ? (float)px[j] : 4096.0f * (float)(i + 1);
     const float fy = alive ? (float)py[j] : 0.0f;
     const float n = fmaf(fy, fy, fx * fx);
     mx2[j] = -2.0f * fx;
     my2[j] = -2.0f * fy;
-    thr[j] = alive ? T - n : -__int_as_float(0x7f800000);
+    thr[j] = alive ? T - n : -inf;
     if (!C::kGhost || j < B - 1 || i < A) {
       sp[i] = make_double2(px[j], py[j]);
       sf[i] = make_float2(fx, fy);
-      sn[i] = n;
+      sn[i] = alive ? n : inf;
     }
   }
   __syncwarp();
@@ -424,7 +427,7 @@ __global__ void __launch_bounds__(kCoopThreads, 5) collision_coop_rollout_kernel
     int collisions = 0;
     collision_coop_env_step<A, S, COMPACT>(px, py, done_bits, adx, ady, a.landmarks + e, ld, a.L, a.size, a.agents_size, s, q,
                                   s_pos + el * C::PA, s_f + el * C::FS, s_n + el * C::NS, s_clip, reward, collisions);
-    if (!active) reward = 0.0;                 // collisions is 0 by itself: every agent is on its sentinel
+    if (!active) reward = 0.0;                 // collisions is 0 by itself: every agent is done
     steps += active ? 1 : 0;
     const float rf = (float)reward;
     const float pf = (float)(lam * (double)collisions);

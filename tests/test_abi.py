@@ -7,6 +7,7 @@ import re
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -157,6 +158,35 @@ def test_register_capped_launchers_reject_bad_agent_counts(lib):
         for A in (0, -1):
             rc = agent_count_call(lib, env, kind, A, 1 << 18)
             assert rc == -3 and b"n_agents=%d outside 1..32" % A in lib.smarl_last_error(), (env, kind, A, rc)
+
+
+def test_collision_rejects_agents_size_without_a_normal_square(lib):
+    """The Collision kernels compare squared distances with agents_size^2 and (2 agents_size)^2 and take the square
+    root only in a relative band around them.  Below 2^-511 that square is subnormal or zero and the band collapses
+    (an agent exactly on its landmark would not reach it: qn = 0 < 0 is false), so every Collision entry point rejects
+    such an agents_size before any CUDA work."""
+    from safe_multiagent_rl_b200 import _lib
+    f = C.c_void_p(0x1000)   # never dereferenced
+    acc = C.byref(_lib.Accounting(0.9, 4, 0, None))
+    pol = C.byref(_lib.GaussianPolicyParams(3, 6, 16, 2, 0, 0, f, f, f, f, f, f, 1, 0, None))
+    tiny = 2.0 ** -511
+    for agents_size in (1e-170, np.nextafter(tiny, 0), 2.0 ** -600, 5e-324):
+        p = C.byref(_lib.CollisionParams(5, 3, 1, 0, float(agents_size), 0, 0))
+        calls = {
+            "reset": lambda: lib.smarl_collision_reset(p, f, f, f, f, f, f, None, None, 16, 16, None),
+            "step": lambda: lib.smarl_collision_step(p, f, f, f, f, f, None, f, f, None, None, None, None, 16, 16, None),
+            "rollout": lambda: lib.smarl_collision_rollout(p, acc, f, f, f, f, None, f, f, f, f, f, f, f, None, None,
+                                                           None, None, 16, 16, None),
+            "policy_rollout": lambda: lib.smarl_collision_policy_rollout(p, pol, acc, f, f, f, None, None, None, None,
+                                                                         f, f, f, f, f, f, f, None, None, None, None,
+                                                                         16, 16, None),
+        }
+        for name, call in calls.items():
+            assert call() == -1 and b"below 2^-511" in lib.smarl_last_error(), (name, agents_size)
+    for agents_size in (0.0, -0.25, float("nan")):
+        p = C.byref(_lib.CollisionParams(5, 3, 1, 0, agents_size, 0, 0))
+        assert lib.smarl_collision_step(p, f, f, f, f, f, None, f, f, None, None, None, None, 16, 16, None) == -1
+        assert b"agents_size must be positive" in lib.smarl_last_error()
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
